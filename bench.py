@@ -7,6 +7,7 @@ seeded synthetic graph of the same shape.
     python bench.py --gpus 1 --steps K --warmup W            # this repo's CUDA path (one JSON line)
     python bench.py --impl reference --steps K --warmup W    # the reference's CPU path (port, oracle/)
     torchrun ... bench.py --gpus N ...                       # entity-sharded over NCCL (strong scaling)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
 A step = one optimiser step (fit + step) on one batch of 512 (s, r) queries.
 `value`       triples/s with the batches already resident in HBM (CUDA events around K steps, CUDA graphs).
@@ -49,6 +50,7 @@ LR = 109.09      # OneCycleLR(max_lr=600, div_factor=5.5) at epoch 1 (train.py:2
 REG = 1e-11      # configs/base_config.py:19
 SEED = 322       # README.md:45
 FFMA_PEAK_TF = 148 * 128 * 2 * 1.965e9 / 1e12      # nominal FP32 FFMA peak at the measured max clock (74.4)
+DUMP_ROWS = 8192  # entity-factor rows --dump-outputs keeps: whole factors are 65 MB (WN18RR) to 1.6 GB (1M entities)
 
 
 def synth_graph(w, seed=1234):
@@ -271,7 +273,7 @@ class Runner:
         from rtucker_b200.engine import SparseTargets
         from rtucker_b200.optim import FusedLoss
         score_fn = self.model(fd[:, 0], fd[:, 1])
-        self.opt.fit(FusedLoss(score_fn, SparseTargets(od, xd), LABEL_SMOOTHING, REG), None)
+        self.rgrad_norm = self.opt.fit(FusedLoss(score_fn, SparseTargets(od, xd), LABEL_SMOOTHING, REG), None)
         self.opt.step()
 
     def max_over_ranks(self, ms):
@@ -294,6 +296,29 @@ class Runner:
         self.barrier()
         self.dev_batches = dev_batches
         return self.max_over_ranks(e0.elapsed_time(e1)), sum(self.triples[warmup:warmup + steps])
+
+    def dump_outputs(self, out_dir):
+        """What the last step returned to its caller, as out_dir/<name>.npy (float32): the loss and ||rgrad|| of fit(),
+        the core and relation factor after step(), and of every entity factor the rows of a fixed seeded sample of
+        DUMP_ROWS global row ids (ascending; the same rows on any number of GPUs).  Written by rank 0."""
+        w, model = self.w, self.model
+        rows = np.sort(np.random.default_rng(SEED).choice(w["N"], size=min(w["N"], DUMP_ROWS), replace=False))
+        out = {"loss": self.opt.loss, "rgrad_norm": self.rgrad_norm, "core": model.core.data, "R": model.R.weight.data}
+        mine = (rows >= self.n_begin) & (rows < self.n_end)
+        for name in ("E",) if w["sym"] else ("S", "O"):
+            local = getattr(model, name).weight.data
+            sample = torch.zeros(len(rows), local.shape[1], dtype=local.dtype, device=self.dev)
+            sample[torch.from_numpy(np.flatnonzero(mine)).to(self.dev)] = \
+                local[torch.from_numpy(rows[mine] - self.n_begin).to(self.dev)]
+            if self.world > 1:
+                torch.distributed.all_reduce(sample)      # each row lives on one rank, the others add zeros
+            out[name] = sample
+        out = {k: v.detach().cpu().numpy() for k, v in out.items()}
+        assert sum(a.nbytes for a in out.values()) <= 64 << 20, "dump exceeds 64 MB: lower DUMP_ROWS"
+        if int(os.environ.get("RANK", "0")) == 0:
+            os.makedirs(out_dir, exist_ok=True)
+            for name, a in out.items():
+                np.save(os.path.join(out_dir, name + ".npy"), a)
 
     def timed_e2e(self, first, steps):
         h2d = d2h = 0
@@ -536,9 +561,14 @@ def main():
     ap.add_argument("--no-strict", action="store_true", help="skip the run with the other score kernel (variant 2 <-> 0)")
     ap.add_argument("--no-c5", action="store_true", help="skip the synthetic 1M-entity sub-record")
     ap.add_argument("--c5-steps", type=int, default=5)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (loss, ||rgrad||, core, relation factor, "
+                         "a seeded sample of entity-factor rows) as DIR/<name>.npy, to compare two builds output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the CUDA path's results: it needs --impl b200")
         return run_reference(args)
 
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -582,6 +612,8 @@ def main():
     launches_eager = int(lib().rt_launch_count() - launches0)
     value = n_tr / (ms * 1e-3)
     eng = run.opt._engine
+    if args.dump_outputs:                    # before the profile and e2e passes below take further steps
+        run.dump_outputs(args.dump_outputs)
 
     progress(f"resident done: {ms / args.steps:.3f} ms/step; stage profile")
     # ---- per-stage profile pass: same steps launched eagerly with CUDA-event brackets around every stage

@@ -1,21 +1,21 @@
 """ORACLE / TEST INFRASTRUCTURE ONLY.
 
-Imports the UNMODIFIED reference (read-only checkout, default /root/reference) with the
-restated ``tucker_riemopt`` from this directory on sys.path, and injects the module
-globals ``train.py`` reads implicitly (train.py:21,25,38-41,72,183-193) -- the recipe of
-SURVEY.md App. E.  Only usable where the reference checkout exists (this container); on the
-GPU box the tests rely on the fixtures under tests/golden/ generated with it.
+Imports the UNMODIFIED reference (a read-only checkout of R-TuckER, named by the environment
+variable RTUCKER_REFERENCE_DIR) with the restated ``tucker_riemopt`` from this directory on
+sys.path, and injects the module globals ``train.py`` reads implicitly (train.py:21,25,38-41,72,
+183-193) -- the recipe of SURVEY.md App. E.  The reference is not part of this repository: without
+it the live comparisons skip and the tests rely on the fixtures under tests/golden/ generated with it.
 """
 import importlib
 import os
 import sys
 
-REF_DIR = os.environ.get("RTUCKER_REFERENCE_DIR", "/root/reference")
+REF_DIR = os.environ.get("RTUCKER_REFERENCE_DIR", "")
 _HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF_DIR, "train.py"))
+    return bool(REF_DIR) and os.path.isfile(os.path.join(REF_DIR, "train.py"))
 
 
 def _paths():

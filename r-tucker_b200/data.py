@@ -176,8 +176,10 @@ def wn18rr_fixture(path=None):
     if not os.path.isfile(path):
         return None
     d = np.load(path)
+    # stored as column-major uint16 (every id < 65536) to keep the file small; callers get row-major int32
+    split = lambda name: np.ascontiguousarray(d[name], dtype=np.int32)  # noqa: E731
     return dict(n_entities=int(d["n_entities"]), n_relations=int(d["n_relations"]),
-                train=d["train"], valid=d["valid"], test=d["test"])
+                train=split("train"), valid=split("valid"), test=split("test"))
 
 
 def datasets_from_ids(ids, label_smoothing=0.1):

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
-"""Generates the golden fixtures under tests/golden/ by IMPORTING THE UNMODIFIED REFERENCE from
-/root/reference (read-only) -- run in the build container only; the GPU box just reads the .npz files.
+"""Generates the golden fixtures under tests/golden/ by IMPORTING THE UNMODIFIED REFERENCE from the read-only
+checkout RTUCKER_REFERENCE_DIR names (oracle/ref_harness.py); the tests only read the .npz files.
 
   scores_{asym,sym}.npz   reference R_TuckER.init (seeded) + forward(s, r)(T) dense probabilities
                           (src/model/*/R_TuckER.py), fp32
@@ -87,6 +87,16 @@ def ranking():
                         hits10=float(m["hits@10"]))
 
 
+def tucker_factors(X, rank):
+    """HOSVD of a dense tensor of multilinear rank ``rank``: {"X_final_core", "X_final_U0".."U2"}, exact up to fp64
+    rounding (tests/golden_util.py rebuilds the dense tensor).  A few KB where the dense fp64 tensor is 1 MB."""
+    Us = [np.linalg.svd(np.moveaxis(X, m, 0).reshape(X.shape[m], -1), full_matrices=False)[0][:, :r]
+          for m, r in enumerate(rank)]
+    out = {f"X_final_U{m}": U for m, U in enumerate(Us)}
+    out["X_final_core"] = np.einsum("abc,ai,bj,ck->ijk", X, *Us)
+    return out
+
+
 def steps(mode, opt_name):
     torch.set_default_dtype(torch.float64)
     ns = ref_harness.load(mode, opt_name)
@@ -124,7 +134,7 @@ def steps(mode, opt_name):
     X = ns.train.extract_tensor(model).to_dense().detach().numpy()
     torch.set_default_dtype(torch.float32)
     np.savez_compressed(os.path.join(HERE, f"steps_{'sym' if sym else 'asym'}_{opt_name}.npz"), N=N, M=M,
-                        rank=np.asarray(rank), ls=ls, reg=reg, lr=lr, beta=0.8, X_final=X,
+                        rank=np.asarray(rank), ls=ls, reg=reg, lr=lr, beta=0.8, **tucker_factors(X, rank),
                         sub=np.stack(rec["sub"]), rel=np.stack(rec["rel"]),
                         off=np.stack(rec["off"]), idx=np.asarray(rec["idx"], dtype=object),
                         loss=np.asarray(rec["loss"]), norm=np.asarray(rec["norm"]),
@@ -157,9 +167,11 @@ def wn18rr_ids():
     ent = {e: i for i, e in enumerate(data.entities)}
     rel = {r: i for i, r in enumerate(data.relations)}
     out = dict(n_entities=len(data.entities), n_relations=len(data.relations))
+    assert len(data.entities) <= 1 << 16
     for split in ("train", "valid", "test"):
         rows = getattr(data, f"{split}_data")
-        out[split] = np.asarray([(ent[a], rel[b], ent[c]) for a, b, c in rows], dtype=np.int32)
+        # uint16, column-major: under 1 MB where int32 rows were not; wn18rr_fixture() returns int32 rows
+        out[split] = np.asfortranarray(np.asarray([(ent[a], rel[b], ent[c]) for a, b, c in rows], dtype=np.uint16))
     np.savez_compressed(os.path.join(HERE, "wn18rr_ids.npz"), **out)
 
 

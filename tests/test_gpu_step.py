@@ -10,6 +10,8 @@ Two checks per configuration:
   * trajectory: the free-running oracle started from the same initial point stays within 1e-3 after
     the same steps (errors are amplified by lr/||g||, SURVEY.md App. B.6).
 """
+import zlib
+
 import pytest
 import torch
 
@@ -65,7 +67,7 @@ def test_step_parity(cuda_device, cfg):
     A.ELEMENTWISE_FP32 = True   # the reference's fp32 sigmoid / log saturation semantics
     name, N, M, rank, B, sym, beta, lr_rel, reg_rel, steps = cfg
     dev = cuda_device
-    g = torch.Generator().manual_seed(hash(name) % 1000)
+    g = torch.Generator().manual_seed(zlib.crc32(name.encode()) % 1000)     # the same problem in every process
     R, S = ortho(M, rank[0], g), ortho(N, rank[1], g)
     O = S if sym else ortho(N, rank[2], g)
     # scale the core so that logits are O(1): exercises the sigmoid away from 0.5

@@ -67,7 +67,7 @@ def test_sparse_dataset_semantics():
     assert idx[off[0]:off[1]].tolist() == [1, 2, 4] and idx[off[1]:off[2]].tolist() == [0, 1]  # filter over ALL splits
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference checkout (with data/WN18RR) not present")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs a reference R-TuckER checkout with data/WN18RR: set RTUCKER_REFERENCE_DIR")
 def test_sparse_dataset_matches_reference_kg_dataset_on_wn18rr():
     import os
     from rtucker_b200.data import from_reference_data

@@ -1,7 +1,7 @@
 """Pins the closed-form oracle (oracle/analytic.py) against
   * the golden trajectories produced by the reference's UNMODIFIED optimisers (tests/golden/steps_*.npz),
   * the port of the reference step (oracle/reference_step.py) at fp32,
-  * the reference's own classes, imported live when /root/reference exists (this container)."""
+  * the reference's own classes, imported live when RTUCKER_REFERENCE_DIR names a checkout (oracle/ref_harness.py)."""
 import numpy as np
 import pytest
 import torch
@@ -99,7 +99,7 @@ def test_closed_form_partials_match_reference_forward_autograd():
     assert float((A.scatter_rows(M, rel, dr) - gR).norm() / gR.norm()) < 1e-12
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference checkout not present")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs a reference R-TuckER checkout: set RTUCKER_REFERENCE_DIR")
 @pytest.mark.parametrize("mode,opt", [("asymmetric", "rsgd"), ("symmetric", "rsgd"), ("symmetric", "rgd")])
 def test_live_reference_optimisers(mode, opt):
     """The reference's own modules, imported unmodified, driven like train.py:78-83, in fp64."""
@@ -141,7 +141,7 @@ def test_live_reference_optimisers(mode, opt):
         torch.set_default_dtype(torch.float32)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference checkout not present (GPU box)")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs a reference R-TuckER checkout: set RTUCKER_REFERENCE_DIR")
 def test_live_reference_sftucker_adam():
     """The analytic Adam twin against the reference's unmodified SFTuckerAdam (symmetric/optim.py:110-167) in fp64.
     The class hard-codes ``device="cuda"`` for its scalar second moment (optim.py:118): that one allocation is

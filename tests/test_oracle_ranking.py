@@ -31,7 +31,7 @@ def test_filtering_semantics():
     assert (int(g[0]), int(e[0]), int(eb[0])) == (0, 5, 3)     # all tied at 0: 3 of them before the target
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference checkout not present")
+@pytest.mark.skipif(not ref_harness.available(), reason="needs a reference R-TuckER checkout: set RTUCKER_REFERENCE_DIR")
 def test_live_reference_metrics():
     ns = ref_harness.load("asymmetric", "rsgd")
     g = torch.Generator().manual_seed(3)

@@ -50,6 +50,7 @@ using rt::cdiv;
 constexpr int kNumT = 8;          // core-sized fp64 temporaries
 constexpr int kMaxSplitCtas = 592;
 constexpr int kDotBlocks = 296;
+constexpr int kMinDotSlots = 2048;
 
 struct Layout {
   int r[3];
@@ -57,6 +58,7 @@ struct Layout {
   int64_t c;  // r0*r1*r2
   size_t C64, Gm[3], Ainv[3], coresq, Tn[kNumT], KC[3], Nn[3], Vf[3], Wv[3], GL[3], GLinv[3], Gs[3],
       tmpM[3], tmpK[3], eig[3], sub[3], sub_shared, exec_bar, gemm_partial, gram_ws, dot_partial, scal, total;
+  int dot_slots;  // doubles at dot_partial: one per kEwChunk elements of the dots recorded between two flushes
 };
 
 Layout make_layout(int r0, int r1, int r2, int B) {
@@ -88,7 +90,13 @@ Layout make_layout(int r0, int r1, int r2, int B) {
   L.gemm_partial = take((size_t)kMaxSplitCtas * GT * GT);
   int rmax = r0 > r1 ? r0 : r1; rmax = rmax > r2 ? rmax : r2;
   { size_t at = o; o += align_up(rt_gram_ws_bytes(B > 0 ? B : 1, rmax, rmax), 256); L.gram_ws = at; }
-  L.dot_partial = take(2048);
+  // The largest dots (rt_small_norm) are one over the core and one over each r_i x r_i Gram, recorded together;
+  // every partial of one dot must fit, or its two-stage sum would write past the slot.
+  auto chunks = [](int64_t n) { return (n + kEwChunk - 1) / kEwChunk; };
+  int64_t slots = chunks(L.c);
+  for (int i = 0; i < 3; ++i) slots += chunks((int64_t)L.r[i] * L.r[i]);
+  L.dot_slots = (int)std::max<int64_t>(kMinDotSlots, slots);
+  L.dot_partial = take((size_t)L.dot_slots);
   L.scal = take(16);
   L.total = o;
   return L;
@@ -100,7 +108,6 @@ struct Range { const char* lo; const char* hi; };
 struct Rec { Op op; Range rd[4]; int nrd; Range wr[2]; int nwr; };
 
 constexpr size_t kPartialArenaBytes = (size_t)kMaxSplitCtas * GT * GT * sizeof(double);
-constexpr int kDotSlots = 2048;
 
 template <typename T> struct DT;
 template <> struct DT<float> { static constexpr int v = DT_F32; };
@@ -366,8 +373,14 @@ struct Ctx {
   // out[0] = (accumulate ? out[0] : 0) + scale * sum x[i] y[i]   (deterministic two-stage sum)
   void dot(const void* x, int tx, const void* y, int ty, int64_t n, double scale, double* out, int accumulate) {
     if (err || n <= 0) return;
-    const int units = (int)((n + kEwChunk - 1) / kEwChunk);
-    if (dot_off + units > kDotSlots) { flush(); }
+    const int64_t units64 = (n + kEwChunk - 1) / kEwChunk;
+    if (units64 > L.dot_slots) {       // the partial count is fixed by kEwChunk: never widen the chunk to make it fit
+      rt::set_error("small stage: a dot over %lld elements needs %lld partial slots, the workspace has %d",
+                    (long long)n, (long long)units64, L.dot_slots);
+      err = 2; return;
+    }
+    const int units = (int)units64;
+    if (dot_off + units > L.dot_slots) { flush(); }
     double* part = p(L.dot_partial) + dot_off;
     dot_off += units;
     Rec rec{};
@@ -411,7 +424,7 @@ struct Ctx {
 
 int finish(Ctx& c, const char* what) {
   c.flush();
-  if (c.err) { rt::set_error("%s: kernel launch failed", what); return 1; }
+  if (c.err) { if (c.err == 1) rt::set_error("%s: kernel launch failed", what); return 1; }
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { rt::set_error("%s: %s", what, cudaGetErrorString(e)); return 1; }
   return 0;
@@ -739,5 +752,7 @@ extern "C" int rt_small_retract(const float* core, const float* dS_dir, const do
     c.axpby(Z1_S, nullptr, Z1_O, (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
     c.axpby(Z2_S, nullptr, Z2_O, (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
   }
+  // SF-Tucker: a separate Mn_O receives the shared mode's transport Gram, as Z1_O / Z2_O do
+  if (sym && Mn_S && Mn_O && Mn_O != Mn_S) c.axpby(Mn_S, nullptr, Mn_O, 2 * (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
   return finish(c, "rt_small_retract");
 }

@@ -200,7 +200,8 @@ class SmallStage:
             L.append((-(M[k] @ Kk)).contiguous())
         return (beta * pS).to(core.dtype), K, L
 
-    def retract(self, core, dS_dir, gram_R, gram_S, gram_O, hyper, transport_out=None):
+    def retract(self, core, dS_dir, gram_R, gram_S, gram_O, hyper, transport_out=None, spectra=None):
+        """``spectra`` (a list, optional) receives the descending eigenvalues of the three unfolding Grams N_i."""
         r, lr = self.r, float(hyper[0])
         grams = [gram_R, gram_S, gram_S if self.sym else gram_O]
         C = self.C
@@ -225,8 +226,12 @@ class SmallStage:
         for i in range(3):
             if self.sym and i == 2:
                 Y.append(Y[1])
+                if spectra is not None:
+                    spectra.append(spectra[1])
                 continue
             w, V = torch.linalg.eigh(N[i])
+            if spectra is not None:
+                spectra.append(w.flip(0))
             Y.append(V[:, torch.argsort(w, descending=True)[:r[i]]])
         Wa = [Y[k][:r[k]].T for k in range(3)]
         Wb = [Y[k][r[k]:].T for k in range(3)]

@@ -9,6 +9,11 @@ Two checks per configuration:
     shapes, random multilinear probes otherwise) -- factors are only defined up to rotation.
   * trajectory: the free-running oracle started from the same initial point stays within 1e-3 after
     the same steps (errors are amplified by lr/||g||, SURVEY.md App. B.6).
+
+tools/step_seed_sweep.py runs the two huge-step configurations over problem seeds 0-39.  On one B200 (1000 W power
+limit) no step of the 80 draws came near a bound: largest one-step point error 1.2e-6 (bound 1e-5), trajectory 2.1e-6
+(1e-3), factor orthonormality defect 4.1e-7 (5e-6).  The small stage itself agrees with its fp64 restatement in that
+regime (test_gpu_small_stage.py::test_small_retract_huge_step).
 """
 import zlib
 

@@ -78,6 +78,27 @@ int rt_score_rank_fused(const float* q, const float* O, int B, int r2, int n_beg
                         int32_t* greater, int32_t* equal, int32_t* equal_before,
                         double* bce_sum, void* ws, void* stream);
 
+/*
+ * Filtered top-k link prediction without materialising P: which k entities best complete (s, r, ?).
+ * q[B, r2] are the query rows (rt_query_fwd), O the entity shard holding global rows [n_begin, n_begin+n_local).
+ * For query b, with filter list F_b = flt_idx[flt_off[b]:flt_off[b+1]] (global ids, ASCENDING within each query, as
+ * the data pipeline produces them; flt_off and flt_idx both NULL: no filtering):
+ *     p_j = sigmoid(q_b . O_j), bit-identical to rt_score_dense;  entities in F_b are excluded;
+ *     order: p descending, then global id ascending (a total order: the entity at position i has filtered rank i + 1
+ *            under rt_rank_filtered / rt_score_rank_fused whenever its p > 0);
+ *     top_idx[b, 0:k] (int32 global ids), top_p[b, 0:k] (the exact p).  Positions beyond the number of unfiltered
+ *            entities of the shard get id -1 and p = -inf, so per-shard lists merge without special cases.
+ * n_cand[b] (may be NULL) tells which path produced query b: >= 0 the number of tensor-core candidates that were
+ * rechecked exactly, -1 the exact full pass.  The path is chosen from the shape and from device flags only.
+ * Limits: 1 <= k <= 256, 1 <= B <= 1024 per call, 1 <= r2 <= 256; anything else returns an error.
+ * The workspace (rt_score_topk_ws_bytes) does not grow with n_local beyond the shard's row norms and a fixed chunk:
+ * tens of MB at B = 512, n_local = 10^6, r2 = 200, k = 100 instead of the 2 GB of the dense probabilities.
+ */
+size_t rt_score_topk_ws_bytes(int B, int n_local, int r2, int k);
+int rt_score_topk(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
+                  const int32_t* flt_off, const int32_t* flt_idx,
+                  int32_t* top_idx, float* top_p, int32_t* n_cand, void* ws, void* stream);
+
 /* Dense compatibility path: P[b, j] = sigmoid(q_b . O_j), what score_fn(T) returns in the reference
  * (src/model/asymmetric/R_TuckER.py:47-48).  Bit-identical to the values the fused kernels use. */
 int rt_score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp,

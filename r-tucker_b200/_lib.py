@@ -32,6 +32,8 @@ PROTOTYPES = {
     "rt_target_prob": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp]),
     "rt_score_rank_ws_bytes": (sz, [i32, i32, i32]),
     "rt_score_rank_fused": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "rt_score_topk_ws_bytes": (sz, [i32, i32, i32, i32]),
+    "rt_score_topk": (i32, [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
     "rt_score_dense": (i32, [vp, vp, i32, i32, i32, vp, i64, vp]),
     "rt_filter_dense": (i32, [vp, i64, vp, i64, i32, i32, vp, vp]),
     "rt_gather_rows": (i32, [vp, i32, i32, i32, vp, i32, vp, vp]),

@@ -22,6 +22,7 @@
 // bulk async copies (TMA, mbarrier complete_tx).
 #include "common.h"
 #include "tc.cuh"
+#include "exact.cuh"
 #include <algorithm>
 #include <math.h>
 
@@ -32,6 +33,7 @@ constexpr int kEpiWarps = 8, kProdWarps = 4, kMmaWarp = 12, kLoadWarp = 13;
 constexpr int kThreads = 512;       // 16 warps = 4 warpgroups: epilogue (2), producers (1), MMA + loader + 2 idle (1)
 constexpr int kRegsEpi = 168, kRegsOther = 88;                  // setmaxnreg: 256 * 168 + 256 * 88 = 64 K registers
 constexpr int kRegsEpiLogits = 176, kRegsOtherLogits = 80;      // rank / score mode: 128 logits + counters per thread
+                                                                // (top-k mode: 128 logits and no counters, the factor-update split)
 constexpr int TM = 128;             // rows per tile
 constexpr int KB = 16;              // contraction elements per staged block (2 MMA k-steps)
 constexpr int GB = 2;               // blocks per partial sum held in tensor memory (factor updates)
@@ -80,6 +82,9 @@ struct Args {
   float* G; int64_t ldg;              // [n_local][ldg] (ldg = 256 * njobs)
   float t_neg, inv_count;
   double* loss_partial;               // [grid]
+  // ---- top-k mode (MODE 3): the rank-mode logits; entities not certainly below the query's threshold are appended to
+  //      its segment seg[b][0, cand_cap) (overflow: cnt[b] > cand_cap; thr and onorms as in rank mode) ----
+  int32_t* topk_seg; int* topk_cnt;
 };
 struct PackArgs {
   const void* K[MAX_JOBS * MAX_TERMS]; int rk[MAX_JOBS * MAX_TERMS]; int blk0[MAX_JOBS * MAX_TERMS + 1];
@@ -272,6 +277,29 @@ __device__ __noinline__ float score_chunk8(float* __restrict__ gdst, bool rv, in
   return lsum;
 }
 
+// ---- top-k candidate epilogue of 8 columns (queries) of one thread's row (entity): append the entity to the segment of
+//      every query whose band it reaches (z >= lo_b - slope_b ||O_j||: not certainly below the sample threshold).
+//      Inlined: one compare per column; with the factor-update register split it does not spill. ----
+__device__ __forceinline__ void topk_chunk8(const float* __restrict__ lop, const float* __restrict__ slp, float onorm, bool rv,
+                                         int ncols, int b0, int e_loc, int* cnt, int32_t* seg, int cap, float z0, float z1,
+                                         float z2, float z3, float z4, float z5, float z6, float z7) {
+  const float zs[8] = {z0, z1, z2, z3, z4, z5, z6, z7};
+  if (!rv) return;
+#pragma unroll
+  for (int u = 0; u < 8; u += 4) {
+    const float4 lo4 = __ldg(reinterpret_cast<const float4*>(lop + u)), sl4 = __ldg(reinterpret_cast<const float4*>(slp + u));
+    const float lo[4] = {lo4.x, lo4.y, lo4.z, lo4.w}, sl[4] = {sl4.x, sl4.y, sl4.z, sl4.w};
+#pragma unroll
+    for (int v = 0; v < 4; ++v) {
+      if (u + v < ncols && zs[u + v] >= lo[v] - sl[v] * onorm) {       // rare: a few hundred entities per query
+        const int b = b0 + u + v;
+        const int pos = atomicAdd(cnt + b, 1);
+        if (pos < cap) seg[(int64_t)b * cap + pos] = e_loc;
+      }
+    }
+  }
+}
+
 // position in this CTA's flattened sequence of (tile, block) pairs
 struct Cursor {
   int tile, job, blk, nblk, kblk0;
@@ -322,7 +350,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
 
   if (warp < kEpiWarps) {
     // ================= epilogue: partial sums -> fp32 running sum (round to nearest) -> Y =================
-    if (MODE == 0) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpi));
+    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpi));
     else asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpiLogits));
     const int quarter = warp & 3, half = warp >> 2;
     constexpr int NACC = HC8 * 8;
@@ -438,6 +466,18 @@ apply_tc_kernel(const __grid_constant__ Args a) {
           lsum += score_chunk8(grow + c8 * 8, rv, a.B - (q0 + c8 * 8), tn, inv, acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2],
                                acc[c8 * 8 + 3], acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
         lacc += (double)lsum;
+      } else if (MODE == 3) {
+        // ---- top-k candidate epilogue: acc[c] = logit of (entity row, query column) ----
+        const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
+        const bool rv = e_loc < J.n;
+        const int q0 = job * 256 + half * halfcols;
+        const int Bp = 256 * a.njobs;
+        const float onorm = rv ? __ldg(a.onorms + e_loc) : 0.0f;
+#pragma unroll
+        for (int c8 = 0; c8 < HC8; ++c8)
+          topk_chunk8(a.thr + q0 + c8 * 8, a.thr + 3 * Bp + q0 + c8 * 8, onorm, rv, a.B - (q0 + c8 * 8), q0 + c8 * 8, e_loc,
+                      a.topk_cnt, a.topk_seg, a.cand_cap, acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3],
+                      acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
       } else {
       const int lt = tile - J.tile0, rep = lt / J.tiles_per_rep;
       const int row0 = (lt - rep * J.tiles_per_rep) * TM;
@@ -484,7 +524,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     if (tid == 0) { PROF_PRINT("epilogue (acc_full, store)"); }
   } else if (warp < kEpiWarps + kProdWarps) {
     // ================= producers: X block -> hi / lo operand images (+ optional raw copy) =================
-    if (MODE == 0) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     const int ptid = tid - kEpiWarps * 32;             // 0 .. kProdWarps*32-1
     // thread -> (16-byte chunk ch of the block's 4, rows r0, r0 + rstep, ...).  Row-major terms: 4 lanes cover the 64
@@ -636,7 +676,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     if (ptid == 0) { PROF_PRINT("producer (empty, produce)"); }
   } else if (warp == kMmaWarp) {
     // ================= MMA issuer =================
-    if (MODE == 0) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     if (lane == 0) {
       const uint32_t idesc = make_idesc_tf32(TM, a.rcp, false, false);
@@ -677,7 +717,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     __syncwarp();
   } else if (warp == kLoadWarp) {
     // ================= K image loader =================
-    if (MODE == 0) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     if (lane == 0) {
       Cursor c;
@@ -700,7 +740,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     }
     __syncwarp();
   } else {
-    if (MODE == 0) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));     // idle warps of the last warpgroup
   }
   fence_before_sync();
@@ -734,29 +774,8 @@ Plan make_plan(int rc) {
 // arithmetic of the dense path (k ascending, one fmaf accumulator, 1 / (1 + expf(-z))), so the counts equal the ones
 // the fp32 kernel produces.  Filtered entities are corrected from their exact probabilities afterwards.
 // ---------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float exact_logit(const float* __restrict__ q, const float* __restrict__ o, int r2) {
-  float z = 0.0f;                                   // same order as score_dense_kernel / target_prob_kernel
-  int k = 0;
-  if ((r2 & 3) == 0 && ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(o)) & 15u) == 0) {
-    // 16-byte loads, eight in flight per operand: one thread walks one row, so the chain is bound by its own loads
-    for (; k + 32 <= r2; k += 32) {
-      float4 a[8], b[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) { a[u] = __ldg(reinterpret_cast<const float4*>(q + k) + u); b[u] = __ldg(reinterpret_cast<const float4*>(o + k) + u); }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        z = fmaf(a[u].x, b[u].x, z); z = fmaf(a[u].y, b[u].y, z); z = fmaf(a[u].z, b[u].z, z); z = fmaf(a[u].w, b[u].w, z);
-      }
-    }
-    for (; k + 4 <= r2; k += 4) {
-      const float4 a = __ldg(reinterpret_cast<const float4*>(q + k)), b = __ldg(reinterpret_cast<const float4*>(o + k));
-      z = fmaf(a.x, b.x, z); z = fmaf(a.y, b.y, z); z = fmaf(a.z, b.z, z); z = fmaf(a.w, b.w, z);
-    }
-  }
-  for (; k < r2; ++k) z = fmaf(__ldg(q + k), __ldg(o + k), z);
-  return z;
-}
-__device__ __forceinline__ float sigmoid_ref(float z) { return 1.0f / (1.0f + expf(-z)); }
+using rt::exact_logit;
+using rt::sigmoid_ref;
 
 // max_j ||O_j||^2 over the shard (bounds the error of a logit); out is a float bit pattern updated with atomicMax
 __global__ void rank_rownorm_kernel(const float* __restrict__ O, int n_local, int r2, unsigned int* out,
@@ -970,6 +989,65 @@ int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_lo
   rank_reset_if_overflow_kernel<<<rt::cdiv(B, 256), 256, 0, s>>>(B, greater, equal, equal_before, scal + 1);
   RT_LAUNCH_CHECK();
   *overflow_flag = scal + 1;
+  return 0;
+}
+
+// ---- top-k mode: the rank-mode pass with the per-query sample threshold p_k in place of p_target (topk.cu) ----
+size_t topk_tc_ws_bytes(int B, int n_local, int r2) {
+  const RankLayout L = rank_layout(B, n_local, r2);
+  return L.cand;                                      // the rank layout up to its candidate list
+}
+}  // namespace rt
+
+namespace {
+// queries the sample already sent to the exact pass get an empty band
+__global__ void topk_empty_band_kernel(float* __restrict__ thr, int B, const int* __restrict__ flag) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < B && flag[b]) thr[b] = INFINITY;
+}
+}  // namespace
+
+namespace rt {
+// Appends to seg[b][0, cap) every entity j of the shard whose tensor-core logit is not certainly below the logit of
+// p_k[b] (the band of rank_thresholds_kernel for p_target = p_k); cnt[b] (zeroed by the caller) ends as the number of
+// such entities, > cap when the segment overflowed.  Queries with flag[b] != 0 are skipped.
+int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
+                 int32_t* seg, int cap, void* ws, cudaStream_t s) {
+  const RankLayout L = rank_layout(B, n_local, r2);
+  const Plan p = make_plan(256);
+  char* base = (char*)ws;
+  unsigned int* maxnorm = (unsigned int*)(base + L.scal + 8);
+  float* thr = (float*)(base + L.thr);
+  float* onorms = (float*)(base + L.norms);
+  RT_CHECK_CUDA(cudaMemsetAsync(maxnorm, 0, sizeof(unsigned int), s));
+  rank_rownorm_kernel<<<rt::sm_count() * 4, 256, 0, s>>>(O, n_local, r2, maxnorm, onorms);
+  RT_LAUNCH_CHECK();
+  rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
+  RT_LAUNCH_CHECK();
+  topk_empty_band_kernel<<<rt::cdiv(B, 256), 256, 0, s>>>(thr, B, flag);
+  RT_LAUNCH_CHECK();
+  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kimg), p.cs_k,
+                                                       p.kimg_bytes);
+  RT_LAUNCH_CHECK();
+  Args a{};
+  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
+  a.stage_bytes = p.stage_bytes; a.Kimg = (const unsigned char*)(base + L.kimg);
+  a.njobs = L.njobs;
+  const int tiles_per_job = rt::cdiv(n_local, TM);
+  for (int j = 0; j < L.njobs; ++j) {
+    Job& J = a.job[j];
+    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
+    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = L.nblk;
+    J.nblk = L.nblk; J.kblk0 = j * L.nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
+    J.reps = 1; J.tiles_per_rep = tiles_per_job;
+  }
+  a.ntiles = L.njobs * tiles_per_job;
+  a.thr = thr; a.onorms = onorms; a.B = B;
+  a.topk_seg = seg; a.topk_cnt = cnt; a.cand_cap = cap;
+  const int grid = a.ntiles < rt::sm_count() ? a.ntiles : rt::sm_count();
+  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 3>, SMEM_LIMIT));
+  apply_tc_kernel<16, 3><<<grid, kThreads, p.smem, s>>>(a);
+  RT_LAUNCH_CHECK();
   return 0;
 }
 }  // namespace rt

@@ -309,10 +309,12 @@ __global__ void target_prob_kernel(const float* __restrict__ q, const float* __r
 
 // Dense compatibility path: P[b, j] = sigmoid(q_b . O_j) written out (what score_fn(T) returns in
 // the reference, R_TuckER.py:47-48).  Same staging and k order as score_kernel, so the values are
-// bit-identical to the ones the fused kernels see.
+// bit-identical to the ones the fused kernels see.  gate (may be NULL): the launch is a no-op unless
+// *gate != 0 (the exact pass of the top-k selection, topk.cu).
 __global__ void __launch_bounds__(256)
 score_dense_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2, int n_local,
-                   float* __restrict__ P, int64_t ldp) {
+                   float* __restrict__ P, int64_t ldp, const int* __restrict__ gate) {
+  if (gate && *gate == 0) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int ldw = row_ld(r2, 1);
   const int k_end = (r2 + 3) / 4 * 4;
@@ -542,15 +544,22 @@ extern "C" int rt_score_rank_fused(const float* q, const float* O, int B, int r2
   return 0;
 }
 
-extern "C" int rt_score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P,
-                              int64_t ldp, void* stream) {
-  RT_REQUIRE(B >= 0 && r2 > 0 && r2 <= 1024 && n_local >= 0 && ldp >= n_local, "rt_score_dense: bad shape");
+namespace rt {
+int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
+                cudaStream_t s) {
   if (B == 0 || n_local == 0) return 0;
   const size_t smem = (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float);
   RT_CHECK_CUDA(cudaFuncSetAttribute(score_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                      (int)smem));
   dim3 grid(rt::cdiv(n_local, NT), rt::cdiv(B, BT));
-  score_dense_kernel<<<grid, 256, smem, (cudaStream_t)stream>>>(q, O, B, r2, n_local, P, ldp);
+  score_dense_kernel<<<grid, 256, smem, s>>>(q, O, B, r2, n_local, P, ldp, gate);
   RT_LAUNCH_CHECK();
   return 0;
+}
+}  // namespace rt
+
+extern "C" int rt_score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P,
+                              int64_t ldp, void* stream) {
+  RT_REQUIRE(B >= 0 && r2 > 0 && r2 <= 1024 && n_local >= 0 && ldp >= n_local, "rt_score_dense: bad shape");
+  return rt::score_dense(q, O, B, r2, n_local, P, ldp, nullptr, (cudaStream_t)stream);
 }

@@ -58,6 +58,38 @@ def score_rank_fused(q, O, target, p_target, flt_off, flt_idx, n_begin=0, want_b
     return out[0], out[1], out[2], bce
 
 
+TOPK_MAX_B, TOPK_MAX_K = 1024, 256
+
+
+def score_topk(q, O, k, flt_off=None, flt_idx=None, n_begin=0):
+    """Filtered top-k of every query row of ``q`` [B, r2] over the entity shard ``O`` (global rows
+    [n_begin, n_begin + n_local)) -- see rt_score_topk in include/rtucker.h.  ``flt_off`` / ``flt_idx``: CSR of the
+    known objects per query (global ids, ascending within a query), or both None.  Returns (top_idx int32 [B, k],
+    top_p f32 [B, k], n_cand int32 [B]); positions without an entity hold id -1 and p -inf.  B > 1024 is split into
+    calls of at most 1024 queries."""
+    require_cuda(q, O, flt_off, flt_idx)
+    if (flt_off is None) != (flt_idx is None):
+        raise RTuckerError("score_topk: pass both flt_off and flt_idx, or neither")
+    B, r2 = q.shape
+    n_local = O.shape[0]
+    k = int(k)
+    dev = q.device
+    top_idx = torch.empty(B, k, dtype=i32, device=dev)
+    top_p = torch.empty(B, k, dtype=f32, device=dev)
+    n_cand = torch.empty(B, dtype=i32, device=dev)
+    q, O = _c(q, f32), _c(O, f32)
+    if flt_off is not None:
+        flt_off, flt_idx = _c(flt_off, i32), _c(flt_idx, i32)
+    ws = _ws(lib().rt_score_topk_ws_bytes(min(max(B, 1), TOPK_MAX_B), n_local, r2, k), dev)
+    for lo in range(0, B, TOPK_MAX_B):
+        hi = min(B, lo + TOPK_MAX_B)
+        check(lib().rt_score_topk(ptr(q[lo:hi]), ptr(O), hi - lo, r2, int(n_begin), n_local, k,
+                                  ptr(flt_off[lo:hi + 1]) if flt_off is not None else None, ptr(flt_idx),
+                                  ptr(top_idx[lo:hi]), ptr(top_p[lo:hi]), ptr(n_cand[lo:hi]), ptr(ws), stream_ptr()),
+              "rt_score_topk")
+    return top_idx, top_p, n_cand
+
+
 # ---------------------------------------------------------------- (a) query contraction
 def gather_rows(table, idx, row_begin=0):
     require_cuda(table, idx)

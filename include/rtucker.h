@@ -174,6 +174,40 @@ int rt_score_bce_tc3(const float* q, const float* qp, const float* O, int B, int
                      int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
                      double* loss_sum, float* H, float* dO, void* ws, void* stream);
 
+/* ---- (b') fused 1-N softmax cross-entropy + backward ------------------------------------ */
+/*
+ * The other standard objective of 1-N scoring (KvsAll / 1vsAll trainers): softmax cross-entropy over ALL entities.
+ * For query b with target set y_b (tgt_idx[tgt_off[b]:tgt_off[b+1]], GLOBAL ids, unique), label smoothing ls,
+ * N = n_total entities and logits z_bj = q_b . O_j:
+ *   t_bj   = (1 - ls) [j in y_b] / |y_b| + ls / N            (sum_j t_bj = 1)
+ *   lse_b  = log sum_j exp(z_bj)                              (over all N entities, all shards)
+ *   loss   = (1/B) sum_b (lse_b - sum_j t_bj z_bj) + reg ||core||^2
+ *   G_bj   = dloss/dz_bj = (exp(z_bj - lse_b) - t_bj) / B
+ * i.e. torch.nn.functional.cross_entropy(z, y / |y|, label_smoothing=ls, reduction="mean").  A query with no targets
+ * (|y_b| = 0: the CSR lives on the device and is not checked) is defined, not rejected: its positive term is 0 and
+ * only the ls / N part of t remains (loss_b = lse_b - (ls/N) sum_j z_bj, G = (softmax - ls/N) / B).  Correct for
+ * any finite fp32 logits (|z| ~ 1e3 included): the max is kept online.
+ *
+ * Two passes per entity shard (global rows [n_begin, n_begin + n_local)):
+ * rt_score_lse: parts[B][2] (fp32) = (m_b, s_b), m_b the largest logit of the shard, s_b = sum_{j in shard}
+ *   exp(z_bj - m_b); an empty shard gives (-inf, 0).  No B x N object is written.
+ * rt_score_ce_fwd_bwd: parts[nparts][B][2] are the rt_score_lse results of ALL shards (nparts = 1 unsharded), merged
+ *   in a fixed order into lse_b.  Outputs as rt_score_bce_fwd_bwd:  H = G O [B, r2] (shard partial),
+ *   dO = G^T qp [n_local, r2] (qp = q when NULL), loss_sum (double[1]) = sum_b sum_{j in shard} t_bj (lse_b - z_bj):
+ *   un-normalised (divide by b_total); summed over the shards it is B times the loss without the regulariser (the
+ *   (1 - ls) lse_b of a query without targets is charged to the shard with n_begin == 0).
+ * variant: 0 = fp32 FFMA (any shape), 3 = 3xTF32 tensor cores (the shapes of rt_score_bce_tc3_supported).  Any other
+ * variant, or nparts < 1, returns an error.  Deterministic: the same inputs give the same bits.
+ */
+size_t rt_score_lse_ws_bytes(int B, int n_local, int r2, int variant);
+int rt_score_lse(const float* q, const float* O, int B, int r2, int n_local, int variant, float* parts, void* ws,
+                 void* stream);
+size_t rt_score_ce_ws_bytes(int B, int n_local, int r2, int variant);
+int rt_score_ce_fwd_bwd(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local,
+                        int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
+                        const float* parts, int nparts, double* loss_sum, float* H, float* dO, int variant, void* ws,
+                        void* stream);
+
 /* ---- (c) tall-skinny passes over the N x r factors ----------------------------------- */
 /* out[ra, rb] (fp64) = A[n, :ra]^T  B[n, :rb]   (deterministic two-stage reduction).
  * precise = 0: fp32 products accumulated in fp32 over 256-row blocks, fp64 across blocks;

@@ -76,6 +76,11 @@ PROTOTYPES = {
     "rt_score_bce_tc3_supported": (i32, [i32, i32, i32]),
     "rt_score_bce_tc3_ws_bytes": (sz, [i32, i32, i32]),
     "rt_score_bce_tc3": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp, vp, vp]),
+    "rt_score_lse_ws_bytes": (sz, [i32, i32, i32, i32]),
+    "rt_score_lse": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp]),
+    "rt_score_ce_ws_bytes": (sz, [i32, i32, i32, i32]),
+    "rt_score_ce_fwd_bwd": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, f32, vp, i32, vp, vp, vp, i32, vp,
+                                  vp]),
     "rt_score_bce_v3_supported": (i32, [i32]),
     "rt_score_bce_v3_ws_bytes": (sz, [i32, i32, i32]),
     "rt_score_v3_set_profile": (i32, [vp]),

@@ -24,6 +24,7 @@
 #include "tc.cuh"
 #include "exact.cuh"
 #include <algorithm>
+#include <limits.h>
 #include <math.h>
 
 namespace {
@@ -300,6 +301,67 @@ __device__ __forceinline__ void topk_chunk8(const float* __restrict__ lop, const
   }
 }
 
+// ---- 1-N softmax cross-entropy, log-sum-exp epilogue of 8 columns (queries) over the warp's 32 rows (entities): per
+//      column m = the largest valid logit (integer warp max on an order-preserving key), s = sum exp(z - m); the 8 sums
+//      by a reduce-scatter butterfly (4 + 2 + 1 shuffles leave lane group j = (lane >> 2) & 7 holding column j, 2 more
+//      finish it) instead of 8 full warp sums.  Lane 4j writes dst[j] = (m_j, s_j).  Rows / columns that do not exist
+//      count as -inf. ----
+__device__ __noinline__ void lse_chunk8(float2* __restrict__ dst, bool rv, int ncols, float z0, float z1, float z2, float z3,
+                                        float z4, float z5, float z6, float z7) {
+  const int lane = threadIdx.x & 31;
+  const float zs[8] = {z0, z1, z2, z3, z4, z5, z6, z7};
+  float m[8], e[8];
+#pragma unroll
+  for (int u = 0; u < 8; ++u) {
+    const bool on = rv && u < ncols;
+    const int bits = __float_as_int(zs[u]);
+    const int key = on ? (bits >= 0 ? bits : bits ^ 0x7fffffff) : INT_MIN;
+    const int mk = __reduce_max_sync(0xffffffffu, key);
+    m[u] = mk == INT_MIN ? -INFINITY : __int_as_float(mk >= 0 ? mk : mk ^ 0x7fffffff);
+    e[u] = on ? ex2_fast((zs[u] - m[u]) * 1.4426950408889634f) : 0.0f;
+  }
+  const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4;
+  float v[4], w[2];
+#pragma unroll
+  for (int i = 0; i < 4; ++i) v[i] = (b4 ? e[i + 4] : e[i]) + __shfl_xor_sync(0xffffffffu, b4 ? e[i] : e[i + 4], 16);
+#pragma unroll
+  for (int i = 0; i < 2; ++i) w[i] = (b3 ? v[i + 2] : v[i]) + __shfl_xor_sync(0xffffffffu, b3 ? v[i] : v[i + 2], 8);
+  float x = (b2 ? w[1] : w[0]) + __shfl_xor_sync(0xffffffffu, b2 ? w[0] : w[1], 4);
+  x += __shfl_xor_sync(0xffffffffu, x, 2);
+  x += __shfl_xor_sync(0xffffffffu, x, 1);
+  const float mlo = b3 ? (b2 ? m[3] : m[2]) : (b2 ? m[1] : m[0]);
+  const float mhi = b3 ? (b2 ? m[7] : m[6]) : (b2 ? m[5] : m[4]);
+  if ((lane & 3) == 0) dst[(lane >> 2) & 7] = make_float2(b4 ? mhi : mlo, x);
+}
+
+// ---- 1-N softmax cross-entropy, gradient epilogue of 8 columns of one thread's row: G[e][b] = (softmax - ls/N) / B for
+//      ALL-NEGATIVE targets, softmax = 2^((z - M_b) log2e - log2 S_b) (one ex2), loss += (ls/N) (lse_b - z); the sparse
+//      positives are fixed up afterwards (score_ce_fix_positives_kernel).  Not inlined, like score_chunk8. ----
+__device__ __noinline__ float ce_chunk8(float* __restrict__ gdst, const float* __restrict__ mp, const float* __restrict__ lp,
+                                        bool rv, int ncols, float tn, float inv, float z0, float z1, float z2, float z3, float z4,
+                                        float z5, float z6, float z7) {
+  const float zs[8] = {z0, z1, z2, z3, z4, z5, z6, z7};
+  const float4 m0 = __ldg(reinterpret_cast<const float4*>(mp)), m1 = __ldg(reinterpret_cast<const float4*>(mp + 4));
+  const float4 l0 = __ldg(reinterpret_cast<const float4*>(lp)), l1 = __ldg(reinterpret_cast<const float4*>(lp + 4));
+  const float M[8] = {m0.x, m0.y, m0.z, m0.w, m1.x, m1.y, m1.z, m1.w};
+  const float L[8] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w};
+  float gv[8];
+  float lsum = 0.0f;
+#pragma unroll
+  for (int u = 0; u < 8; ++u) {
+    const float d = zs[u] - M[u];
+    const float p = ex2_fast(fmaf(d, 1.4426950408889634f, -L[u]));
+    const bool on = rv && u < ncols;
+    if (on) lsum += tn * fmaf(L[u], 0.6931471805599453f, -d);
+    gv[u] = on ? (p - tn) * inv : 0.0f;
+  }
+  if (rv) {
+    *reinterpret_cast<float4*>(gdst) = make_float4(gv[0], gv[1], gv[2], gv[3]);
+    *reinterpret_cast<float4*>(gdst + 4) = make_float4(gv[4], gv[5], gv[6], gv[7]);
+  }
+  return lsum;
+}
+
 // position in this CTA's flattened sequence of (tile, block) pairs
 struct Cursor {
   int tile, job, blk, nblk, kblk0;
@@ -478,6 +540,31 @@ apply_tc_kernel(const __grid_constant__ Args a) {
           topk_chunk8(a.thr + q0 + c8 * 8, a.thr + 3 * Bp + q0 + c8 * 8, onorm, rv, a.B - (q0 + c8 * 8), q0 + c8 * 8, e_loc,
                       a.topk_cnt, a.topk_seg, a.cand_cap, acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3],
                       acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
+      } else if (MODE == 4) {
+        // ---- CE log-sum-exp epilogue: (m, s) of this warp's 32 rows per query column -> part[row group][column]
+        //      (G reinterpreted as float2 [4 * tiles per job][ldg]) ----
+        const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
+        const bool rv = e_loc < J.n;
+        const int q0 = job * 256 + half * halfcols;
+        float2* dst = reinterpret_cast<float2*>(a.G) + (int64_t)((tile - J.tile0) * 4 + quarter) * a.ldg + q0;
+#pragma unroll
+        for (int c8 = 0; c8 < HC8; ++c8)
+          lse_chunk8(dst + c8 * 8, rv, a.B - (q0 + c8 * 8), acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3],
+                     acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
+      } else if (MODE == 5) {
+        // ---- CE gradient epilogue: thr = row statistics [M_b | log2 S_b] with stride ldg (ce_row_stats) ----
+        const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
+        const bool rv = e_loc < J.n;
+        const int q0 = job * 256 + half * halfcols;
+        float* grow = a.G + (int64_t)e_loc * a.ldg + q0;
+        const float tn = a.t_neg, inv = a.inv_count;
+        float lsum = 0.0f;
+#pragma unroll
+        for (int c8 = 0; c8 < HC8; ++c8)
+          lsum += ce_chunk8(grow + c8 * 8, a.thr + q0 + c8 * 8, a.thr + a.ldg + q0 + c8 * 8, rv, a.B - (q0 + c8 * 8), tn, inv,
+                            acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3], acc[c8 * 8 + 4], acc[c8 * 8 + 5],
+                            acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
+        lacc += (double)lsum;
       } else {
       const int lt = tile - J.tile0, rep = lt / J.tiles_per_rep;
       const int row0 = (lt - rep * J.tiles_per_rep) * TM;
@@ -516,7 +603,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
       for (int o = 16; o > 0; o >>= 1) lacc += __shfl_xor_sync(0xffffffffu, lacc, o);
       if (lane == 0 && lacc != 0.0) atomicAdd(a.loss_sum, lacc);
     }
-    if (MODE == 2) {                                  // one slot per epilogue warp: summed later in a fixed order
+    if (MODE == 2 || MODE == 5) {                     // one slot per epilogue warp: summed later in a fixed order
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) lacc += __shfl_xor_sync(0xffffffffu, lacc, o);
       if (lane == 0) a.loss_partial[blockIdx.x * kEpiWarps + warp] = lacc;
@@ -1227,6 +1314,35 @@ ScoreLayout score_layout(int B, int n_local, int r2) {
 }
 }  // namespace
 
+// steps 3 and 4 of the score mode (shared by the BCE and the CE paths): dO = G qp, H = G^T O, loss reduction
+static int score_tc3_backward(const float* q, const float* qp, const float* O, int B, int r2, int n_local,
+                              const ScoreLayout& L, char* base, double* loss_sum, float* H, float* dO, cudaStream_t s) {
+  float* G = (float*)(base + L.G);
+  // ---- 3. dO = G Q'  (Q' = qp = q A_O when the caller folds the right factor of the projection in, else q) ----
+  {
+    JobSpec j{};
+    j.Y = dO; j.ldy = r2; j.n = n_local; j.nk = 1; j.reps = 1;
+    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].rk = B; j.t[0].K = qp ? qp : q; j.t[0].k_f32 = 1; j.t[0].rows_total = B;
+    int rc = run_apply(1, &j, r2, base + L.kws, s);
+    if (rc) return rc;
+  }
+  // ---- 4. H = G^T O in entity chunks ----
+  {
+    JobSpec j{};
+    float* Hpart = (float*)(base + L.hpart);
+    j.Y = Hpart; j.ldy = r2; j.n = B; j.nk = 1; j.reps = L.reps; j.y_rep = (int64_t)B * r2;
+    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].xt = 1; j.t[0].rk = L.chunk; j.t[0].x_rep = (int64_t)L.chunk * L.Bp;
+    j.t[0].K = O; j.t[0].k_f32 = 1; j.t[0].rows_total = n_local;
+    int rc = run_apply(1, &j, r2, base + L.kws, s);
+    if (rc) return rc;
+    score_finish_kernel<<<rt::cdiv(B * r2, 256), 256, 0, s>>>(Hpart, L.reps, B * r2, H, (const double*)(base + L.slots),
+                                                              rt::sm_count() * kEpiWarps, (const double*)(base + L.delta), B,
+                                                              loss_sum);
+    RT_LAUNCH_CHECK();
+  }
+  return 0;
+}
+
 extern "C" int rt_score_bce_tc3_supported(int B, int n_local, int r2) {
   return (B >= 1 && B <= 256 * MAX_JOBS && r2 >= 64 && r2 <= RCP_MAX && n_local >= 1024 && make_plan(256).nstages >= 3 &&
           make_plan(r2).nstages >= 3) ? 1 : 0;
@@ -1276,30 +1392,140 @@ extern "C" int rt_score_bce_tc3(const float* q, const float* qp, const float* O,
   score_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx, t_pos, t_neg,
                                                             inv_count, G, L.Bp, (double*)(base + L.delta));
   RT_LAUNCH_CHECK();
-  // ---- 3. dO = G Q'  (Q' = qp = q A_O when the caller folds the right factor of the projection in, else q) ----
-  {
-    JobSpec j{};
-    j.Y = dO; j.ldy = r2; j.n = n_local; j.nk = 1; j.reps = 1;
-    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].rk = B; j.t[0].K = qp ? qp : q; j.t[0].k_f32 = 1; j.t[0].rows_total = B;
-    int rc = run_apply(1, &j, r2, base + L.kws, s);
-    if (rc) return rc;
+  return score_tc3_backward(q, qp, O, B, r2, n_local, L, base, loss_sum, H, dO, s);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// 1-N softmax cross-entropy on the tensor cores (variant 3 of rt_score_lse / rt_score_ce_fwd_bwd, rtucker.h).
+//   log-sum-exp pass: the score mode's logits (same query images, job layout and 3xTF32 accumulation), epilogue mode 4
+//     writes (m, s) per (32-row group, query); lse_combine (score_bce.cu) merges the groups in a fixed order;
+//   gradient pass: ce_row_stats turns the parts of all shards into (M_b, log2 S_b), epilogue mode 5 writes
+//     G = (softmax - ls/N) / B and the ls/N part of the loss, score_ce_fix_positives_kernel patches the positives,
+//     then steps 3 and 4 of the score mode unchanged.
+// ---------------------------------------------------------------------------------------------------------------
+namespace rt {
+int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
+int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
+}  // namespace rt
+
+namespace {
+// the logits launch of the score mode: rows = the n_local entities, 256 queries per job, query images at kq
+Args score_logit_args(const float* O, int B, int r2, int n_local, const unsigned char* kq) {
+  const Plan p = make_plan(256);
+  Args a{};
+  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
+  a.stage_bytes = p.stage_bytes; a.Kimg = kq;
+  a.njobs = rt::cdiv(B, 256);
+  const int nblk = rt::cdiv(r2, KB), tiles_per_job = rt::cdiv(n_local, TM);
+  for (int j = 0; j < a.njobs; ++j) {
+    Job& J = a.job[j];
+    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
+    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = nblk;
+    J.nblk = nblk; J.kblk0 = j * nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
+    J.reps = 1; J.tiles_per_rep = tiles_per_job;
   }
-  // ---- 4. H = G^T O in entity chunks ----
+  a.ntiles = a.njobs * tiles_per_job;
+  a.B = B;
+  return a;
+}
+
+struct LseLayout { size_t kq, part, total; int groups, Bp, nblk, njobs; };
+LseLayout lse_layout(int B, int n_local, int r2) {
+  LseLayout L;
+  const Plan p256 = make_plan(256);
+  L.njobs = rt::cdiv(B, 256); L.Bp = 256 * L.njobs; L.nblk = rt::cdiv(r2, KB);
+  L.groups = 4 * rt::cdiv(n_local, TM);                      // 32-row groups of one job's tiles
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
+  L.kq = take((size_t)L.njobs * L.nblk * p256.kimg_bytes);
+  L.part = take(sizeof(float2) * (size_t)L.groups * L.Bp);
+  L.total = o;
+  return L;
+}
+
+__global__ void score_ce_fix_positives_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2,
+                                              int n_begin, int n_local, const int32_t* __restrict__ off,
+                                              const int32_t* __restrict__ idx, float one_minus_ls, float t_neg,
+                                              float inv_count, const float* __restrict__ stats, int ldst,
+                                              float* __restrict__ G, int64_t ldg, double* __restrict__ delta) {
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  const int e0 = __ldg(off + b), e1 = __ldg(off + b + 1);
+  const float tp = e1 > e0 ? one_minus_ls / (float)(e1 - e0) : 0.0f;    // (1 - ls) / |y_b| from the FULL target list
+  const float M = __ldg(stats + b), L2 = __ldg(stats + ldst + b);
+  double dl = 0.0;
+  for (int i = e0 + lane; i < e1; i += 32) {
+    const int fl = __ldg(idx + i) - n_begin;
+    if (fl < 0 || fl >= n_local) continue;
+    const float d = exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2) - M;
+    const float p = ex2_fast(fmaf(d, 1.4426950408889634f, -L2));
+    G[(int64_t)fl * ldg + b] = (p - (tp + t_neg)) * inv_count;
+    dl += (double)tp * ((double)L2 * 0.6931471805599453 - (double)d);   // the epilogue charged the ls/N part
+  }
+  // a query without targets: loss_b = lse_b - (ls/N) sum_j z_bj, i.e. (1 - ls) lse_b beyond the ls/N part, charged
+  // once, to the shard that starts at entity 0
+  if (lane == 0 && e1 == e0 && n_begin == 0 && L2 < INFINITY) dl += (double)one_minus_ls * ((double)M + (double)L2 * 0.6931471805599453);
+  dl = rt::warp_sum(dl);
+  if (lane == 0) delta[b] = dl;
+}
+}  // namespace
+
+namespace rt {
+size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2) { return lse_layout(B, n_local, r2).total; }
+
+int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s) {
+  const LseLayout L = lse_layout(B, n_local, r2);
+  const Plan p = make_plan(256);
+  char* base = (char*)ws;
+  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kq), p.cs_k, p.kimg_bytes);
+  RT_LAUNCH_CHECK();
+  Args a = score_logit_args(O, B, r2, n_local, (const unsigned char*)(base + L.kq));
+  a.G = (float*)(base + L.part); a.ldg = L.Bp;
+  const int grid = std::min(rt::sm_count(), a.ntiles);
+  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 4>, SMEM_LIMIT));
+  apply_tc_kernel<16, 4><<<grid, kThreads, p.smem, s>>>(a);
+  RT_LAUNCH_CHECK();
+  return lse_combine((const float2*)(base + L.part), L.groups, L.Bp, B, parts, s);
+}
+
+size_t score_ce_tc3_ws_bytes(int B, int n_local, int r2) {
+  const ScoreLayout L = score_layout(B, n_local, r2);
+  return L.total + rt::align_up(sizeof(float) * 2 * (size_t)L.Bp, 256);
+}
+
+int score_ce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* parts,
+                 int nparts, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s) {
+  const ScoreLayout L = score_layout(B, n_local, r2);
+  const Plan p = make_plan(256);
+  char* base = (char*)ws;
+  float* G = (float*)(base + L.G);
+  float* stats = (float*)(base + L.total);                   // [M_b | log2 S_b], stride Bp
+  const float t_neg = label_smoothing / (float)n_total;
+  const float inv_count = (float)(1.0 / (double)b_total);
+  if (int rc = ce_row_stats(parts, nparts, B, L.Bp, stats, s)) return rc;
+  const size_t pad_rows = (size_t)L.reps * L.chunk - n_local;
+  if (pad_rows) RT_CHECK_CUDA(cudaMemsetAsync(G + (size_t)n_local * L.Bp, 0, pad_rows * L.Bp * sizeof(float), s));
+  // ---- 1. logits -> ls/N part of the loss, G for all-negative targets ----
+  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kq), p.cs_k, p.kimg_bytes);
+  RT_LAUNCH_CHECK();
   {
-    JobSpec j{};
-    float* Hpart = (float*)(base + L.hpart);
-    j.Y = Hpart; j.ldy = r2; j.n = B; j.nk = 1; j.reps = L.reps; j.y_rep = (int64_t)B * r2;
-    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].xt = 1; j.t[0].rk = L.chunk; j.t[0].x_rep = (int64_t)L.chunk * L.Bp;
-    j.t[0].K = O; j.t[0].k_f32 = 1; j.t[0].rows_total = n_local;
-    int rc = run_apply(1, &j, r2, base + L.kws, s);
-    if (rc) return rc;
-    score_finish_kernel<<<rt::cdiv(B * r2, 256), 256, 0, s>>>(Hpart, L.reps, B * r2, H, (const double*)(base + L.slots),
-                                                              rt::sm_count() * kEpiWarps, (const double*)(base + L.delta), B,
-                                                              loss_sum);
+    Args a = score_logit_args(O, B, r2, n_local, (const unsigned char*)(base + L.kq));
+    a.n_begin = n_begin; a.G = G; a.ldg = L.Bp; a.t_neg = t_neg; a.inv_count = inv_count; a.thr = stats;
+    a.loss_partial = (double*)(base + L.slots);
+    RT_CHECK_CUDA(cudaMemsetAsync(a.loss_partial, 0, sizeof(double) * (size_t)rt::sm_count() * kEpiWarps, s));
+    RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 5>, SMEM_LIMIT));
+    apply_tc_kernel<16, 5><<<L.grid, kThreads, p.smem, s>>>(a);
     RT_LAUNCH_CHECK();
   }
-  return 0;
+  // ---- 2. positives ----
+  score_ce_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx,
+                                                               1.0f - label_smoothing, t_neg, inv_count, stats, L.Bp, G,
+                                                               L.Bp, (double*)(base + L.delta));
+  RT_LAUNCH_CHECK();
+  return score_tc3_backward(q, qp, O, B, r2, n_local, L, base, loss_sum, H, dO, s);
 }
+}  // namespace rt
 
 extern "C" int rt_apply_multi(int njobs, const rt_apply_job* jobs, int rc, void* ws, void* stream) {
   RT_REQUIRE(njobs >= 1 && njobs <= MAX_JOBS, "rt_apply_multi: 1..%d jobs per launch, got %d", MAX_JOBS, njobs);

@@ -74,7 +74,12 @@ __device__ __forceinline__ void gemm_k64(const float* __restrict__ Gk, const flo
   }
 }
 
-template <int CPT, bool EVAL>
+__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
+constexpr float kLog2e = 1.4426950408889634f, kLn2 = 0.6931471805599453f;
+
+// CE (1-N softmax cross-entropy) reuses ScoreArgs: p_target = row statistics [2][B] (max logit M_b, log2 S_b of the
+// whole batch row, see ce_row_stats_kernel), t_pos = 1 - ls, t_neg = ls / n_total, inv_count = 1 / B_total.
+template <int CPT, bool EVAL, bool CE = false>
 __global__ void __launch_bounds__(256, 1)
 score_kernel(ScoreArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -170,12 +175,31 @@ score_kernel(ScoreArgs a) {
         float pt = 0.0f;
         int tcol = -1;
         if (EVAL && b < a.B) { pt = a.p_target[b]; tcol = a.target[b] - a.n_begin - n0; }
+        float rowM = 0.0f, rowL = 0.0f, tpos = 0.0f;
+        if (CE && b < a.B) {
+          rowM = a.p_target[b]; rowL = a.p_target[a.B + b];
+          const int cnt = a.off[b + 1] - a.off[b];
+          tpos = (cnt > 0 ? a.t_pos / (float)cnt : 0.0f) + a.t_neg;
+        }
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
           const int cc = tx + 16 * j;
           const bool valid = (b < a.B) && (n0 + cc < a.n_local);
           const bool pos = (m >> cc) & 1ull;
           const float zz = z[i][j];
+          if (CE) {
+            // G = (softmax - t) / B_total with softmax = 2^((z - M) log2e - log2 S); loss += t (lse - z)
+            const float t = pos ? tpos : a.t_neg;
+            float g = 0.0f;
+            if (valid) {
+              const float d = zz - rowM;
+              g = (ex2_approx(fmaf(d, kLog2e, -rowL)) - t) * a.inv_count;
+              loss_t += t * fmaf(rowL, kLn2, -d);
+            }
+            Gz[rr * GLD + cc] = g;
+            GzT[cc * GLD + rr] = g;
+            continue;
+          }
           const float p = 1.0f / (1.0f + expf(-zz));
           const float lp = fmaxf(logf(p), -100.0f);
           const float lq = fmaxf(log1pf(-p), -100.0f);
@@ -380,24 +404,150 @@ Plan make_plan(int n_local, int r2, bool eval) {
   return p;
 }
 
-template <int CPT, bool EVAL>
+template <int CPT, bool EVAL, bool CE = false>
 int launch(const ScoreArgs& a, const Plan& p, cudaStream_t s) {
-  RT_CHECK_CUDA(cudaFuncSetAttribute(score_kernel<CPT, EVAL>,
+  RT_CHECK_CUDA(cudaFuncSetAttribute(score_kernel<CPT, EVAL, CE>,
                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem));
-  score_kernel<CPT, EVAL><<<p.grid, 256, p.smem, s>>>(a);
+  score_kernel<CPT, EVAL, CE><<<p.grid, 256, p.smem, s>>>(a);
   RT_LAUNCH_CHECK();
   return 0;
 }
 
-template <bool EVAL>
+template <bool EVAL, bool CE = false>
 int dispatch(const ScoreArgs& a, const Plan& p, cudaStream_t s) {
   switch (p.cpt) {
-    case 2: return launch<2, EVAL>(a, p, s);
-    case 4: return launch<4, EVAL>(a, p, s);
-    case 7: return launch<7, EVAL>(a, p, s);
-    case 13: return launch<13, EVAL>(a, p, s);
-    default: return launch<16, EVAL>(a, p, s);
+    case 2: return launch<2, EVAL, CE>(a, p, s);
+    case 4: return launch<4, EVAL, CE>(a, p, s);
+    case 7: return launch<7, EVAL, CE>(a, p, s);
+    case 13: return launch<13, EVAL, CE>(a, p, s);
+    default: return launch<16, EVAL, CE>(a, p, s);
   }
+}
+
+// ---- 1-N softmax cross-entropy, FFMA path: the log-sum-exp pass --------------------------------------------------
+// Tile of 64 queries x 64 entities per CTA with score_dense_kernel's staging and k order (the logits are bit-identical
+// to the ones score_kernel<., false, true> sees).  Per query row and tile: m = the largest logit, s = sum exp(z - m)
+// (online max: no fixed shift can keep every term of a trained query from underflowing), written to part[tile][b].
+__device__ __forceinline__ void lse_merge(float& m, float& s, float m2, float s2) {
+  if (m2 == -INFINITY) return;
+  if (m == -INFINITY) { m = m2; s = s2; return; }
+  const float mn = fmaxf(m, m2);
+  s = s * ex2_approx((m - mn) * kLog2e) + s2 * ex2_approx((m2 - mn) * kLog2e);
+  m = mn;
+}
+
+__global__ void __launch_bounds__(256)
+score_lse_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2, int n_local,
+                 float2* __restrict__ part) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int ldw = row_ld(r2, 1);
+  const int k_end = (r2 + 3) / 4 * 4;
+  float* Os = reinterpret_cast<float*>(smem_raw);
+  float* Qs = Os + NT * ldw;
+  const int n0 = blockIdx.x * NT, b0 = blockIdx.y * BT;
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  for (int e = threadIdx.x; e < NT * ldw; e += 256) {
+    const int rr = e / ldw, cc = e - rr * ldw;
+    Os[e] = (n0 + rr < n_local && cc < r2) ? __ldg(O + (int64_t)(n0 + rr) * r2 + cc) : 0.0f;
+    Qs[e] = (b0 + rr < B && cc < r2) ? __ldg(q + (int64_t)(b0 + rr) * r2 + cc) : 0.0f;
+  }
+  __syncthreads();
+  float z[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) z[i][j] = 0.0f;
+  for (int k = 0; k < k_end; k += 4) {
+    float4 qv[4], ov[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) qv[i] = *reinterpret_cast<const float4*>(Qs + (ty + 16 * i) * ldw + k);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) ov[j] = *reinterpret_cast<const float4*>(Os + (tx + 16 * j) * ldw + k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        z[i][j] = fmaf(qv[i].x, ov[j].x, z[i][j]);
+        z[i][j] = fmaf(qv[i].y, ov[j].y, z[i][j]);
+        z[i][j] = fmaf(qv[i].z, ov[j].z, z[i][j]);
+        z[i][j] = fmaf(qv[i].w, ov[j].w, z[i][j]);
+      }
+  }
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int b = b0 + ty + 16 * i;
+    float m = -INFINITY, s = 0.0f;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (n0 + tx + 16 * j < n_local) m = fmaxf(m, z[i][j]);
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      if (n0 + tx + 16 * j < n_local) s += ex2_approx((z[i][j] - m) * kLog2e);
+    // the 16 lanes of this row: butterfly (merge is commutative, so every lane ends with the same bits)
+#pragma unroll
+    for (int o = 8; o > 0; o >>= 1) {
+      const float m2 = __shfl_xor_sync(0xffffffffu, m, o), s2 = __shfl_xor_sync(0xffffffffu, s, o);
+      lse_merge(m, s, m2, s2);
+    }
+    if (tx == 0 && b < B) part[(int64_t)blockIdx.x * B + b] = make_float2(m, s);
+  }
+}
+
+// out[b] = (m, s) of query b merged over part[g][b], g < ngroups (row stride ld), in a fixed order: one warp per query,
+// lane-strided groups, then a butterfly.  fp64 inside.  ngroups == 0 gives the empty part (-inf, 0).
+__global__ void lse_combine_kernel(const float2* __restrict__ part, int ngroups, int64_t ld, int B,
+                                   float* __restrict__ out) {
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= B) return;
+  double m = -INFINITY, s = 0.0;
+  for (int g = lane; g < ngroups; g += 32) {
+    const float2 p = __ldg(part + (int64_t)g * ld + b);
+    if (p.x == -INFINITY) continue;
+    const double pm = p.x;
+    if (pm > m) { s = s * exp(m - pm) + (double)p.y; m = pm; }
+    else s += (double)p.y * exp(pm - m);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const double m2 = __shfl_xor_sync(0xffffffffu, m, o), s2 = __shfl_xor_sync(0xffffffffu, s, o);
+    if (m2 != -INFINITY) {
+      if (m == -INFINITY) { m = m2; s = s2; }
+      else { const double mn = fmax(m, m2); s = s * exp(m - mn) + s2 * exp(m2 - mn); m = mn; }
+    }
+  }
+  if (lane == 0) { out[2 * b] = (float)m; out[2 * b + 1] = (float)s; }
+}
+
+// Row statistics of the whole batch from the shard parts [nparts][B][2] (fixed order over the parts):
+// stats[b] = M_b (largest logit over all shards), stats[ld + b] = log2 S_b with S_b = sum_p s_p 2^((m_p - M_b) log2e),
+// so that lse_b = M_b + ln 2 * log2 S_b.  Columns b in [B, ld) get (0, +inf): softmax 0.
+__global__ void ce_row_stats_kernel(const float* __restrict__ parts, int nparts, int B, int ld, float* __restrict__ stats) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= ld) return;
+  double M = -INFINITY, S = 0.0;
+  if (b < B) {
+    for (int p = 0; p < nparts; ++p) M = fmax(M, (double)parts[((int64_t)p * B + b) * 2]);
+    if (M != -INFINITY)
+      for (int p = 0; p < nparts; ++p) {
+        const double m = parts[((int64_t)p * B + b) * 2], s = parts[((int64_t)p * B + b) * 2 + 1];
+        if (m != -INFINITY) S += s * exp(m - M);
+      }
+  }
+  const bool ok = S > 0.0;
+  stats[b] = ok ? (float)M : 0.0f;
+  stats[ld + b] = ok ? (float)log2(S) : INFINITY;
+}
+
+// loss_sum += sum over the queries WITHOUT targets of (1 - ls) lse_b: their loss is lse_b - (ls/N) sum_j z_bj and the
+// elementwise pass charged the ls/N part.  One warp, fixed order.  Called for the shard that starts at entity 0.
+__global__ void ce_empty_rows_kernel(const int32_t* __restrict__ off, int B, const float* __restrict__ stats, int ld,
+                                     float one_minus_ls, double* __restrict__ loss_sum) {
+  double v = 0.0;
+  for (int b = threadIdx.x; b < B; b += 32)
+    if (off[b + 1] == off[b] && stats[ld + b] < INFINITY)
+      v += (double)one_minus_ls * ((double)stats[b] + (double)stats[ld + b] * 0.6931471805599453);
+  v = rt::warp_sum(v);
+  if (threadIdx.x == 0) loss_sum[0] += v;
 }
 
 }  // namespace
@@ -562,4 +712,107 @@ extern "C" int rt_score_dense(const float* q, const float* O, int B, int r2, int
                               int64_t ldp, void* stream) {
   RT_REQUIRE(B >= 0 && r2 > 0 && r2 <= 1024 && n_local >= 0 && ldp >= n_local, "rt_score_dense: bad shape");
   return rt::score_dense(q, O, B, r2, n_local, P, ldp, nullptr, (cudaStream_t)stream);
+}
+
+// ---- 1-N softmax cross-entropy (rtucker.h: rt_score_lse / rt_score_ce_fwd_bwd) ------------------------------------
+// Variant 3 lives in apply_tc.cu (log-sum-exp and CE epilogue modes of apply_tc_kernel); variant 0 is the FFMA path:
+// score_lse_kernel + lse_combine_kernel, then ce_row_stats_kernel + score_kernel<., false, true>.
+namespace rt {
+int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s) {
+  lse_combine_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(part, ngroups, ld, B, out);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s) {
+  ce_row_stats_kernel<<<rt::cdiv(ld, 256), 256, 0, s>>>(parts, nparts, B, ld, stats);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2);
+int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s);
+size_t score_ce_tc3_ws_bytes(int B, int n_local, int r2);
+int score_ce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* parts,
+                 int nparts, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s);
+}  // namespace rt
+
+static int ce_check_variant(const char* fn, int variant, int B, int n_local, int r2) {
+  RT_REQUIRE(variant == 0 || variant == 3, "%s: variant %d has no cross-entropy path (0 = FFMA, 3 = tensor cores)", fn,
+             variant);
+  RT_REQUIRE(variant == 0 || rt_score_bce_tc3_supported(B, n_local, r2),
+             "%s: variant 3 needs r2 >= 64, n_local >= 1024 and B <= 1024 (got B=%d n_local=%d r2=%d); use variant 0", fn,
+             B, n_local, r2);
+  return 0;
+}
+
+extern "C" size_t rt_score_lse_ws_bytes(int B, int n_local, int r2, int variant) {
+  if (variant == 3) return rt::score_lse_tc3_ws_bytes(B, n_local, r2);
+  return (size_t)rt::cdiv(n_local, NT) * (size_t)B * sizeof(float2) + 256;
+}
+
+extern "C" int rt_score_lse(const float* q, const float* O, int B, int r2, int n_local, int variant, float* parts,
+                            void* ws, void* stream) {
+  RT_REQUIRE(B > 0 && r2 > 0 && r2 <= 256 && n_local >= 0, "rt_score_lse: bad shape B=%d r2=%d n_local=%d", B, r2,
+             n_local);
+  RT_REQUIRE(ws != nullptr && parts != nullptr, "rt_score_lse: workspace or parts is NULL");
+  if (int rc = ce_check_variant("rt_score_lse", variant, B, n_local, r2)) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (variant == 3) return rt::score_lse_tc3(q, O, B, r2, n_local, parts, ws, s);
+  const int n_tiles = rt::cdiv(n_local, NT);
+  float2* part = (float2*)ws;
+  if (n_tiles > 0) {
+    const size_t smem = (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float);
+    RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)score_lse_kernel, smem));
+    score_lse_kernel<<<dim3(n_tiles, rt::cdiv(B, BT)), 256, smem, s>>>(q, O, B, r2, n_local, part);
+    RT_LAUNCH_CHECK();
+  }
+  return rt::lse_combine(part, n_tiles, B, B, parts, s);
+}
+
+extern "C" size_t rt_score_ce_ws_bytes(int B, int n_local, int r2, int variant) {
+  if (variant == 3) return rt::score_ce_tc3_ws_bytes(B, n_local, r2);
+  return rt::align_up(rt_score_bce_ws_bytes(B, n_local, r2, 0), 256) + 2 * (size_t)B * sizeof(float);
+}
+
+extern "C" int rt_score_ce_fwd_bwd(const float* q, const float* qp, const float* O, int B, int r2, int n_begin,
+                                   int n_local, int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx,
+                                   float label_smoothing, const float* parts, int nparts, double* loss_sum, float* H,
+                                   float* dO, int variant, void* ws, void* stream) {
+  RT_REQUIRE(B > 0 && r2 > 0 && r2 <= 256 && n_local >= 0 && n_total > 0 && b_total > 0,
+             "rt_score_ce_fwd_bwd: bad shape B=%d r2=%d n_local=%d", B, r2, n_local);
+  RT_REQUIRE(nparts >= 1, "rt_score_ce_fwd_bwd: nparts must be >= 1 (got %d)", nparts);
+  RT_REQUIRE(ws != nullptr && parts != nullptr, "rt_score_ce_fwd_bwd: workspace or parts is NULL");
+  if (int rc = ce_check_variant("rt_score_ce_fwd_bwd", variant, B, n_local, r2)) return rc;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (variant == 3)
+    return rt::score_ce_tc3(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx, label_smoothing,
+                            parts, nparts, loss_sum, H, dO, ws, s);
+  Plan p = make_plan(n_local, r2, false);
+  const size_t bce_bytes = rt::align_up(rt_score_bce_ws_bytes(B, n_local, r2, 0), 256);
+  float* stats = (float*)((char*)ws + bce_bytes);
+  if (int rc = rt::ce_row_stats(parts, nparts, B, B, stats, s)) return rc;
+  ScoreArgs a{};
+  a.q = q; a.qp = qp ? qp : q; a.O = O;
+  a.B = B; a.r2 = r2; a.n_begin = n_begin; a.n_local = n_local; a.n_total = n_total;
+  a.off = tgt_off; a.idx = tgt_idx;
+  a.t_neg = label_smoothing / (float)n_total;
+  a.t_pos = 1.0f - label_smoothing;
+  a.inv_count = (float)(1.0 / (double)b_total);
+  a.p_target = stats;
+  a.H_ws = (float*)ws;
+  a.loss_partial = (double*)((char*)ws + rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256));
+  a.dO = dO;
+  a.n_tiles = p.n_tiles;
+  int rc = dispatch<false, true>(a, p, s);
+  if (rc) return rc;
+  const int64_t count = (int64_t)B * r2;
+  reduce_H_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
+  RT_LAUNCH_CHECK();
+  reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, loss_sum, 0);
+  RT_LAUNCH_CHECK();
+  if (n_begin == 0) {
+    ce_empty_rows_kernel<<<1, 32, 0, s>>>(tgt_off, B, stats, B, 1.0f - label_smoothing, loss_sum);
+    RT_LAUNCH_CHECK();
+  }
+  return 0;
 }

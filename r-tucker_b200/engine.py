@@ -30,6 +30,16 @@ f32, f64 = torch.float32, torch.float64
 GRAPHS_WITH_NCCL = os.environ.get("RT_GRAPH_NCCL", "1") == "1"
 
 
+LOSSES = ("bce", "ce")
+
+
+def check_loss(loss):
+    """The training objectives the fused score stage implements: "bce" (label-smoothed sigmoid BCE, the reference's)
+    and "ce" (1-N softmax cross-entropy)."""
+    if loss not in LOSSES:
+        raise ValueError(f"loss must be one of {LOSSES}, got {loss!r}")
+
+
 @dataclass
 class SparseTargets:
     """Multi-hot targets of a batch in CSR form: objects of query b are idx[off[b]:off[b+1]]
@@ -193,7 +203,12 @@ class StepEngine:
 
     # -------------------------------------------------------------------------------------------
     def fit(self, rel_idx, sub_idx, targets: SparseTargets, label_smoothing, reg, lr_hint=0.0,
-            normalize_grad=1.0):
+            normalize_grad=1.0, loss="bce"):
+        """Riemannian gradient and step direction of ``loss`` at the current point: "bce" (the reference's
+        label-smoothed sigmoid BCE, the default) or "ce" (1-N softmax cross-entropy over all entities,
+        rtucker.h: rt_score_ce_fwd_bwd)."""
+        check_loss(loss)
+        loss_kind = loss
         ops, small, sym = self.ops, self.small, self.sym
         r0, r1, r2 = self.rank
         core = self.core.data
@@ -219,6 +234,8 @@ class StepEngine:
         # variant 3 = the same at fp32 accuracy (3xTF32 tensor-core kernels); it falls back to variant 0 on shapes the
         # tensor-core path does not take (thin ranks, short shards)
         variant = self.score_variant
+        if loss_kind == "ce" and variant not in (0, 3):
+            raise ValueError(f"loss='ce' runs on score variants 0 (FFMA) and 3 (tensor cores), not {variant}")
         if variant == 3 and not (getattr(ops, "HAS_SCORE_V3", False) and ops.score_tc3_supported(B, O.shape[0], r2)):
             variant = 0
         # variant 2 returns dO = G^T q and leaves the right factor A_O to the projection apply ("fold"): measured on real
@@ -226,20 +243,23 @@ class StepEngine:
         # components along the weak directions of the core; variants 0 and 3 contract with qp = q A_O directly
         fold_a = variant == 2 and getattr(ops, "HAS_SCORE_V3", False) and ops.score_v3_supported(r2)
         dO_raw = self.dV_new[k_obj] if fold_a else None
-        with self._stage("score_bce_fwd_bwd"):
-            if fold_a:
-                ops.score_bce_fwd_bwd(q, None, O, targets.off, targets.idx, label_smoothing, n_total=self.n_total,
-                                      b_total=B, n_begin=self.n_begin, variant=2, out=(bce_sum, H, dO_raw),
-                                      o_absmax=1.0,     # factors of a point on the manifold are orthonormal
-                                      centre=self.score_centre)
-            else:
-                ops.score_bce_fwd_bwd(q, qp, O, targets.off, targets.idx, label_smoothing, n_total=self.n_total,
-                                      b_total=B, n_begin=self.n_begin, variant=variant if variant == 3 else min(variant, 1),
-                                      out=(bce_sum, H, dOp))
+        if loss_kind == "ce":
+            self._score_ce(q, qp, O, targets, label_smoothing, variant, (bce_sum, H, dOp))
+        else:
+            with self._stage("score_bce_fwd_bwd"):
+                if fold_a:
+                    ops.score_bce_fwd_bwd(q, None, O, targets.off, targets.idx, label_smoothing, n_total=self.n_total,
+                                          b_total=B, n_begin=self.n_begin, variant=2, out=(bce_sum, H, dO_raw),
+                                          o_absmax=1.0,     # factors of a point on the manifold are orthonormal
+                                          centre=self.score_centre)
+                else:
+                    ops.score_bce_fwd_bwd(q, qp, O, targets.off, targets.idx, label_smoothing, n_total=self.n_total,
+                                          b_total=B, n_begin=self.n_begin, variant=variant if variant == 3 else min(variant, 1),
+                                          out=(bce_sum, H, dOp))
         self._allreduce(H, bce_sum)
         with self._stage("query_bwd"):
             d_core, ds_rows, dr_rows = ops.query_bwd(core, r_rows, s_rows, H)
-        inv_count = 1.0 / (float(B) * float(self.n_total))
+        inv_count = 1.0 / float(B) if loss_kind == "ce" else 1.0 / (float(B) * float(self.n_total))
         with self._stage("small_grad"):
             dS_g, loss, drA, dsA, P_R, P_S, P_O = small.grad(core, d_core, qp, H, r_rows, s_rows, dr_rows,
                                                              ds_rows, bce_sum, inv_count, self.hyper)
@@ -294,6 +314,25 @@ class StepEngine:
         self.loss = self.loss_buf
         self.rgrad_norm = self.norm_buf
         return self.norm_buf
+
+    def _score_ce(self, q, qp, O, targets, label_smoothing, variant, out):
+        """1-N softmax cross-entropy: the log-sum-exp pass over this shard, the (m, s) parts of every shard (one
+        all-reduce of a zero-filled [world, B, 2] buffer in which each rank fills its own slot), then the gradient
+        pass.  The loss scalar and H are all-reduced by the caller as for the BCE."""
+        ops = self.ops
+        B = q.shape[0]
+        with self._stage("score_lse"):
+            parts = ops.score_lse(q, O, variant=variant)
+        if self.group is not None:
+            import torch.distributed as dist
+            world, rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+            allp = torch.zeros(world, B, 2, dtype=parts.dtype, device=parts.device)
+            allp[rank].copy_(parts)
+            self._allreduce(allp)
+            parts = allp
+        with self._stage("score_ce_fwd_bwd"):
+            ops.score_ce_fwd_bwd(q, qp, O, targets.off, targets.idx, label_smoothing, parts, n_total=self.n_total,
+                                 b_total=B, n_begin=self.n_begin, variant=variant, out=out)
 
     # -------------------------------------------------------------------------------------------
     def step(self, lr):
@@ -456,11 +495,13 @@ class StepEngine:
                 and self.ops is cuda_ops and getattr(self, "timers", None) is None)
 
     def fit_auto(self, rel_idx, sub_idx, targets: SparseTargets, label_smoothing, reg, lr_hint=0.0,
-                 normalize_grad=1.0):
-        """fit() through a captured CUDA graph once the state machine is in steady state."""
+                 normalize_grad=1.0, loss="bce"):
+        """fit() through a captured CUDA graph once the state machine is in steady state (one graph per batch size,
+        label smoothing and loss kind)."""
+        check_loss(loss)
         steady = self._eager_steps >= 1 and (self.beta is None or self.has_old)
         if not (self._graphs_ok() and steady):
-            return self.fit(rel_idx, sub_idx, targets, label_smoothing, reg, lr_hint, normalize_grad)
+            return self.fit(rel_idx, sub_idx, targets, label_smoothing, reg, lr_hint, normalize_grad, loss=loss)
         B, nnz = rel_idx.shape[0], targets.idx.shape[0]
         si = self._static_in
         if si is None or si["B"] != B or si["cap"] < nnz:
@@ -477,13 +518,13 @@ class StepEngine:
         si["off"].copy_(targets.off, non_blocking=True)
         si["idx"][:nnz].copy_(targets.idx, non_blocking=True)
         self._set_hyper(self._hyper_vals[0], reg, self.beta, normalize_grad if normalize_grad else 0.0)
-        key = ("fit", B, float(label_smoothing))
+        key = ("fit", B, float(label_smoothing), loss)
         g = self._graphs.get(key)
         if g is None:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self.fit(si["rel"], si["sub"], SparseTargets(si["off"], si["idx"]), label_smoothing, reg,
-                         lr_hint, normalize_grad)
+                         lr_hint, normalize_grad, loss=loss)
             self._graphs[key] = g
         g.replay()
         self.pending = (self.dS_dir, self.dV_new)

@@ -206,6 +206,48 @@ def score_bce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, n_total=None,
     return loss, H, dO
 
 
+# ---------------------------------------------------------------- (b') fused 1-N softmax cross-entropy + backward
+def score_lse(q, O, variant=0, out=None, ws=None):
+    """Shard-local log-sum-exp parts of every query row of ``q`` [B, r2] over the entity shard ``O``: returns
+    parts f32 [B, 2] = (m_b, s_b), m_b the largest logit, s_b = sum_j exp(z_bj - m_b) -- see rt_score_lse.
+    variant 3 (tensor cores) or 0 (FFMA)."""
+    require_cuda(q, O)
+    B, r2 = q.shape
+    n_local = O.shape[0]
+    parts = out if out is not None else torch.empty(B, 2, dtype=f32, device=q.device)
+    ws = ws if ws is not None else _ws(lib().rt_score_lse_ws_bytes(B, n_local, r2, int(variant)), q.device)
+    check(lib().rt_score_lse(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, n_local, int(variant), ptr(_c(parts, f32)),
+                             ptr(ws), stream_ptr()), "rt_score_lse")
+    return parts
+
+
+def score_ce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, parts, n_total=None, b_total=None, n_begin=0,
+                     variant=0, out=None, ws=None):
+    """1-N softmax cross-entropy and its backward (rt_score_ce_fwd_bwd).  ``parts`` f32 [nparts, B, 2] (or [B, 2]):
+    the score_lse results of every entity shard.  Returns (loss_sum[1] f64 -- un-normalised: divide by b_total,
+    H [B, r2], dO [n_local, r2])."""
+    require_cuda(q, qp, O, tgt_off, tgt_idx, parts)
+    B, r2 = q.shape
+    n_local = O.shape[0]
+    n_total = n_local if n_total is None else n_total
+    b_total = B if b_total is None else b_total
+    parts = _c(parts, f32)
+    nparts = 1 if parts.dim() == 2 else parts.shape[0]
+    if parts.shape[-2:] != (B, 2):
+        raise RTuckerError(f"score_ce_fwd_bwd: parts must be [nparts, {B}, 2], got {tuple(parts.shape)}")
+    dev = q.device
+    if out is None:
+        out = (torch.empty(1, dtype=f64, device=dev), torch.empty(B, r2, dtype=f32, device=dev),
+               torch.empty(n_local, r2, dtype=f32, device=dev))
+    loss, H, dO = out
+    ws = ws if ws is not None else _ws(lib().rt_score_ce_ws_bytes(B, n_local, r2, int(variant)), dev)
+    check(lib().rt_score_ce_fwd_bwd(ptr(_c(q, f32)), ptr(qp), ptr(_c(O, f32)), B, r2, int(n_begin), n_local,
+                                    int(n_total), int(b_total), ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)),
+                                    float(label_smoothing), ptr(parts), nparts, ptr(loss), ptr(H), ptr(dO),
+                                    int(variant), ptr(ws), stream_ptr()), "rt_score_ce_fwd_bwd")
+    return loss, H, dO
+
+
 # ---------------------------------------------------------------- (c) tall-skinny
 # The N x r x r passes run on tcgen05 (3xTF32 with round-to-nearest partial-sum accumulation: fp32 accuracy, see
 # csrc/apply_tc.cu) whenever the shape is wide enough to fill an MMA tile; thin ranks (d_e = 20) and short factors

@@ -17,7 +17,7 @@ from typing import Optional
 import torch
 from torch.optim import Optimizer
 
-from .engine import SparseTargets, StepEngine
+from .engine import SparseTargets, StepEngine, check_loss
 from .model import ScoreFn
 
 
@@ -25,11 +25,16 @@ class FusedLoss:
     """BCE(score_fn(T), targets) + reg * ||T||^2  (train.py:79) with sparse targets.
 
     Stands where the reference passes ``lambda T: criterion(score_fn(T), targets) + reg * T.norm()**2``.
+    ``loss="ce"`` selects the 1-N softmax cross-entropy over all entities instead of the BCE (the same targets,
+    normalised to 1 per query, with the same label smoothing; include/rtucker.h, rt_score_ce_fwd_bwd).
     """
 
-    def __init__(self, score_fn: ScoreFn, targets: SparseTargets, label_smoothing: float, reg_coeff: float):
+    def __init__(self, score_fn: ScoreFn, targets: SparseTargets, label_smoothing: float, reg_coeff: float,
+                 loss: str = "bce"):
+        check_loss(loss)
         self.score_fn, self.targets = score_fn, targets
         self.label_smoothing, self.reg_coeff = float(label_smoothing), float(reg_coeff)
+        self.loss = loss
 
 
 class _RiemannianBase(Optimizer):
@@ -112,7 +117,8 @@ class _RiemannianBase(Optimizer):
         if self.adam is not None:
             normalize_grad = 0.0       # SFTuckerAdam.fit never normalises (its normalize_grad argument is unused)
         norm = eng.fit_auto(sf.relation_idx, sf.subject_idx, loss_fn.targets, loss_fn.label_smoothing,
-                            loss_fn.reg_coeff, lr_hint=self.param_groups[0]["lr"], normalize_grad=normalize_grad)
+                            loss_fn.reg_coeff, lr_hint=self.param_groups[0]["lr"], normalize_grad=normalize_grad,
+                            loss=loss_fn.loss)
         self.loss = eng.loss.float().reshape(())
         self.direction = eng.pending
         return norm.float().reshape(())

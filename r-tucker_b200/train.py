@@ -9,8 +9,12 @@ Differences that follow from the fused path: the loaders are ``data.DeviceEpoch`
 epoch, on-device shuffle) yielding ``(features, SparseTargets)``; the loss closure is a ``FusedLoss``; losses and
 gradient norms are accumulated in device scalars and read back ONCE per epoch (the reference formats a device
 tensor into its tqdm bar every step, train.py:88: an implicit synchronisation per step); checkpoints carry the
-optimiser state (checkpoint.py).  ``criterion`` is accepted for signature compatibility: the fused kernels implement
-``nn.BCELoss(reduction="mean")`` (train.py:136) and nothing else.
+optimiser state (checkpoint.py).  ``criterion`` selects the training objective among the two the fused kernels
+implement: ``nn.BCELoss(reduction="mean")`` (train.py:136, the default) and ``nn.CrossEntropyLoss(reduction="mean")``
+(1-N softmax cross-entropy over all entities; no ``weight``, no ``ignore_index``, ``label_smoothing=0``: the smoothing
+comes from the loader, as for the BCE).  Evaluation is the same for both: the reference's BCE evaluation loss and the
+filtered ranks.  Ranks, ``evaluation.predict_topk`` and ``score_fn(T)`` use z or sigmoid(z), both monotone in the logit
+z, so they do not depend on which loss trained the model.
 """
 import os
 import time
@@ -32,15 +36,22 @@ def extract_tensor(model):
 
 
 def _check_criterion(criterion):
+    """The fused loss kind ("bce" or "ce") a criterion selects; TypeError for anything the kernels do not implement."""
     if criterion is None:
-        return
-    if not isinstance(criterion, nn.BCELoss) or criterion.reduction != "mean":
-        raise TypeError("the fused path implements nn.BCELoss(reduction='mean') (train.py:136); got %r" % (criterion,))
+        return "bce"
+    if isinstance(criterion, nn.BCELoss) and criterion.reduction == "mean":
+        return "bce"
+    if (isinstance(criterion, nn.CrossEntropyLoss) and criterion.reduction == "mean" and criterion.weight is None
+            and criterion.ignore_index == -100 and criterion.label_smoothing == 0.0):
+        return "ce"
+    raise TypeError("the fused path implements nn.BCELoss(reduction='mean') (train.py:136) and "
+                    "nn.CrossEntropyLoss(reduction='mean') without weight, ignore_index or label_smoothing "
+                    "(the smoothing comes from the loader); got %r" % (criterion,))
 
 
 def train_one_epoch(model, optimizer, criterion, train_loader, regularization_coeff=1e-4):
     """One pass over ``train_loader``; returns (mean loss, mean ||rgrad||) like train.py:91."""
-    _check_criterion(criterion)
+    loss_kind = _check_criterion(criterion)
     model.train()
     device = model.core.device
     n_batches = len(train_loader)
@@ -48,7 +59,7 @@ def train_one_epoch(model, optimizer, criterion, train_loader, regularization_co
     train_grad_norm = torch.zeros((), device=device)
     for features, targets in train_loader:
         score_fn = model(features[:, 0], features[:, 1])
-        loss_fn = FusedLoss(score_fn, targets, train_loader.label_smoothing, regularization_coeff)
+        loss_fn = FusedLoss(score_fn, targets, train_loader.label_smoothing, regularization_coeff, loss=loss_kind)
         x_k = extract_tensor(model)
         grad_norm = optimizer.fit(loss_fn, x_k)
         optimizer.step()
@@ -61,7 +72,8 @@ def train_one_epoch(model, optimizer, criterion, train_loader, regularization_co
 @torch.no_grad()
 def evaluate(model, criterion, dataloader, n_begin=0, group=None):
     """Filtered ranking + BCE over ``dataloader`` (features (s, r, o), targets = filter lists over all splits);
-    returns (metrics dict, mean batch loss) like train.py:124-125."""
+    returns (metrics dict, mean batch loss) like train.py:124-125.  The loss is the reference's BCE whichever
+    criterion trained the model."""
     _check_criterion(criterion)
     model.eval()
     device = model.core.device
@@ -82,11 +94,14 @@ def evaluate(model, criterion, dataloader, n_begin=0, group=None):
 
 
 def train(model, optimizer, train_loader, val_loader, test_loader, config, regulizer, scheduler=None, log_fn=None,
-          start_epoch=None, num_epoches=None, history=None):
+          start_epoch=None, num_epoches=None, history=None, criterion=None):
     """train.py:128-167: evaluate once, then per epoch: regulariser step, train epoch, validate, test, snapshot
     (now with the optimiser state), scheduler step.  ``config`` needs ``train_cfg.num_epoches`` and
-    ``train_cfg.checkpoint_path`` (configs/base_config.py); ``log_fn(record)`` replaces wandb_log."""
-    criterion = nn.BCELoss(reduction="mean")
+    ``train_cfg.checkpoint_path`` (configs/base_config.py); ``log_fn(record)`` replaces wandb_log.  ``criterion``:
+    the training objective, ``nn.BCELoss(reduction="mean")`` (the reference's, the default) or
+    ``nn.CrossEntropyLoss(reduction="mean")`` (see the module docstring); evaluation reports the BCE either way."""
+    criterion = nn.BCELoss(reduction="mean") if criterion is None else criterion
+    _check_criterion(criterion)
     num_epoches = num_epoches if num_epoches is not None else config.train_cfg.num_epoches
     start_epoch = start_epoch if start_epoch is not None else 1
     history = history if history is not None else []

@@ -65,6 +65,9 @@ def main():
     ap.add_argument("--eval-every", type=int, default=5)
     ap.add_argument("--recipe", default="head", choices=["head", "readme"])
     ap.add_argument("--total-epochs", type=int, default=500, help="length of the HEAD recipe's one-cycle schedule")
+    ap.add_argument("--loss", default="bce", choices=["bce", "ce"],
+                    help="training objective: the reference's label-smoothed BCE or the 1-N softmax cross-entropy "
+                         "(evaluation reports the BCE and the filtered ranks either way)")
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
@@ -91,7 +94,7 @@ def main():
     train_loader = DeviceEpoch(train_ds, 512, dev, shuffle="host", drop_last=True)
     val_loader = DeviceEpoch(valid_ds, 512, dev, shuffle=False)
     test_loader = DeviceEpoch(test_ds, 512, dev, shuffle=False)
-    crit = torch.nn.BCELoss(reduction="mean")
+    crit = torch.nn.CrossEntropyLoss(reduction="mean") if args.loss == "ce" else torch.nn.BCELoss(reduction="mean")
     hist = []
     t_start = time.perf_counter()
     for epoch in range(1, args.epochs + 1):
@@ -123,6 +126,7 @@ def main():
     summary = dict(config=dict(dataset="WN18RR (real triples, tests/golden/wn18rr_ids.npz)", mode=args.mode, rank=rank,
                                batch=512, optim="rsgd", recipe=args.recipe,
                                momentum=0.8, label_smoothing=0.1, seed=args.seed, score_variant=args.variant,
+                               loss=args.loss,
                                epochs=args.epochs, steps_per_epoch=len(train_loader)),
                    wall_s=time.perf_counter() - t_start, history=hist)
     if args.out:

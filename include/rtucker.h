@@ -107,6 +107,41 @@ int rt_score_dense(const float* q, const float* O, int B, int r2, int n_local, f
 int rt_filter_dense(float* P, int64_t ldp, float* T, int64_t ldt, int B, int N,
                     const int32_t* filter_col, void* stream);
 
+/* ---- (d') evaluation and prediction in logit space ----------------------------------- */
+/*
+ * For models trained with the softmax cross-entropy (rt_score_ce_fwd_bwd), whose top logits sit where the fp32 sigmoid
+ * has saturated (p == 1.0f from z = 16.6 on, coarse steps of p well below): ranks and top-k on the exact fp32 logit
+ * z_bj = q_b . O_j (k ascending, one fmaf accumulator: the value rt_score_dense passes to the sigmoid) instead of p.
+ *
+ * rt_score_dense_logits: Z[b, j] = z_bj, bit-identical to the logits inside rt_score_dense.
+ * rt_target_logit: z_target[b] = z_{b, target[b]} on the shard that owns the target, 0 elsewhere (sum over shards).
+ * rt_score_rank_logit: filtered counts in logit space, as shard partial sums.  Filtered entities are REMOVED (not
+ *   scored 0 as in rt_score_rank_fused: 0 is an ordinary logit).  With F_b = flt_idx[flt_off[b]:flt_off[b+1]] (global
+ *   ids, unique; flt_off and flt_idx both NULL: no filter), t = target[b], zt = z_target[b] (summed over shards):
+ *     greater[b]      = #{ j in shard, j not in F_b, j != t : z_bj >  zt }
+ *     equal[b]        = #{ j in shard, j not in F_b, j != t : z_bj == zt }
+ *     equal_before[b] = the same as equal, restricted to j < t           (rank = 1 + greater + equal_before)
+ *     pos_sum[b]      = sum_{j in F_b and in shard} z_bj (double; pos_sum may be NULL), summed in a fixed order.
+ *   With lse_b from rt_score_lse, lse_b - pos_sum[b] / |F_b| is the cross-entropy of the un-smoothed multi-hot target
+ *   y / |y|.  Limits: 1 <= B <= 65535, 1 <= r2 <= 256.  Deterministic; no host synchronisation.
+ * rt_score_topk_logit: rt_score_topk (same arguments, limits and workspace, rt_score_topk_ws_bytes) with z in place of
+ *   p: order z descending, then global id ascending; top_z the exact z, bit-identical to rt_score_dense_logits;
+ *   padding id -1, z = -inf.
+ */
+int rt_score_dense_logits(const float* q, const float* O, int B, int r2, int n_local, float* Z, int64_t ldz,
+                          void* stream);
+int rt_target_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local,
+                    const int32_t* target, float* z_target, void* stream);
+size_t rt_score_rank_logit_ws_bytes(int B, int n_local, int r2);
+int rt_score_rank_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local,
+                        const int32_t* target, const float* z_target,
+                        const int32_t* flt_off, const int32_t* flt_idx,
+                        int32_t* greater, int32_t* equal, int32_t* equal_before,
+                        double* pos_sum, void* ws, void* stream);
+int rt_score_topk_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
+                        const int32_t* flt_off, const int32_t* flt_idx,
+                        int32_t* top_idx, float* top_z, int32_t* n_cand, void* ws, void* stream);
+
 /* ---- (a) query contraction ----------------------------------------------------------- */
 /* out[b,:] = table[idx[b] - row_begin, :] if row_begin <= idx[b] < row_begin+rows else 0.
  * Replaces the gathers at src/model/asymmetric/R_TuckER.py:43-44 (shard-aware). */

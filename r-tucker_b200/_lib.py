@@ -35,6 +35,11 @@ PROTOTYPES = {
     "rt_score_topk_ws_bytes": (sz, [i32, i32, i32, i32]),
     "rt_score_topk": (i32, [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
     "rt_score_dense": (i32, [vp, vp, i32, i32, i32, vp, i64, vp]),
+    "rt_score_dense_logits": (i32, [vp, vp, i32, i32, i32, vp, i64, vp]),
+    "rt_target_logit": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp]),
+    "rt_score_rank_logit_ws_bytes": (sz, [i32, i32, i32]),
+    "rt_score_rank_logit": (i32, [vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "rt_score_topk_logit": (i32, [vp, vp, i32, i32, i32, i32, i32, vp, vp, vp, vp, vp, vp, vp]),
     "rt_filter_dense": (i32, [vp, i64, vp, i64, i32, i32, vp, vp]),
     "rt_gather_rows": (i32, [vp, i32, i32, i32, vp, i32, vp, vp]),
     "rt_scatter_rows_add": (i32, [vp, i32, i32, i32, vp, i32, vp, vp]),

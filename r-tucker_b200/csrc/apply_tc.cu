@@ -886,18 +886,22 @@ __global__ void rank_rownorm_kernel(const float* __restrict__ O, int n_local, in
 // bound of a logit is proportional to ||q_b|| ||O_j|| with the entity's OWN norm -- with the shard maximum the band
 // of every entity was as wide as the heaviest row needs (rows 8x heavier than average after a few hundred steps: the
 // candidate list filled up and the evaluation batch went from 0.9 to 4 ms).  Queries >= B get an empty band.
+// slope of query b's band (one warp): |z_fp32 - z_tensor| <= (r2 * 2^-24 + 1e-6) * ||q|| ||o||  (fp32 recurrence +
+// 3xTF32); factor 2 of safety, and 1e-3 relative for the fp32 evaluation of lo0 - slope * norm in the epilogue
+__device__ __forceinline__ float rank_band_slope(const float* __restrict__ q, int b, int r2, int lane) {
+  float s = 0.0f;
+  for (int k = lane; k < r2; k += 32) { const float v = __ldg(q + (int64_t)b * r2 + k); s = fmaf(v, v, s); }
+  s = rt::warp_sum(s);
+  return (float)(2.0 * ((double)r2 * 5.96e-8 + 1e-6) * sqrt((double)s) * 1.001) + 1e-30f;
+}
+
 __global__ void rank_thresholds_kernel(const float* __restrict__ q, const float* __restrict__ p_target, int B, int Bp,
                                        int r2, float* __restrict__ thr) {
   const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (b >= Bp) return;
   float lo = INFINITY, hi = INFINITY, eqlo = INFINITY, slope = 0.0f;
   if (b < B) {
-    float s = 0.0f;
-    for (int k = lane; k < r2; k += 32) { const float v = __ldg(q + (int64_t)b * r2 + k); s = fmaf(v, v, s); }
-    s = rt::warp_sum(s);
-    // |z_fp32 - z_tensor| <= (r2 * 2^-24 + 1e-6) * ||q|| ||o||  (fp32 recurrence + 3xTF32); factor 2 of safety, and
-    // 1e-3 relative for the fp32 evaluation of lo0 - slope * norm in the epilogue
-    slope = (float)(2.0 * ((double)r2 * 5.96e-8 + 1e-6) * sqrt((double)s) * 1.001) + 1e-30f;
+    slope = rank_band_slope(q, b, r2, lane);
     const double margin = 2e-6;                      // absolute part of the old margin (+ the conversions to fp32)
     const float pt = __ldg(p_target + b);
     if (pt >= 1.0f) {                 // saturated target: nothing is greater; z > 18 certainly gives p == 1
@@ -914,6 +918,28 @@ __global__ void rank_thresholds_kernel(const float* __restrict__ q, const float*
     }
   }
   if (lane == 0) { thr[b] = lo; thr[Bp + b] = hi; thr[2 * Bp + b] = eqlo; thr[3 * Bp + b] = slope; }
+}
+
+// Logit space (rt_score_rank_logit, rt_score_topk_logit): thresholds of a per-query reference LOGIT z_ref (the target's
+// exact fp32 logit, or the top-k sample threshold z_k).  lo0 = hi0 = z_ref widened by 4e-7 |z_ref| and one ulp, eqlo0 =
+// +inf (no saturated-target test: logits do not saturate), slope as above.  The bound: the epilogue classifies the
+// tensor-core logit z' of entity j against lo_u = fl(lo0 - m), hi_u = fl(hi0 + m), m = fl(slope ||O_j||) >= 2 E_j,
+// E_j = the error bound above, so |z - z'| <= E_j for the exact fp32 logit z.  Round to nearest moves hi0 + m by at
+// most 2^-24 |hi0 + m| <= 6e-8 (|hi0| + m): the widening of hi0 covers the |hi0| part, the factor 2 of m its m part,
+// so hi_u >= z_ref + E_j and z' > hi_u gives z > z_ref (certainly greater); symmetrically z' < lo_u gives z < z_ref.
+// Everything in [lo_u, hi_u] is a candidate and is recounted from its exact logit.  Queries >= B: empty band.
+__global__ void logit_thresholds_kernel(const float* __restrict__ q, const float* __restrict__ z_ref, int B, int Bp,
+                                        int r2, float* __restrict__ thr) {
+  const int b = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (b >= Bp) return;
+  float lo = INFINITY, hi = INFINITY, slope = 0.0f;
+  if (b < B) {
+    slope = rank_band_slope(q, b, r2, lane);
+    const double z = (double)__ldg(z_ref + b);
+    lo = nextafterf((float)(z - 4e-7 * fabs(z)), -INFINITY);
+    hi = nextafterf((float)(z + 4e-7 * fabs(z)), INFINITY);
+  }
+  if (lane == 0) { thr[b] = lo; thr[Bp + b] = hi; thr[2 * Bp + b] = INFINITY; thr[3 * Bp + b] = slope; }
 }
 
 // K images of the query chunks: job j, block kb: element (c, kk) = q[256 j + c][kb * KB + kk]
@@ -934,6 +960,8 @@ __global__ void rank_pack_q_kernel(const float* __restrict__ q, int B, int r2, i
   }
 }
 
+// LOGIT: compare exact logits with the target's logit (p_target then holds z_target)
+template <bool LOGIT>
 __global__ void rank_candidates_kernel(const float* __restrict__ q, const float* __restrict__ O, int r2, int n_begin,
                                        const int32_t* __restrict__ target, const float* __restrict__ p_target,
                                        const int2* __restrict__ cand, const int* __restrict__ cand_count, int cap,
@@ -944,7 +972,8 @@ __global__ void rank_candidates_kernel(const float* __restrict__ q, const float*
     const int2 c = cand[i];
     const int j = n_begin + c.x, b = c.y, t = __ldg(target + b);
     if (j == t) continue;
-    const float p = sigmoid_ref(exact_logit(q + (int64_t)b * r2, O + (int64_t)c.x * r2, r2));
+    const float z = exact_logit(q + (int64_t)b * r2, O + (int64_t)c.x * r2, r2);
+    const float p = LOGIT ? z : sigmoid_ref(z);
     const float pt = __ldg(p_target + b);
     if (p > pt) atomicAdd(greater + b, 1);
     else if (p == pt) { atomicAdd(equal + b, 1); if (j < t) atomicAdd(equal_before + b, 1); }
@@ -1022,11 +1051,31 @@ bool rank_tc_supported(int B, int n_local, int r2) {
   return B >= 1 && B <= 256 * MAX_JOBS && r2 >= 64 && r2 <= 1024 && n_local >= 1024 && make_plan(256).nstages >= 3;
 }
 size_t rank_tc_ws_bytes(int B, int n_local, int r2) { return rank_layout(B, n_local, r2).total; }
+static int rank_tc_impl(bool logit, const float* q, const float* O, int B, int r2, int n_begin, int n_local,
+                        const int32_t* target, const float* p_target, const int32_t* flt_off, const int32_t* flt_idx,
+                        int32_t* greater, int32_t* equal, int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s,
+                        const int** overflow_flag);
 // Counts and BCE of one evaluation batch on the tensor cores; *overflow_flag (device int inside ws, returned) is set
 // when the candidate list did not fit: the caller then runs the fp32 kernel gated on that flag.
 int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
             const float* p_target, const int32_t* flt_off, const int32_t* flt_idx, int32_t* greater, int32_t* equal,
             int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s, const int** overflow_flag) {
+  return rank_tc_impl(false, q, O, B, r2, n_begin, n_local, target, p_target, flt_off, flt_idx, greater, equal,
+                      equal_before, bce_sum, ws, s, overflow_flag);
+}
+// Logit space (rank_logit.cu): counts of every entity of the shard against z_target, the target itself excluded and
+// the filter list NOT applied (the caller removes it); counts are zeroed when the candidate list overflowed, with
+// *overflow_flag set as above.  The epilogue's BCE sum goes to a scratch slot of ws.
+int rank_tc_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
+                  const float* z_target, int32_t* greater, int32_t* equal, int32_t* equal_before, void* ws,
+                  cudaStream_t s, const int** overflow_flag) {
+  return rank_tc_impl(true, q, O, B, r2, n_begin, n_local, target, z_target, nullptr, nullptr, greater, equal,
+                      equal_before, nullptr, ws, s, overflow_flag);
+}
+static int rank_tc_impl(bool logit, const float* q, const float* O, int B, int r2, int n_begin, int n_local,
+                        const int32_t* target, const float* p_target, const int32_t* flt_off, const int32_t* flt_idx,
+                        int32_t* greater, int32_t* equal, int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s,
+                        const int** overflow_flag) {
   const RankLayout L = rank_layout(B, n_local, r2);
   const Plan p = make_plan(256);
   char* base = (char*)ws;
@@ -1037,7 +1086,8 @@ int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_lo
   float* onorms = (float*)(base + L.norms);
   rank_rownorm_kernel<<<rt::sm_count() * 4, 256, 0, s>>>(O, n_local, r2, (unsigned int*)(scal + 2), onorms);
   RT_LAUNCH_CHECK();
-  rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_target, B, L.Bp, r2, thr);
+  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_target, B, L.Bp, r2, thr);
+  else rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_target, B, L.Bp, r2, thr);
   RT_LAUNCH_CHECK();
   rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kimg), p.cs_k,
                                                        p.kimg_bytes);
@@ -1065,8 +1115,17 @@ int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_lo
   RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 1>, SMEM_LIMIT));
   apply_tc_kernel<16, 1><<<grid, kThreads, p.smem, s>>>(a);
   RT_LAUNCH_CHECK();
-  rank_candidates_kernel<<<rt::sm_count() * 2, 256, 0, s>>>(q, O, r2, n_begin, target, p_target, a.cand, scal, L.cap,
-                                                            greater, equal, equal_before, scal + 1);
+  if (logit) {
+    rank_candidates_kernel<true><<<rt::sm_count() * 2, 256, 0, s>>>(q, O, r2, n_begin, target, p_target, a.cand, scal,
+                                                                    L.cap, greater, equal, equal_before, scal + 1);
+    RT_LAUNCH_CHECK();
+    rank_reset_if_overflow_kernel<<<rt::cdiv(B, 256), 256, 0, s>>>(B, greater, equal, equal_before, scal + 1);
+    RT_LAUNCH_CHECK();
+    *overflow_flag = scal + 1;
+    return 0;
+  }
+  rank_candidates_kernel<false><<<rt::sm_count() * 2, 256, 0, s>>>(q, O, r2, n_begin, target, p_target, a.cand, scal,
+                                                                   L.cap, greater, equal, equal_before, scal + 1);
   RT_LAUNCH_CHECK();
   rank_filter_fix_kernel<<<rt::sm_count() * 2, 128, 0, s>>>(q, O, B, r2, n_begin, n_local, target, p_target, flt_off, flt_idx,
                                                         greater, equal, equal_before, loss, scal + 1);
@@ -1098,8 +1157,9 @@ namespace rt {
 // Appends to seg[b][0, cap) every entity j of the shard whose tensor-core logit is not certainly below the logit of
 // p_k[b] (the band of rank_thresholds_kernel for p_target = p_k); cnt[b] (zeroed by the caller) ends as the number of
 // such entities, > cap when the segment overflowed.  Queries with flag[b] != 0 are skipped.
+// logit: p_k holds the sample's logit threshold z_k and the band is logit_thresholds_kernel's.
 int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
-                 int32_t* seg, int cap, void* ws, cudaStream_t s) {
+                 int32_t* seg, int cap, void* ws, cudaStream_t s, bool logit) {
   const RankLayout L = rank_layout(B, n_local, r2);
   const Plan p = make_plan(256);
   char* base = (char*)ws;
@@ -1109,7 +1169,8 @@ int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, con
   RT_CHECK_CUDA(cudaMemsetAsync(maxnorm, 0, sizeof(unsigned int), s));
   rank_rownorm_kernel<<<rt::sm_count() * 4, 256, 0, s>>>(O, n_local, r2, maxnorm, onorms);
   RT_LAUNCH_CHECK();
-  rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
+  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
+  else rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
   RT_LAUNCH_CHECK();
   topk_empty_band_kernel<<<rt::cdiv(B, 256), 256, 0, s>>>(thr, B, flag);
   RT_LAUNCH_CHECK();

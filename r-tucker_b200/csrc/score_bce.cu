@@ -334,7 +334,9 @@ __global__ void target_prob_kernel(const float* __restrict__ q, const float* __r
 // Dense compatibility path: P[b, j] = sigmoid(q_b . O_j) written out (what score_fn(T) returns in
 // the reference, R_TuckER.py:47-48).  Same staging and k order as score_kernel, so the values are
 // bit-identical to the ones the fused kernels see.  gate (may be NULL): the launch is a no-op unless
-// *gate != 0 (the exact pass of the top-k selection, topk.cu).
+// *gate != 0 (the exact passes of the top-k selection, topk.cu, and of the logit-space ranking, rank_logit.cu).
+// LOGIT: the logits z themselves (rt_score_dense_logits).
+template <bool LOGIT = false>
 __global__ void __launch_bounds__(256)
 score_dense_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2, int n_local,
                    float* __restrict__ P, int64_t ldp, const int* __restrict__ gate) {
@@ -380,7 +382,7 @@ score_dense_kernel(const float* __restrict__ q, const float* __restrict__ O, int
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int n = n0 + tx + 16 * j;
-      if (n < n_local) P[(int64_t)b * ldp + n] = 1.0f / (1.0f + expf(-z[i][j]));
+      if (n < n_local) P[(int64_t)b * ldp + n] = LOGIT ? z[i][j] : 1.0f / (1.0f + expf(-z[i][j]));
     }
   }
 }
@@ -696,13 +698,19 @@ extern "C" int rt_score_rank_fused(const float* q, const float* O, int B, int r2
 
 namespace rt {
 int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
-                cudaStream_t s) {
+                cudaStream_t s, bool logits) {
   if (B == 0 || n_local == 0) return 0;
   const size_t smem = (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float);
-  RT_CHECK_CUDA(cudaFuncSetAttribute(score_dense_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)smem));
   dim3 grid(rt::cdiv(n_local, NT), rt::cdiv(B, BT));
-  score_dense_kernel<<<grid, 256, smem, s>>>(q, O, B, r2, n_local, P, ldp, gate);
+  if (logits) {
+    RT_CHECK_CUDA(cudaFuncSetAttribute(score_dense_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
+    score_dense_kernel<true><<<grid, 256, smem, s>>>(q, O, B, r2, n_local, P, ldp, gate);
+  } else {
+    RT_CHECK_CUDA(cudaFuncSetAttribute(score_dense_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)smem));
+    score_dense_kernel<false><<<grid, 256, smem, s>>>(q, O, B, r2, n_local, P, ldp, gate);
+  }
   RT_LAUNCH_CHECK();
   return 0;
 }
@@ -711,7 +719,13 @@ int score_dense(const float* q, const float* O, int B, int r2, int n_local, floa
 extern "C" int rt_score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P,
                               int64_t ldp, void* stream) {
   RT_REQUIRE(B >= 0 && r2 > 0 && r2 <= 1024 && n_local >= 0 && ldp >= n_local, "rt_score_dense: bad shape");
-  return rt::score_dense(q, O, B, r2, n_local, P, ldp, nullptr, (cudaStream_t)stream);
+  return rt::score_dense(q, O, B, r2, n_local, P, ldp, nullptr, (cudaStream_t)stream, false);
+}
+
+extern "C" int rt_score_dense_logits(const float* q, const float* O, int B, int r2, int n_local, float* Z, int64_t ldz,
+                                     void* stream) {
+  RT_REQUIRE(B >= 0 && r2 > 0 && r2 <= 1024 && n_local >= 0 && ldz >= n_local, "rt_score_dense_logits: bad shape");
+  return rt::score_dense(q, O, B, r2, n_local, Z, ldz, nullptr, (cudaStream_t)stream, true);
 }
 
 // ---- 1-N softmax cross-entropy (rtucker.h: rt_score_lse / rt_score_ce_fwd_bwd) ------------------------------------

@@ -15,6 +15,10 @@
 //      per flagged query.  Gated on a device flag "some query is flagged", so it is a no-op when nothing overflowed.
 //      It is the whole path where the tensor-core pass is not supported (thin ranks, shards under 1024 rows).
 // Steps 1, 3 and 4 share one block-level top-k routine over 64-bit (p, id) keys.
+//
+// Logit space (rt_score_topk_logit): the same four steps on the exact fp32 logit z instead of p, instantiated with
+// LOGIT = true: the key maps z's bit pattern order-preservingly (negative z included), the sample gives a logit
+// threshold z_k and the tensor-core band is the logit band of apply_tc.cu (logit_thresholds_kernel).
 #include "common.h"
 #include "exact.cuh"
 #include <algorithm>
@@ -24,9 +28,9 @@ namespace rt {
 bool rank_tc_supported(int B, int n_local, int r2);
 size_t topk_tc_ws_bytes(int B, int n_local, int r2);
 int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
-                 int32_t* seg, int cap, void* ws, cudaStream_t s);
+                 int32_t* seg, int cap, void* ws, cudaStream_t s, bool logit);
 int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
-                cudaStream_t s);
+                cudaStream_t s, bool logits);
 }  // namespace rt
 
 namespace {
@@ -46,6 +50,25 @@ __device__ __forceinline__ u64 make_key(float p, int id) {
 }
 __device__ __forceinline__ float key_p(u64 key) { return key ? __uint_as_float((uint32_t)(key >> 32) - 1u) : -INFINITY; }
 __device__ __forceinline__ int key_id(u64 key) { return key ? (int)(0xffffffffu - (uint32_t)key) : -1; }
+
+// Key of (z, id) for a logit of either sign: the bit pattern with the sign bit set for z >= +0 and all bits inverted for
+// z < 0 orders like the value (-inf lowest); 0 stays the empty key (only the pattern 0xffffffff, a negative NaN, maps
+// there).  -0 orders just below +0.
+__device__ __forceinline__ u64 make_key_z(float z, int id) {
+  const uint32_t b = __float_as_uint(z);
+  return ((u64)((b & 0x80000000u) ? ~b : (b | 0x80000000u)) << 32) | (u64)(0xffffffffu - (uint32_t)id);
+}
+__device__ __forceinline__ float key_z(u64 key) {
+  const uint32_t h = (uint32_t)(key >> 32);
+  return key ? __uint_as_float((h & 0x80000000u) ? (h & 0x7fffffffu) : ~h) : -INFINITY;
+}
+
+// the score of an exact logit and its key: p = sigmoid(z) (rt_score_topk) or z itself (rt_score_topk_logit)
+template <bool LOGIT> __device__ __forceinline__ float score_of(float z) { return LOGIT ? z : rt::sigmoid_ref(z); }
+template <bool LOGIT> __device__ __forceinline__ u64 key_of_score(float v, int id) {
+  return LOGIT ? make_key_z(v, id) : make_key(v, id);
+}
+template <bool LOGIT> __device__ __forceinline__ float score_of_key(u64 key) { return LOGIT ? key_z(key) : key_p(key); }
 
 // id in the ascending filter list flt_idx[f0, f1)?
 __device__ __forceinline__ bool filtered(const int32_t* __restrict__ flt_idx, int f0, int f1, int id) {
@@ -95,14 +118,16 @@ __device__ __forceinline__ void clear_keys(u64* s, int kp) {
   __syncthreads();
 }
 
+template <bool LOGIT>
 __device__ __forceinline__ void write_out(const u64* s, int k, int b, int32_t* top_idx, float* top_p) {
   for (int i = threadIdx.x; i < k; i += blockDim.x) {
     top_idx[(int64_t)b * k + i] = key_id(s[i]);
-    top_p[(int64_t)b * k + i] = key_p(s[i]);
+    top_p[(int64_t)b * k + i] = score_of_key<LOGIT>(s[i]);
   }
 }
 
 // 1. per query: the k-th best exact p among the unfiltered entities 0, stride, 2 stride, ... (m of them)
+template <bool LOGIT>
 __global__ void __launch_bounds__(kThreads)
 topk_sample_kernel(const float* __restrict__ q, const float* __restrict__ O, int r2, int n_begin, int stride, int m,
                    int k, const int32_t* __restrict__ flt_off, const int32_t* __restrict__ flt_idx,
@@ -115,16 +140,17 @@ topk_sample_kernel(const float* __restrict__ q, const float* __restrict__ O, int
   topk_merge(s, k, m, [&](int i) {
     const int e = i * stride, id = n_begin + e;
     if (filtered(flt_idx, f0, f1, id)) return 0ull;
-    return make_key(rt::sigmoid_ref(rt::exact_logit(qb, O + (int64_t)e * r2, r2)), id);
+    return key_of_score<LOGIT>(score_of<LOGIT>(rt::exact_logit(qb, O + (int64_t)e * r2, r2)), id);
   });
   if (threadIdx.x == 0) {
     const u64 kth = s[k - 1];
     flag[b] = kth == 0ull;
-    p_k[b] = kth ? key_p(kth) : 1.0f;
+    p_k[b] = kth ? score_of_key<LOGIT>(kth) : (LOGIT ? INFINITY : 1.0f);
   }
 }
 
 // 3. per query: exact p of the candidates, best k; flags the query when its segment overflowed
+template <bool LOGIT>
 __global__ void __launch_bounds__(kThreads)
 topk_select_kernel(const float* __restrict__ q, const float* __restrict__ O, int r2, int n_begin, int k,
                    const int32_t* __restrict__ flt_off, const int32_t* __restrict__ flt_idx,
@@ -145,14 +171,15 @@ topk_select_kernel(const float* __restrict__ q, const float* __restrict__ O, int
   topk_merge(s, k, c, [&](int i) {
     const int e = __ldg(sb + i), id = n_begin + e;
     if (filtered(flt_idx, f0, f1, id)) return 0ull;
-    return make_key(rt::sigmoid_ref(rt::exact_logit(qb, O + (int64_t)e * r2, r2)), id);
+    return key_of_score<LOGIT>(score_of<LOGIT>(rt::exact_logit(qb, O + (int64_t)e * r2, r2)), id);
   });
-  write_out(s, k, b, top_idx, top_p);
+  write_out<LOGIT>(s, k, b, top_idx, top_p);
   if (n_cand && threadIdx.x == 0) n_cand[b] = c;
 }
 
 // 4. per query: merge the staged exact probabilities P[b][0, len) of entities id0 .. id0 + len - 1 into the running
 //    best k (run[b]); the last chunk writes the outputs.  flag == NULL: every query; gate == NULL: always.
+template <bool LOGIT>
 __global__ void __launch_bounds__(kThreads)
 topk_exact_merge_kernel(const float* __restrict__ P, int64_t ldp, int len, int id0, int k,
                         const int32_t* __restrict__ flt_off, const int32_t* __restrict__ flt_idx,
@@ -173,10 +200,10 @@ topk_exact_merge_kernel(const float* __restrict__ P, int64_t ldp, int len, int i
   topk_merge(s, k, len, [&](int i) {
     const int id = id0 + i;
     if (filtered(flt_idx, f0, f1, id)) return 0ull;
-    return make_key(__ldg(pb + i), id);
+    return key_of_score<LOGIT>(__ldg(pb + i), id);
   });
   if (last) {
-    write_out(s, k, b, top_idx, top_p);
+    write_out<LOGIT>(s, k, b, top_idx, top_p);
     if (n_cand && threadIdx.x == 0) n_cand[b] = -1;
   } else {
     for (int i = threadIdx.x; i < k; i += blockDim.x) rb[i] = s[i];
@@ -209,20 +236,17 @@ TopkLayout topk_layout(int B, int n_local, int r2, int k) {
   return L;
 }
 
-}  // namespace
-
-extern "C" size_t rt_score_topk_ws_bytes(int B, int n_local, int r2, int k) { return topk_layout(B, n_local, r2, k).total; }
-
-extern "C" int rt_score_topk(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
-                             const int32_t* flt_off, const int32_t* flt_idx, int32_t* top_idx, float* top_p,
-                             int32_t* n_cand, void* ws, void* stream) {
-  RT_REQUIRE(k >= 1 && k <= kMaxK, "rt_score_topk: k=%d outside 1..%d", k, kMaxK);
-  RT_REQUIRE(B >= 1 && B <= kMaxB, "rt_score_topk: B=%d outside 1..%d queries per call", B, kMaxB);
-  RT_REQUIRE(r2 >= 1 && r2 <= kMaxR2, "rt_score_topk: r2=%d outside 1..%d", r2, kMaxR2);
-  RT_REQUIRE(n_local >= 0 && n_begin >= 0, "rt_score_topk: bad shard n_begin=%d n_local=%d", n_begin, n_local);
-  RT_REQUIRE((flt_off == nullptr) == (flt_idx == nullptr), "rt_score_topk: flt_off and flt_idx must both be NULL or both set");
-  RT_REQUIRE(q && (O || n_local == 0) && top_idx && top_p, "rt_score_topk: NULL input or output");
-  RT_REQUIRE(ws != nullptr, "rt_score_topk: workspace is NULL");
+template <bool LOGIT>
+int score_topk(const char* fn, const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
+               const int32_t* flt_off, const int32_t* flt_idx, int32_t* top_idx, float* top_p, int32_t* n_cand, void* ws,
+               void* stream) {
+  RT_REQUIRE(k >= 1 && k <= kMaxK, "%s: k=%d outside 1..%d", fn, k, kMaxK);
+  RT_REQUIRE(B >= 1 && B <= kMaxB, "%s: B=%d outside 1..%d queries per call", fn, B, kMaxB);
+  RT_REQUIRE(r2 >= 1 && r2 <= kMaxR2, "%s: r2=%d outside 1..%d", fn, r2, kMaxR2);
+  RT_REQUIRE(n_local >= 0 && n_begin >= 0, "%s: bad shard n_begin=%d n_local=%d", fn, n_begin, n_local);
+  RT_REQUIRE((flt_off == nullptr) == (flt_idx == nullptr), "%s: flt_off and flt_idx must both be NULL or both set", fn);
+  RT_REQUIRE(q && (O || n_local == 0) && top_idx && top_p, "%s: NULL input or output", fn);
+  RT_REQUIRE(ws != nullptr, "%s: workspace is NULL", fn);
   cudaStream_t s = (cudaStream_t)stream;
   const TopkLayout L = topk_layout(B, n_local, r2, k);
   char* base = (char*)ws;
@@ -240,12 +264,12 @@ extern "C" int rt_score_topk(const float* q, const float* O, int B, int r2, int 
     const double m_target = std::max({2.0 * sqrt(kn), 4.0 * kn / kCap, (double)k});
     const int stride = std::max(1, (int)(n_local / m_target));
     const int m = rt::cdiv(n_local, stride);
-    topk_sample_kernel<<<B, kThreads, 0, s>>>(q, O, r2, n_begin, stride, m, k, flt_off, flt_idx, p_k, flag);
+    topk_sample_kernel<LOGIT><<<B, kThreads, 0, s>>>(q, O, r2, n_begin, stride, m, k, flt_off, flt_idx, p_k, flag);
     RT_LAUNCH_CHECK();
     int32_t* seg = (int32_t*)(base + L.seg);
-    int rc = rt::topk_tc_pass(q, O, B, r2, n_local, p_k, flag, cnt, seg, kCap, base + L.tc, s);
+    int rc = rt::topk_tc_pass(q, O, B, r2, n_local, p_k, flag, cnt, seg, kCap, base + L.tc, s, LOGIT);
     if (rc) return rc;
-    topk_select_kernel<<<B, kThreads, 0, s>>>(q, O, r2, n_begin, k, flt_off, flt_idx, cnt, seg, kCap, flag, any_flag,
+    topk_select_kernel<LOGIT><<<B, kThreads, 0, s>>>(q, O, r2, n_begin, k, flt_off, flt_idx, cnt, seg, kCap, flag, any_flag,
                                               top_idx, top_p, n_cand);
     RT_LAUNCH_CHECK();
     gate = any_flag;
@@ -254,12 +278,30 @@ extern "C" int rt_score_topk(const float* q, const float* O, int B, int r2, int 
   u64* run = (u64*)(base + L.run);
   for (int c = 0; c < L.nchunks; ++c) {
     const int c0 = c * L.chunk_len, len = std::min(L.chunk_len, n_local - c0);
-    int rc = rt::score_dense(q, O + (int64_t)c0 * r2, B, r2, len, P, L.chunk_len, gate, s);
+    int rc = rt::score_dense(q, O + (int64_t)c0 * r2, B, r2, len, P, L.chunk_len, gate, s, LOGIT);
     if (rc) return rc;
-    topk_exact_merge_kernel<<<B, kThreads, 0, s>>>(P, L.chunk_len, len, n_begin + c0, k, flt_off, flt_idx,
+    topk_exact_merge_kernel<LOGIT><<<B, kThreads, 0, s>>>(P, L.chunk_len, len, n_begin + c0, k, flt_off, flt_idx,
                                                    L.use_tc ? flag : nullptr, gate, run, c == 0, c == L.nchunks - 1,
                                                    top_idx, top_p, n_cand);
     RT_LAUNCH_CHECK();
   }
   return 0;
+}
+
+}  // namespace
+
+extern "C" size_t rt_score_topk_ws_bytes(int B, int n_local, int r2, int k) { return topk_layout(B, n_local, r2, k).total; }
+
+extern "C" int rt_score_topk(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
+                             const int32_t* flt_off, const int32_t* flt_idx, int32_t* top_idx, float* top_p,
+                             int32_t* n_cand, void* ws, void* stream) {
+  return score_topk<false>("rt_score_topk", q, O, B, r2, n_begin, n_local, k, flt_off, flt_idx, top_idx, top_p, n_cand,
+                           ws, stream);
+}
+
+extern "C" int rt_score_topk_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int k,
+                                   const int32_t* flt_off, const int32_t* flt_idx, int32_t* top_idx, float* top_z,
+                                   int32_t* n_cand, void* ws, void* stream) {
+  return score_topk<true>("rt_score_topk_logit", q, O, B, r2, n_begin, n_local, k, flt_off, flt_idx, top_idx, top_z,
+                          n_cand, ws, stream);
 }

@@ -67,9 +67,19 @@ def score_topk(q, O, k, flt_off=None, flt_idx=None, n_begin=0):
     known objects per query (global ids, ascending within a query), or both None.  Returns (top_idx int32 [B, k],
     top_p f32 [B, k], n_cand int32 [B]); positions without an entity hold id -1 and p -inf.  B > 1024 is split into
     calls of at most 1024 queries."""
+    return _score_topk("rt_score_topk", q, O, k, flt_off, flt_idx, n_begin)
+
+
+def score_topk_logit(q, O, k, flt_off=None, flt_idx=None, n_begin=0):
+    """``score_topk`` on the exact logit z instead of p = sigmoid(z) (rt_score_topk_logit): order z descending, then
+    id ascending; returns (top_idx int32 [B, k], top_z f32 [B, k], n_cand int32 [B]), padding id -1 and z -inf."""
+    return _score_topk("rt_score_topk_logit", q, O, k, flt_off, flt_idx, n_begin)
+
+
+def _score_topk(fn, q, O, k, flt_off, flt_idx, n_begin):
     require_cuda(q, O, flt_off, flt_idx)
     if (flt_off is None) != (flt_idx is None):
-        raise RTuckerError("score_topk: pass both flt_off and flt_idx, or neither")
+        raise RTuckerError(f"{fn[3:]}: pass both flt_off and flt_idx, or neither")
     B, r2 = q.shape
     n_local = O.shape[0]
     k = int(k)
@@ -83,11 +93,43 @@ def score_topk(q, O, k, flt_off=None, flt_idx=None, n_begin=0):
     ws = _ws(lib().rt_score_topk_ws_bytes(min(max(B, 1), TOPK_MAX_B), n_local, r2, k), dev)
     for lo in range(0, B, TOPK_MAX_B):
         hi = min(B, lo + TOPK_MAX_B)
-        check(lib().rt_score_topk(ptr(q[lo:hi]), ptr(O), hi - lo, r2, int(n_begin), n_local, k,
-                                  ptr(flt_off[lo:hi + 1]) if flt_off is not None else None, ptr(flt_idx),
-                                  ptr(top_idx[lo:hi]), ptr(top_p[lo:hi]), ptr(n_cand[lo:hi]), ptr(ws), stream_ptr()),
-              "rt_score_topk")
+        check(getattr(lib(), fn)(ptr(q[lo:hi]), ptr(O), hi - lo, r2, int(n_begin), n_local, k,
+                                 ptr(flt_off[lo:hi + 1]) if flt_off is not None else None, ptr(flt_idx),
+                                 ptr(top_idx[lo:hi]), ptr(top_p[lo:hi]), ptr(n_cand[lo:hi]), ptr(ws), stream_ptr()),
+              fn)
     return top_idx, top_p, n_cand
+
+
+# ---------------------------------------------------------------- (d') logit space (rtucker.h section d')
+def target_logit(q, O, target, n_begin=0):
+    """Exact fp32 logit of every query's target on the shard that owns it, 0 elsewhere (rt_target_logit)."""
+    require_cuda(q, O, target)
+    B, r2 = q.shape
+    out = torch.empty(B, dtype=f32, device=q.device)
+    check(lib().rt_target_logit(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, int(n_begin), O.shape[0],
+                                ptr(_c(target, i32)), ptr(out), stream_ptr()), "rt_target_logit")
+    return out
+
+
+def score_rank_logit(q, O, target, z_target, flt_off=None, flt_idx=None, n_begin=0, want_pos=True):
+    """Filtered counts in logit space (rt_score_rank_logit): filtered entities removed, ties with the target's logit
+    ``z_target`` (summed over shards) counted as equal.  Returns (greater, equal, equal_before) int32 [B] each and
+    pos_sum f64 [B] = the sum of the logits of the filter list on this shard (None unless ``want_pos``)."""
+    require_cuda(q, O, target, z_target, flt_off, flt_idx)
+    if (flt_off is None) != (flt_idx is None):
+        raise RTuckerError("score_rank_logit: pass both flt_off and flt_idx, or neither")
+    B, r2 = q.shape
+    n_local = O.shape[0]
+    out = torch.empty(3, B, dtype=i32, device=q.device)
+    pos = torch.empty(B, dtype=f64, device=q.device) if want_pos else None
+    ws = _ws(lib().rt_score_rank_logit_ws_bytes(B, n_local, r2), q.device)
+    check(lib().rt_score_rank_logit(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, int(n_begin), n_local,
+                                    ptr(_c(target, i32)), ptr(_c(z_target, f32)),
+                                    ptr(_c(flt_off, i32)) if flt_off is not None else None,
+                                    ptr(_c(flt_idx, i32)) if flt_idx is not None else None,
+                                    ptr(out[0]), ptr(out[1]), ptr(out[2]), ptr(pos), ptr(ws), stream_ptr()),
+          "rt_score_rank_logit")
+    return out[0], out[1], out[2], pos
 
 
 # ---------------------------------------------------------------- (a) query contraction
@@ -471,6 +513,17 @@ def score_dense(q, O, out=None):
     check(lib().rt_score_dense(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, n, ptr(P), P.stride(0), stream_ptr()),
           "rt_score_dense")
     return P
+
+
+def score_dense_logits(q, O, out=None):
+    """Dense logits Z[B, n] = q O^T, bit-identical to the logits inside score_dense (rt_score_dense_logits)."""
+    require_cuda(q, O)
+    B, r2 = q.shape
+    n = O.shape[0]
+    Z = out if out is not None else torch.empty(B, n, dtype=f32, device=q.device)
+    check(lib().rt_score_dense_logits(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, n, ptr(Z), Z.stride(0), stream_ptr()),
+          "rt_score_dense_logits")
+    return Z
 
 
 def filter_dense_(P, T, filter_col):

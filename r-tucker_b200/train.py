@@ -12,9 +12,10 @@ tensor into its tqdm bar every step, train.py:88: an implicit synchronisation pe
 optimiser state (checkpoint.py).  ``criterion`` selects the training objective among the two the fused kernels
 implement: ``nn.BCELoss(reduction="mean")`` (train.py:136, the default) and ``nn.CrossEntropyLoss(reduction="mean")``
 (1-N softmax cross-entropy over all entities; no ``weight``, no ``ignore_index``, ``label_smoothing=0``: the smoothing
-comes from the loader, as for the BCE).  Evaluation is the same for both: the reference's BCE evaluation loss and the
-filtered ranks.  Ranks, ``evaluation.predict_topk`` and ``score_fn(T)`` use z or sigmoid(z), both monotone in the logit
-z, so they do not depend on which loss trained the model.
+comes from the loader, as for the BCE).  Evaluation is the same for both unless asked otherwise: the reference's BCE
+evaluation loss and the probability-space filtered ranks.  ``evaluate(space="logit")`` / ``train(eval_space="logit")``
+rank the exact logits and report the cross-entropy instead, which is what a cross-entropy model needs: its top logits
+sit where the fp32 sigmoid has saturated to 1.0.
 """
 import os
 import time
@@ -23,7 +24,7 @@ import torch
 from torch import nn
 
 from . import checkpoint
-from .evaluation import _sums_from_ranks, rank_batch
+from .evaluation import _check_space, _sums_from_ranks, rank_batch
 from .manifold import SFTucker, Tucker
 from .optim import FusedLoss
 
@@ -70,11 +71,13 @@ def train_one_epoch(model, optimizer, criterion, train_loader, regularization_co
 
 
 @torch.no_grad()
-def evaluate(model, criterion, dataloader, n_begin=0, group=None):
-    """Filtered ranking + BCE over ``dataloader`` (features (s, r, o), targets = filter lists over all splits);
-    returns (metrics dict, mean batch loss) like train.py:124-125.  The loss is the reference's BCE whichever
-    criterion trained the model."""
+def evaluate(model, criterion, dataloader, n_begin=0, group=None, space="prob"):
+    """Filtered ranking + loss over ``dataloader`` (features (s, r, o), targets = filter lists over all splits);
+    returns (metrics dict, mean batch loss) like train.py:124-125.  space="prob" (the default): probability-space
+    ranks and the reference's BCE, whichever criterion trained the model; space="logit": logit-space ranks and the
+    cross-entropy of the un-smoothed filter lists (evaluation.py), comparable with the CE training loss."""
     _check_criterion(criterion)
+    _check_space(space, ("prob", "logit"))
     model.eval()
     device = model.core.device
     point = extract_tensor(model)
@@ -83,10 +86,13 @@ def evaluate(model, criterion, dataloader, n_begin=0, group=None):
     val_loss = torch.zeros(1, dtype=torch.float64, device=device)
     denom = 0
     for features, filters in dataloader:
-        ranks, bce, _ = rank_batch(point, features, filters, n_begin, group)
+        ranks, bl, _ = rank_batch(point, features, filters, n_begin, group, space)
         s = _sums_from_ranks(ranks)
         sums = s if sums is None else {k: sums[k] + s[k] for k in s}
-        val_loss += bce / (features.shape[0] * n_ent)       # BCELoss(mean) of the batch (train.py:113)
+        if space == "logit":
+            val_loss += bl / features.shape[0]              # cross_entropy(mean) of the batch
+        else:
+            val_loss += bl / (features.shape[0] * n_ent)    # BCELoss(mean) of the batch (train.py:113)
         denom += features.shape[0]
     n_batches = len(dataloader)
     metrics = {k: v.item() / denom for k, v in sums.items()}
@@ -94,18 +100,21 @@ def evaluate(model, criterion, dataloader, n_begin=0, group=None):
 
 
 def train(model, optimizer, train_loader, val_loader, test_loader, config, regulizer, scheduler=None, log_fn=None,
-          start_epoch=None, num_epoches=None, history=None, criterion=None):
+          start_epoch=None, num_epoches=None, history=None, criterion=None, eval_space="prob"):
     """train.py:128-167: evaluate once, then per epoch: regulariser step, train epoch, validate, test, snapshot
     (now with the optimiser state), scheduler step.  ``config`` needs ``train_cfg.num_epoches`` and
     ``train_cfg.checkpoint_path`` (configs/base_config.py); ``log_fn(record)`` replaces wandb_log.  ``criterion``:
     the training objective, ``nn.BCELoss(reduction="mean")`` (the reference's, the default) or
-    ``nn.CrossEntropyLoss(reduction="mean")`` (see the module docstring); evaluation reports the BCE either way."""
+    ``nn.CrossEntropyLoss(reduction="mean")`` (see the module docstring).  ``eval_space``: the ``space`` of
+    ``evaluate`` ("prob", the default: BCE and probability ranks whichever the criterion; "logit"); each record
+    names it."""
     criterion = nn.BCELoss(reduction="mean") if criterion is None else criterion
     _check_criterion(criterion)
+    _check_space(eval_space, ("prob", "logit"))
     num_epoches = num_epoches if num_epoches is not None else config.train_cfg.num_epoches
     start_epoch = start_epoch if start_epoch is not None else 1
     history = history if history is not None else []
-    prev_val_mrr = evaluate(model, criterion, val_loader)[0]["mrr"]
+    prev_val_mrr = evaluate(model, criterion, val_loader, space=eval_space)[0]["mrr"]
     state = None
     for epoch in range(start_epoch, num_epoches + start_epoch):
         regularization_coeff = regulizer.step()
@@ -113,14 +122,14 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
         train_loss, train_norm = train_one_epoch(model, optimizer, criterion, train_loader,
                                                  regularization_coeff=regularization_coeff)
         epoch_time = time.perf_counter() - t0
-        val_metrics, val_loss = evaluate(model, criterion, val_loader)
+        val_metrics, val_loss = evaluate(model, criterion, val_loader, space=eval_space)
         t0 = time.perf_counter()
-        test_metrics, test_loss = evaluate(model, criterion, test_loader)
+        test_metrics, test_loss = evaluate(model, criterion, test_loader, space=eval_space)
         torch.cuda.synchronize()
         eval_time = time.perf_counter() - t0
         record = dict(epoch=epoch, train_loss=train_loss, grad_norm=train_norm, val_loss=float(val_loss),
                       test_loss=float(test_loss), lr=optimizer.param_groups[0]["lr"], reg_coeff=regularization_coeff,
-                      epoch_time=epoch_time, eval_time=eval_time,
+                      epoch_time=epoch_time, eval_time=eval_time, eval_space=eval_space,
                       **{"val_" + k: v for k, v in val_metrics.items()},
                       **{"test_" + k: v for k, v in test_metrics.items()})
         history.append(record)

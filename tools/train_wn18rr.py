@@ -9,7 +9,10 @@ train.py:69-167), rank (10, 200, 200), batch 512, rsgd momentum 0.8, label smoot
 
     python tools/train_wn18rr.py --epochs 150 --variant 2 --out profiles/r02_train_wn18rr_v2.json
 
-Writes one JSON record per epoch (train loss, ||rgrad||, validation / test MRR and Hits@k, epoch seconds).  The score
+Writes one JSON record per epoch (train loss, ||rgrad||, validation / test MRR and Hits@k, epoch seconds).
+--eval-space logit adds, next to those (which stay the probability-space ones), per split: the logit-space metrics
+(<split>_logit_mrr, ...), the cross-entropy evaluation loss (<split>_ce_loss) and the number of queries whose target
+ties with an unfiltered entity (equal > 0) in each space (<split>_ties_prob, <split>_ties_logit).  The score
 kernel variant 2 (fp16-operand tcgen05) and variant 0 (fp32 FFMA, the 1e-5 parity path) are run on identical seeds
 and batches (host shuffle = the reference's RandomSampler draw) so that their curves can be compared point by point.
 """
@@ -27,6 +30,7 @@ sys.path.insert(0, ROOT)
 from rtucker_b200 import asymmetric, symmetric                      # noqa: E402
 from rtucker_b200 import train as T                                  # noqa: E402
 from rtucker_b200.data import DeviceEpoch, datasets_from_ids, wn18rr_fixture   # noqa: E402
+from rtucker_b200.evaluation import rank_batch                      # noqa: E402
 
 
 class LinearRegulariser:
@@ -54,6 +58,17 @@ class ExpRegulariser:
         return self.val
 
 
+@torch.no_grad()
+def tie_census(model, loader):
+    """Queries of ``loader`` whose target ties with at least one unfiltered entity, in probability and logit space."""
+    point = T.extract_tensor(model)
+    ties = {"prob": 0, "logit": 0}
+    for features, filters in loader:
+        for space in ties:
+            ties[space] += int((rank_batch(point, features, filters, space=space)[2][1] > 0).sum())
+    return ties
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--epochs", type=int, default=100)
@@ -68,6 +83,8 @@ def main():
     ap.add_argument("--loss", default="bce", choices=["bce", "ce"],
                     help="training objective: the reference's label-smoothed BCE or the 1-N softmax cross-entropy "
                          "(evaluation reports the BCE and the filtered ranks either way)")
+    ap.add_argument("--eval-space", default="prob", choices=["prob", "logit"],
+                    help="logit: also report logit-space ranks, the cross-entropy evaluation loss and tie counts")
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
@@ -119,6 +136,13 @@ def main():
             rec.update(ortho_defect=defect)
             rec.update(eval_s=time.perf_counter() - t0, val_loss=float(vl), test_loss=float(tl),
                        **{"val_" + k: v for k, v in vm.items()}, **{"test_" + k: v for k, v in tm.items()})
+            if args.eval_space == "logit":
+                for split, loader in (("val", val_loader), ("test", test_loader)):
+                    lm, ll = T.evaluate(model, crit, loader, space="logit")
+                    ties = tie_census(model, loader)
+                    rec.update({f"{split}_logit_{k}": v for k, v in lm.items()})
+                    rec.update({f"{split}_ce_loss": float(ll), f"{split}_ties_prob": ties["prob"],
+                                f"{split}_ties_logit": ties["logit"], f"{split}_queries": len(loader.dataset)})
         if not (args.recipe == "head" and epoch >= args.total_epochs):
             sched.step()
         hist.append(rec)
@@ -126,13 +150,25 @@ def main():
     summary = dict(config=dict(dataset="WN18RR (real triples, tests/golden/wn18rr_ids.npz)", mode=args.mode, rank=rank,
                                batch=512, optim="rsgd", recipe=args.recipe,
                                momentum=0.8, label_smoothing=0.1, seed=args.seed, score_variant=args.variant,
-                               loss=args.loss,
+                               loss=args.loss, eval_space=args.eval_space,
+                               device=torch.cuda.get_device_name(dev), power_limit_w=_power_limit(),
                                epochs=args.epochs, steps_per_epoch=len(train_loader)),
                    wall_s=time.perf_counter() - t_start, history=hist)
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, "w") as f:
             json.dump(summary, f)
+
+
+def _power_limit():
+    """The card's power limit in W, read next to the measurement (None where nvidia-smi is not available)."""
+    import subprocess
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits", "-i", "0"],
+                             capture_output=True, text=True, timeout=30).stdout.strip()
+        return float(out.splitlines()[0])
+    except (OSError, ValueError, IndexError, subprocess.SubprocessError):
+        return None
 
 
 if __name__ == "__main__":

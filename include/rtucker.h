@@ -385,6 +385,18 @@ int rt_eigh(double* A, int n, double* w, double* V, void* ws, void* stream);
 size_t rt_dominant_subspace_ws_bytes(int n, int r);
 int rt_dominant_subspace(const double* A, int n, int r, double* Y, int* info, void* ws, void* stream);
 
+/* ---- (e) rank change ------------------------------------------------------------------- */
+/*
+ * rt_fill_normal: out[rows, cols] (row-major, dense) <- standard normal fp32 values, counter-based (csrc/fill.cu:
+ * Philox4x32-10, Box-Muller).  The value at (row, col) depends only on (seed, stream_id, row_begin + row, col): a
+ * shard that passes its first global row as row_begin draws exactly those rows of the draw over all rows, and every
+ * caller that passes the same arguments gets the same bits.  stream_id separates independent draws under one seed.
+ * Used by set_rank (rank.py) for the new factor directions and core entries of a rank increase.  rows == 0 or
+ * cols == 0 launches nothing.
+ */
+int rt_fill_normal(float* out, int rows, int cols, int64_t row_begin, uint64_t seed, uint32_t stream_id,
+                   void* stream);
+
 
 #ifdef __cplusplus
 }

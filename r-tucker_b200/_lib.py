@@ -74,6 +74,7 @@ PROTOTYPES = {
     "rt_eigh": (i32, [vp, i32, vp, vp, vp, vp]),
     "rt_dominant_subspace_ws_bytes": (sz, [i32, i32]),
     "rt_dominant_subspace": (i32, [vp, i32, i32, vp, vp, vp, vp]),
+    "rt_fill_normal": (i32, [vp, i32, i32, i64, C.c_uint64, C.c_uint32, vp]),
     "rt_tc_selftest": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, vp]),
     "rt_tc_selftest16": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, vp]),
     "rt_bulk_reduce_selftest": (i32, [vp, vp, vp, i32, vp]),

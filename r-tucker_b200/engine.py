@@ -40,6 +40,50 @@ def check_loss(loss):
         raise ValueError(f"loss must be one of {LOSSES}, got {loss!r}")
 
 
+def core_mode_product(ops, core, K, mode):
+    """``core`` x_mode K^T, i.e. core[.., j, ..] <- sum_j' core[.., j', ..] K[j', j] for K fp64 [r_mode, rc]: ONE
+    ops.apply over a permuted copy of the core that puts ``mode`` last.  Returns a (possibly non-contiguous) view of
+    shape ``core.shape`` with rc at ``mode``."""
+    r0, r1, r2 = core.shape
+    rc = K.shape[1]
+    if mode == 2:
+        c = core.reshape(r0 * r1, r2)
+        out = torch.empty(r0 * r1, rc, dtype=core.dtype, device=core.device)
+        ops.apply(out, None, None, [(c, K)])
+        return out.view(r0, r1, rc)
+    if mode == 1:
+        c = core.permute(0, 2, 1).contiguous().reshape(r0 * r2, r1)
+        out = torch.empty(r0 * r2, rc, dtype=core.dtype, device=core.device)
+        ops.apply(out, None, None, [(c, K)])
+        return out.view(r0, r2, rc).permute(0, 2, 1)
+    c = core.permute(1, 2, 0).contiguous().reshape(r1 * r2, r0)
+    out = torch.empty(r1 * r2, rc, dtype=core.dtype, device=core.device)
+    ops.apply(out, None, None, [(c, K)])
+    return out.view(r1, r2, rc).permute(2, 0, 1)
+
+
+def polar_gauge(ops, core, jobs, reduce=None):
+    """Pull factors back to orthonormal columns WITHOUT moving the point (a change of gauge), in place.
+
+    jobs = [(U, core_modes, spare)]: U <- U K with K = (3 I - U^T U) / 2, one Newton-Schulz step of the polar
+    decomposition from the exact fp64 Gram (it squares the orthonormality defect); the core absorbs K^-1 =
+    (I + U^T U) / 2 (exact to the same second order) on each of ``core_modes`` (both shared modes of SF-Tucker), so
+    the tensor moves by O(defect^2) only.  ``spare``: scratch of U's shape.  ``reduce(grams)`` completes the Grams
+    of entity-sharded factors before they are used.  Returns the Grams U^T U."""
+    grams = [ops.gram(U, U, precise=True) for U, _, _ in jobs]
+    if reduce is not None:
+        reduce(grams)
+    for (U, modes, spare), G in zip(jobs, grams):
+        eye = torch.eye(U.shape[1], dtype=f64, device=U.device)
+        K = 1.5 * eye - 0.5 * G
+        Kinv = 0.5 * (eye + G)
+        ops.apply(spare, None, None, [(U, K)])
+        U.copy_(spare)
+        for mode in modes:
+            core.copy_(core_mode_product(ops, core, Kinv, mode))
+    return grams
+
+
 @dataclass
 class SparseTargets:
     """Multi-hot targets of a batch in CSR form: objects of query b are idx[off[b]:off[b+1]]
@@ -390,41 +434,22 @@ class StepEngine:
         an fp32 cancellation (dV = g A - U (U^T g A) with the in-span part of g much larger than dV), the reference
         hides the same residue inside the QR of [U | dV] it runs every step (tucker_riemopt round, call site
         src/model/asymmetric/optim.py:108), here it would accumulate in the factors: measured on real WN18RR,
-        max |O^T O - I| = 3e-2 after 200 steps.  One Newton-Schulz step of the polar decomposition,
+        max |O^T O - I| = 3e-2 after 200 steps.  One Newton-Schulz step of the polar decomposition (polar_gauge),
         U <- U K with K = (3 I - U^T U) / 2 from the exact fp64 Gram, squares the defect; the core absorbs K^-1
         (K^-1 = (I + U^T U) / 2 up to the same second order), so the TENSOR is unchanged to O(defect^2), and the transport
         Grams of the kept direction follow the new basis (M <- K M)."""
         ops = self.ops
         if not hasattr(ops, "gram") or self.dev.type != "cuda":
             return
-        core = self.core.data
-        r0, r1, r2 = self.rank
-        for k in self._entity_factor_ids():
-            U = self._U(k)
-            r = U.shape[1]
-            G = ops.gram(U, U, precise=True)
-            self._allreduce(G)
-            eye = torch.eye(r, dtype=f64, device=self.dev)
-            K = 1.5 * eye - 0.5 * G
-            Kinv = 0.5 * (eye + G)
-            ops.apply(self.spare[k], None, None, [(U, K)])
-            U.copy_(self.spare[k])
-            modes = (1, 2) if self.sym else (k,)
-            for mode in modes:
-                if mode == 2:        # core[a, i, j] <- sum_j' core[a, i, j'] Kinv[j', j]   (Kinv symmetric)
-                    c2 = core.reshape(r0 * r1, r2)
-                    out = torch.empty_like(c2)
-                    ops.apply(out, None, None, [(c2, Kinv)])
-                    core.copy_(out.view(r0, r1, r2))
-                else:                # mode 1: the same on the transposed view
-                    ct = core.permute(0, 2, 1).contiguous().reshape(r0 * r2, r1)
-                    out = torch.empty_like(ct)
-                    ops.apply(out, None, None, [(ct, Kinv)])
-                    core.copy_(out.view(r0, r2, r1).permute(0, 2, 1))
+        ent = self._entity_factor_ids()
+        jobs = [(self._U(k), (1, 2) if self.sym else (k,), self.spare[k]) for k in ent]
+        grams = polar_gauge(ops, self.core.data, jobs, reduce=lambda gs: self._allreduce(*gs))
+        for k, G in zip(ent, grams):
             if self.beta is not None and self.has_old and self.M_next[k] is not None:
                 # M <- K M = M - (G - I) M / 2 with this library's Gram kernel (A^T B, exact products, fp64 sums): the
                 # correction term is second-order small, its fp32 operands cost nothing; no cuBLAS on the path (its lazy
                 # initialisation inside a timed step was measured as a 120 ms one-off)
+                eye = torch.eye(G.shape[0], dtype=f64, device=self.dev)
                 D32 = (G - eye).to(f32).contiguous()              # symmetric: D^T = D
                 M32 = self.M_next[k].to(f32).contiguous()
                 self.M_next[k].sub_(0.5 * ops.gram(D32, M32, precise=True))

@@ -504,6 +504,16 @@ def dominant_subspace(A, r):
     return Y, info
 
 
+def fill_normal(out, seed, stream_id=0, row_begin=0):
+    """``out`` (contiguous f32 [rows, cols]) <- standard normal values that depend only on (seed, stream_id,
+    row_begin + row, col) -- see rt_fill_normal.  Returns ``out``."""
+    require_cuda(out)
+    rows, cols = out.shape
+    check(lib().rt_fill_normal(ptr(_c(out, f32)), rows, cols, int(row_begin), int(seed) & (2 ** 64 - 1),
+                               int(stream_id) & 0xFFFFFFFF, stream_ptr()), "rt_fill_normal")
+    return out
+
+
 def score_dense(q, O, out=None):
     """Dense sigmoid scores P[B, n] (compat path of R_TuckER.py:47-48)."""
     require_cuda(q, O)

@@ -27,6 +27,7 @@ from . import checkpoint
 from .evaluation import _check_space, _sums_from_ranks, rank_batch
 from .manifold import SFTucker, Tucker
 from .optim import FusedLoss
+from .rank import set_rank
 
 
 def extract_tensor(model):
@@ -100,14 +101,16 @@ def evaluate(model, criterion, dataloader, n_begin=0, group=None, space="prob"):
 
 
 def train(model, optimizer, train_loader, val_loader, test_loader, config, regulizer, scheduler=None, log_fn=None,
-          start_epoch=None, num_epoches=None, history=None, criterion=None, eval_space="prob"):
+          start_epoch=None, num_epoches=None, history=None, criterion=None, eval_space="prob", rank_schedule=None):
     """train.py:128-167: evaluate once, then per epoch: regulariser step, train epoch, validate, test, snapshot
     (now with the optimiser state), scheduler step.  ``config`` needs ``train_cfg.num_epoches`` and
     ``train_cfg.checkpoint_path`` (configs/base_config.py); ``log_fn(record)`` replaces wandb_log.  ``criterion``:
     the training objective, ``nn.BCELoss(reduction="mean")`` (the reference's, the default) or
     ``nn.CrossEntropyLoss(reduction="mean")`` (see the module docstring).  ``eval_space``: the ``space`` of
     ``evaluate`` ("prob", the default: BCE and probability ranks whichever the criterion; "logit"); each record
-    names it."""
+    names it.  ``rank_schedule``: {epoch: (r0, r1, r2)}; ``rank.set_rank(model, rank, optimizer)`` runs at the start of
+    that epoch (truncation or growth; the optimiser's momentum restarts, the scheduler is untouched).  Each record
+    names the rank the epoch trained at."""
     criterion = nn.BCELoss(reduction="mean") if criterion is None else criterion
     _check_criterion(criterion)
     _check_space(eval_space, ("prob", "logit"))
@@ -117,6 +120,8 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
     prev_val_mrr = evaluate(model, criterion, val_loader, space=eval_space)[0]["mrr"]
     state = None
     for epoch in range(start_epoch, num_epoches + start_epoch):
+        if rank_schedule and epoch in rank_schedule:
+            set_rank(model, rank_schedule[epoch], optimizer)
         regularization_coeff = regulizer.step()
         t0 = time.perf_counter()
         train_loss, train_norm = train_one_epoch(model, optimizer, criterion, train_loader,
@@ -129,7 +134,7 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
         eval_time = time.perf_counter() - t0
         record = dict(epoch=epoch, train_loss=train_loss, grad_norm=train_norm, val_loss=float(val_loss),
                       test_loss=float(test_loss), lr=optimizer.param_groups[0]["lr"], reg_coeff=regularization_coeff,
-                      epoch_time=epoch_time, eval_time=eval_time, eval_space=eval_space,
+                      epoch_time=epoch_time, eval_time=eval_time, eval_space=eval_space, rank=list(model.core.shape),
                       **{"val_" + k: v for k, v in val_metrics.items()},
                       **{"test_" + k: v for k, v in test_metrics.items()})
         history.append(record)

@@ -9,7 +9,11 @@ train.py:69-167), rank (10, 200, 200), batch 512, rsgd momentum 0.8, label smoot
 
     python tools/train_wn18rr.py --epochs 150 --variant 2 --out profiles/r02_train_wn18rr_v2.json
 
-Writes one JSON record per epoch (train loss, ||rgrad||, validation / test MRR and Hits@k, epoch seconds).
+Writes one JSON record per epoch (train loss, ||rgrad||, validation / test MRR and Hits@k, epoch seconds, the rank the
+epoch trained at, seconds since the start).
+--rank r0,r1,r2 sets the starting rank; --rank-schedule "epoch:r0,r1,r2;..." changes it with rank.set_rank at the start
+of those epochs (--growth: the relative size of a rank increase).  The record of such an epoch carries the change's
+report and the test metrics measured right after the change, before any training at the new rank (after_change).
 --eval-space logit adds, next to those (which stay the probability-space ones), per split: the logit-space metrics
 (<split>_logit_mrr, ...), the cross-entropy evaluation loss (<split>_ce_loss) and the number of queries whose target
 ties with an unfiltered entity (equal > 0) in each space (<split>_ties_prob, <split>_ties_logit).  The score
@@ -31,6 +35,7 @@ from rtucker_b200 import asymmetric, symmetric                      # noqa: E402
 from rtucker_b200 import train as T                                  # noqa: E402
 from rtucker_b200.data import DeviceEpoch, datasets_from_ids, wn18rr_fixture   # noqa: E402
 from rtucker_b200.evaluation import rank_batch                      # noqa: E402
+from rtucker_b200.rank import DEFAULT_GROWTH, set_rank              # noqa: E402
 
 
 class LinearRegulariser:
@@ -69,6 +74,22 @@ def tie_census(model, loader):
     return ties
 
 
+def parse_rank(text):
+    r = tuple(int(x) for x in text.split(","))
+    if len(r) != 3:
+        raise argparse.ArgumentTypeError(f"a rank is r0,r1,r2, got {text!r}")
+    return r
+
+
+def parse_schedule(text):
+    """"epoch:r0,r1,r2;epoch:r0,r1,r2" -> {epoch: (r0, r1, r2)}"""
+    out = {}
+    for item in filter(None, (t.strip() for t in text.split(";"))):
+        epoch, rank = item.split(":")
+        out[int(epoch)] = parse_rank(rank)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--epochs", type=int, default=100)
@@ -85,13 +106,18 @@ def main():
                          "(evaluation reports the BCE and the filtered ranks either way)")
     ap.add_argument("--eval-space", default="prob", choices=["prob", "logit"],
                     help="logit: also report logit-space ranks, the cross-entropy evaluation loss and tie counts")
+    ap.add_argument("--rank", type=parse_rank, default=(10, 200, 200), help="starting rank r0,r1,r2")
+    ap.add_argument("--rank-schedule", type=parse_schedule, default={},
+                    help='rank changes at the start of epochs: "epoch:r0,r1,r2;epoch:r0,r1,r2"')
+    ap.add_argument("--growth", type=float, default=DEFAULT_GROWTH,
+                    help="||X' - X|| / ||X|| of a rank increase (rank.set_rank)")
     ap.add_argument("--out", default="")
     args = ap.parse_args()
     dev = torch.device("cuda:0")
     ids = wn18rr_fixture()
     assert ids is not None, "tests/golden/wn18rr_ids.npz is missing"
     train_ds, valid_ds, test_ds = datasets_from_ids(ids, label_smoothing=0.1)
-    rank = (10, 200, 200)
+    rank = args.rank
     torch.manual_seed(args.seed)
     mod = asymmetric if args.mode == "asymmetric" else symmetric
     model = mod.R_TuckER((ids["n_entities"], ids["n_relations"]), rank)
@@ -115,13 +141,24 @@ def main():
     hist = []
     t_start = time.perf_counter()
     for epoch in range(1, args.epochs + 1):
+        change = None
+        if epoch in args.rank_schedule:
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            info = set_rank(model, args.rank_schedule[epoch], opt, growth=args.growth)
+            torch.cuda.synchronize()
+            change = dict(info, set_rank_s=time.perf_counter() - t0)
+            tm, _ = T.evaluate(model, crit, test_loader)
+            change.update({"test_" + k: v for k, v in tm.items()})
         r = reg.step()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
         loss, gnorm = T.train_one_epoch(model, opt, crit, train_loader, regularization_coeff=r)
         torch.cuda.synchronize()
-        rec = dict(epoch=epoch, train_loss=loss, grad_norm=gnorm, lr=opt.param_groups[0]["lr"], reg=r,
-                   epoch_s=time.perf_counter() - t0)
+        rec = dict(epoch=epoch, rank=list(model.core.shape), train_loss=loss, grad_norm=gnorm,
+                   lr=opt.param_groups[0]["lr"], reg=r, epoch_s=time.perf_counter() - t0)
+        if change is not None:
+            rec["after_change"] = change
         if epoch % args.eval_every == 0 or epoch == 1 or epoch == args.epochs:
             t0 = time.perf_counter()
             vm, vl = T.evaluate(model, crit, val_loader)
@@ -145,9 +182,11 @@ def main():
                                 f"{split}_ties_logit": ties["logit"], f"{split}_queries": len(loader.dataset)})
         if not (args.recipe == "head" and epoch >= args.total_epochs):
             sched.step()
+        rec["wall_s"] = time.perf_counter() - t_start
         hist.append(rec)
         print(json.dumps(rec), flush=True)
     summary = dict(config=dict(dataset="WN18RR (real triples, tests/golden/wn18rr_ids.npz)", mode=args.mode, rank=rank,
+                               rank_schedule={str(k): v for k, v in args.rank_schedule.items()}, growth=args.growth,
                                batch=512, optim="rsgd", recipe=args.recipe,
                                momentum=0.8, label_smoothing=0.1, seed=args.seed, score_variant=args.variant,
                                loss=args.loss, eval_space=args.eval_space,

@@ -51,6 +51,10 @@ constexpr uint32_t X_HALF = (KB / 4) * CS_X;            // one image (hi or lo) 
 constexpr int RCP_MAX = 256;
 constexpr int MAX_JOBS = 4, MAX_TERMS = 4;
 constexpr size_t SMEM_LIMIT = 226 * 1024;
+// epilogue modes of apply_tc_kernel (its MODE parameter): the factor update Y = a0 X0 + sum X_t K_t, and the logits
+// passes (rows = entities, 256 queries per job) of the filtered ranking, the BCE score, the top-k candidates, the
+// log-sum-exp parts and the cross-entropy score
+constexpr int kModeApply = 0, kModeRank = 1, kModeScore = 2, kModeTopk = 3, kModeLse = 4, kModeCe = 5;
 
 struct Job {
   float* Y; int64_t ldy;
@@ -71,7 +75,7 @@ struct Args {
   const unsigned char* Kimg;          // [total blocks][hi | lo][KB/4 chunks][cs_k bytes]
   uint32_t cs_k, kimg_bytes, stage_bytes;
   int debug;                          // profiling build only (RT_APPLY_DEBUG): 1 no X loads, 2 no K loads, 4 no MMAs, 8 ld.cg
-  // ---- rank mode (MODE 1): rows = entities of the shard, columns of job j = queries [256 j, 256 j + 256) ----
+  // ---- rank mode (kModeRank): rows = entities of the shard, columns of job j = queries [256 j, 256 j + 256) ----
   const float* thr;                   // [4][Bp]: lo0, hi0, eqlo0, slope per query (Bp = 256 * njobs), see rank_thresholds_kernel
   const float* onorms;                // [n_local] upper bounds of the entity row norms
   const int32_t* target;              // [B] global id of the target entity
@@ -79,12 +83,12 @@ struct Args {
   int32_t* greater; int32_t* equal; int32_t* equal_before;
   int2* cand; int* cand_count; int cand_cap;   // (local entity, query) pairs whose probability must be recomputed exactly
   double* loss_sum;                   // sum of softplus(z) over every valid (entity, query)
-  // ---- score mode (MODE 2): the same logits; the epilogue writes G[e][b] = dBCE/dz for all-negative targets ----
+  // ---- score mode (kModeScore): the same logits; the epilogue writes G[e][b] = dBCE/dz for all-negative targets ----
   float* G; int64_t ldg;              // [n_local][ldg] (ldg = 256 * njobs)
   float t_neg, inv_count;
   double* loss_partial;               // [grid]
-  // ---- top-k mode (MODE 3): the rank-mode logits; entities not certainly below the query's threshold are appended to
-  //      its segment seg[b][0, cand_cap) (overflow: cnt[b] > cand_cap; thr and onorms as in rank mode) ----
+  // ---- top-k mode (kModeTopk): the rank-mode logits; entities not certainly below the query's threshold are
+  //      appended to its segment seg[b][0, cand_cap) (overflow: cnt[b] > cand_cap; thr and onorms as in rank mode) ----
   int32_t* topk_seg; int* topk_cnt;
 };
 struct PackArgs {
@@ -389,7 +393,7 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
 __device__ __forceinline__ float rcp_fast(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 // HC8 = 8-column groups of the accumulator owned by one epilogue warp (rcp / 16): 13 for r = 200, 16 = any rcp <= 256
-template <int HC8, int MODE = 0>
+template <int HC8, int MODE = kModeApply>
 __global__ void __launch_bounds__(kThreads, 1)
 apply_tc_kernel(const __grid_constant__ Args a) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -397,6 +401,8 @@ apply_tc_kernel(const __grid_constant__ Args a) {
   __shared__ uint32_t tmem_slot;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int NS = a.nstages;
+  // register split: the factor update's, or the logits passes' (top-k, with 128 logits and no counters, takes the former)
+  constexpr bool kUpdateRegs = MODE == kModeApply || MODE == kModeTopk;
   if (tid == 0) {
     for (int s = 0; s < NS; ++s) { mbar_init(&bar_full[s], kProdWarps + 1); mbar_init(&bar_empty[s], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&bar_acc_full[i], 1); mbar_init(&bar_acc_empty[i], kEpiWarps); }
@@ -412,7 +418,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
 
   if (warp < kEpiWarps) {
     // ================= epilogue: partial sums -> fp32 running sum (round to nearest) -> Y =================
-    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpi));
+    if (kUpdateRegs) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpi));
     else asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;\n" :: "n"(kRegsEpiLogits));
     const int quarter = warp & 3, half = warp >> 2;
     constexpr int NACC = HC8 * 8;
@@ -428,7 +434,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     for (int u = 0; u < HC8; ++u) cntw[u] = 0u;
     // sum the counters over the lanes and add them to greater[] (job = query block the counters belong to)
     auto flush_counts = [&](int job_of) {
-      if (MODE != 1 || job_of < 0) return;
+      if (MODE != kModeRank || job_of < 0) return;
       const int q0 = job_of * 256 + (warp >> 2) * halfcols;
 #pragma unroll
       for (int c = 0; c < HC8 * 8; ++c) {
@@ -480,7 +486,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
         if (lane == 0) mbar_arrive(&bar_acc_empty[ab]);
       }
       PROF_BEGIN;
-      if (MODE == 1) {
+      if (MODE == kModeRank) {
         // ---- filtered-ranking epilogue: acc[c] = logit of (entity row, query column) ----
         if (job != cnt_job || cnt_tiles == 15) { flush_counts(cnt_job); cnt_job = job; cnt_tiles = 0; }
         ++cnt_tiles;
@@ -513,7 +519,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
           lsum += o.lsum;
         }
         lacc += (double)lsum;
-      } else if (MODE == 2) {
+      } else if (MODE == kModeScore) {
         // ---- score epilogue: G[e][b] = dBCE/dz and the BCE itself for ALL-NEGATIVE targets (t = t_neg), with the
         //      reference's fp32 semantics (score_bce.cu: p = 1 / (1 + expf(-z)), log terms clamped at -100, gradient
         //      scaled by p (1 - p) / max(p (1 - p), 1e-12)); the sparse positives are fixed up afterwards ----
@@ -528,7 +534,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
           lsum += score_chunk8(grow + c8 * 8, rv, a.B - (q0 + c8 * 8), tn, inv, acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2],
                                acc[c8 * 8 + 3], acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
         lacc += (double)lsum;
-      } else if (MODE == 3) {
+      } else if (MODE == kModeTopk) {
         // ---- top-k candidate epilogue: acc[c] = logit of (entity row, query column) ----
         const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
         const bool rv = e_loc < J.n;
@@ -540,7 +546,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
           topk_chunk8(a.thr + q0 + c8 * 8, a.thr + 3 * Bp + q0 + c8 * 8, onorm, rv, a.B - (q0 + c8 * 8), q0 + c8 * 8, e_loc,
                       a.topk_cnt, a.topk_seg, a.cand_cap, acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3],
                       acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
-      } else if (MODE == 4) {
+      } else if (MODE == kModeLse) {
         // ---- CE log-sum-exp epilogue: (m, s) of this warp's 32 rows per query column -> part[row group][column]
         //      (G reinterpreted as float2 [4 * tiles per job][ldg]) ----
         const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
@@ -551,7 +557,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
         for (int c8 = 0; c8 < HC8; ++c8)
           lse_chunk8(dst + c8 * 8, rv, a.B - (q0 + c8 * 8), acc[c8 * 8], acc[c8 * 8 + 1], acc[c8 * 8 + 2], acc[c8 * 8 + 3],
                      acc[c8 * 8 + 4], acc[c8 * 8 + 5], acc[c8 * 8 + 6], acc[c8 * 8 + 7]);
-      } else if (MODE == 5) {
+      } else if (MODE == kModeCe) {
         // ---- CE gradient epilogue: thr = row statistics [M_b | log2 S_b] with stride ldg (ce_row_stats) ----
         const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
         const bool rv = e_loc < J.n;
@@ -597,13 +603,13 @@ apply_tc_kernel(const __grid_constant__ Args a) {
       }
       PROF_END(pw1);
     }
-    if (MODE == 1) {
+    if (MODE == kModeRank) {
       flush_counts(cnt_job);
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) lacc += __shfl_xor_sync(0xffffffffu, lacc, o);
       if (lane == 0 && lacc != 0.0) atomicAdd(a.loss_sum, lacc);
     }
-    if (MODE == 2 || MODE == 5) {                     // one slot per epilogue warp: summed later in a fixed order
+    if (MODE == kModeScore || MODE == kModeCe) {   // one slot per epilogue warp: summed later in a fixed order
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) lacc += __shfl_xor_sync(0xffffffffu, lacc, o);
       if (lane == 0) a.loss_partial[blockIdx.x * kEpiWarps + warp] = lacc;
@@ -611,7 +617,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     if (tid == 0) { PROF_PRINT("epilogue (acc_full, store)"); }
   } else if (warp < kEpiWarps + kProdWarps) {
     // ================= producers: X block -> hi / lo operand images (+ optional raw copy) =================
-    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (kUpdateRegs) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     const int ptid = tid - kEpiWarps * 32;             // 0 .. kProdWarps*32-1
     // thread -> (16-byte chunk ch of the block's 4, rows r0, r0 + rstep, ...).  Row-major terms: 4 lanes cover the 64
@@ -763,7 +769,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     if (ptid == 0) { PROF_PRINT("producer (empty, produce)"); }
   } else if (warp == kMmaWarp) {
     // ================= MMA issuer =================
-    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (kUpdateRegs) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     if (lane == 0) {
       const uint32_t idesc = make_idesc_tf32(TM, a.rcp, false, false);
@@ -804,7 +810,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     __syncwarp();
   } else if (warp == kLoadWarp) {
     // ================= K image loader =================
-    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (kUpdateRegs) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));
     if (lane == 0) {
       Cursor c;
@@ -827,7 +833,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
     }
     __syncwarp();
   } else {
-    if (MODE == 0 || MODE == 3) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
+    if (kUpdateRegs) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOther));
     else asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;\n" :: "n"(kRegsOtherLogits));     // idle warps of the last warpgroup
   }
   fence_before_sync();
@@ -1026,27 +1032,79 @@ __global__ void rank_reset_if_overflow_kernel(int B, int32_t* greater, int32_t* 
   }
 }
 
-struct RankLayout { size_t scal, thr, norms, kimg, cand, total; int cap, nblk, njobs, Bp; };
-RankLayout rank_layout(int B, int n_local, int r2) {
-  RankLayout L;
+// ---------------------------------------------------------------------------------------------------------------
+// The logits passes (rank, top-k, BCE score, log-sum-exp, CE score): Z = O q^T on apply_tc_kernel, rows = the n_local
+// entities of the shard, the B queries in jobs of 256 columns, contraction over r2; the epilogue mode decides what
+// becomes of the logits.  Their shapes: rt::rank_tc_supported.
+// ---------------------------------------------------------------------------------------------------------------
+struct LogitGeom { int njobs, Bp, nblk, tiles_per_job; size_t kimg_bytes; };   // kimg_bytes: all query images
+LogitGeom logit_geom(int B, int n_local, int r2) {
+  LogitGeom g;
+  g.njobs = rt::cdiv(B, 256); g.Bp = 256 * g.njobs; g.nblk = rt::cdiv(r2, KB); g.tiles_per_job = rt::cdiv(n_local, TM);
+  g.kimg_bytes = (size_t)g.njobs * g.nblk * make_plan(256).kimg_bytes;
+  return g;
+}
+
+// Packs q into the query images at kimg and runs the logits pass with epilogue MODE on min(tiles, SMs) persistent
+// CTAs.  `a` carries the mode's own fields (thresholds and counters, G and loss slots, top-k segments); the modes with
+// loss slots get them zeroed before the launch.
+template <int MODE>
+int launch_logits(Args a, const float* q, const float* O, int B, int r2, int n_local, unsigned char* kimg,
+                  cudaStream_t s) {
   const Plan p = make_plan(256);
-  L.njobs = rt::cdiv(B, 256); L.Bp = 256 * L.njobs; L.nblk = rt::cdiv(r2, KB);
-  const long long all = (long long)B * n_local;
-  L.cap = (int)std::min<long long>(std::max<long long>(all / 8, 1 << 16), 1 << 22);
+  const LogitGeom g = logit_geom(B, n_local, r2);
+  rank_pack_q_kernel<<<g.njobs * g.nblk, 256, 0, s>>>(q, B, r2, g.nblk, p.rcp, kimg, p.cs_k, p.kimg_bytes);
+  RT_LAUNCH_CHECK();
+  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
+  a.stage_bytes = p.stage_bytes; a.Kimg = kimg;
+  a.njobs = g.njobs; a.ntiles = g.njobs * g.tiles_per_job; a.B = B;
+  for (int j = 0; j < g.njobs; ++j) {
+    Job& J = a.job[j];
+    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
+    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = g.nblk;
+    J.nblk = g.nblk; J.kblk0 = j * g.nblk; J.tile0 = j * g.tiles_per_job; J.ntiles = g.tiles_per_job;
+    J.reps = 1; J.tiles_per_rep = g.tiles_per_job;
+  }
+#ifdef RT_APPLY_PROF
+  a.debug = getenv("RT_APPLY_DEBUG") ? atoi(getenv("RT_APPLY_DEBUG")) : 0;
+#endif
+  if (MODE == kModeScore || MODE == kModeCe)
+    RT_CHECK_CUDA(cudaMemsetAsync(a.loss_partial, 0, sizeof(double) * (size_t)rt::sm_count() * kEpiWarps, s));
+  const int grid = std::min(a.ntiles, rt::sm_count());
+  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, MODE>, SMEM_LIMIT));
+  apply_tc_kernel<16, MODE><<<grid, kThreads, p.smem, s>>>(a);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+
+// Workspace of the rank and top-k passes: scalars, per-query band thresholds [4][Bp], entity norms, query images, and
+// a candidate list of `cap` (local entity, query) pairs (the rank pass; top-k keeps its candidates in the per-query
+// segments of its caller and passes cap = 0)
+struct BandLayout { LogitGeom g; size_t scal, thr, norms, kimg, cand, total; int cap; };
+BandLayout band_layout(int B, int n_local, int r2, int cap) {
+  BandLayout L;
+  L.g = logit_geom(B, n_local, r2);
+  L.cap = cap;
   size_t o = 0;
   auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
   L.scal = take(256);                                 // [0] cand_count, [1] overflow, [2] max ||O_j||^2, [4..5] loss (double)
-  L.thr = take(sizeof(float) * 4 * L.Bp);
+  L.thr = take(sizeof(float) * 4 * L.g.Bp);
   L.norms = take(sizeof(float) * (size_t)(n_local > 0 ? n_local : 1));
-  L.kimg = take((size_t)L.njobs * L.nblk * p.kimg_bytes);
-  L.cand = take(sizeof(int2) * (size_t)L.cap);
+  L.kimg = take(L.g.kimg_bytes);
+  L.cand = take(sizeof(int2) * (size_t)cap);
   L.total = o;
   return L;
+}
+BandLayout rank_layout(int B, int n_local, int r2) {
+  const long long all = (long long)B * n_local;
+  return band_layout(B, n_local, r2, (int)std::min<long long>(std::max<long long>(all / 8, 1 << 16), 1 << 22));
 }
 
 }  // namespace
 
 namespace rt {
+// the shapes of every logits pass: at most MAX_JOBS jobs of 256 queries, a contraction of 64 .. 1024, shards of at
+// least 1024 rows, three pipeline stages at width 256
 bool rank_tc_supported(int B, int n_local, int r2) {
   return B >= 1 && B <= 256 * MAX_JOBS && r2 >= 64 && r2 <= 1024 && n_local >= 1024 && make_plan(256).nstages >= 3;
 }
@@ -1076,8 +1134,7 @@ static int rank_tc_impl(bool logit, const float* q, const float* O, int B, int r
                         const int32_t* target, const float* p_target, const int32_t* flt_off, const int32_t* flt_idx,
                         int32_t* greater, int32_t* equal, int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s,
                         const int** overflow_flag) {
-  const RankLayout L = rank_layout(B, n_local, r2);
-  const Plan p = make_plan(256);
+  const BandLayout L = rank_layout(B, n_local, r2);
   char* base = (char*)ws;
   int* scal = (int*)(base + L.scal);
   double* loss = (double*)(base + L.scal + 16);
@@ -1086,35 +1143,14 @@ static int rank_tc_impl(bool logit, const float* q, const float* O, int B, int r
   float* onorms = (float*)(base + L.norms);
   rank_rownorm_kernel<<<rt::sm_count() * 4, 256, 0, s>>>(O, n_local, r2, (unsigned int*)(scal + 2), onorms);
   RT_LAUNCH_CHECK();
-  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_target, B, L.Bp, r2, thr);
-  else rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_target, B, L.Bp, r2, thr);
-  RT_LAUNCH_CHECK();
-  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kimg), p.cs_k,
-                                                       p.kimg_bytes);
+  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.g.Bp, 8), 256, 0, s>>>(q, p_target, B, L.g.Bp, r2, thr);
+  else rank_thresholds_kernel<<<rt::cdiv(L.g.Bp, 8), 256, 0, s>>>(q, p_target, B, L.g.Bp, r2, thr);
   RT_LAUNCH_CHECK();
   Args a{};
-  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
-  a.stage_bytes = p.stage_bytes; a.Kimg = (const unsigned char*)(base + L.kimg);
-  a.njobs = L.njobs;
-  const int tiles_per_job = rt::cdiv(n_local, TM);
-  for (int j = 0; j < L.njobs; ++j) {
-    Job& J = a.job[j];
-    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
-    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = L.nblk;
-    J.nblk = L.nblk; J.kblk0 = j * L.nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
-    J.reps = 1; J.tiles_per_rep = tiles_per_job;
-  }
-  a.ntiles = L.njobs * tiles_per_job;
-#ifdef RT_APPLY_PROF
-  a.debug = getenv("RT_APPLY_DEBUG") ? atoi(getenv("RT_APPLY_DEBUG")) : 0;
-#endif
-  a.thr = thr; a.onorms = onorms; a.target = target; a.B = B; a.n_begin = n_begin;
+  a.thr = thr; a.onorms = onorms; a.target = target; a.n_begin = n_begin;
   a.greater = greater; a.equal = equal; a.equal_before = equal_before;
   a.cand = (int2*)(base + L.cand); a.cand_count = scal; a.cand_cap = L.cap; a.loss_sum = loss;
-  const int grid = a.ntiles < rt::sm_count() ? a.ntiles : rt::sm_count();
-  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 1>, SMEM_LIMIT));
-  apply_tc_kernel<16, 1><<<grid, kThreads, p.smem, s>>>(a);
-  RT_LAUNCH_CHECK();
+  if (int rc = launch_logits<kModeRank>(a, q, O, B, r2, n_local, (unsigned char*)(base + L.kimg), s)) return rc;
   if (logit) {
     rank_candidates_kernel<true><<<rt::sm_count() * 2, 256, 0, s>>>(q, O, r2, n_begin, target, p_target, a.cand, scal,
                                                                     L.cap, greater, equal, equal_before, scal + 1);
@@ -1139,10 +1175,7 @@ static int rank_tc_impl(bool logit, const float* q, const float* O, int B, int r
 }
 
 // ---- top-k mode: the rank-mode pass with the per-query sample threshold p_k in place of p_target (topk.cu) ----
-size_t topk_tc_ws_bytes(int B, int n_local, int r2) {
-  const RankLayout L = rank_layout(B, n_local, r2);
-  return L.cand;                                      // the rank layout up to its candidate list
-}
+size_t topk_tc_ws_bytes(int B, int n_local, int r2) { return band_layout(B, n_local, r2, 0).total; }
 }  // namespace rt
 
 namespace {
@@ -1160,8 +1193,7 @@ namespace rt {
 // logit: p_k holds the sample's logit threshold z_k and the band is logit_thresholds_kernel's.
 int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
                  int32_t* seg, int cap, void* ws, cudaStream_t s, bool logit) {
-  const RankLayout L = rank_layout(B, n_local, r2);
-  const Plan p = make_plan(256);
+  const BandLayout L = band_layout(B, n_local, r2, 0);
   char* base = (char*)ws;
   unsigned int* maxnorm = (unsigned int*)(base + L.scal + 8);
   float* thr = (float*)(base + L.thr);
@@ -1169,34 +1201,15 @@ int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, con
   RT_CHECK_CUDA(cudaMemsetAsync(maxnorm, 0, sizeof(unsigned int), s));
   rank_rownorm_kernel<<<rt::sm_count() * 4, 256, 0, s>>>(O, n_local, r2, maxnorm, onorms);
   RT_LAUNCH_CHECK();
-  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
-  else rank_thresholds_kernel<<<rt::cdiv(L.Bp, 8), 256, 0, s>>>(q, p_k, B, L.Bp, r2, thr);
+  if (logit) logit_thresholds_kernel<<<rt::cdiv(L.g.Bp, 8), 256, 0, s>>>(q, p_k, B, L.g.Bp, r2, thr);
+  else rank_thresholds_kernel<<<rt::cdiv(L.g.Bp, 8), 256, 0, s>>>(q, p_k, B, L.g.Bp, r2, thr);
   RT_LAUNCH_CHECK();
   topk_empty_band_kernel<<<rt::cdiv(B, 256), 256, 0, s>>>(thr, B, flag);
   RT_LAUNCH_CHECK();
-  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kimg), p.cs_k,
-                                                       p.kimg_bytes);
-  RT_LAUNCH_CHECK();
   Args a{};
-  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
-  a.stage_bytes = p.stage_bytes; a.Kimg = (const unsigned char*)(base + L.kimg);
-  a.njobs = L.njobs;
-  const int tiles_per_job = rt::cdiv(n_local, TM);
-  for (int j = 0; j < L.njobs; ++j) {
-    Job& J = a.job[j];
-    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
-    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = L.nblk;
-    J.nblk = L.nblk; J.kblk0 = j * L.nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
-    J.reps = 1; J.tiles_per_rep = tiles_per_job;
-  }
-  a.ntiles = L.njobs * tiles_per_job;
-  a.thr = thr; a.onorms = onorms; a.B = B;
+  a.thr = thr; a.onorms = onorms;
   a.topk_seg = seg; a.topk_cnt = cnt; a.cand_cap = cap;
-  const int grid = a.ntiles < rt::sm_count() ? a.ntiles : rt::sm_count();
-  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 3>, SMEM_LIMIT));
-  apply_tc_kernel<16, 3><<<grid, kThreads, p.smem, s>>>(a);
-  RT_LAUNCH_CHECK();
-  return 0;
+  return launch_logits<kModeTopk>(a, q, O, B, r2, n_local, (unsigned char*)(base + L.kimg), s);
 }
 }  // namespace rt
 
@@ -1308,6 +1321,12 @@ int run_apply(int njobs, const JobSpec* jobs, int rc, void* ws, cudaStream_t s) 
 //                          chunks (replicated job) whose partial results are summed in a fixed order.
 // The logit / probability matrices never exist; G (B x N fp32, 84 MB at WN18RR size) is staged between the three
 // launches and stays resident in the 126 MB L2.
+//
+// 1-N softmax cross-entropy on the tensor cores (variant 3 of rt_score_lse / rt_score_ce_fwd_bwd, rtucker.h).
+//   log-sum-exp pass: the score mode's logits (same query images, job layout and 3xTF32 accumulation), epilogue
+//     kModeLse writes (m, s) per (32-row group, query); lse_combine (score_bce.cu) merges the groups in a fixed order;
+//   gradient pass: ce_row_stats turns the parts of all shards into (M_b, log2 S_b), then the four steps above with
+//     epilogue kModeCe (G = (softmax - ls/N) / B and the ls/N part of the loss) and score_ce_fix_positives_kernel.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void score_fix_positives_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2,
                                            int n_begin, int n_local, const int32_t* __restrict__ off,
@@ -1328,180 +1347,6 @@ __global__ void score_fix_positives_kernel(const float* __restrict__ q, const fl
   }
   dl = rt::warp_sum(dl);
   if (lane == 0) delta[b] = dl;
-}
-
-__global__ void score_finish_kernel(const float* __restrict__ Hpart, int reps, int count, float* __restrict__ H,
-                                    const double* __restrict__ loss_slots, int nslots, const double* __restrict__ delta,
-                                    int B, double* __restrict__ loss_out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < count) {
-    float s = 0.0f;
-    for (int r = 0; r < reps; ++r) s += Hpart[(size_t)r * count + i];      // fixed order
-    H[i] = s;
-  }
-  if (blockIdx.x == 0 && threadIdx.x < 32) {       // lane-strided partial sums + butterfly: the same association every run
-    double t = 0.0;
-    for (int k = threadIdx.x; k < nslots; k += 32) t += loss_slots[k];
-    for (int b = threadIdx.x; b < B; b += 32) t += delta[b];
-    t = rt::warp_sum(t);
-    if (threadIdx.x == 0) loss_out[0] = t;
-  }
-}
-
-struct ScoreLayout { size_t G, kq, kws, hpart, slots, delta, total; int njobs, Bp, nblk, chunk, reps, grid; };
-ScoreLayout score_layout(int B, int n_local, int r2) {
-  ScoreLayout L;
-  const Plan p256 = make_plan(256);
-  L.njobs = rt::cdiv(B, 256); L.Bp = 256 * L.njobs; L.nblk = rt::cdiv(r2, KB);
-  // H = G^T O: chunks of the entity range so that (query tiles) x (chunks) fills the SMs about once
-  const int qtiles = rt::cdiv(B, TM);
-  int reps = std::max(1, rt::sm_count() / qtiles);
-  int chunk = rt::cdiv(rt::cdiv(n_local, reps), KB) * KB;
-  if (chunk < 256) chunk = 256;
-  L.chunk = chunk; L.reps = rt::cdiv(n_local, chunk);
-  L.grid = std::min(rt::sm_count(), L.njobs * rt::cdiv(n_local, TM));
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.G = take(sizeof(float) * (size_t)L.reps * L.chunk * L.Bp);
-  L.kq = take((size_t)L.njobs * L.nblk * p256.kimg_bytes);
-  JobSpec j2{}; j2.n = n_local; j2.nk = 1; j2.t[0].rk = B; j2.reps = 1;
-  JobSpec j3{}; j3.n = B; j3.nk = 1; j3.t[0].rk = L.chunk; j3.reps = L.reps;
-  L.kws = take(std::max(run_apply_ws_bytes(1, &j2, r2), run_apply_ws_bytes(1, &j3, r2)));
-  L.hpart = take(sizeof(float) * (size_t)L.reps * B * r2);
-  L.slots = take(sizeof(double) * (size_t)rt::sm_count() * kEpiWarps);
-  L.delta = take(sizeof(double) * (size_t)B);
-  L.total = o;
-  return L;
-}
-}  // namespace
-
-// steps 3 and 4 of the score mode (shared by the BCE and the CE paths): dO = G qp, H = G^T O, loss reduction
-static int score_tc3_backward(const float* q, const float* qp, const float* O, int B, int r2, int n_local,
-                              const ScoreLayout& L, char* base, double* loss_sum, float* H, float* dO, cudaStream_t s) {
-  float* G = (float*)(base + L.G);
-  // ---- 3. dO = G Q'  (Q' = qp = q A_O when the caller folds the right factor of the projection in, else q) ----
-  {
-    JobSpec j{};
-    j.Y = dO; j.ldy = r2; j.n = n_local; j.nk = 1; j.reps = 1;
-    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].rk = B; j.t[0].K = qp ? qp : q; j.t[0].k_f32 = 1; j.t[0].rows_total = B;
-    int rc = run_apply(1, &j, r2, base + L.kws, s);
-    if (rc) return rc;
-  }
-  // ---- 4. H = G^T O in entity chunks ----
-  {
-    JobSpec j{};
-    float* Hpart = (float*)(base + L.hpart);
-    j.Y = Hpart; j.ldy = r2; j.n = B; j.nk = 1; j.reps = L.reps; j.y_rep = (int64_t)B * r2;
-    j.t[0].X = G; j.t[0].ldx = L.Bp; j.t[0].xt = 1; j.t[0].rk = L.chunk; j.t[0].x_rep = (int64_t)L.chunk * L.Bp;
-    j.t[0].K = O; j.t[0].k_f32 = 1; j.t[0].rows_total = n_local;
-    int rc = run_apply(1, &j, r2, base + L.kws, s);
-    if (rc) return rc;
-    score_finish_kernel<<<rt::cdiv(B * r2, 256), 256, 0, s>>>(Hpart, L.reps, B * r2, H, (const double*)(base + L.slots),
-                                                              rt::sm_count() * kEpiWarps, (const double*)(base + L.delta), B,
-                                                              loss_sum);
-    RT_LAUNCH_CHECK();
-  }
-  return 0;
-}
-
-extern "C" int rt_score_bce_tc3_supported(int B, int n_local, int r2) {
-  return (B >= 1 && B <= 256 * MAX_JOBS && r2 >= 64 && r2 <= RCP_MAX && n_local >= 1024 && make_plan(256).nstages >= 3 &&
-          make_plan(r2).nstages >= 3) ? 1 : 0;
-}
-extern "C" size_t rt_score_bce_tc3_ws_bytes(int B, int n_local, int r2) { return score_layout(B, n_local, r2).total; }
-
-extern "C" int rt_score_bce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local,
-                                int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx,
-                                float label_smoothing, double* loss_sum, float* H, float* dO, void* ws, void* stream) {
-  RT_REQUIRE(rt_score_bce_tc3_supported(B, n_local, r2), "rt_score_bce_tc3: unsupported shape B=%d n_local=%d r2=%d", B, n_local, r2);
-  RT_REQUIRE(ws != nullptr, "rt_score_bce_tc3: workspace is NULL");
-  cudaStream_t s = (cudaStream_t)stream;
-  const ScoreLayout L = score_layout(B, n_local, r2);
-  const Plan p = make_plan(256);
-  char* base = (char*)ws;
-  float* G = (float*)(base + L.G);
-  const float t_neg = label_smoothing / (float)n_total, t_pos = (1.0f - label_smoothing) + t_neg;
-  const float inv_count = (float)(1.0 / ((double)b_total * (double)n_total));
-  // rows [n_local, reps * chunk) of G are contraction padding of step 4
-  const size_t pad_rows = (size_t)L.reps * L.chunk - n_local;
-  if (pad_rows) RT_CHECK_CUDA(cudaMemsetAsync(G + (size_t)n_local * L.Bp, 0, pad_rows * L.Bp * sizeof(float), s));
-  // ---- 1. logits -> loss, G ----
-  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kq), p.cs_k, p.kimg_bytes);
-  RT_LAUNCH_CHECK();
-  {
-    Args a{};
-    a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
-    a.stage_bytes = p.stage_bytes; a.Kimg = (const unsigned char*)(base + L.kq);
-    a.njobs = L.njobs;
-    const int tiles_per_job = rt::cdiv(n_local, TM);
-    for (int j = 0; j < L.njobs; ++j) {
-      Job& J = a.job[j];
-      J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
-      for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = L.nblk;
-      J.nblk = L.nblk; J.kblk0 = j * L.nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
-      J.reps = 1; J.tiles_per_rep = tiles_per_job;
-    }
-    a.ntiles = L.njobs * tiles_per_job;
-    a.B = B; a.n_begin = n_begin; a.G = G; a.ldg = L.Bp; a.t_neg = t_neg; a.inv_count = inv_count;
-    a.loss_partial = (double*)(base + L.slots);
-    RT_CHECK_CUDA(cudaMemsetAsync(a.loss_partial, 0, sizeof(double) * (size_t)rt::sm_count() * kEpiWarps, s));
-    RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 2>, SMEM_LIMIT));
-    apply_tc_kernel<16, 2><<<L.grid, kThreads, p.smem, s>>>(a);
-    RT_LAUNCH_CHECK();
-  }
-  // ---- 2. positives ----
-  score_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx, t_pos, t_neg,
-                                                            inv_count, G, L.Bp, (double*)(base + L.delta));
-  RT_LAUNCH_CHECK();
-  return score_tc3_backward(q, qp, O, B, r2, n_local, L, base, loss_sum, H, dO, s);
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// 1-N softmax cross-entropy on the tensor cores (variant 3 of rt_score_lse / rt_score_ce_fwd_bwd, rtucker.h).
-//   log-sum-exp pass: the score mode's logits (same query images, job layout and 3xTF32 accumulation), epilogue mode 4
-//     writes (m, s) per (32-row group, query); lse_combine (score_bce.cu) merges the groups in a fixed order;
-//   gradient pass: ce_row_stats turns the parts of all shards into (M_b, log2 S_b), epilogue mode 5 writes
-//     G = (softmax - ls/N) / B and the ls/N part of the loss, score_ce_fix_positives_kernel patches the positives,
-//     then steps 3 and 4 of the score mode unchanged.
-// ---------------------------------------------------------------------------------------------------------------
-namespace rt {
-int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
-int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
-}  // namespace rt
-
-namespace {
-// the logits launch of the score mode: rows = the n_local entities, 256 queries per job, query images at kq
-Args score_logit_args(const float* O, int B, int r2, int n_local, const unsigned char* kq) {
-  const Plan p = make_plan(256);
-  Args a{};
-  a.rc = 256; a.rcp = p.rcp; a.nstages = p.nstages; a.cs_k = p.cs_k; a.kimg_bytes = p.kimg_bytes; a.gb = GB_LOGITS;
-  a.stage_bytes = p.stage_bytes; a.Kimg = kq;
-  a.njobs = rt::cdiv(B, 256);
-  const int nblk = rt::cdiv(r2, KB), tiles_per_job = rt::cdiv(n_local, TM);
-  for (int j = 0; j < a.njobs; ++j) {
-    Job& J = a.job[j];
-    J.n = n_local; J.nk = 1; J.X[0] = O; J.ldx[0] = r2; J.rk[0] = r2;
-    for (int t = 0; t < MAX_TERMS; ++t) J.blk_end[t] = nblk;
-    J.nblk = nblk; J.kblk0 = j * nblk; J.tile0 = j * tiles_per_job; J.ntiles = tiles_per_job;
-    J.reps = 1; J.tiles_per_rep = tiles_per_job;
-  }
-  a.ntiles = a.njobs * tiles_per_job;
-  a.B = B;
-  return a;
-}
-
-struct LseLayout { size_t kq, part, total; int groups, Bp, nblk, njobs; };
-LseLayout lse_layout(int B, int n_local, int r2) {
-  LseLayout L;
-  const Plan p256 = make_plan(256);
-  L.njobs = rt::cdiv(B, 256); L.Bp = 256 * L.njobs; L.nblk = rt::cdiv(r2, KB);
-  L.groups = 4 * rt::cdiv(n_local, TM);                      // 32-row groups of one job's tiles
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.kq = take((size_t)L.njobs * L.nblk * p256.kimg_bytes);
-  L.part = take(sizeof(float2) * (size_t)L.groups * L.Bp);
-  L.total = o;
-  return L;
 }
 
 __global__ void score_ce_fix_positives_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2,
@@ -1529,62 +1374,161 @@ __global__ void score_ce_fix_positives_kernel(const float* __restrict__ q, const
   dl = rt::warp_sum(dl);
   if (lane == 0) delta[b] = dl;
 }
+
+__global__ void score_finish_kernel(const float* __restrict__ Hpart, int reps, int count, float* __restrict__ H,
+                                    const double* __restrict__ loss_slots, int nslots, const double* __restrict__ delta,
+                                    int B, double* __restrict__ loss_out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < count) {
+    float s = 0.0f;
+    for (int r = 0; r < reps; ++r) s += Hpart[(size_t)r * count + i];      // fixed order
+    H[i] = s;
+  }
+  if (blockIdx.x == 0 && threadIdx.x < 32) {       // lane-strided partial sums + butterfly: the same association every run
+    double t = 0.0;
+    for (int k = threadIdx.x; k < nslots; k += 32) t += loss_slots[k];
+    for (int b = threadIdx.x; b < B; b += 32) t += delta[b];
+    t = rt::warp_sum(t);
+    if (threadIdx.x == 0) loss_out[0] = t;
+  }
+}
+
+struct ScoreLayout { LogitGeom g; size_t G, kq, kws, hpart, slots, delta, total; int chunk, reps; };
+ScoreLayout score_layout(int B, int n_local, int r2) {
+  ScoreLayout L;
+  L.g = logit_geom(B, n_local, r2);
+  // H = G^T O: chunks of the entity range so that (query tiles) x (chunks) fills the SMs about once
+  const int qtiles = rt::cdiv(B, TM);
+  int reps = std::max(1, rt::sm_count() / qtiles);
+  int chunk = rt::cdiv(rt::cdiv(n_local, reps), KB) * KB;
+  if (chunk < 256) chunk = 256;
+  L.chunk = chunk; L.reps = rt::cdiv(n_local, chunk);
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
+  L.G = take(sizeof(float) * (size_t)L.reps * L.chunk * L.g.Bp);
+  L.kq = take(L.g.kimg_bytes);
+  JobSpec j2{}; j2.n = n_local; j2.nk = 1; j2.t[0].rk = B; j2.reps = 1;
+  JobSpec j3{}; j3.n = B; j3.nk = 1; j3.t[0].rk = L.chunk; j3.reps = L.reps;
+  L.kws = take(std::max(run_apply_ws_bytes(1, &j2, r2), run_apply_ws_bytes(1, &j3, r2)));
+  L.hpart = take(sizeof(float) * (size_t)L.reps * B * r2);
+  L.slots = take(sizeof(double) * (size_t)rt::sm_count() * kEpiWarps);
+  L.delta = take(sizeof(double) * (size_t)B);
+  L.total = o;
+  return L;
+}
+
+// The four steps with epilogue MODE: kModeScore (label-smoothed BCE) or kModeCe (softmax cross-entropy; stats = the
+// row statistics [M_b | log2 S_b] of ce_row_stats, stride Bp).
+template <int MODE>
+int score_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+              int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* stats,
+              double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s) {
+  const ScoreLayout L = score_layout(B, n_local, r2);
+  const int Bp = L.g.Bp;
+  char* base = (char*)ws;
+  float* G = (float*)(base + L.G);
+  double* delta = (double*)(base + L.delta);
+  const float t_neg = label_smoothing / (float)n_total;
+  const float inv_count = MODE == kModeCe ? (float)(1.0 / (double)b_total)
+                                          : (float)(1.0 / ((double)b_total * (double)n_total));
+  // rows [n_local, reps * chunk) of G are contraction padding of step 4
+  const size_t pad_rows = (size_t)L.reps * L.chunk - n_local;
+  if (pad_rows) RT_CHECK_CUDA(cudaMemsetAsync(G + (size_t)n_local * Bp, 0, pad_rows * Bp * sizeof(float), s));
+  // ---- 1. logits -> loss, G for all-negative targets ----
+  Args a{};
+  a.n_begin = n_begin; a.G = G; a.ldg = Bp; a.t_neg = t_neg; a.inv_count = inv_count; a.thr = stats;
+  a.loss_partial = (double*)(base + L.slots);
+  if (int rc = launch_logits<MODE>(a, q, O, B, r2, n_local, (unsigned char*)(base + L.kq), s)) return rc;
+  // ---- 2. positives ----
+  if (MODE == kModeCe)
+    score_ce_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx,
+                                                                 1.0f - label_smoothing, t_neg, inv_count, stats, Bp, G,
+                                                                 Bp, delta);
+  else
+    score_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx,
+                                                              (1.0f - label_smoothing) + t_neg, t_neg, inv_count, G, Bp,
+                                                              delta);
+  RT_LAUNCH_CHECK();
+  // ---- 3. dO = G Q'  (Q' = qp = q A_O when the caller folds the right factor of the projection in, else q) ----
+  {
+    JobSpec j{};
+    j.Y = dO; j.ldy = r2; j.n = n_local; j.nk = 1; j.reps = 1;
+    j.t[0].X = G; j.t[0].ldx = Bp; j.t[0].rk = B; j.t[0].K = qp ? qp : q; j.t[0].k_f32 = 1; j.t[0].rows_total = B;
+    int rc = run_apply(1, &j, r2, base + L.kws, s);
+    if (rc) return rc;
+  }
+  // ---- 4. H = G^T O in entity chunks ----
+  {
+    JobSpec j{};
+    float* Hpart = (float*)(base + L.hpart);
+    j.Y = Hpart; j.ldy = r2; j.n = B; j.nk = 1; j.reps = L.reps; j.y_rep = (int64_t)B * r2;
+    j.t[0].X = G; j.t[0].ldx = Bp; j.t[0].xt = 1; j.t[0].rk = L.chunk; j.t[0].x_rep = (int64_t)L.chunk * Bp;
+    j.t[0].K = O; j.t[0].k_f32 = 1; j.t[0].rows_total = n_local;
+    int rc = run_apply(1, &j, r2, base + L.kws, s);
+    if (rc) return rc;
+    score_finish_kernel<<<rt::cdiv(B * r2, 256), 256, 0, s>>>(Hpart, L.reps, B * r2, H, (const double*)(base + L.slots),
+                                                              rt::sm_count() * kEpiWarps, delta, B, loss_sum);
+    RT_LAUNCH_CHECK();
+  }
+  return 0;
+}
+
+struct LseLayout { LogitGeom g; size_t kq, part, total; int groups; };
+LseLayout lse_layout(int B, int n_local, int r2) {
+  LseLayout L;
+  L.g = logit_geom(B, n_local, r2);
+  L.groups = 4 * L.g.tiles_per_job;                          // 32-row groups of one job's tiles
+  size_t o = 0;
+  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
+  L.kq = take(L.g.kimg_bytes);
+  L.part = take(sizeof(float2) * (size_t)L.groups * L.g.Bp);
+  L.total = o;
+  return L;
+}
 }  // namespace
 
+extern "C" int rt_score_bce_tc3_supported(int B, int n_local, int r2) {
+  return (rt::rank_tc_supported(B, n_local, r2) && r2 <= RCP_MAX && make_plan(r2).nstages >= 3) ? 1 : 0;
+}
+extern "C" size_t rt_score_bce_tc3_ws_bytes(int B, int n_local, int r2) { return score_layout(B, n_local, r2).total; }
+
+extern "C" int rt_score_bce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local,
+                                int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx,
+                                float label_smoothing, double* loss_sum, float* H, float* dO, void* ws, void* stream) {
+  RT_REQUIRE(rt_score_bce_tc3_supported(B, n_local, r2), "rt_score_bce_tc3: unsupported shape B=%d n_local=%d r2=%d", B, n_local, r2);
+  RT_REQUIRE(ws != nullptr, "rt_score_bce_tc3: workspace is NULL");
+  return score_tc3<kModeScore>(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx, label_smoothing,
+                               nullptr, loss_sum, H, dO, ws, (cudaStream_t)stream);
+}
+
 namespace rt {
+int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
+int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
+
 size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2) { return lse_layout(B, n_local, r2).total; }
 
 int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s) {
   const LseLayout L = lse_layout(B, n_local, r2);
-  const Plan p = make_plan(256);
   char* base = (char*)ws;
-  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kq), p.cs_k, p.kimg_bytes);
-  RT_LAUNCH_CHECK();
-  Args a = score_logit_args(O, B, r2, n_local, (const unsigned char*)(base + L.kq));
-  a.G = (float*)(base + L.part); a.ldg = L.Bp;
-  const int grid = std::min(rt::sm_count(), a.ntiles);
-  RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 4>, SMEM_LIMIT));
-  apply_tc_kernel<16, 4><<<grid, kThreads, p.smem, s>>>(a);
-  RT_LAUNCH_CHECK();
-  return lse_combine((const float2*)(base + L.part), L.groups, L.Bp, B, parts, s);
+  Args a{};
+  a.G = (float*)(base + L.part); a.ldg = L.g.Bp;
+  if (int rc = launch_logits<kModeLse>(a, q, O, B, r2, n_local, (unsigned char*)(base + L.kq), s)) return rc;
+  return lse_combine((const float2*)(base + L.part), L.groups, L.g.Bp, B, parts, s);
 }
 
 size_t score_ce_tc3_ws_bytes(int B, int n_local, int r2) {
   const ScoreLayout L = score_layout(B, n_local, r2);
-  return L.total + rt::align_up(sizeof(float) * 2 * (size_t)L.Bp, 256);
+  return L.total + rt::align_up(sizeof(float) * 2 * (size_t)L.g.Bp, 256);
 }
 
 int score_ce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
                  int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* parts,
                  int nparts, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s) {
   const ScoreLayout L = score_layout(B, n_local, r2);
-  const Plan p = make_plan(256);
-  char* base = (char*)ws;
-  float* G = (float*)(base + L.G);
-  float* stats = (float*)(base + L.total);                   // [M_b | log2 S_b], stride Bp
-  const float t_neg = label_smoothing / (float)n_total;
-  const float inv_count = (float)(1.0 / (double)b_total);
-  if (int rc = ce_row_stats(parts, nparts, B, L.Bp, stats, s)) return rc;
-  const size_t pad_rows = (size_t)L.reps * L.chunk - n_local;
-  if (pad_rows) RT_CHECK_CUDA(cudaMemsetAsync(G + (size_t)n_local * L.Bp, 0, pad_rows * L.Bp * sizeof(float), s));
-  // ---- 1. logits -> ls/N part of the loss, G for all-negative targets ----
-  rank_pack_q_kernel<<<L.njobs * L.nblk, 256, 0, s>>>(q, B, r2, L.nblk, p.rcp, (unsigned char*)(base + L.kq), p.cs_k, p.kimg_bytes);
-  RT_LAUNCH_CHECK();
-  {
-    Args a = score_logit_args(O, B, r2, n_local, (const unsigned char*)(base + L.kq));
-    a.n_begin = n_begin; a.G = G; a.ldg = L.Bp; a.t_neg = t_neg; a.inv_count = inv_count; a.thr = stats;
-    a.loss_partial = (double*)(base + L.slots);
-    RT_CHECK_CUDA(cudaMemsetAsync(a.loss_partial, 0, sizeof(double) * (size_t)rt::sm_count() * kEpiWarps, s));
-    RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)apply_tc_kernel<16, 5>, SMEM_LIMIT));
-    apply_tc_kernel<16, 5><<<L.grid, kThreads, p.smem, s>>>(a);
-    RT_LAUNCH_CHECK();
-  }
-  // ---- 2. positives ----
-  score_ce_fix_positives_kernel<<<rt::cdiv(B, 8), 256, 0, s>>>(q, O, B, r2, n_begin, n_local, tgt_off, tgt_idx,
-                                                               1.0f - label_smoothing, t_neg, inv_count, stats, L.Bp, G,
-                                                               L.Bp, (double*)(base + L.delta));
-  RT_LAUNCH_CHECK();
-  return score_tc3_backward(q, qp, O, B, r2, n_local, L, base, loss_sum, H, dO, s);
+  float* stats = (float*)((char*)ws + L.total);              // [M_b | log2 S_b], stride Bp
+  if (int rc = ce_row_stats(parts, nparts, B, L.g.Bp, stats, s)) return rc;
+  return score_tc3<kModeCe>(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx, label_smoothing,
+                            stats, loss_sum, H, dO, ws, s);
 }
 }  // namespace rt
 

@@ -15,7 +15,6 @@
 // H_chunk += G O_tile (accumulated in this CTA's private workspace slice, summed over CTAs in a
 // fixed order afterwards)  and  dO_tile += G^T QP_chunk (registers, across the chunk loop).
 #include "common.h"
-#include <stdlib.h>
 #include <math.h>
 
 namespace {
@@ -426,6 +425,35 @@ int dispatch(const ScoreArgs& a, const Plan& p, cudaStream_t s) {
   }
 }
 
+// Variant 0 of the training passes, BCE (CE = false) or softmax cross-entropy (CE = true, stats = the row statistics
+// of ce_row_stats): score_kernel over the shard, then H and the loss summed over the CTAs in a fixed order.
+// ws: [grid][B][r2] partial H, then [grid] partial losses (rt_score_bce_ws_bytes).
+template <bool CE>
+int score_train_ffma(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local,
+                     int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
+                     const float* stats, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s) {
+  const Plan p = make_plan(n_local, r2, false);
+  ScoreArgs a{};
+  a.q = q; a.qp = qp ? qp : q; a.O = O;
+  a.B = B; a.r2 = r2; a.n_begin = n_begin; a.n_local = n_local; a.n_total = n_total;
+  a.off = tgt_off; a.idx = tgt_idx;
+  a.t_neg = label_smoothing / (float)n_total;
+  a.t_pos = CE ? 1.0f - label_smoothing : (1.0f - label_smoothing) + a.t_neg;
+  a.inv_count = CE ? (float)(1.0 / (double)b_total) : (float)(1.0 / ((double)b_total * (double)n_total));
+  a.p_target = stats;
+  a.H_ws = (float*)ws;
+  a.loss_partial = (double*)((char*)ws + rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256));
+  a.dO = dO;
+  a.n_tiles = p.n_tiles;
+  if (int rc = dispatch<false, CE>(a, p, s)) return rc;
+  const int64_t count = (int64_t)B * r2;
+  reduce_H_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
+  RT_LAUNCH_CHECK();
+  reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, loss_sum, 0);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+
 // ---- 1-N softmax cross-entropy, FFMA path: the log-sum-exp pass --------------------------------------------------
 // Tile of 64 queries x 64 entities per CTA with score_dense_kernel's staging and k order (the logits are bit-identical
 // to the ones score_kernel<., false, true> sees).  Per query row and tile: m = the largest logit, s = sum exp(z - m)
@@ -594,27 +622,8 @@ extern "C" int rt_score_bce_fwd_bwd(const float* q, const float* qp, const float
                            loss_sum, H, dO, nullptr, ws, stream);
   }
   RT_REQUIRE(variant == 0, "rt_score_bce_fwd_bwd: unknown variant %d", variant);
-  cudaStream_t s = (cudaStream_t)stream;
-  Plan p = make_plan(n_local, r2, false);
-  ScoreArgs a{};
-  a.q = q; a.qp = qp ? qp : q; a.O = O;
-  a.B = B; a.r2 = r2; a.n_begin = n_begin; a.n_local = n_local; a.n_total = n_total;
-  a.off = tgt_off; a.idx = tgt_idx;
-  a.t_neg = label_smoothing / (float)n_total;
-  a.t_pos = (1.0f - label_smoothing) + a.t_neg;
-  a.inv_count = (float)(1.0 / ((double)b_total * (double)n_total));
-  a.H_ws = (float*)ws;
-  a.loss_partial = (double*)((char*)ws + rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256));
-  a.dO = dO;
-  a.n_tiles = p.n_tiles;
-  int rc = dispatch<false>(a, p, s);
-  if (rc) return rc;
-  const int64_t count = (int64_t)B * r2;
-  reduce_H_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
-  RT_LAUNCH_CHECK();
-  reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, loss_sum, 0);
-  RT_LAUNCH_CHECK();
-  return 0;
+  return score_train_ffma<false>(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx, label_smoothing,
+                                 nullptr, loss_sum, H, dO, ws, (cudaStream_t)stream);
 }
 
 extern "C" int rt_target_prob(const float* q, const float* O, int B, int r2, int n_begin, int n_local,
@@ -641,11 +650,6 @@ __global__ void gated_reduce_loss_kernel(const double* __restrict__ partial, int
   for (int i = 0; i < n; ++i) s += partial[i];
   out[0] = s;
 }
-// RT_RANK_TC=0 keeps the evaluation on the fp32 FFMA kernel (A/B timing, cross-checks)
-static bool rank_tc_enabled() {
-  static const bool v = [] { const char* e = getenv("RT_RANK_TC"); return !(e && e[0] == '0'); }();
-  return v;
-}
 
 extern "C" size_t rt_score_rank_ws_bytes(int B, int n_local, int r2) {
   Plan p = make_plan(n_local, r2, true);
@@ -670,7 +674,7 @@ extern "C" int rt_score_rank_fused(const float* q, const float* O, int B, int r2
   // probability could tie with or cross the target's (apply_tc.cu, rank mode); the fp32 kernel below then only
   // runs -- gated on a device flag, no host synchronisation -- when that candidate list overflowed
   const int* gate = nullptr;
-  if (rank_tc_enabled() && rt::rank_tc_supported(B, n_local, r2)) {
+  if (rt::rank_tc_supported(B, n_local, r2)) {
     char* tc_ws = (char*)ws + rt::align_up((size_t)p.grid * sizeof(double) + 256, 256);
     int rc = rt::rank_tc(q, O, B, r2, n_begin, n_local, target, p_target, flt_off, flt_idx, greater, equal,
                          equal_before, bce_sum, tc_ws, s, &gate);
@@ -801,29 +805,12 @@ extern "C" int rt_score_ce_fwd_bwd(const float* q, const float* qp, const float*
   if (variant == 3)
     return rt::score_ce_tc3(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx, label_smoothing,
                             parts, nparts, loss_sum, H, dO, ws, s);
-  Plan p = make_plan(n_local, r2, false);
   const size_t bce_bytes = rt::align_up(rt_score_bce_ws_bytes(B, n_local, r2, 0), 256);
   float* stats = (float*)((char*)ws + bce_bytes);
   if (int rc = rt::ce_row_stats(parts, nparts, B, B, stats, s)) return rc;
-  ScoreArgs a{};
-  a.q = q; a.qp = qp ? qp : q; a.O = O;
-  a.B = B; a.r2 = r2; a.n_begin = n_begin; a.n_local = n_local; a.n_total = n_total;
-  a.off = tgt_off; a.idx = tgt_idx;
-  a.t_neg = label_smoothing / (float)n_total;
-  a.t_pos = 1.0f - label_smoothing;
-  a.inv_count = (float)(1.0 / (double)b_total);
-  a.p_target = stats;
-  a.H_ws = (float*)ws;
-  a.loss_partial = (double*)((char*)ws + rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256));
-  a.dO = dO;
-  a.n_tiles = p.n_tiles;
-  int rc = dispatch<false, true>(a, p, s);
-  if (rc) return rc;
-  const int64_t count = (int64_t)B * r2;
-  reduce_H_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
-  RT_LAUNCH_CHECK();
-  reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, loss_sum, 0);
-  RT_LAUNCH_CHECK();
+  if (int rc = score_train_ffma<true>(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx,
+                                      label_smoothing, stats, loss_sum, H, dO, ws, s))
+    return rc;
   if (n_begin == 0) {
     ce_empty_rows_kernel<<<1, 32, 0, s>>>(tgt_off, B, stats, B, 1.0f - label_smoothing, loss_sum);
     RT_LAUNCH_CHECK();

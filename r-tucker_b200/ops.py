@@ -188,6 +188,19 @@ def score_v3_supported(r2):
 def score_tc3_supported(B, n_local, r2):
     return bool(lib().rt_score_bce_tc3_supported(int(B), int(n_local), int(r2)))
 
+
+def _score_prologue(q, O, n_total, b_total, out):
+    """Shapes and outputs of the fused training losses: (B, r2, n_local, n_total, b_total, (loss, H, dO)), with
+    n_total / b_total defaulting to this shard and this batch and the outputs allocated unless ``out`` is given."""
+    B, r2 = q.shape
+    n_local = O.shape[0]
+    if out is None:
+        dev = q.device
+        out = (torch.empty(1, dtype=f64, device=dev), torch.empty(B, r2, dtype=f32, device=dev),
+               torch.empty(n_local, r2, dtype=f32, device=dev))
+    return (B, r2, n_local, n_local if n_total is None else n_total, B if b_total is None else b_total, out)
+
+
 def score_bce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, n_total=None, b_total=None,
                       n_begin=0, variant=0, out=None, ws=None, o_absmax=None, phases=7, centre=None):
     """Returns (loss_sum[1] f64 -- un-normalised, H [B,r2], dO [n_local,r2]).
@@ -196,55 +209,26 @@ def score_bce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, n_total=None,
     ``phases`` (variant 2 only) selects packing (1), fused kernel (2), reduction (4) for timing; ``centre`` (variant 2,
     device float[2], persistent across steps, [1] initialised to 0.5) enables the centred gradient operand."""
     require_cuda(q, qp, O, tgt_off, tgt_idx, centre)
+    if variant == 2 and qp is not None and qp is not q:
+        raise RTuckerError("score_bce_fwd_bwd(variant=2) computes dO = G^T q: pass qp=None")
+    B, r2, n_local, n_total, b_total, (loss, H, dO) = _score_prologue(q, O, n_total, b_total, out)
+    if ws is None:
+        ws = _ws(lib().rt_score_bce_tc3_ws_bytes(B, n_local, r2) if variant == 3 else
+                 lib().rt_score_bce_ws_bytes(B, n_local, r2, variant), q.device)
     if variant == 3:
-        B, r2 = q.shape
-        n_local = O.shape[0]
-        n_total = n_local if n_total is None else n_total
-        b_total = B if b_total is None else b_total
-        dev = q.device
-        if out is None:
-            out = (torch.empty(1, dtype=f64, device=dev), torch.empty(B, r2, dtype=f32, device=dev),
-                   torch.empty(n_local, r2, dtype=f32, device=dev))
-        loss, H, dO = out
-        ws = ws if ws is not None else _ws(lib().rt_score_bce_tc3_ws_bytes(B, n_local, r2), dev)
         check(lib().rt_score_bce_tc3(ptr(_c(q, f32)), ptr(qp), ptr(_c(O, f32)), B, r2, n_begin, n_local, n_total, b_total,
                                      ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)), float(label_smoothing), ptr(loss),
                                      ptr(H), ptr(dO), ptr(ws), stream_ptr()), "rt_score_bce_tc3")
-        return loss, H, dO
-    if variant == 2:
-        if qp is not None and qp is not q:
-            raise RTuckerError("score_bce_fwd_bwd(variant=2) computes dO = G^T q: pass qp=None")
-        B, r2 = q.shape
-        n_local = O.shape[0]
-        n_total = n_local if n_total is None else n_total
-        b_total = B if b_total is None else b_total
-        dev = q.device
-        if out is None:
-            out = (torch.empty(1, dtype=f64, device=dev), torch.empty(B, r2, dtype=f32, device=dev),
-                   torch.empty(n_local, r2, dtype=f32, device=dev))
-        loss, H, dO = out
-        ws = ws if ws is not None else _ws(lib().rt_score_bce_v3_ws_bytes(B, n_local, r2), dev)
+    elif variant == 2:
         check(lib().rt_score_bce_v3_phases(ptr(_c(q, f32)), ptr(_c(O, f32)), B, r2, n_begin, n_local, n_total,
                                            b_total, ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)),
                                            float(label_smoothing), float(o_absmax or 0.0), ptr(loss), ptr(H),
                                            ptr(dO), ptr(centre), ptr(ws), stream_ptr(), int(phases)), "rt_score_bce_v3")
-        return loss, H, dO
-    B, r2 = q.shape
-    n_local = O.shape[0]
-    n_total = n_local if n_total is None else n_total
-    b_total = B if b_total is None else b_total
-    dev = q.device
-    if out is None:
-        loss = torch.empty(1, dtype=f64, device=dev)
-        H = torch.empty(B, r2, dtype=f32, device=dev)
-        dO = torch.empty(n_local, r2, dtype=f32, device=dev)
     else:
-        loss, H, dO = out
-    ws = ws if ws is not None else _ws(lib().rt_score_bce_ws_bytes(B, n_local, r2, variant), dev)
-    check(lib().rt_score_bce_fwd_bwd(ptr(_c(q, f32)), ptr(_c(qp, f32)), ptr(_c(O, f32)), B, r2, n_begin,
-                                     n_local, n_total, b_total, ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)),
-                                     float(label_smoothing), ptr(loss), ptr(H), ptr(dO), variant, ptr(ws),
-                                     stream_ptr()), "rt_score_bce_fwd_bwd")
+        check(lib().rt_score_bce_fwd_bwd(ptr(_c(q, f32)), ptr(_c(qp, f32)), ptr(_c(O, f32)), B, r2, n_begin,
+                                         n_local, n_total, b_total, ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)),
+                                         float(label_smoothing), ptr(loss), ptr(H), ptr(dO), variant, ptr(ws),
+                                         stream_ptr()), "rt_score_bce_fwd_bwd")
     return loss, H, dO
 
 
@@ -269,20 +253,12 @@ def score_ce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, parts, n_total
     the score_lse results of every entity shard.  Returns (loss_sum[1] f64 -- un-normalised: divide by b_total,
     H [B, r2], dO [n_local, r2])."""
     require_cuda(q, qp, O, tgt_off, tgt_idx, parts)
-    B, r2 = q.shape
-    n_local = O.shape[0]
-    n_total = n_local if n_total is None else n_total
-    b_total = B if b_total is None else b_total
+    B, r2, n_local, n_total, b_total, (loss, H, dO) = _score_prologue(q, O, n_total, b_total, out)
     parts = _c(parts, f32)
     nparts = 1 if parts.dim() == 2 else parts.shape[0]
     if parts.shape[-2:] != (B, 2):
         raise RTuckerError(f"score_ce_fwd_bwd: parts must be [nparts, {B}, 2], got {tuple(parts.shape)}")
-    dev = q.device
-    if out is None:
-        out = (torch.empty(1, dtype=f64, device=dev), torch.empty(B, r2, dtype=f32, device=dev),
-               torch.empty(n_local, r2, dtype=f32, device=dev))
-    loss, H, dO = out
-    ws = ws if ws is not None else _ws(lib().rt_score_ce_ws_bytes(B, n_local, r2, int(variant)), dev)
+    ws = ws if ws is not None else _ws(lib().rt_score_ce_ws_bytes(B, n_local, r2, int(variant)), q.device)
     check(lib().rt_score_ce_fwd_bwd(ptr(_c(q, f32)), ptr(qp), ptr(_c(O, f32)), B, r2, int(n_begin), n_local,
                                     int(n_total), int(b_total), ptr(_c(tgt_off, i32)), ptr(_c(tgt_idx, i32)),
                                     float(label_smoothing), ptr(parts), nparts, ptr(loss), ptr(H), ptr(dO),

@@ -1,4 +1,4 @@
-"""Filtered-ranking batch (rt_score_rank_fused) at the WN18RR shape: tensor-core path vs fp32 kernel (RT_RANK_TC=0)."""
+"""Filtered-ranking batch (rt_score_rank_fused) at the WN18RR shape, on the path the library picks for it."""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
@@ -13,4 +13,4 @@ for name, scale in (("trained-like logits (std 3)", 3.0 * (N / r) ** 0.5), ("ini
     q = (scale * torch.randn(B, r, generator=g) / r ** 0.5).to(dev)
     pt = ops.target_prob(q, O, tgt)
     ms = timeit(lambda: ops.score_rank_fused(q, O, tgt, pt, off, idx), iters=20)
-    print(f"{name}: {ms:.3f} ms per batch of {B} = {B / ms * 1e3 / 1e6:.2f} M queries/s (RT_RANK_TC={os.environ.get('RT_RANK_TC', '1')})")
+    print(f"{name}: {ms:.3f} ms per batch of {B} = {B / ms * 1e3 / 1e6:.2f} M queries/s")

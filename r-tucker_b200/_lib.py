@@ -90,6 +90,8 @@ PROTOTYPES = {
     "rt_score_bce_v3_supported": (i32, [i32]),
     "rt_score_bce_v3_ws_bytes": (sz, [i32, i32, i32]),
     "rt_score_v3_set_profile": (i32, [vp]),
+    "rt_score_tc_set_profile": (i32, [vp]),
+    "rt_eigh_set_profile": (i32, [vp]),
     "rt_score_bce_v3_phases": (i32, [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, f32, f32, vp, vp, vp, vp, vp, vp, i32]),
     "rt_score_bce_v3": (i32, [vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, f32, f32, vp, vp, vp, vp, vp, vp]),
 }

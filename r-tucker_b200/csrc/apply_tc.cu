@@ -1502,9 +1502,6 @@ extern "C" int rt_score_bce_tc3(const float* q, const float* qp, const float* O,
 }
 
 namespace rt {
-int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
-int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
-
 size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2) { return lse_layout(B, n_local, r2).total; }
 
 int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s) {

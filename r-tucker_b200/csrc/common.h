@@ -85,4 +85,63 @@ __device__ __forceinline__ int warp_sum(int v) {
   return v;
 }
 
+// ---- functions shared between translation units ---------------------------------------------------------------------
+// Each is defined in the file named above its group and called from at least one other.  They return 0 or an error
+// code with rt_last_error() set, like the C ABI, unless they return a size or a flag.
+
+// apply_tc.cu: the logits passes of apply_tc_kernel (3xTF32 tensor cores)
+bool rank_tc_supported(int B, int n_local, int r2);
+size_t rank_tc_ws_bytes(int B, int n_local, int r2);
+int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
+            const float* p_target, const int32_t* flt_off, const int32_t* flt_idx, int32_t* greater, int32_t* equal,
+            int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s, const int** overflow_flag);
+int rank_tc_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
+                  const float* z_target, int32_t* greater, int32_t* equal, int32_t* equal_before, void* ws,
+                  cudaStream_t s, const int** overflow_flag);
+size_t topk_tc_ws_bytes(int B, int n_local, int r2);
+int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
+                 int32_t* seg, int cap, void* ws, cudaStream_t s, bool logit);
+size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2);
+int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s);
+size_t score_ce_tc3_ws_bytes(int B, int n_local, int r2);
+int score_ce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* parts,
+                 int nparts, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s);
+
+// score_bce.cu: exact fp32 probabilities or logits, and the log-sum-exp reductions of the cross-entropy
+int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
+                cudaStream_t s, bool logits);
+int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
+int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
+
+// score_bce_tc.cu: BCE score variant 1 (TF32 tensor cores)
+size_t score_bce_tc_ws_bytes(int B, int n_local, int r2);
+int score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, double* loss_sum,
+                 float* H, float* dO, void* ws, void* stream);
+
+// gram_sym.cu: X^T X on the fp64 tensor cores
+bool gram_sym_supported(int r);
+size_t gram_sym_ws_bytes(int n, int r);
+int gram_sym(const float* X, int64_t ld, int n, int r, double* out, void* ws, cudaStream_t s);
+
+// tallskinny_v2.cu: register-tiled FP32 Gram and factor update
+size_t gram_v2_ws_bytes(int n, int ra, int rb);
+int gram_v2(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int ra, int rb, double* out, void* ws,
+            void* stream);
+int apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0, int64_t ldx0, const double* a0_dev, int nk,
+             const float* const* X_host, const int64_t* ldx_host, const int* rk_host, const double* const* K_host,
+             void* stream);
+
+// eig.cu: batched symmetric eigen-decomposition (block Jacobi)
+int eig_batch(int count, const double* const* A, const int* n, double* const* w, double* const* V, void* const* ws,
+              cudaStream_t s, double stop);
+size_t eig_ws_bytes(int n);
+
+// subspace.cu: batched dominant invariant subspaces
+int subspace_batch(int count, const double* const* N, const int* n, const int* r, double* const* Y, const int* ldy,
+                   void* const* ws, void* shared_ws, int* const* info, cudaStream_t s);
+size_t subspace_ws_bytes(int n, int r);
+size_t subspace_shared_ws_bytes();
+
 }  // namespace rt

@@ -21,16 +21,6 @@
 #include <algorithm>
 #include <math.h>
 
-namespace rt {
-bool rank_tc_supported(int B, int n_local, int r2);
-size_t rank_tc_ws_bytes(int B, int n_local, int r2);
-int rank_tc_logit(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
-                  const float* z_target, int32_t* greater, int32_t* equal, int32_t* equal_before, void* ws,
-                  cudaStream_t s, const int** overflow_flag);
-int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
-                cudaStream_t s, bool logits);
-}  // namespace rt
-
 namespace {
 
 constexpr int kMaxB = 65535, kMaxR2 = 256;

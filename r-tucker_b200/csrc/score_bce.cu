@@ -582,23 +582,9 @@ __global__ void ce_empty_rows_kernel(const int32_t* __restrict__ off, int B, con
 
 }  // namespace
 
-// tcgen05 variant (score_bce_tc.cu)
-extern "C" size_t rt_score_bce_tc_ws_bytes(int B, int n_local, int r2);
-extern "C" int rt_score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2,
-                               int n_begin, int n_local, int n_total, int b_total,
-                               const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
-                               double* loss_sum, float* H, float* dO, void* ws, void* stream);
-
-// warp-specialised fp16 tcgen05 variant (score_bce_v3.cu)
-extern "C" int rt_score_bce_v3_supported(int r2);
-extern "C" size_t rt_score_bce_v3_ws_bytes(int B, int n_local, int r2);
-extern "C" int rt_score_bce_v3(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
-                               int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
-                               float o_absmax_hint, double* loss_sum, float* H, float* dO, float* centre_state, void* ws,
-                               void* stream);
-
+// variant 1: tcgen05 TF32 (score_bce_tc.cu); variant 2: warp-specialised fp16 tcgen05 (score_bce_v3.cu)
 extern "C" size_t rt_score_bce_ws_bytes(int B, int n_local, int r2, int variant) {
-  if (variant == 1) return rt_score_bce_tc_ws_bytes(B, n_local, r2);
+  if (variant == 1) return rt::score_bce_tc_ws_bytes(B, n_local, r2);
   if (variant == 2) return rt_score_bce_v3_ws_bytes(B, n_local, r2);
   Plan p = make_plan(n_local, r2, false);
   return rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256) + (size_t)p.grid * sizeof(double);
@@ -613,8 +599,8 @@ extern "C" int rt_score_bce_fwd_bwd(const float* q, const float* qp, const float
              "rt_score_bce_fwd_bwd: bad shape B=%d r2=%d n_local=%d", B, r2, n_local);
   RT_REQUIRE(ws != nullptr, "rt_score_bce_fwd_bwd: workspace is NULL");
   if (variant == 1)
-    return rt_score_bce_tc(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx,
-                           label_smoothing, loss_sum, H, dO, ws, stream);
+    return rt::score_bce_tc(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx,
+                            label_smoothing, loss_sum, H, dO, ws, stream);
   if (variant == 2) {
     RT_REQUIRE(qp == nullptr || qp == q, "rt_score_bce_fwd_bwd: variant 2 computes dO = G^T q only (pass qp = NULL and "
                "fold the right factor into the following rt_apply)");
@@ -636,13 +622,6 @@ extern "C" int rt_target_prob(const float* q, const float* O, int B, int r2, int
   return 0;
 }
 
-namespace rt {
-bool rank_tc_supported(int B, int n_local, int r2);
-size_t rank_tc_ws_bytes(int B, int n_local, int r2);
-int rank_tc(const float* q, const float* O, int B, int r2, int n_begin, int n_local, const int32_t* target,
-            const float* p_target, const int32_t* flt_off, const int32_t* flt_idx, int32_t* greater, int32_t* equal,
-            int32_t* equal_before, double* bce_sum, void* ws, cudaStream_t s, const int** overflow_flag);
-}  // namespace rt
 __global__ void gated_reduce_loss_kernel(const double* __restrict__ partial, int n, double* __restrict__ out,
                                          const int* __restrict__ gate) {
   if (*gate == 0 || threadIdx.x != 0 || blockIdx.x != 0) return;
@@ -746,12 +725,6 @@ int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cu
   RT_LAUNCH_CHECK();
   return 0;
 }
-size_t score_lse_tc3_ws_bytes(int B, int n_local, int r2);
-int score_lse_tc3(const float* q, const float* O, int B, int r2, int n_local, float* parts, void* ws, cudaStream_t s);
-size_t score_ce_tc3_ws_bytes(int B, int n_local, int r2);
-int score_ce_tc3(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
-                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, const float* parts,
-                 int nparts, double* loss_sum, float* H, float* dO, void* ws, cudaStream_t s);
 }  // namespace rt
 
 static int ce_check_variant(const char* fn, int variant, int B, int n_local, int r2) {

@@ -633,12 +633,12 @@ static TcLayout tc_layout(int B, int n_local, int r2) {
   return L;
 }
 
-extern "C" size_t rt_score_bce_tc_ws_bytes(int B, int n_local, int r2) { return tc_layout(B, n_local, r2).total; }
+namespace rt {
+size_t score_bce_tc_ws_bytes(int B, int n_local, int r2) { return tc_layout(B, n_local, r2).total; }
 
-extern "C" int rt_score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2, int n_begin,
-                               int n_local, int n_total, int b_total, const int32_t* tgt_off,
-                               const int32_t* tgt_idx, float label_smoothing, double* loss_sum, float* H,
-                               float* dO, void* ws, void* stream) {
+int score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
+                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, double* loss_sum,
+                 float* H, float* dO, void* ws, void* stream) {
   RT_REQUIRE(r2 >= 1 && r2 <= 256, "rt_score_bce_tc: r2=%d out of range (1..256)", r2);
   cudaStream_t s = (cudaStream_t)stream;
   const TcLayout L = tc_layout(B, n_local, r2);
@@ -680,6 +680,7 @@ extern "C" int rt_score_bce_tc(const float* q, const float* qp, const float* O, 
   RT_LAUNCH_CHECK();
   return 0;
 }
+}  // namespace rt
 
-// Debug: per-CTA cycle counters of score_tc_kernel ([grid][8] int64), NULL to disable.
+// Debug: per-CTA, per-phase cycle counters of score_tc_kernel ([grid][12] int64), NULL to disable.
 extern "C" int rt_score_tc_set_profile(long long* dev_buf) { g_tc_prof = dev_buf; return 0; }

@@ -781,14 +781,6 @@ extern "C" int rt_score_bce_v3_supported(int r2) { return r2 >= 1 && r2 <= R2P_M
 
 extern "C" size_t rt_score_bce_v3_ws_bytes(int B, int n_local, int r2) { return v3_layout(B, n_local, r2).total; }
 
-// phases: bit 0 = operand scaling + packing, bit 1 = the fused kernel, bit 2 = H / loss reduction.  Running a
-// single phase needs a workspace already prepared by the earlier phases on the same inputs (bench.py times the
-// fused kernel alone this way).
-extern "C" int rt_score_bce_v3_phases(const float* q, const float* O, int B, int r2, int n_begin, int n_local,
-                                      int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx,
-                                      float label_smoothing, float o_absmax_hint, double* loss_sum, float* H, float* dO,
-                                      float* centre_state, void* ws, void* stream, int phases);
-
 extern "C" int rt_score_bce_v3(const float* q, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
                                int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing,
                                float o_absmax_hint, double* loss_sum, float* H, float* dO, float* centre_state, void* ws,
@@ -797,6 +789,9 @@ extern "C" int rt_score_bce_v3(const float* q, const float* O, int B, int r2, in
                                 o_absmax_hint, loss_sum, H, dO, centre_state, ws, stream, 7);
 }
 
+// phases: bit 0 = operand scaling + packing, bit 1 = the fused kernel, bit 2 = H / loss reduction.  Running a
+// single phase needs a workspace already prepared by the earlier phases on the same inputs (bench.py times the
+// fused kernel alone this way).
 extern "C" int rt_score_bce_v3_phases(const float* q, const float* O, int B, int r2, int n_begin, int n_local,
                                       int n_total, int b_total, const int32_t* tgt_off, const int32_t* tgt_idx,
                                       float label_smoothing, float o_absmax_hint, double* loss_sum, float* H, float* dO,

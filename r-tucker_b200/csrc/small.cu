@@ -23,24 +23,12 @@ static double hosvd_stop() {
   return v;
 }
 
-namespace rt {
-int eig_batch(int count, const double* const* A, const int* n, double* const* w, double* const* V,
-              void* const* ws, cudaStream_t s, double stop);
-size_t eig_ws_bytes(int n);
-int subspace_batch(int count, const double* const* N, const int* n, const int* r, double* const* Y, const int* ldy,
-                   void* const* ws, void* shared_ws, int* const* info, cudaStream_t s);
-size_t subspace_ws_bytes(int n, int r);
-size_t subspace_shared_ws_bytes();
-}  // namespace rt
-
 // HOSVD route: 1 (default) = dominant subspaces by purification + Newton-Schulz on the fp64 tensor cores
 // (subspace.cu); 0 = full eigen-decomposition by block Jacobi (eig.cu, round 1).  RT_HOSVD=jacobi selects 0.
 static int hosvd_route() {
   static const int v = [] { const char* e = std::getenv("RT_HOSVD"); return (e && e[0] == 'j') ? 0 : 1; }();
   return v;
 }
-
-extern "C" size_t rt_gram_ws_bytes(int n, int ra, int rb);
 
 namespace {
 using namespace rt::small;
@@ -503,9 +491,6 @@ extern "C" int rt_rows_times_ainv(const float* A, int m, int mode, int r0, int r
   RT_LAUNCH_CHECK();
   return 0;
 }
-
-extern "C" int rt_gram(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int ra, int rb,
-                       double* out, int precise, void* ws, void* stream);
 
 extern "C" int rt_small_grad(const float* core, const float* d_core, const float* qp, const float* H,
                              const float* r_rows, const float* s_rows, const float* dr_rows,

@@ -224,24 +224,11 @@ extern "C" int rt_core_axpby(const float* dS_g, const double* alpha_dev, const f
   return 0;
 }
 
-// register-tiled FP32 kernels (tallskinny_v2.cu): the default for the non-precise Gram and for apply
-extern "C" size_t rt_gram_v2_ws_bytes(int n, int ra, int rb);
-extern "C" int rt_gram_v2(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int ra, int rb,
-                          double* out, void* ws, void* stream);
-extern "C" int rt_apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0, int64_t ldx0, const double* a0_dev,
-                           int nk, const float* const* X_host, const int64_t* ldx_host, const int* rk_host,
-                           const double* const* K_host, void* stream);
-
-namespace rt {
-bool gram_sym_supported(int r);
-size_t gram_sym_ws_bytes(int n, int r);
-int gram_sym(const float* X, int64_t ld, int n, int r, double* out, void* ws, cudaStream_t s);
-}  // namespace rt
-
+// the register-tiled FP32 kernels of tallskinny_v2.cu are the default for the non-precise Gram and for apply
 extern "C" size_t rt_gram_ws_bytes(int n, int ra, int rb) {
   if (n <= 0 || ra <= 0 || rb <= 0) return 0;
   GramPlan p = gram_plan(n, ra, rb);
-  const size_t v1 = (size_t)p.nsplit * ra * rb * sizeof(double), v2 = rt_gram_v2_ws_bytes(n, ra, rb);
+  const size_t v1 = (size_t)p.nsplit * ra * rb * sizeof(double), v2 = rt::gram_v2_ws_bytes(n, ra, rb);
   const size_t v3 = (ra == rb && rt::gram_sym_supported(ra)) ? rt::gram_sym_ws_bytes(n, ra) : 0;
   return std::max(v1, std::max(v2, v3));
 }
@@ -259,7 +246,7 @@ extern "C" int rt_gram(const float* A, int64_t lda, const float* B, int64_t ldb,
   // A^T A (the norm and retraction Grams of a step): upper triangle on the fp64 tensor cores, exact accumulation
   if (A == B && lda == ldb && ra == rb && rt::gram_sym_supported(ra) && n >= 64)
     return rt::gram_sym(A, lda, n, ra, out, ws, s);
-  if (!precise) return rt_gram_v2(A, lda, B, ldb, n, ra, rb, out, ws, stream);
+  if (!precise) return rt::gram_v2(A, lda, B, ldb, n, ra, rb, out, ws, stream);
   GramPlan p = gram_plan(n, ra, rb);
   dim3 grid(p.tiles_a * p.tiles_b, p.nsplit);
   gram_dmma_kernel<<<grid, 256, 0, s>>>(A, lda, B, ldb, n, ra, rb, p.tiles_b, p.rows_per_split, (double*)ws);
@@ -278,5 +265,5 @@ extern "C" int rt_apply(float* Y, int64_t ldy, int n, int rc, const float* X0, i
   RT_REQUIRE(nk >= 0 && nk <= 4, "rt_apply: nk=%d out of range (max 4)", nk);
   RT_REQUIRE(X0 != nullptr || nk > 0, "rt_apply: nothing to compute");
   if (n == 0) return 0;
-  return rt_apply_v2(Y, ldy, n, rc, X0, ldx0, a0_dev, nk, X_host, ldx_host, rk_host, K_host, stream);
+  return rt::apply_v2(Y, ldy, n, rc, X0, ldx0, a0_dev, nk, X_host, ldx_host, rk_host, K_host, stream);
 }

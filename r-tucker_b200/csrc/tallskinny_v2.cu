@@ -261,14 +261,15 @@ apply_v2_kernel(float* __restrict__ Y, int64_t ldy, int n, int rc, const float* 
 
 }  // namespace
 
-extern "C" size_t rt_gram_v2_ws_bytes(int n, int ra, int rb) {
+namespace rt {
+size_t gram_v2_ws_bytes(int n, int ra, int rb) {
   if (n <= 0) return 16;
   GramV2Plan p = gram_v2_plan(n, ra, rb);
   return (size_t)p.nsplit * ra * rb * sizeof(float);
 }
 
-extern "C" int rt_gram_v2(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int ra, int rb,
-                          double* out, void* ws, void* stream) {
+int gram_v2(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int ra, int rb, double* out, void* ws,
+            void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
   if (n == 0) { RT_CHECK_CUDA(cudaMemsetAsync(out, 0, sizeof(double) * ra * rb, s)); return 0; }
   RT_REQUIRE(ws != nullptr, "rt_gram_v2: workspace is NULL");
@@ -284,9 +285,9 @@ extern "C" int rt_gram_v2(const float* A, int64_t lda, const float* B, int64_t l
   return 0;
 }
 
-extern "C" int rt_apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0, int64_t ldx0, const double* a0_dev,
-                           int nk, const float* const* X_host, const int64_t* ldx_host, const int* rk_host,
-                           const double* const* K_host, void* stream) {
+int apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0, int64_t ldx0, const double* a0_dev, int nk,
+             const float* const* X_host, const int64_t* ldx_host, const int* rk_host, const double* const* K_host,
+             void* stream) {
   RT_REQUIRE(nk >= 0 && nk <= kMaxTerms, "rt_apply_v2: nk out of range");
   if (n == 0) return 0;
   ApplyV2Args a{};
@@ -301,3 +302,4 @@ extern "C" int rt_apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0
   RT_LAUNCH_CHECK();
   return 0;
 }
+}  // namespace rt

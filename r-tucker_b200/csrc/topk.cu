@@ -24,15 +24,6 @@
 #include <algorithm>
 #include <math.h>
 
-namespace rt {
-bool rank_tc_supported(int B, int n_local, int r2);
-size_t topk_tc_ws_bytes(int B, int n_local, int r2);
-int topk_tc_pass(const float* q, const float* O, int B, int r2, int n_local, const float* p_k, const int* flag, int* cnt,
-                 int32_t* seg, int cap, void* ws, cudaStream_t s, bool logit);
-int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
-                cudaStream_t s, bool logits);
-}  // namespace rt
-
 namespace {
 
 typedef unsigned long long u64;

@@ -1,21 +1,39 @@
-"""The C-ABI shared library loads on a CPU-only host and exports every symbol include/rtucker.h declares."""
+"""The C-ABI shared library loads on a CPU-only host and exports exactly the symbols include/rtucker.h and
+include/rtucker_debug.h declare, with the ctypes signatures of _lib.PROTOTYPES."""
 import ctypes
 import os
 import re
+import subprocess
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+HEADERS = ("rtucker.h", "rtucker_debug.h")
 
 
-def declared_symbols(headers=("rtucker.h", "rtucker_debug.h")):
+def header_text(h):
+    """One header with its comments stripped."""
+    text = open(os.path.join(ROOT, "include", h)).read()
+    return re.sub(r"/\*.*?\*/", "", text, flags=re.S)
+
+
+def declared_symbols(headers=HEADERS):
     """Entry points of the drop-in boundary (rtucker.h) and of the debug / self-test header (rtucker_debug.h)."""
     syms = set()
     for h in headers:
-        text = open(os.path.join(ROOT, "include", h)).read()
-        text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-        syms |= set(re.findall(r"\b(rt_[a-z0-9_]+)\s*\(", text))
+        syms |= set(re.findall(r"\b(rt_[a-z0-9_]+)\s*\(", header_text(h)))
     return sorted(syms)
+
+
+def declarations():
+    """name -> (return type, [parameter declarations]) of every function the two headers declare."""
+    decls = {}
+    for h in HEADERS:
+        text = re.sub(r"^\s*#.*$", "", header_text(h), flags=re.M)
+        for ret, name, params in re.findall(r"([^;{}()]*?)\b(rt_[a-z0-9_]+)\s*\(([^()]*)\)\s*;", text):
+            params = [" ".join(p.split()) for p in params.split(",")]
+            decls[name] = (" ".join(ret.split()), [] if params == ["void"] else params)
+    return decls
 
 
 def test_debug_entry_points_are_not_in_the_public_header():
@@ -41,9 +59,46 @@ def test_library_exports_every_declared_symbol():
     assert handle.rt_abi_version() == 1
 
 
+def test_library_exports_only_declared_symbols():
+    """Helpers shared between the library's own source files are C++ functions, not exported rt_* symbols."""
+    import rtucker_b200
+    if not os.path.isfile(rtucker_b200.LIB_PATH):
+        pytest.skip("library not built (run __graft_entry__.build())")
+    out = subprocess.run(["nm", "-D", "--defined-only", rtucker_b200.LIB_PATH], check=True, capture_output=True,
+                         text=True).stdout
+    exported = sorted({f[-1] for f in map(str.split, out.splitlines()) if f and f[-1].startswith("rt_")})
+    assert exported == declared_symbols(), sorted(set(exported) ^ set(declared_symbols()))
+
+
 def test_prototypes_cover_the_header():
     from rtucker_b200._lib import PROTOTYPES
     assert sorted(PROTOTYPES) == declared_symbols()
+
+
+SCALARS = {"int": ctypes.c_int, "int32_t": ctypes.c_int, "int64_t": ctypes.c_int64, "size_t": ctypes.c_size_t,
+           "float": ctypes.c_float, "double": ctypes.c_double, "unsigned long long": ctypes.c_ulonglong,
+           "uint64_t": ctypes.c_uint64, "uint32_t": ctypes.c_uint32}
+
+
+def test_prototypes_match_the_headers():
+    """Argument count, scalar types and pointer-ness of every PROTOTYPES entry agree with its header declaration."""
+    from rtucker_b200._lib import PROTOTYPES
+    decls = declarations()
+    assert sorted(decls) == declared_symbols()
+    for name, (ret, params) in decls.items():
+        res, args = PROTOTYPES[name]
+        want_res = ctypes.c_char_p if ret == "const char*" else SCALARS.get(ret)
+        assert want_res is not None, f"{name}: no ctypes mapping for return type {ret!r}"
+        assert res is want_res, f"{name}: returns {ret}, PROTOTYPES says {res.__name__}"
+        assert len(args) == len(params), f"{name}: {len(params)} parameters, PROTOTYPES lists {len(args)}"
+        for i, (p, a) in enumerate(zip(params, args)):
+            if "*" in p:
+                assert a is ctypes.c_void_p or issubclass(a, ctypes._Pointer), \
+                    f"{name} parameter {i} ({p}): pointer, PROTOTYPES says {a.__name__}"
+            else:
+                ctype = p.rsplit(" ", 1)[0]
+                assert ctype in SCALARS, f"{name} parameter {i} ({p}): no ctypes mapping for {ctype!r}"
+                assert a is SCALARS[ctype], f"{name} parameter {i} ({p}): PROTOTYPES says {a.__name__}"
 
 
 def test_no_cpu_fallback():

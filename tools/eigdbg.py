@@ -14,7 +14,7 @@ for n in (20, 400):
     scal=ws[off_scal:off_scal+8*24].view(torch.float64).cpu()
     print(n,'norm2',scal[0].item(),'off per sweep',[f'{x:.1e}' for x in scal[1:21].tolist()],'scale',scal[21].item())
 # per-phase cycle profile
-L = lib(); L.rt_eigh_set_profile.argtypes=[C.c_void_p]; L.rt_eigh_set_profile.restype=C.c_int
+L = lib()
 for n in (20, 400):
     prof=torch.zeros(148*4,dtype=torch.int64,device='cuda')
     L.rt_eigh_set_profile(C.c_void_p(prof.data_ptr()))

@@ -1,7 +1,7 @@
 import sys, torch, ctypes as C
 sys.path.insert(0,'/root/repo')
 from rtucker_b200._lib import lib, ptr, stream_ptr, check
-L = lib(); L.rt_eigh_set_profile.argtypes=[C.c_void_p]; L.rt_eigh_set_profile.restype=C.c_int
+L = lib()
 n=400
 prof=torch.zeros(148*4,dtype=torch.int64,device='cuda')
 X=torch.randn(n,4*n,dtype=torch.float64,device='cuda'); A=(X@X.T).contiguous()

@@ -2,7 +2,7 @@ import sys, torch, ctypes as C
 sys.path.insert(0,'/root/repo')
 from rtucker_b200 import ops
 from rtucker_b200._lib import lib
-L=lib(); L.rt_score_tc_set_profile.argtypes=[C.c_void_p]; L.rt_score_tc_set_profile.restype=C.c_int
+L=lib()
 dev=torch.device('cuda'); N,B,r2=40943,512,200
 q=torch.randn(B,r2,device=dev)/r2**0.5; O=torch.randn(N,r2,device=dev)
 off=torch.arange(0,(B+1)*2,2,device=dev,dtype=torch.int32); idx=torch.randint(0,N,(B*2,),device=dev,dtype=torch.int32)

@@ -390,8 +390,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&v)[8]) {
                : "r"(taddr) : "memory");
 }
 
-__device__ __forceinline__ float rcp_fast(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-
 // HC8 = 8-column groups of the accumulator owned by one epilogue warp (rcp / 16): 13 for r = 200, 16 = any rcp <= 256
 template <int HC8, int MODE = kModeApply>
 __global__ void __launch_bounds__(kThreads, 1)

@@ -133,11 +133,6 @@ int apply_v2(float* Y, int64_t ldy, int n, int rc, const float* X0, int64_t ldx0
              const float* const* X_host, const int64_t* ldx_host, const int* rk_host, const double* const* K_host,
              void* stream);
 
-// eig.cu: batched symmetric eigen-decomposition (block Jacobi)
-int eig_batch(int count, const double* const* A, const int* n, double* const* w, double* const* V, void* const* ws,
-              cudaStream_t s, double stop);
-size_t eig_ws_bytes(int n);
-
 // subspace.cu: batched dominant invariant subspaces
 int subspace_batch(int count, const double* const* N, const int* n, const int* r, double* const* Y, const int* ldy,
                    void* const* ws, void* shared_ws, int* const* info, cudaStream_t s);

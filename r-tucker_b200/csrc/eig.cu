@@ -687,13 +687,13 @@ EigLayout eig_layout(int n) {
   return L;
 }
 
-size_t eig_ws_bytes(int n) { return eig_layout(n).total; }
+static size_t eig_ws_bytes(int n) { return eig_layout(n).total; }
 
 // Solve `count` (<= 4) independent problems in one cooperative launch.
 long long* g_eig_prof = nullptr;   // set through rt_eigh_set_profile (debug)
 
-int eig_batch(int count, const double* const* A, const int* n, double* const* w, double* const* V,
-              void* const* ws, cudaStream_t s, double stop) {
+static int eig_batch(int count, const double* const* A, const int* n, double* const* w, double* const* V,
+                     void* const* ws, cudaStream_t s, double stop) {
   RT_REQUIRE(count >= 1 && count <= kMaxProblems, "eig_batch: count=%d out of range", count);
   EigBatch b{};
   b.count = count;

@@ -5,8 +5,8 @@
 // (call sites src/model/asymmetric/optim.py:89, symmetric/optim.py:83), `TangentVector.norm`
 // (asymmetric/optim.py:90), `project` (asymmetric/optim.py:86) and the core part of
 // `construct().round(rank)` (asymmetric/optim.py:108) -- the latter as the structured HOSVD of
-// SURVEY.md App. A.5 (Cholesky of the W_i Grams, block-structured rank-2r core, eigenvectors of the
-// unfolding Grams by block Jacobi) instead of QR(N x 2r) + SVD(2r_i x prod 2r_j).
+// SURVEY.md App. A.5 (Cholesky of the W_i Grams, block-structured rank-2r core, dominant invariant
+// subspaces of the unfolding Grams, subspace.cu) instead of QR(N x 2r) + SVD(2r_i x prod 2r_j).
 //
 // Everything here costs O(poly(r)) and is replicated on every GPU of an entity-sharded run.
 #include "small_kernels.cuh"
@@ -15,37 +15,23 @@
 #include <algorithm>
 #include <vector>
 
-#include <cstdlib>
-// Stop criterion of the HOSVD eigenproblems (off-diagonal mass SEEN in a sweep, relative to ||A||_F^2).
-// RT_HOSVD_STOP overrides it for experiments.
-static double hosvd_stop() {
-  static const double v = [] { const char* e = std::getenv("RT_HOSVD_STOP"); return e ? std::atof(e) : 1e-10; }();
-  return v;
-}
-
-// HOSVD route: 1 (default) = dominant subspaces by purification + Newton-Schulz on the fp64 tensor cores
-// (subspace.cu); 0 = full eigen-decomposition by block Jacobi (eig.cu, round 1).  RT_HOSVD=jacobi selects 0.
-static int hosvd_route() {
-  static const int v = [] { const char* e = std::getenv("RT_HOSVD"); return (e && e[0] == 'j') ? 0 : 1; }();
-  return v;
-}
-
 namespace {
 using namespace rt::small;
 using rt::align_up;
 using rt::cdiv;
 
 constexpr int kNumT = 8;          // core-sized fp64 temporaries
-constexpr int kMaxSplitCtas = 592;
-constexpr int kDotBlocks = 296;
 constexpr int kMinDotSlots = 2048;
+// Arena of the executor's split-K partial sums: 592 tiles of 64 x 64 doubles.  Ctx::gemm_any splits a GEMM over K only
+// when its partials fit here, so this size fixes the order of the sums: changing it changes results in the last bits.
+constexpr size_t kPartialArenaBytes = (size_t)592 * 64 * 64 * sizeof(double);
 
 struct Layout {
   int r[3];
   int B;
   int64_t c;  // r0*r1*r2
-  size_t C64, Gm[3], Ainv[3], coresq, Tn[kNumT], KC[3], Nn[3], Vf[3], Wv[3], GL[3], GLinv[3], Gs[3],
-      tmpM[3], tmpK[3], eig[3], sub[3], sub_shared, exec_bar, gemm_partial, gram_ws, dot_partial, scal, total;
+  size_t C64, Gm[3], Ainv[3], coresq, Tn[kNumT], KC[3], Nn[3], Vf[3], GL[3], GLinv[3], Gs[3],
+      tmpM[3], tmpK[3], sub[3], sub_shared, exec_bar, gemm_partial, gram_ws, dot_partial, scal, total;
   int dot_slots;  // doubles at dot_partial: one per kEwChunk elements of the dots recorded between two flushes
 };
 
@@ -64,18 +50,16 @@ Layout make_layout(int r0, int r1, int r2, int B) {
     L.KC[i] = take(2 * r * r);
     L.Nn[i] = take(4 * r * r);
     L.Vf[i] = take(4 * r * r);
-    L.Wv[i] = take(2 * r);
     L.GL[i] = take(r * r);
     L.GLinv[i] = take(r * r);
     L.Gs[i] = take(r * r);
     L.tmpM[i] = take(2 * r * r);
     L.tmpK[i] = take(2 * r * r);
-    size_t at = o; o += align_up(rt::eig_ws_bytes(2 * (int)r), 256); L.eig[i] = at;
-    at = o; o += align_up(rt::subspace_ws_bytes(2 * (int)r, (int)r), 256); L.sub[i] = at;
+    size_t at = o; o += align_up(rt::subspace_ws_bytes(2 * (int)r, (int)r), 256); L.sub[i] = at;
   }
   { size_t at = o; o += align_up(rt::subspace_shared_ws_bytes(), 256); L.sub_shared = at; }
   L.exec_bar = take(32);
-  L.gemm_partial = take((size_t)kMaxSplitCtas * GT * GT);
+  L.gemm_partial = take(kPartialArenaBytes / sizeof(double));
   int rmax = r0 > r1 ? r0 : r1; rmax = rmax > r2 ? rmax : r2;
   { size_t at = o; o += align_up(rt_gram_ws_bytes(B > 0 ? B : 1, rmax, rmax), 256); L.gram_ws = at; }
   // The largest dots (rt_small_norm) are one over the core and one over each r_i x r_i Gram, recorded together;
@@ -95,7 +79,19 @@ Layout make_layout(int r0, int r1, int r2, int B) {
 struct Range { const char* lo; const char* hi; };
 struct Rec { Op op; Range rd[4]; int nrd; Range wr[2]; int nwr; };
 
-constexpr size_t kPartialArenaBytes = (size_t)kMaxSplitCtas * GT * GT * sizeof(double);
+// C[m,n] = alpha * sum_{k1<K1,k2<K2} A[m,(k1,k2)] B[(k1,k2),n] + beta * C[m,n]      (batched): what Ctx::mode_prod and
+// Ctx::unfold_gram hand to Ctx::gemm
+template <typename T>
+struct GemmT {
+  const T* A; const T* B; T* C;
+  int m, n, K1, K2;
+  int64_t a_m, a_k1, a_k2;
+  int64_t b_k1, b_k2, b_n;
+  int64_t c_m, c_n;
+  int batch; int64_t a_b, b_b, c_b;
+  double alpha, beta;
+  int sym;                  // C is symmetric (A = B with equal strides): compute the upper triangle of tiles only
+};
 
 template <typename T> struct DT;
 template <> struct DT<float> { static constexpr int v = DT_F32; };
@@ -313,7 +309,6 @@ struct Ctx {
   void to32plain(const double* x, float* y, int64_t n) { cvt(x, DT_F64, y, DT_F32, n); }
   void scale32(const float* x, float* y, int64_t n, double a_host, const double* a_dev) { cvt(x, DT_F32, y, DT_F32, n, a_host, a_dev); }
   void to64(const float* x, double* y, int64_t n) { cvt(x, DT_F32, y, DT_F64, n); }
-  void to32(const double* x, float* y, int64_t n, double a_host, const double* a_dev) { cvt(x, DT_F64, y, DT_F32, n, a_host, a_dev); }
   void axpby(const double* x, const double* y, double* z, int64_t n, double a, const double* a_dev,
              double b, const double* b_dev) {
     ew(EW_AXPBY64, x, DT_F64, n * 8, y, n * 8, z, DT_F64, n * 8, n, a, a_dev, b, b_dev);
@@ -399,9 +394,8 @@ struct Ctx {
     if (smem > smem_limit || nmax > 256) {
       rt::set_error("small stage: rank %d exceeds the in-shared-memory Cholesky limit (230)", nmax); return 2; }
     // tensor-core phases need one more [8][n] block; the largest ranks keep the plain fp64 path
-    static const bool dmma_off = getenv("RT_SPD_DMMA") && atoi(getenv("RT_SPD_DMMA")) == 0;
     SpdBatch bb = b;
-    bb.dmma = (!dmma_off && smem + (size_t)SPD_NB * nmax * sizeof(double) <= smem_limit) ? 1 : 0;
+    bb.dmma = (smem + (size_t)SPD_NB * nmax * sizeof(double) <= smem_limit) ? 1 : 0;
     if (bb.dmma) smem += (size_t)SPD_NB * nmax * sizeof(double);
     if (cudaFuncSetAttribute(spd_blocked_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
       rt::set_error("small stage: cannot raise shared memory to %zu", smem); return 1; }
@@ -679,21 +673,12 @@ extern "C" int rt_small_retract(const float* core, const float* dS_dir, const do
   if (sym) c.axpby(Nn[1], Nn[2], Nn[1], 4 * (int64_t)d[1] * d[1], 1.0, nullptr, 1.0, nullptr);
   c.flush();
   if (c.err) return finish(c, "rt_small_retract");
-  if (hosvd_route() == 1) {
-    const double* Ain[3]; int nn[3]; int rr[3]; int ldy[3]; double* Yv[3]; void* sws[3];
-    for (int i = 0; i < nm; ++i) {
-      Ain[i] = Nn[i]; nn[i] = 2 * d[i]; rr[i] = d[i]; ldy[i] = 2 * d[i]; Yv[i] = c.p(c.L.Vf[i]);
-      sws[i] = c.base + c.L.sub[i];
-    }
-    if ((rc = rt::subspace_batch(nm, Ain, nn, rr, Yv, ldy, sws, c.base + c.L.sub_shared, nullptr, s))) return rc;
-  } else {
-    const double* Ain[3]; int nn[3]; double* wv[3]; double* Vv[3]; void* ews[3];
-    for (int i = 0; i < nm; ++i) {
-      Ain[i] = Nn[i]; nn[i] = 2 * d[i]; wv[i] = c.p(c.L.Wv[i]); Vv[i] = c.p(c.L.Vf[i]);
-      ews[i] = c.base + c.L.eig[i];
-    }
-    if ((rc = rt::eig_batch(nm, Ain, nn, wv, Vv, ews, s, hosvd_stop()))) return rc;   // see eig.cu
+  const double* Ain[3]; int nn[3]; int rr[3]; int ldy[3]; double* Yv[3]; void* sws[3];
+  for (int i = 0; i < nm; ++i) {
+    Ain[i] = Nn[i]; nn[i] = 2 * d[i]; rr[i] = d[i]; ldy[i] = 2 * d[i]; Yv[i] = c.p(c.L.Vf[i]);
+    sws[i] = c.base + c.L.sub[i];
   }
+  if ((rc = rt::subspace_batch(nm, Ain, nn, rr, Yv, ldy, sws, c.base + c.L.sub_shared, nullptr, s))) return rc;
   // Y_i = V_i[:, :r_i]  (2r_i x r_i, row stride 2r_i);  W_i = Y_i^T = [Y_ia^T | Y_ib^T]
   const double* Y[3] = {c.p(c.L.Vf[0]), c.p(c.L.Vf[1]), c.p(c.L.Vf[sym ? 1 : 2])};
   // core_new = T x_i Y_i^T through the block structure, in fp32 (the output is fp32): fp32 images of C', B_k

@@ -1,232 +1,12 @@
-// Device kernels of the N-independent ("small") stage: generic strided fp64 GEMM with a two-level
-// K index (covers mode products and unfolding Grams of r0 x r1 x r2 tensors without permuting
-// them), SPD factorisation / inverse, small elementwise helpers.  Internal to small.cu.
+// Device kernels of the N-independent ("small") stage that small.cu launches directly, outside the recorded
+// executor of small_exec.cuh: the SPD factorisation / inverse, and the rows-times-inverse product of
+// rt_rows_times_ainv.  Internal to small.cu.
 #pragma once
 #include "common.h"
 #include <math.h>
 
 namespace rt {
 namespace small {
-
-// C[m,n] = alpha * sum_{k1<K1,k2<K2} A[m,(k1,k2)] B[(k1,k2),n] + beta * C[m,n]      (batched)
-template <typename T>
-struct GemmT {
-  const T* A; const T* B; T* C;
-  int m, n, K1, K2;
-  int64_t a_m, a_k1, a_k2;
-  int64_t b_k1, b_k2, b_n;
-  int64_t c_m, c_n;
-  int batch; int64_t a_b, b_b, c_b;
-  double alpha, beta;
-  int ksplit, k_per_split;  // split over the flattened K (batch == 1 only)
-  T* partial;               // [ksplit][m][n] when ksplit > 1
-  int sym;                  // C is symmetric (A = B with equal strides): compute the upper triangle of tiles only
-};
-using Gemm = GemmT<double>;
-
-constexpr int GT = 64, GK = 16;
-
-template <typename T>
-__global__ void __launch_bounds__(256)
-gemm64_kernel(GemmT<T> g) {
-  __shared__ T As[GK][GT + 2];
-  __shared__ T Bs[GK][GT + 2];
-  const int m0 = blockIdx.x * GT, n0 = blockIdx.y * GT;
-  int z = blockIdx.z, split = 0, bidx = 0;
-  if (g.ksplit > 1) split = z; else bidx = z;
-  const T* A = g.A + (int64_t)bidx * g.a_b;
-  const T* B = g.B + (int64_t)bidx * g.b_b;
-  const int K = g.K1 * g.K2;
-  const int kbeg = split * g.k_per_split;
-  const int kend = (g.ksplit > 1) ? min(K, kbeg + g.k_per_split) : K;
-  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  const bool a_lanes_m = (g.a_m == 1);   // lanes along m when m is the contiguous index
-  const bool b_lanes_n = (g.b_n == 1);
-  T acc[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = (T)0;
-  // software pipeline: the global loads of chunk k0+GK are in flight while chunk k0 is multiplied
-  T va[(GT * GK) / 256], vb[(GT * GK) / 256];
-  auto load_chunk = [&](int k0) {
-#pragma unroll
-    for (int it = 0; it < (GT * GK) / 256; ++it) {
-      const int e = it * 256 + threadIdx.x;
-      int rr, kk;
-      if (a_lanes_m) { kk = e / GT; rr = e % GT; } else { rr = e / GK; kk = e % GK; }
-      int k = k0 + kk;
-      T v = (T)0;
-      if (m0 + rr < g.m && k < kend) {
-        const int k1 = k / g.K2, k2 = k - k1 * g.K2;
-        v = A[(int64_t)(m0 + rr) * g.a_m + (int64_t)k1 * g.a_k1 + (int64_t)k2 * g.a_k2];
-      }
-      va[it] = v;
-      int cc, kb;
-      if (b_lanes_n) { kb = e / GT; cc = e % GT; } else { cc = e / GK; kb = e % GK; }
-      k = k0 + kb;
-      v = (T)0;
-      if (n0 + cc < g.n && k < kend) {
-        const int k1 = k / g.K2, k2 = k - k1 * g.K2;
-        v = B[(int64_t)k1 * g.b_k1 + (int64_t)k2 * g.b_k2 + (int64_t)(n0 + cc) * g.b_n];
-      }
-      vb[it] = v;
-    }
-  };
-  if (kbeg < kend) load_chunk(kbeg);
-  for (int k0 = kbeg; k0 < kend; k0 += GK) {
-#pragma unroll
-    for (int it = 0; it < (GT * GK) / 256; ++it) {
-      const int e = it * 256 + threadIdx.x;
-      int rr, kk, cc, kb;
-      if (a_lanes_m) { kk = e / GT; rr = e % GT; } else { rr = e / GK; kk = e % GK; }
-      if (b_lanes_n) { kb = e / GT; cc = e % GT; } else { cc = e / GK; kb = e % GK; }
-      As[kk][rr] = va[it];
-      Bs[kb][cc] = vb[it];
-    }
-    __syncthreads();
-    if (k0 + GK < kend) load_chunk(k0 + GK);
-#pragma unroll
-    for (int kk = 0; kk < GK; ++kk) {
-      T a[4], b[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] = As[kk][ty + 16 * i];
-#pragma unroll
-      for (int j = 0; j < 4; ++j) b[j] = Bs[kk][tx + 16 * j];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = fma(a[i], b[j], acc[i][j]);
-    }
-    __syncthreads();
-  }
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int mm = m0 + ty + 16 * i;
-    if (mm >= g.m) continue;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int nn = n0 + tx + 16 * j;
-      if (nn >= g.n) continue;
-      if (g.ksplit > 1) {
-        g.partial[((int64_t)split * g.m + mm) * g.n + nn] = acc[i][j];
-      } else {
-        T* c = g.C + (int64_t)bidx * g.c_b + (int64_t)mm * g.c_m + (int64_t)nn * g.c_n;
-        *c = (T)g.alpha * acc[i][j] + (g.beta != 0.0 ? (T)g.beta * (*c) : (T)0);
-      }
-    }
-  }
-}
-
-// LANES threads per output element: lane l sums the splits l, l + LANES, ... in index order, then the lanes are
-// combined by a fixed xor tree -- a fixed order whatever the schedule, hence deterministic.  LANES = 1: consecutive
-// threads read consecutive elements of each partial slab.  LANES = 32 is for the tiny outputs of very long
-// contractions (e.g. 10 x 10 from K = 10^5, 278 splits): one thread per element walked the 278 slabs as one
-// dependent chain of L2 round trips and fp64 additions (60 us under ncu, six times per step).
-template <typename T, int LANES>
-__global__ void gemm64_reduce_kernel(GemmT<T> g) {
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  const int64_t e = t / LANES;
-  const int lane = (int)(t % LANES);
-  const int64_t mn = (int64_t)g.m * g.n;
-  const bool live = e < mn;                   // a whole group of LANES threads is live or not (blockDim % LANES == 0)
-  T s = (T)0;
-  if (live) {
-#pragma unroll 4
-    for (int k = lane; k < g.ksplit; k += LANES) s += g.partial[(int64_t)k * mn + e];
-  }
-#pragma unroll
-  for (int o = LANES / 2; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
-  if (live && lane == 0) {
-    const int mm = (int)(e / g.n), nn = (int)(e - (int64_t)mm * g.n);
-    T* c = g.C + (int64_t)mm * g.c_m + (int64_t)nn * g.c_n;
-    *c = (T)g.alpha * s + (g.beta != 0.0 ? (T)g.beta * (*c) : (T)0);
-  }
-}
-
-// ---- elementwise helpers ----------------------------------------------------------------
-__global__ void f32_to_f64_kernel(const float* __restrict__ x, double* __restrict__ y, int64_t n) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    y[i] = (double)x[i];
-}
-// y(f32) = a * x(f64), a = a_host * (a_dev ? *a_dev : 1)
-__global__ void f64_to_f32_scaled_kernel(const double* __restrict__ x, float* __restrict__ y, int64_t n,
-                                         double a_host, const double* __restrict__ a_dev) {
-  const double a = a_host * (a_dev ? *a_dev : 1.0);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    y[i] = (float)(a * x[i]);
-}
-// z = a*x + b*y (fp64), scalars = host * optional device factor
-__global__ void axpby64_kernel(const double* __restrict__ x, const double* __restrict__ y,
-                               double* __restrict__ z, int64_t n, double a_host,
-                               const double* __restrict__ a_dev, double b_host,
-                               const double* __restrict__ b_dev) {
-  const double a = a_host * (a_dev ? *a_dev : 1.0);
-  const double b = b_host * (b_dev ? *b_dev : 1.0);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    z[i] = a * x[i] + (y ? b * y[i] : 0.0);
-}
-// out(f64) = x32 - lr * y32   (lr from device)
-__global__ void core_minus_lr_kernel(const float* __restrict__ x, const float* __restrict__ y,
-                                     const double* __restrict__ lr, double* __restrict__ out, int64_t n) {
-  const double l = *lr;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    out[i] = (double)x[i] - l * (double)y[i];
-}
-// dS_g(f32) = d_core + 2*reg*core
-__global__ void grad_core_kernel(const float* __restrict__ d_core, const float* __restrict__ core,
-                                 const double* __restrict__ hyper, float* __restrict__ out, int64_t n) {
-  const float two_reg = (float)(2.0 * hyper[1]);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    out[i] = fmaf(two_reg, core[i], d_core[i]);
-}
-
-__global__ void f64_to_f32_kernel(const double* __restrict__ x, float* __restrict__ y, int64_t n) {
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    y[i] = (float)x[i];
-}
-// dst[i, j] (ld ldd) = (float) src[i, j] (ld lds) for i < rows, j < cols
-__global__ void f64_to_f32_strided_kernel(const double* __restrict__ src, int64_t lds, float* __restrict__ dst,
-                                          int64_t ldd, int rows, int cols) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= rows * cols) return;
-  const int i = e / cols, j = e - i * cols;
-  dst[(int64_t)i * ldd + j] = (float)src[(int64_t)i * lds + j];
-}
-// y(f32) = a * x(f32), a = a_host * (a_dev ? *a_dev : 1)
-__global__ void scale_f32_kernel(const float* __restrict__ x, float* __restrict__ y, int64_t n, double a_host,
-                                 const double* __restrict__ a_dev) {
-  const float a = (float)(a_host * (a_dev ? *a_dev : 1.0));
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    y[i] = a * x[i];
-}
-
-// Deterministic two-stage sum of squares / dot product.  stage 1: grid partials; stage 2: 1 block.
-template <typename TA, typename TB>
-__global__ void dot_partial_kernel(const TA* __restrict__ x, const TB* __restrict__ y, int64_t n,
-                                   double* __restrict__ partial) {
-  __shared__ double red[8];
-  double s = 0.0;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-    s += (double)x[i] * (double)y[i];
-  s = rt::warp_sum(s);
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double t = 0.0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) t += red[w];
-    partial[blockIdx.x] = t;
-  }
-}
-// out[0] = scale * sum(partial) (+ out[0] if accumulate)
-__global__ void dot_final_kernel(const double* __restrict__ partial, int n, double scale,
-                                 double* __restrict__ out, int accumulate) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    double s = 0.0;
-    for (int i = 0; i < n; ++i) s += partial[i];
-    out[0] = (accumulate ? out[0] : 0.0) + scale * s;
-  }
-}
 
 // C(f32)[m, r] = A(f32)[m, r] . K(f64)[r, r]
 __global__ void __launch_bounds__(256)
@@ -256,34 +36,7 @@ rows_times_mat_kernel(const float* __restrict__ A, int m, int r, const double* _
   }
 }
 
-// dst[a, b] (row stride ldd) = src[b, a]  for an n x n matrix
-__global__ void transpose_into_kernel(const double* __restrict__ src, int n, double* __restrict__ dst, int64_t ldd) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n * n) return;
-  const int a = e / n, b = e - a * n;
-  dst[(int64_t)a * ldd + b] = src[(int64_t)b * n + a];
-}
-
-// lower -> full symmetric
-__global__ void symmetrize_lower_kernel(double* A, int n) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n * n) return;
-  const int i = e / n, j = e - i * n;
-  if (j > i) A[e] = A[(int64_t)j * n + i];
-}
-
-// out = scale_host * (*scale_dev)^pow * in   (pow in {1,2})
-__global__ void scale_mat_kernel(const double* __restrict__ in, double* __restrict__ out, int n,
-                                 double scale_host, const double* __restrict__ scale_dev, int pow2) {
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= n) return;
-  double s = scale_host;
-  if (scale_dev) s *= pow2 ? (*scale_dev) * (*scale_dev) : (*scale_dev);
-  out[e] = s * in[e];
-}
-
 // ---- SPD factorisation: G = L L^T (packed in smem), Linv = L^-1, Ginv = Linv^T Linv ---------
-// One CTA per problem.  Pivots <= tol * max diag are treated as zero (pseudo-inverse on the rest).
 struct SpdProblem {
   const double* G;   // [n][n]
   double* L;         // [n][n] lower (may be NULL)
@@ -303,10 +56,12 @@ __device__ __forceinline__ double spd_sum8(const double (&c)[8][2], int e) {
   return ((c[0][e] + c[1][e]) + (c[2][e] + c[3][e])) + ((c[4][e] + c[5][e]) + (c[6][e] + c[7][e]));
 }
 
-// Blocked variant (what the small stage launches): same contract and the same zero-pivot semantics as
-// spd_factor_kernel below, but ~10x fewer block barriers.  Two threads per matrix row.
+// One CTA per problem of the batch.  It reads G, symmetrised as (G + G^T) / 2, and writes each of L, Linv and Ginv that
+// is not NULL as a full n x n row-major matrix: the lower Cholesky factor with G = L L^T, its lower-triangular inverse
+// L^-1, and G^-1 = Linv^T Linv.  A pivot <= 1e-12 x the largest diagonal entry of G counts as zero: that column of L
+// and that row and column of Linv are zero, so Ginv inverts G on the other columns only.
 //   Cholesky, left looking in blocks of 8 columns: (1) every row subtracts the contribution of all earlier
-//   columns from its 8 block entries (the 8 "pivot rows" are broadcast reads), (2) one thread factors the 8x8
+//   columns from its 8 block entries (the 8 "pivot rows" are broadcast reads), (2) warp 0 factors the 8x8
 //   diagonal block, (3) every row below solves its 8 entries against that block.
 //   Inverse, in blocks of 8 rows: the rows of L are staged, then thread group j produces column j of the 8 new rows
 //   of L^-1 from its own (already inverted) column above.
@@ -681,99 +436,6 @@ spd_blocked_kernel(SpdBatch batch) {
 #ifdef RT_SPD_PROF
   if (tid == 0) printf("spd n=%d inverse %lld write Linv %lld Ginv %lld\n", n, t_a, t_b, t_c);
 #endif
-}
-
-__global__ void __launch_bounds__(1024, 1)
-spd_factor_kernel(SpdBatch batch) {
-  extern __shared__ double sm[];
-  const SpdProblem P = batch.p[blockIdx.x];
-  const int n = P.n;
-  if (n <= 0) return;
-  double* Lp = sm;                       // packed lower n(n+1)/2
-  double* col = sm + n * (n + 1) / 2;    // [n] scratch column
-  __shared__ double s_piv, s_maxd;
-  const int tid = threadIdx.x, nt = blockDim.x;
-  for (int e = tid; e < n * (n + 1) / 2; e += nt) {
-    // invert pk: find i with i(i+1)/2 <= e
-    int i = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
-    while (i * (i + 1) / 2 > e) --i;
-    while ((i + 1) * (i + 2) / 2 <= e) ++i;
-    const int j = e - i * (i + 1) / 2;
-    Lp[e] = 0.5 * (P.G[(int64_t)i * n + j] + P.G[(int64_t)j * n + i]);
-  }
-  __syncthreads();
-  if (tid == 0) {
-    double m = 0.0;
-    for (int i = 0; i < n; ++i) m = fmax(m, Lp[pk(i, i)]);
-    s_maxd = m;
-  }
-  __syncthreads();
-  const double tol = 1e-12 * s_maxd;
-  for (int k = 0; k < n; ++k) {
-    if (tid == 0) {
-      const double d = Lp[pk(k, k)];
-      s_piv = (d > tol) ? sqrt(d) : 0.0;
-    }
-    __syncthreads();
-    const double piv = s_piv;
-    const double inv = piv > 0.0 ? 1.0 / piv : 0.0;
-    for (int i = k + tid; i < n; i += nt) {
-      const double v = (i == k) ? piv : Lp[pk(i, k)] * inv;
-      Lp[pk(i, k)] = v;
-      col[i] = v;
-    }
-    __syncthreads();
-    // trailing update: rows i > k, cols k < j <= i  (warp w takes rows k+1+w, +32, ...; lanes run along j)
-    {
-      const int w = tid >> 5, ln = tid & 31, nw = nt >> 5;
-      for (int i = k + 1 + w; i < n; i += nw) {
-        const double ci = col[i];
-        for (int j = k + 1 + ln; j <= i; j += 32) Lp[pk(i, j)] -= ci * col[j];
-      }
-    }
-    __syncthreads();
-  }
-  if (P.L) {
-    for (int e = tid; e < n * n; e += nt) {
-      const int i = e / n, j = e - i * n;
-      P.L[e] = (j <= i) ? Lp[pk(i, j)] : 0.0;
-    }
-  }
-  if (!P.Linv && !P.Ginv) return;
-  __syncthreads();
-  // in-place inverse of the packed lower triangle (column by column from the right, dtrti2 style)
-  const int sub = tid & 3, row_t = tid >> 2;  // 4 threads per row
-  for (int j = n - 1; j >= 0; --j) {
-    const double d = Lp[pk(j, j)];
-    const double dinv = d > 0.0 ? 1.0 / d : 0.0;
-    for (int i = j + 1 + tid; i < n; i += nt) col[i] = Lp[pk(i, j)];
-    __syncthreads();
-    for (int i0 = j + 1; i0 < n; i0 += nt / 4) {
-      const int i = i0 + row_t;
-      double s = 0.0;
-      if (i < n)
-        for (int k = j + 1 + sub; k <= i; k += 4) s += Lp[pk(i, k)] * col[k];
-      s += __shfl_xor_sync(0xffffffffu, s, 1);
-      s += __shfl_xor_sync(0xffffffffu, s, 2);
-      if (i < n && sub == 0) Lp[pk(i, j)] = -s * dinv;
-    }
-    if (tid == 0) Lp[pk(j, j)] = dinv;
-    __syncthreads();
-  }
-  if (P.Linv) {
-    for (int e = tid; e < n * n; e += nt) {
-      const int i = e / n, j = e - i * n;
-      P.Linv[e] = (j <= i) ? Lp[pk(i, j)] : 0.0;
-    }
-  }
-  if (P.Ginv) {
-    for (int e = tid; e < n * n; e += nt) {
-      const int i = e / n, j = e - i * n;
-      double s = 0.0;
-      for (int k = (i > j ? i : j); k < n; ++k) s += Lp[pk(k, i)] * Lp[pk(k, j)];
-      P.Ginv[e] = s;
-    }
-  }
 }
 
 }  // namespace small

@@ -80,7 +80,6 @@ __global__ void core_axpby_kernel(const float* __restrict__ x, const double* __r
 // ------------------------------------------------------------------------------------------
 constexpr int GT = 64;       // output tile edge
 constexpr int GKC = 32;      // rows per smem chunk
-constexpr int GFLUSH = 8;    // chunks accumulated in fp32 before flushing to fp64
 
 // Exact Gram A^T B for A != B (A^T A takes gram_sym.cu): 64 x 64 tiles, two-stage fixed-order reduction; the products of two fp32
 // values are exact in fp64 and accumulated in fp64 by mma.sync m8n8k4 (DMMA).  A CTA owns a 64 x 64 output tile over

@@ -151,8 +151,6 @@ __device__ __forceinline__ void bulk_s2g_add_f32(void* dst, const void* src_smem
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;\n" ::: "memory"); }
 template <int N>
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;\n" :: "n"(N) : "memory"); }
-template <int N>
 __device__ __forceinline__ void bulk_wait() { asm volatile("cp.async.bulk.wait_group %0;\n" :: "n"(N) : "memory"); }
 
 // byte offset of element (row, col) of a 16-bit array in the interleaved format: 8 rows x 16 bytes

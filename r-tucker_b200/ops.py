@@ -2,7 +2,6 @@
 and the current CUDA stream only; all arithmetic happens in librtucker_b200.so.
 """
 import ctypes as C
-import os
 
 import torch
 
@@ -269,8 +268,7 @@ def score_ce_fwd_bwd(q, qp, O, tgt_off, tgt_idx, label_smoothing, parts, n_total
 # ---------------------------------------------------------------- (c) tall-skinny
 # The N x r x r passes run on tcgen05 (3xTF32 with round-to-nearest partial-sum accumulation: fp32 accuracy, see
 # csrc/apply_tc.cu) whenever the shape is wide enough to fill an MMA tile; thin ranks (d_e = 20) and short factors
-# (the relation factor) stay on the fp32 FFMA kernels.  RT_TALLSKINNY_TC=0 forces the FFMA kernels everywhere.
-USE_TENSOR_CORES = os.environ.get("RT_TALLSKINNY_TC", "1") == "1"
+# (the relation factor) stay on the fp32 FFMA kernels.
 TC_MIN_ROWS, TC_MIN_WIDTH = 1024, 64
 
 
@@ -291,7 +289,7 @@ def gram(A, B, out=None, ws=None, precise=False):
 def apply_tc_ok(n, rc, rks):
     """True when Y[n,rc] = ... + sum X_k[n,rk] K_k runs on the tcgen05 kernel (apply_multi)."""
     nk = len(rks)
-    if not (USE_TENSOR_CORES and 1 <= nk <= 4 and n >= TC_MIN_ROWS and rc >= TC_MIN_WIDTH):
+    if not (1 <= nk <= 4 and n >= TC_MIN_ROWS and rc >= TC_MIN_WIDTH):
         return False
     return bool(lib().rt_apply_tc_supported(rc, nk, (C.c_int * nk)(*rks)))
 

@@ -93,7 +93,7 @@ def core_axpby(dS_g, alpha_dev, pS_beta, out=None):
 
 def chol_psd(G, tol=1e-12):
     """Unpivoted Cholesky of a PSD matrix; pivots <= tol*max(diag) become zero columns (as the
-    spd_factor_kernel of csrc/small_kernels.cuh does).  Returns (L, Linv) with the matching
+    spd_blocked_kernel of csrc/small_kernels.cuh does).  Returns (L, Linv) with the matching
     rows/columns of Linv zeroed (inverse on the non-degenerate part)."""
     n = G.shape[0]
     A = 0.5 * (G + G.T).clone()

@@ -1,6 +1,7 @@
 """The C-ABI shared library loads on a CPU-only host and exports exactly the symbols include/rtucker.h and
 include/rtucker_debug.h declare, with the ctypes signatures of _lib.PROTOTYPES."""
 import ctypes
+import glob
 import os
 import re
 import subprocess
@@ -99,6 +100,20 @@ def test_prototypes_match_the_headers():
                 ctype = p.rsplit(" ", 1)[0]
                 assert ctype in SCALARS, f"{name} parameter {i} ({p}): no ctypes mapping for {ctype!r}"
                 assert a is SCALARS[ctype], f"{name} parameter {i} ({p}): PROTOTYPES says {a.__name__}"
+
+
+def test_every_kernel_is_referenced():
+    """Every __global__ function in csrc/ is named somewhere besides its own definition: a kernel nothing launches
+    still compiles into the library and reads as a live path."""
+    text = ""
+    for ext in ("cu", "cuh", "h"):
+        for path in sorted(glob.glob(os.path.join(ROOT, "r-tucker_b200", "csrc", "*." + ext))):
+            text += re.sub(r"//[^\n]*|/\*.*?\*/", "", open(path).read(), flags=re.S) + "\n"
+    text = re.sub(r"__launch_bounds__\s*\([^()]*\)", "", text)
+    definitions = re.findall(r"__global__\s[^;{}()]*?\b(\w+)\s*\(", text)
+    unreferenced = sorted(k for k in set(definitions)
+                          if len(re.findall(r"\b%s\b" % k, text)) <= definitions.count(k))
+    assert not unreferenced, "never referenced: " + " ".join(unreferenced)
 
 
 def test_no_cpu_fallback():

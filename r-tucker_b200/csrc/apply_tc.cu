@@ -156,7 +156,6 @@ __global__ void pack_K_kernel(PackArgs a) {
 #define PROF_PRINT(role)
 #endif
 
-__device__ __forceinline__ float ex2_fast(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ float lg2_fast(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 // ---- filtered-ranking epilogue of 8 columns (queries) of one thread's row (entity) --------------------------------
 // NOT inlined: the epilogue of a tile is 128 columns per thread, and as one unrolled block it was ~30 000 instructions
@@ -228,10 +227,10 @@ __device__ __noinline__ RankChunkOut rank_chunk8(const RankChunkCtx& cx, int c0,
       // -log(1 - p) with the reference's fp32 semantics: for z >= 0 through the fp32 probability itself (1 - p
       // is quantised to multiples of 2^-24 there: up to 0.35 per element near saturation, 2e-4 of a batch's
       // BCE), p == 1 from z = 24 ln 2 on (BCELoss clamps log(1 - p) at -100); for z < 0 log(1 + e^z)
-      const float en = ex2_fast(-1.4426950408889634f * fabsf(z));
+      const float en = rt::ex2_approx(-rt::kLog2e * fabsf(z));
       const float sden = 1.0f + en;
       const bool pos = z >= 0.0f;                                      // branch-free: both signs share every warp
-      const float lg = 0.6931471805599453f * lg2_fast(pos ? 1.0f - __frcp_rn(sden) : sden);
+      const float lg = rt::kLn2 * lg2_fast(pos ? 1.0f - __frcp_rn(sden) : sden);
       float sp = pos ? -lg : lg;
       sp = (!pos && en < 1e-3f) ? en * (1.0f - 0.5f * en) : sp;
       sp = (pos && z >= 16.635532f) ? 100.0f : sp;
@@ -242,7 +241,7 @@ __device__ __noinline__ RankChunkOut rank_chunk8(const RankChunkCtx& cx, int c0,
 }
 
 // ---- score epilogue of 8 columns (queries) of one thread's row (entity): G[e][b] = dBCE/dz and the BCE itself for
-//      ALL-NEGATIVE targets (t = t_neg), with the reference's fp32 semantics (score_bce.cu: p = 1 / (1 + expf(-z)), log
+//      ALL-NEGATIVE targets (t = t_neg), with the reference's fp32 semantics (exact.cuh: p = 1 / (1 + expf(-z)), log
 //      terms clamped at -100, gradient scaled by p (1 - p) / max(p (1 - p), 1e-12)); the sparse positives are fixed up
 //      afterwards.  Not inlined for the same reason as rank_chunk8 (instruction footprint of 128 unrolled columns). ----
 __device__ __noinline__ float score_chunk8(float* __restrict__ gdst, bool rv, int ncols, float tn, float inv, float z0, float z1,
@@ -255,14 +254,14 @@ __device__ __noinline__ float score_chunk8(float* __restrict__ gdst, bool rv, in
     const float z = zs[u];
     // three special-function operations per element (ex2, rcp, lg2), BRANCH-FREE (the two signs of z share every warp:
     // as if / else both sides ran for every element)
-    const float en = ex2_fast(-1.4426950408889634f * fabsf(z));                      // e^-|z|
+    const float en = rt::ex2_approx(-rt::kLog2e * fabsf(z));                                 // e^-|z|
     const float sden = 1.0f + en;
     const float rq = __frcp_rn(sden);                                                 // 1 / (1 + e^-|z|)
     const bool pos = z >= 0.0f;
     // z >= 0: p in [0.5, 1] is the fp32 quotient, 1 - p is exact, log(1 - p) from it (p == 1 from z = 24 ln 2 on);
     // z <  0: p = e^z / (1 + e^z), log(1 - p) = -log(1 + e^z) (series for tiny e^z)
     const float p = pos ? rq : en * rq;
-    const float lg = 0.6931471805599453f * lg2_fast(pos ? 1.0f - rq : sden);
+    const float lg = rt::kLn2 * lg2_fast(pos ? 1.0f - rq : sden);
     float lq = pos ? lg : -lg;
     lq = (!pos && en < 1e-3f) ? -(en * (1.0f - 0.5f * en)) : lq;
     lq = (pos && z >= 16.635532f) ? -100.0f : lq;
@@ -322,7 +321,7 @@ __device__ __noinline__ void lse_chunk8(float2* __restrict__ dst, bool rv, int n
     const int key = on ? (bits >= 0 ? bits : bits ^ 0x7fffffff) : INT_MIN;
     const int mk = __reduce_max_sync(0xffffffffu, key);
     m[u] = mk == INT_MIN ? -INFINITY : __int_as_float(mk >= 0 ? mk : mk ^ 0x7fffffff);
-    e[u] = on ? ex2_fast((zs[u] - m[u]) * 1.4426950408889634f) : 0.0f;
+    e[u] = on ? rt::ex2_approx((zs[u] - m[u]) * rt::kLog2e) : 0.0f;
   }
   const bool b4 = lane & 16, b3 = lane & 8, b2 = lane & 4;
   float v[4], w[2];
@@ -354,9 +353,9 @@ __device__ __noinline__ float ce_chunk8(float* __restrict__ gdst, const float* _
 #pragma unroll
   for (int u = 0; u < 8; ++u) {
     const float d = zs[u] - M[u];
-    const float p = ex2_fast(fmaf(d, 1.4426950408889634f, -L[u]));
+    const float p = rt::ce_softmax(d, L[u]);
     const bool on = rv && u < ncols;
-    if (on) lsum += tn * fmaf(L[u], 0.6931471805599453f, -d);
+    if (on) lsum += rt::ce_loss_term(tn, d, L[u]);
     gv[u] = on ? (p - tn) * inv : 0.0f;
   }
   if (rv) {
@@ -519,7 +518,7 @@ apply_tc_kernel(const __grid_constant__ Args a) {
         lacc += (double)lsum;
       } else if (MODE == kModeScore) {
         // ---- score epilogue: G[e][b] = dBCE/dz and the BCE itself for ALL-NEGATIVE targets (t = t_neg), with the
-        //      reference's fp32 semantics (score_bce.cu: p = 1 / (1 + expf(-z)), log terms clamped at -100, gradient
+        //      reference's fp32 semantics (exact.cuh: p = 1 / (1 + expf(-z)), log terms clamped at -100, gradient
         //      scaled by p (1 - p) / max(p (1 - p), 1e-12)); the sparse positives are fixed up afterwards ----
         const int e_loc = (tile - J.tile0) * TM + quarter * 32 + lane;
         const bool rv = e_loc < J.n;
@@ -862,11 +861,9 @@ Plan make_plan(int rc) {
 // thresholds derived from the target's probability: above `hi` the entity certainly has p > p_t, below `lo`
 // certainly p < p_t, above `eqlo` (only when p_t == 1) certainly p == 1 == p_t.  Everything in between -- a few
 // entities per query -- goes to a candidate list and is recomputed by rank_candidates_kernel with the EXACT fp32
-// arithmetic of the dense path (k ascending, one fmaf accumulator, 1 / (1 + expf(-z))), so the counts equal the ones
-// the fp32 kernel produces.  Filtered entities are corrected from their exact probabilities afterwards.
+// arithmetic of the dense path (exact.cuh), so the counts equal the ones the fp32 kernel produces.  Filtered entities
+// are corrected from their exact probabilities afterwards.
 // ---------------------------------------------------------------------------------------------------------------
-using rt::exact_logit;
-using rt::sigmoid_ref;
 
 // max_j ||O_j||^2 over the shard (bounds the error of a logit); out is a float bit pattern updated with atomicMax
 __global__ void rank_rownorm_kernel(const float* __restrict__ O, int n_local, int r2, unsigned int* out,
@@ -976,8 +973,8 @@ __global__ void rank_candidates_kernel(const float* __restrict__ q, const float*
     const int2 c = cand[i];
     const int j = n_begin + c.x, b = c.y, t = __ldg(target + b);
     if (j == t) continue;
-    const float z = exact_logit(q + (int64_t)b * r2, O + (int64_t)c.x * r2, r2);
-    const float p = LOGIT ? z : sigmoid_ref(z);
+    const float z = rt::exact_logit(q + (int64_t)b * r2, O + (int64_t)c.x * r2, r2);
+    const float p = LOGIT ? z : rt::sigmoid_ref(z);
     const float pt = __ldg(p_target + b);
     if (p > pt) atomicAdd(greater + b, 1);
     else if (p == pt) { atomicAdd(equal + b, 1); if (j < t) atomicAdd(equal_before + b, 1); }
@@ -1002,9 +999,9 @@ __global__ void rank_filter_fix_kernel(const float* __restrict__ q, const float*
     if (fl < 0 || fl >= n_local) continue;
     const int t = __ldg(target + b);
     const float pt = __ldg(p_target + b);
-    const float z = exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2);
-    const float p = sigmoid_ref(z);
-    const float lp = fmaxf(logf(p), -100.0f), lq = fmaxf(log1pf(-p), -100.0f);
+    const float z = rt::exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2);
+    const float p = rt::sigmoid_ref(z);
+    const float lp = rt::bce_log_p(p), lq = rt::bce_log_q(p);
     dl += (double)(-lp) - (double)(-lq);              // the pass over all entities charged -log(1 - p)
     if (f != t) {
       const int was_eq = (p == pt), is_eq = (0.0f == pt);
@@ -1336,11 +1333,10 @@ __global__ void score_fix_positives_kernel(const float* __restrict__ q, const fl
   for (int i = __ldg(off + b) + lane; i < __ldg(off + b + 1); i += 32) {
     const int fl = __ldg(idx + i) - n_begin;
     if (fl < 0 || fl >= n_local) continue;
-    const float z = exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2);
-    const float p = sigmoid_ref(z);
-    const float lp = fmaxf(logf(p), -100.0f), lq = fmaxf(log1pf(-p), -100.0f);
-    const float pq = (1.0f - p) * p;
-    G[(int64_t)fl * ldg + b] = (p - t_pos) / fmaxf(pq, 1e-12f) * inv_count * pq;
+    const float z = rt::exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2);
+    const float p = rt::sigmoid_ref(z);
+    const float lp = rt::bce_log_p(p), lq = rt::bce_log_q(p);
+    G[(int64_t)fl * ldg + b] = rt::bce_grad(p, t_pos, inv_count);
     dl += -(double)(t_pos - t_neg) * ((double)lp - (double)lq);     // the kernel charged the negative-target term
   }
   dl = rt::warp_sum(dl);
@@ -1361,8 +1357,8 @@ __global__ void score_ce_fix_positives_kernel(const float* __restrict__ q, const
   for (int i = e0 + lane; i < e1; i += 32) {
     const int fl = __ldg(idx + i) - n_begin;
     if (fl < 0 || fl >= n_local) continue;
-    const float d = exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2) - M;
-    const float p = ex2_fast(fmaf(d, 1.4426950408889634f, -L2));
+    const float d = rt::exact_logit(q + (int64_t)b * r2, O + (int64_t)fl * r2, r2) - M;
+    const float p = rt::ce_softmax(d, L2);
     G[(int64_t)fl * ldg + b] = (p - (tp + t_neg)) * inv_count;
     dl += (double)tp * ((double)L2 * 0.6931471805599453 - (double)d);   // the epilogue charged the ls/N part
   }

@@ -15,6 +15,7 @@
 // H_chunk += G O_tile (accumulated in this CTA's private workspace slice, summed over CTAs in a
 // fixed order afterwards)  and  dO_tile += G^T QP_chunk (registers, across the chunk loop).
 #include "common.h"
+#include "exact.cuh"
 #include <math.h>
 
 namespace {
@@ -29,6 +30,54 @@ __host__ __device__ inline int row_ld(int r2, int cpt) {
   int w = r2 > 16 * cpt ? r2 : 16 * cpt;
   w = (w + 3) / 4 * 4;
   return ((w / 4) & 1) ? w : w + 4;
+}
+
+// Dynamic shared memory of one staged 64-entity + 64-query tile (stage_logit_tile).
+size_t logit_tile_smem(int r2) { return (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float); }
+
+// The logits of the staged tiles (pitch ldw, zero padded beyond r2): z[i][j] = q_b . O_n for query row ty + 16 i and
+// entity row tx + 16 j, one fmaf accumulator, k ascending -- the order of exact_logit, the padding adds exact zeros.
+// k_end = r2 rounded up to a multiple of 4, computed by the caller outside its tile loops.
+struct LogitTile { float z[4][4]; };
+__device__ __forceinline__ LogitTile logit_tile(const float* Qs, const float* Os, int ldw, int k_end) {
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  LogitTile t;
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) t.z[i][j] = 0.0f;
+  for (int k = 0; k < k_end; k += 4) {
+    float4 qv[4], ov[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) qv[i] = *reinterpret_cast<const float4*>(Qs + (ty + 16 * i) * ldw + k);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) ov[j] = *reinterpret_cast<const float4*>(Os + (tx + 16 * j) * ldw + k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        t.z[i][j] = fmaf(qv[i].x, ov[j].x, t.z[i][j]);
+        t.z[i][j] = fmaf(qv[i].y, ov[j].y, t.z[i][j]);
+        t.z[i][j] = fmaf(qv[i].z, ov[j].z, t.z[i][j]);
+        t.z[i][j] = fmaf(qv[i].w, ov[j].w, t.z[i][j]);
+      }
+  }
+  return t;
+}
+
+// Stages entities [n0, n0 + 64) and queries [b0, b0 + 64) in smem (logit_tile_smem bytes) and returns their logits.
+__device__ __forceinline__ LogitTile stage_logit_tile(const float* __restrict__ q, const float* __restrict__ O, int B,
+                                                      int r2, int n_local, int n0, int b0, unsigned char* smem) {
+  const int ldw = row_ld(r2, 1);
+  float* Os = reinterpret_cast<float*>(smem);
+  float* Qs = Os + NT * ldw;
+  for (int e = threadIdx.x; e < NT * ldw; e += 256) {
+    const int rr = e / ldw, cc = e - rr * ldw;
+    Os[e] = (n0 + rr < n_local && cc < r2) ? __ldg(O + (int64_t)(n0 + rr) * r2 + cc) : 0.0f;
+    Qs[e] = (b0 + rr < B && cc < r2) ? __ldg(q + (int64_t)(b0 + rr) * r2 + cc) : 0.0f;
+  }
+  __syncthreads();
+  return logit_tile(Qs, Os, ldw, (r2 + 3) / 4 * 4);
 }
 
 struct ScoreArgs {
@@ -72,9 +121,6 @@ __device__ __forceinline__ void gemm_k64(const float* __restrict__ Gk, const flo
     }
   }
 }
-
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-constexpr float kLog2e = 1.4426950408889634f, kLn2 = 0.6931471805599453f;
 
 // CE (1-N softmax cross-entropy) reuses ScoreArgs: p_target = row statistics [2][B] (max logit M_b, log2 S_b of the
 // whole batch row, see ce_row_stats_kernel), t_pos = 1 - ls, t_neg = ls / n_total, inv_count = 1 / B_total.
@@ -140,28 +186,8 @@ score_kernel(ScoreArgs a) {
           if (m) atomicOr(&mask[rr], m);
         }
       }
-      // ---- GEMM1: Z[b][n], b = ty + 16 i, n = tx + 16 j; k ascending, single accumulator ----
-      float z[4][4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) z[i][j] = 0.0f;
-      for (int k = 0; k < k_end; k += 4) {
-        float4 qv[4], ov[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) qv[i] = *reinterpret_cast<const float4*>(Qs + (ty + 16 * i) * ldw + k);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) ov[j] = *reinterpret_cast<const float4*>(Os + (tx + 16 * j) * ldw + k);
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            z[i][j] = fmaf(qv[i].x, ov[j].x, z[i][j]);
-            z[i][j] = fmaf(qv[i].y, ov[j].y, z[i][j]);
-            z[i][j] = fmaf(qv[i].z, ov[j].z, z[i][j]);
-            z[i][j] = fmaf(qv[i].w, ov[j].w, z[i][j]);
-          }
-      }
+      // ---- GEMM1: Z[b][n], b = ty + 16 i, n = tx + 16 j ----
+      const LogitTile lt = logit_tile(Qs, Os, ldw, k_end);
       __syncthreads();  // mask complete
       // ---- elementwise ----
       float loss_t = 0.0f;
@@ -185,23 +211,22 @@ score_kernel(ScoreArgs a) {
           const int cc = tx + 16 * j;
           const bool valid = (b < a.B) && (n0 + cc < a.n_local);
           const bool pos = (m >> cc) & 1ull;
-          const float zz = z[i][j];
+          const float zz = lt.z[i][j];
           if (CE) {
             // G = (softmax - t) / B_total with softmax = 2^((z - M) log2e - log2 S); loss += t (lse - z)
             const float t = pos ? tpos : a.t_neg;
             float g = 0.0f;
             if (valid) {
               const float d = zz - rowM;
-              g = (ex2_approx(fmaf(d, kLog2e, -rowL)) - t) * a.inv_count;
-              loss_t += t * fmaf(rowL, kLn2, -d);
+              g = (rt::ce_softmax(d, rowL) - t) * a.inv_count;
+              loss_t += rt::ce_loss_term(t, d, rowL);
             }
             Gz[rr * GLD + cc] = g;
             GzT[cc * GLD + rr] = g;
             continue;
           }
-          const float p = 1.0f / (1.0f + expf(-zz));
-          const float lp = fmaxf(logf(p), -100.0f);
-          const float lq = fmaxf(log1pf(-p), -100.0f);
+          const float p = rt::sigmoid_ref(zz);
+          const float lp = rt::bce_log_p(p), lq = rt::bce_log_q(p);
           if (EVAL) {
             const float t = pos ? 1.0f : 0.0f;
             if (valid) {
@@ -219,8 +244,7 @@ score_kernel(ScoreArgs a) {
             float g = 0.0f;
             if (valid) {
               loss_t -= t * lp + (1.0f - t) * lq;
-              const float pq = (1.0f - p) * p;
-              g = (p - t) / fmaxf(pq, 1e-12f) * a.inv_count * pq;
+              g = rt::bce_grad(p, t, a.inv_count);
             }
             Gz[rr * GLD + cc] = g;
             GzT[cc * GLD + rr] = g;
@@ -321,19 +345,13 @@ __global__ void target_prob_kernel(const float* __restrict__ q, const float* __r
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int t = target[b] - n_begin;
-  float p = 0.0f;
-  if (t >= 0 && t < n_local) {
-    float z = 0.0f;  // same order as the tile kernel: k ascending, one accumulator
-    for (int k = 0; k < r2; ++k) z = fmaf(q[(int64_t)b * r2 + k], O[(int64_t)t * r2 + k], z);
-    p = 1.0f / (1.0f + expf(-z));
-  }
-  p_target[b] = p;
+  const bool local = t >= 0 && t < n_local;
+  p_target[b] = local ? rt::sigmoid_ref(rt::exact_logit(q + (int64_t)b * r2, O + (int64_t)t * r2, r2)) : 0.0f;
 }
 
 // Dense compatibility path: P[b, j] = sigmoid(q_b . O_j) written out (what score_fn(T) returns in
-// the reference, R_TuckER.py:47-48).  Same staging and k order as score_kernel, so the values are
-// bit-identical to the ones the fused kernels see.  gate (may be NULL): the launch is a no-op unless
-// *gate != 0 (the exact passes of the top-k selection, topk.cu, and of the logit-space ranking, rank_logit.cu).
+// the reference, R_TuckER.py:47-48).  gate (may be NULL): the launch is a no-op unless *gate != 0 (the exact
+// passes of the top-k selection, topk.cu, and of the logit-space ranking, rank_logit.cu).
 // LOGIT: the logits z themselves (rt_score_dense_logits).
 template <bool LOGIT = false>
 __global__ void __launch_bounds__(256)
@@ -341,39 +359,9 @@ score_dense_kernel(const float* __restrict__ q, const float* __restrict__ O, int
                    float* __restrict__ P, int64_t ldp, const int* __restrict__ gate) {
   if (gate && *gate == 0) return;
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int ldw = row_ld(r2, 1);
-  const int k_end = (r2 + 3) / 4 * 4;
-  float* Os = reinterpret_cast<float*>(smem_raw);
-  float* Qs = Os + NT * ldw;
   const int n0 = blockIdx.x * NT, b0 = blockIdx.y * BT;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  for (int e = threadIdx.x; e < NT * ldw; e += 256) {
-    const int rr = e / ldw, cc = e - rr * ldw;
-    Os[e] = (n0 + rr < n_local && cc < r2) ? __ldg(O + (int64_t)(n0 + rr) * r2 + cc) : 0.0f;
-    Qs[e] = (b0 + rr < B && cc < r2) ? __ldg(q + (int64_t)(b0 + rr) * r2 + cc) : 0.0f;
-  }
-  __syncthreads();
-  float z[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) z[i][j] = 0.0f;
-  for (int k = 0; k < k_end; k += 4) {
-    float4 qv[4], ov[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) qv[i] = *reinterpret_cast<const float4*>(Qs + (ty + 16 * i) * ldw + k);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) ov[j] = *reinterpret_cast<const float4*>(Os + (tx + 16 * j) * ldw + k);
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        z[i][j] = fmaf(qv[i].x, ov[j].x, z[i][j]);
-        z[i][j] = fmaf(qv[i].y, ov[j].y, z[i][j]);
-        z[i][j] = fmaf(qv[i].z, ov[j].z, z[i][j]);
-        z[i][j] = fmaf(qv[i].w, ov[j].w, z[i][j]);
-      }
-  }
+  const LogitTile lt = stage_logit_tile(q, O, B, r2, n_local, n0, b0, smem_raw);
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int b = b0 + ty + 16 * i;
@@ -381,7 +369,7 @@ score_dense_kernel(const float* __restrict__ q, const float* __restrict__ O, int
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int n = n0 + tx + 16 * j;
-      if (n < n_local) P[(int64_t)b * ldp + n] = LOGIT ? z[i][j] : 1.0f / (1.0f + expf(-z[i][j]));
+      if (n < n_local) P[(int64_t)b * ldp + n] = LOGIT ? lt.z[i][j] : rt::sigmoid_ref(lt.z[i][j]);
     }
   }
 }
@@ -455,14 +443,14 @@ int score_train_ffma(const float* q, const float* qp, const float* O, int B, int
 }
 
 // ---- 1-N softmax cross-entropy, FFMA path: the log-sum-exp pass --------------------------------------------------
-// Tile of 64 queries x 64 entities per CTA with score_dense_kernel's staging and k order (the logits are bit-identical
-// to the ones score_kernel<., false, true> sees).  Per query row and tile: m = the largest logit, s = sum exp(z - m)
-// (online max: no fixed shift can keep every term of a trained query from underflowing), written to part[tile][b].
+// Tile of 64 queries x 64 entities per CTA, the logits of score_dense_kernel.  Per query row and tile: m = the largest
+// logit, s = sum exp(z - m) (online max: no fixed shift can keep every term of a trained query from underflowing),
+// written to part[tile][b].
 __device__ __forceinline__ void lse_merge(float& m, float& s, float m2, float s2) {
   if (m2 == -INFINITY) return;
   if (m == -INFINITY) { m = m2; s = s2; return; }
   const float mn = fmaxf(m, m2);
-  s = s * ex2_approx((m - mn) * kLog2e) + s2 * ex2_approx((m2 - mn) * kLog2e);
+  s = s * rt::ex2_approx((m - mn) * rt::kLog2e) + s2 * rt::ex2_approx((m2 - mn) * rt::kLog2e);
   m = mn;
 }
 
@@ -470,49 +458,19 @@ __global__ void __launch_bounds__(256)
 score_lse_kernel(const float* __restrict__ q, const float* __restrict__ O, int B, int r2, int n_local,
                  float2* __restrict__ part) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  const int ldw = row_ld(r2, 1);
-  const int k_end = (r2 + 3) / 4 * 4;
-  float* Os = reinterpret_cast<float*>(smem_raw);
-  float* Qs = Os + NT * ldw;
   const int n0 = blockIdx.x * NT, b0 = blockIdx.y * BT;
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-  for (int e = threadIdx.x; e < NT * ldw; e += 256) {
-    const int rr = e / ldw, cc = e - rr * ldw;
-    Os[e] = (n0 + rr < n_local && cc < r2) ? __ldg(O + (int64_t)(n0 + rr) * r2 + cc) : 0.0f;
-    Qs[e] = (b0 + rr < B && cc < r2) ? __ldg(q + (int64_t)(b0 + rr) * r2 + cc) : 0.0f;
-  }
-  __syncthreads();
-  float z[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) z[i][j] = 0.0f;
-  for (int k = 0; k < k_end; k += 4) {
-    float4 qv[4], ov[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) qv[i] = *reinterpret_cast<const float4*>(Qs + (ty + 16 * i) * ldw + k);
-#pragma unroll
-    for (int j = 0; j < 4; ++j) ov[j] = *reinterpret_cast<const float4*>(Os + (tx + 16 * j) * ldw + k);
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        z[i][j] = fmaf(qv[i].x, ov[j].x, z[i][j]);
-        z[i][j] = fmaf(qv[i].y, ov[j].y, z[i][j]);
-        z[i][j] = fmaf(qv[i].z, ov[j].z, z[i][j]);
-        z[i][j] = fmaf(qv[i].w, ov[j].w, z[i][j]);
-      }
-  }
+  const LogitTile lt = stage_logit_tile(q, O, B, r2, n_local, n0, b0, smem_raw);
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int b = b0 + ty + 16 * i;
     float m = -INFINITY, s = 0.0f;
 #pragma unroll
     for (int j = 0; j < 4; ++j)
-      if (n0 + tx + 16 * j < n_local) m = fmaxf(m, z[i][j]);
+      if (n0 + tx + 16 * j < n_local) m = fmaxf(m, lt.z[i][j]);
 #pragma unroll
     for (int j = 0; j < 4; ++j)
-      if (n0 + tx + 16 * j < n_local) s += ex2_approx((z[i][j] - m) * kLog2e);
+      if (n0 + tx + 16 * j < n_local) s += rt::ex2_approx((lt.z[i][j] - m) * rt::kLog2e);
     // the 16 lanes of this row: butterfly (merge is commutative, so every lane ends with the same bits)
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) {
@@ -683,7 +641,7 @@ namespace rt {
 int score_dense(const float* q, const float* O, int B, int r2, int n_local, float* P, int64_t ldp, const int* gate,
                 cudaStream_t s, bool logits) {
   if (B == 0 || n_local == 0) return 0;
-  const size_t smem = (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float);
+  const size_t smem = logit_tile_smem(r2);
   dim3 grid(rt::cdiv(n_local, NT), rt::cdiv(B, BT));
   if (logits) {
     RT_CHECK_CUDA(cudaFuncSetAttribute(score_dense_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -752,7 +710,7 @@ extern "C" int rt_score_lse(const float* q, const float* O, int B, int r2, int n
   const int n_tiles = rt::cdiv(n_local, NT);
   float2* part = (float2*)ws;
   if (n_tiles > 0) {
-    const size_t smem = (size_t)(NT + BT) * row_ld(r2, 1) * sizeof(float);
+    const size_t smem = logit_tile_smem(r2);
     RT_CHECK_CUDA(rt::ensure_dyn_smem((const void*)score_lse_kernel, smem));
     score_lse_kernel<<<dim3(n_tiles, rt::cdiv(B, BT)), 256, smem, s>>>(q, O, B, r2, n_local, part);
     RT_LAUNCH_CHECK();

@@ -102,18 +102,37 @@ def test_prototypes_match_the_headers():
                 assert a is SCALARS[ctype], f"{name} parameter {i} ({p}): PROTOTYPES says {a.__name__}"
 
 
+def csrc_sources():
+    """file name -> text with comments stripped, for every .cu, .cuh and .h under csrc/."""
+    sources = {}
+    for ext in ("cu", "cuh", "h"):
+        for path in sorted(glob.glob(os.path.join(ROOT, "r-tucker_b200", "csrc", "*." + ext))):
+            sources[os.path.basename(path)] = re.sub(r"//[^\n]*|/\*.*?\*/", "", open(path).read(), flags=re.S)
+    return sources
+
+
 def test_every_kernel_is_referenced():
     """Every __global__ function in csrc/ is named somewhere besides its own definition: a kernel nothing launches
     still compiles into the library and reads as a live path."""
-    text = ""
-    for ext in ("cu", "cuh", "h"):
-        for path in sorted(glob.glob(os.path.join(ROOT, "r-tucker_b200", "csrc", "*." + ext))):
-            text += re.sub(r"//[^\n]*|/\*.*?\*/", "", open(path).read(), flags=re.S) + "\n"
+    text = "\n".join(csrc_sources().values())
     text = re.sub(r"__launch_bounds__\s*\([^()]*\)", "", text)
     definitions = re.findall(r"__global__\s[^;{}()]*?\b(\w+)\s*\(", text)
     unreferenced = sorted(k for k in set(definitions)
                           if len(re.findall(r"\b%s\b" % k, text)) <= definitions.count(k))
     assert not unreferenced, "never referenced: " + " ".join(unreferenced)
+
+
+def test_exact_score_arithmetic_is_written_once():
+    """The element arithmetic that the dense, fused and recheck kernels must share bit for bit (accurate sigmoid,
+    clamped BCE logs, guarded BCE gradient, ex2.approx of the softmax) is spelled out only in exact.cuh.  The fp16
+    score variant (score_bce_v3.cu) keeps its own approximate ex2."""
+    rules = {"log1pf(": r"\blog1pf\(", "fmaxf(.., 1e-12f)": r"\bfmaxf\([^();]*\b1e-12f",
+             "expf(-": r"(?<!\w)expf\(\s*-", "ex2.approx": r"ex2\.approx"}
+    found = {rule: sorted(f for f, text in csrc_sources().items() if re.search(pattern, text))
+             for rule, pattern in rules.items()}
+    for rule in ("log1pf(", "fmaxf(.., 1e-12f)", "expf(-"):
+        assert found[rule] == ["exact.cuh"], (rule, found[rule])
+    assert len([f for f in found["ex2.approx"] if f != "score_bce_v3.cu"]) <= 1, found["ex2.approx"]
 
 
 def test_no_cpu_fallback():

@@ -161,6 +161,15 @@ int rt_query_fwd(const float* core, const float* r_rows, const float* s_rows,
 int rt_query_bwd(const float* core, const float* r_rows, const float* s_rows, const float* H,
                  int B, int r0, int r1, int r2,
                  float* d_core, float* ds_rows, float* dr_rows, void* ws, void* stream);
+/* t[b,:] = core x_2 s_rows[b] x_3 o_rows[b]: t[b,a] = sum_{i,j} core[a,i,j] s_rows[b,i] o_rows[b,j]  [B, r0].
+ * The relation-mode query of relation prediction (s, ?, o): z_bm = R[m] . t_b scores every relation, so the
+ * entity-side ranking, top-k and log-sum-exp entry points take t as the query rows and the relation factor as O.
+ * Reads the core in place (no permuted copy).  Bit-identical to rt_query_fwd on core permuted to (r1, r2, r0)
+ * with (s_rows, o_rows) in place of (r_rows, s_rows): same products, same split plan, same summation order.
+ * Deterministic; B == 0 launches nothing. */
+size_t rt_pair_ws_bytes(int B, int r0, int r1, int r2);
+int rt_pair_fwd(const float* core, const float* s_rows, const float* o_rows,
+                int B, int r0, int r1, int r2, float* t, void* ws, void* stream);
 
 /* ---- (b) fused 1-N score + sigmoid + label-smoothed BCE + backward ------------------- */
 /*

@@ -5,6 +5,8 @@
 //   reduces it; here q[b,:] = sum_{a,i} r[b,a] s[b,i] core[a,i,:] is ONE GEMM whose left operand
 //   r[b,a]*s[b,i] is generated on the fly (never stored), K = r0*r1, split-K for occupancy.
 // Backward is what autograd would compute for those two lines.
+// Pair contraction (relation prediction, (s, ?, o)): t[b,a] = sum_{i,j} core[a,i,j] s[b,i] o[b,j], the same GEMM with
+// K = r1*r2, the left operand s[b,i]*o[b,j] generated on the fly and the core read in place (no permuted copy).
 //
 // FP32 FFMA, deterministic (split partials reduced in a fixed order).
 // Flops: fwd 2*B*r0*r1*r2, bwd 3x that.  Bytes: core once per pass (L2 resident) + rows.
@@ -86,6 +88,44 @@ query_fwd_kernel(const float* __restrict__ core, const float* __restrict__ r_row
     for (int j = 0; j < 4; ++j) {
       const int jj = j0 + tx * 4 + j;
       if (jj < r2) partial[((int64_t)split * B + b) * r2 + jj] = acc[i][j];
+    }
+  }
+}
+
+// ---- pair contraction: partial[split][b][a] = sum_{k=(i,j) in split} s[b,i] o[b,j] core[a*K + k] ---------
+// The relation-mode query of (s, ?, o).  Same loop as query_fwd_kernel run on the core permuted to (r1, r2, r0), with
+// the permutation folded into the B operand's addressing (lanes along K: core[a, :, :] is contiguous in k), so the
+// products and the order they are added in are those of rt_query_fwd on that permuted core.
+__global__ void __launch_bounds__(256)
+pair_fwd_kernel(const float* __restrict__ core, const float* __restrict__ s_rows,
+                const float* __restrict__ o_rows, int B, int r0, int r1, int r2, int k_per_split,
+                float* __restrict__ partial) {
+  __shared__ Smem As, Bs;
+  const int b0 = blockIdx.x * T, a0 = blockIdx.y * T, split = blockIdx.z;
+  const int K = r1 * r2;
+  const int kbeg = split * k_per_split, kend = min(K, kbeg + k_per_split);
+  float acc[4][4];
+  zero_acc(acc);
+  auto la = [&](int rr, int k) -> float {
+    const int b = b0 + rr;
+    if (b >= B) return 0.0f;
+    const int i = k / r2, j = k - i * r2;
+    return __ldg(s_rows + (int64_t)b * r1 + i) * __ldg(o_rows + (int64_t)b * r2 + j);
+  };
+  auto lb = [&](int k, int cc) -> float {
+    const int a = a0 + cc;
+    return (a < r0) ? __ldg(core + (int64_t)a * K + k) : 0.0f;
+  };
+  tile_mainloop<true, false>(kbeg, kend, la, lb, acc, As, Bs);
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int b = b0 + ty * 4 + i;
+    if (b >= B) continue;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int a = a0 + tx * 4 + j;
+      if (a < r0) partial[((int64_t)split * B + b) * r0 + a] = acc[i][j];
     }
   }
 }
@@ -254,6 +294,29 @@ extern "C" int rt_query_fwd(const float* core, const float* r_rows, const float*
   RT_LAUNCH_CHECK();
   const int64_t count = (int64_t)B * r2;
   reduce_splits_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>((const float*)ws, p.ksplit, count, q);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+
+// The forward split plan of the permuted core (r1, r2, r0): the plan, and so the partial sums, of rt_query_fwd there.
+extern "C" size_t rt_pair_ws_bytes(int B, int r0, int r1, int r2) {
+  if (B <= 0) return 16;
+  QueryPlan p = query_plan(B, r1, r2, r0);
+  return sizeof(float) * (size_t)p.ksplit * B * r0;
+}
+
+extern "C" int rt_pair_fwd(const float* core, const float* s_rows, const float* o_rows, int B, int r0, int r1,
+                           int r2, float* t, void* ws, void* stream) {
+  RT_REQUIRE(B >= 0 && r0 > 0 && r1 > 0 && r2 > 0, "rt_pair_fwd: bad shape");
+  if (B == 0) return 0;
+  RT_REQUIRE(ws != nullptr, "rt_pair_fwd: workspace is NULL");
+  cudaStream_t s = (cudaStream_t)stream;
+  QueryPlan p = query_plan(B, r1, r2, r0);
+  dim3 grid(rt::cdiv(B, T), rt::cdiv(r0, T), p.ksplit);
+  pair_fwd_kernel<<<grid, 256, 0, s>>>(core, s_rows, o_rows, B, r0, r1, r2, p.k_per_split, (float*)ws);
+  RT_LAUNCH_CHECK();
+  const int64_t count = (int64_t)B * r0;
+  reduce_splits_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>((const float*)ws, p.ksplit, count, t);
   RT_LAUNCH_CHECK();
   return 0;
 }

@@ -190,3 +190,15 @@ def datasets_from_ids(ids, label_smoothing=0.1):
     valid = SparseKGDataset(ids["valid"], n, all_triples=allt, test_set=True)
     test = SparseKGDataset(ids["test"], n, all_triples=allt, test_set=True)
     return train, valid, test
+
+
+def relation_datasets_from_ids(ids):
+    """(valid, test) relation-prediction datasets (s, ?, o) of an id-triple dictionary (wn18rr_fixture): each a
+    SparseKGDataset over the split's directed triples (reverse triples included) with the columns permuted to
+    (s, o, r), so its features are (s, o, r), its n_entities is the number of relations M (the candidates) and its
+    filter lists are the relations known for (s, o) in any split, ascending (evaluation.evaluate_relations)."""
+    cols = [0, 2, 1]
+    allt = np.concatenate([ids["train"], ids["valid"], ids["test"]])[:, cols]
+    m = ids["n_relations"]
+    return tuple(SparseKGDataset(np.asarray(ids[split])[:, cols], m, all_triples=allt, test_set=True)
+                 for split in ("valid", "test"))

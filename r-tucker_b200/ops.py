@@ -162,6 +162,19 @@ def query_fwd(core, r_rows, s_rows, ws=None):
     return q
 
 
+def pair_fwd(core, s_rows, o_rows, ws=None):
+    """t [B, r0] with t[b, a] = sum_{i,j} core[a, i, j] s_rows[b, i] o_rows[b, j] (rt_pair_fwd): the relation-mode
+    query of (s, ?, o), bit-identical to query_fwd(core.permute(1, 2, 0).contiguous(), s_rows, o_rows)."""
+    require_cuda(core, s_rows, o_rows)
+    r0, r1, r2 = core.shape
+    B = s_rows.shape[0]
+    t = torch.empty(B, r0, dtype=f32, device=core.device)
+    ws = ws if ws is not None else _ws(lib().rt_pair_ws_bytes(B, r0, r1, r2), core.device)
+    check(lib().rt_pair_fwd(ptr(_c(core, f32)), ptr(_c(s_rows, f32)), ptr(_c(o_rows, f32)), B, r0, r1, r2,
+                            ptr(t), ptr(ws), stream_ptr()), "rt_pair_fwd")
+    return t
+
+
 def query_bwd(core, r_rows, s_rows, H, ws=None):
     require_cuda(core, r_rows, s_rows, H)
     r0, r1, r2 = core.shape

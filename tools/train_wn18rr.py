@@ -19,6 +19,9 @@ report and the test metrics measured right after the change, before any training
 ties with an unfiltered entity (equal > 0) in each space (<split>_ties_prob, <split>_ties_logit).  The score
 kernel variant 2 (fp16-operand tcgen05) and variant 0 (fp32 FFMA, the 1e-5 parity path) are run on identical seeds
 and batches (host shuffle = the reference's RandomSampler draw) so that their curves can be compared point by point.
+--relation-eval adds relation prediction (s, ?, o) over all relations, reverse relations included, per split: the
+filtered probability-space metrics (<split>_rel_mrr, <split>_rel_hits@k), the BCE over the relations
+(<split>_rel_loss) and the seconds the two splits took (rel_eval_s); the model is trained as before (1-N over entities).
 """
 import argparse
 import json
@@ -33,8 +36,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from rtucker_b200 import asymmetric, symmetric                      # noqa: E402
 from rtucker_b200 import train as T                                  # noqa: E402
-from rtucker_b200.data import DeviceEpoch, datasets_from_ids, wn18rr_fixture   # noqa: E402
-from rtucker_b200.evaluation import rank_batch                      # noqa: E402
+from rtucker_b200.data import DeviceEpoch, datasets_from_ids, relation_datasets_from_ids, wn18rr_fixture  # noqa: E402
+from rtucker_b200.evaluation import evaluate_relations, rank_batch  # noqa: E402
 from rtucker_b200.rank import DEFAULT_GROWTH, set_rank              # noqa: E402
 
 
@@ -106,6 +109,8 @@ def main():
                          "(evaluation reports the BCE and the filtered ranks either way)")
     ap.add_argument("--eval-space", default="prob", choices=["prob", "logit"],
                     help="logit: also report logit-space ranks, the cross-entropy evaluation loss and tie counts")
+    ap.add_argument("--relation-eval", action="store_true",
+                    help="also report filtered relation prediction (s, ?, o) metrics and loss per split")
     ap.add_argument("--rank", type=parse_rank, default=(10, 200, 200), help="starting rank r0,r1,r2")
     ap.add_argument("--rank-schedule", type=parse_schedule, default={},
                     help='rank changes at the start of epochs: "epoch:r0,r1,r2;epoch:r0,r1,r2"')
@@ -117,6 +122,7 @@ def main():
     ids = wn18rr_fixture()
     assert ids is not None, "tests/golden/wn18rr_ids.npz is missing"
     train_ds, valid_ds, test_ds = datasets_from_ids(ids, label_smoothing=0.1)
+    rel_ds = dict(zip(("val", "test"), relation_datasets_from_ids(ids))) if args.relation_eval else {}
     rank = args.rank
     torch.manual_seed(args.seed)
     mod = asymmetric if args.mode == "asymmetric" else symmetric
@@ -180,6 +186,14 @@ def main():
                     rec.update({f"{split}_logit_{k}": v for k, v in lm.items()})
                     rec.update({f"{split}_ce_loss": float(ll), f"{split}_ties_prob": ties["prob"],
                                 f"{split}_ties_logit": ties["logit"], f"{split}_queries": len(loader.dataset)})
+            if rel_ds:
+                t0 = time.perf_counter()
+                for split, ds in rel_ds.items():
+                    rm, rl = evaluate_relations(model, ds, 512, dev)
+                    rec.update({f"{split}_rel_{k}": v for k, v in rm.items()})
+                    rec[f"{split}_rel_loss"] = float(rl)
+                torch.cuda.synchronize()
+                rec["rel_eval_s"] = time.perf_counter() - t0
         if not (args.recipe == "head" and epoch >= args.total_epochs):
             sched.step()
         rec["wall_s"] = time.perf_counter() - t_start
@@ -189,7 +203,7 @@ def main():
                                rank_schedule={str(k): v for k, v in args.rank_schedule.items()}, growth=args.growth,
                                batch=512, optim="rsgd", recipe=args.recipe,
                                momentum=0.8, label_smoothing=0.1, seed=args.seed, score_variant=args.variant,
-                               loss=args.loss, eval_space=args.eval_space,
+                               loss=args.loss, eval_space=args.eval_space, relation_eval=args.relation_eval,
                                device=torch.cuda.get_device_name(dev), power_limit_w=_power_limit(),
                                epochs=args.epochs, steps_per_epoch=len(train_loader)),
                    wall_s=time.perf_counter() - t_start, history=hist)

@@ -156,7 +156,6 @@ __global__ void pack_K_kernel(PackArgs a) {
 #define PROF_PRINT(role)
 #endif
 
-__device__ __forceinline__ float lg2_fast(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 // ---- filtered-ranking epilogue of 8 columns (queries) of one thread's row (entity) --------------------------------
 // NOT inlined: the epilogue of a tile is 128 columns per thread, and as one unrolled block it was ~30 000 instructions
 // (0.5 MB) executed once per tile -- ncu showed the epilogue warps stalled on instruction fetch (stall_no_inst at every
@@ -230,7 +229,7 @@ __device__ __noinline__ RankChunkOut rank_chunk8(const RankChunkCtx& cx, int c0,
       const float en = rt::ex2_approx(-rt::kLog2e * fabsf(z));
       const float sden = 1.0f + en;
       const bool pos = z >= 0.0f;                                      // branch-free: both signs share every warp
-      const float lg = rt::kLn2 * lg2_fast(pos ? 1.0f - __frcp_rn(sden) : sden);
+      const float lg = rt::kLn2 * rt::lg2_approx(pos ? 1.0f - __frcp_rn(sden) : sden);
       float sp = pos ? -lg : lg;
       sp = (!pos && en < 1e-3f) ? en * (1.0f - 0.5f * en) : sp;
       sp = (pos && z >= 16.635532f) ? 100.0f : sp;
@@ -261,7 +260,7 @@ __device__ __noinline__ float score_chunk8(float* __restrict__ gdst, bool rv, in
     // z >= 0: p in [0.5, 1] is the fp32 quotient, 1 - p is exact, log(1 - p) from it (p == 1 from z = 24 ln 2 on);
     // z <  0: p = e^z / (1 + e^z), log(1 - p) = -log(1 + e^z) (series for tiny e^z)
     const float p = pos ? rq : en * rq;
-    const float lg = rt::kLn2 * lg2_fast(pos ? 1.0f - rq : sden);
+    const float lg = rt::kLn2 * rt::lg2_approx(pos ? 1.0f - rq : sden);
     float lq = pos ? lg : -lg;
     lq = (!pos && en < 1e-3f) ? -(en * (1.0f - 0.5f * en)) : lq;
     lq = (pos && z >= 16.635532f) ? -100.0f : lq;
@@ -1080,14 +1079,13 @@ BandLayout band_layout(int B, int n_local, int r2, int cap) {
   BandLayout L;
   L.g = logit_geom(B, n_local, r2);
   L.cap = cap;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.scal = take(256);                                 // [0] cand_count, [1] overflow, [2] max ||O_j||^2, [4..5] loss (double)
-  L.thr = take(sizeof(float) * 4 * L.g.Bp);
-  L.norms = take(sizeof(float) * (size_t)(n_local > 0 ? n_local : 1));
-  L.kimg = take(L.g.kimg_bytes);
-  L.cand = take(sizeof(int2) * (size_t)cap);
-  L.total = o;
+  rt::WsArena ws;
+  L.scal = ws.take(256);                              // [0] cand_count, [1] overflow, [2] max ||O_j||^2, [4..5] loss (double)
+  L.thr = ws.take(sizeof(float) * 4 * L.g.Bp);
+  L.norms = ws.take(sizeof(float) * (size_t)(n_local > 0 ? n_local : 1));
+  L.kimg = ws.take(L.g.kimg_bytes);
+  L.cand = ws.take(sizeof(int2) * (size_t)cap);
+  L.total = ws.o;
   return L;
 }
 BandLayout rank_layout(int B, int n_local, int r2) {
@@ -1397,17 +1395,16 @@ ScoreLayout score_layout(int B, int n_local, int r2) {
   int chunk = rt::cdiv(rt::cdiv(n_local, reps), KB) * KB;
   if (chunk < 256) chunk = 256;
   L.chunk = chunk; L.reps = rt::cdiv(n_local, chunk);
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.G = take(sizeof(float) * (size_t)L.reps * L.chunk * L.g.Bp);
-  L.kq = take(L.g.kimg_bytes);
+  rt::WsArena ws;
+  L.G = ws.take(sizeof(float) * (size_t)L.reps * L.chunk * L.g.Bp);
+  L.kq = ws.take(L.g.kimg_bytes);
   JobSpec j2{}; j2.n = n_local; j2.nk = 1; j2.t[0].rk = B; j2.reps = 1;
   JobSpec j3{}; j3.n = B; j3.nk = 1; j3.t[0].rk = L.chunk; j3.reps = L.reps;
-  L.kws = take(std::max(run_apply_ws_bytes(1, &j2, r2), run_apply_ws_bytes(1, &j3, r2)));
-  L.hpart = take(sizeof(float) * (size_t)L.reps * B * r2);
-  L.slots = take(sizeof(double) * (size_t)rt::sm_count() * kEpiWarps);
-  L.delta = take(sizeof(double) * (size_t)B);
-  L.total = o;
+  L.kws = ws.take(std::max(run_apply_ws_bytes(1, &j2, r2), run_apply_ws_bytes(1, &j3, r2)));
+  L.hpart = ws.take(sizeof(float) * (size_t)L.reps * B * r2);
+  L.slots = ws.take(sizeof(double) * (size_t)rt::sm_count() * kEpiWarps);
+  L.delta = ws.take(sizeof(double) * (size_t)B);
+  L.total = ws.o;
   return L;
 }
 
@@ -1472,11 +1469,10 @@ LseLayout lse_layout(int B, int n_local, int r2) {
   LseLayout L;
   L.g = logit_geom(B, n_local, r2);
   L.groups = 4 * L.g.tiles_per_job;                          // 32-row groups of one job's tiles
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.kq = take(L.g.kimg_bytes);
-  L.part = take(sizeof(float2) * (size_t)L.groups * L.g.Bp);
-  L.total = o;
+  rt::WsArena ws;
+  L.kq = ws.take(L.g.kimg_bytes);
+  L.part = ws.take(sizeof(float2) * (size_t)L.groups * L.g.Bp);
+  L.total = ws.o;
   return L;
 }
 }  // namespace

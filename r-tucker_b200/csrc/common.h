@@ -69,6 +69,13 @@ inline cudaError_t ensure_dyn_smem(const void* func, size_t bytes) {
 static inline int cdiv(int a, int b) { return (a + b - 1) / b; }
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+// Carves a workspace into regions in call order: take() returns the next region's byte offset and advances by its size
+// rounded up to 256 bytes; o is then the total.
+struct WsArena {
+  size_t o = 0;
+  size_t take(size_t bytes) { const size_t at = o; o += align_up(bytes, 256); return at; }
+};
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -11,7 +11,7 @@
 //   phase B: every 32x32 tile (pair k rows, pair l cols) becomes Q_k^T A_kl Q_l, and V <- V Q.
 // grid.sync() separates the phases.  N-independent, latency-bound: reported separately from the
 // HBM / tensor rooflines (SURVEY.md section 8d "N-independent serial part").
-#include "common.h"
+#include "prims.cuh"
 #include "tc.cuh"
 #include <cooperative_groups.h>
 #include <math.h>
@@ -87,18 +87,6 @@ __device__ __forceinline__ void renormalise(float c0f, float s0f, double& c, dou
   const double f = fma(e, fma(e, 0.375, -0.5), 1.0);     // (1 + e)^(-1/2) to O(e^3)
   c = c0 * f;
   s = s0 * f;
-}
-
-__device__ __forceinline__ void cp_async16_d(double* dst_smem, const double* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n"
-               :: "r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all_d() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
-
-// fp64 tensor-core MMA: D(8x8) += A(8x4) B(4x8); lane l holds A[l>>2][l&3], B[l&3][l>>2], C[l>>2][2*(l&3)+{0,1}]
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
 }
 
 // C(32x32) = op(A) * B for one warp on the fp64 tensor cores.  A element (i, m) is read from
@@ -366,24 +354,9 @@ __device__ __forceinline__ void cta_visit(bool intra) {
   __syncthreads();
 }
 
-// Grid barrier of the round loop (two per round, ~230 rounds per problem: a fifth of the kernel's time went into
-// cooperative-groups grid.sync).  Arrival is a fire-and-forget reduction, the wait polls the same word in L2: one L2
-// round trip less than an atomic with a return value followed by the poll.  The launch is cooperative (all CTAs are
-// resident); the counter only grows during a launch and is reset by CTA 0 before the kernel's first grid.sync.
+// Counter of the round loop's grid_barrier (two per round, ~230 rounds per problem: a fifth of the kernel's time went
+// into cooperative-groups grid.sync).  CTA 0 resets it before the kernel's first grid.sync.
 __device__ unsigned int g_eig_barrier;
-__device__ __forceinline__ void round_barrier(unsigned int& target) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    target += gridDim.x;
-    // release: this CTA's writes (ordered before thread 0 by the barrier above) become visible with the arrival
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;\n" :: "l"(&g_eig_barrier) : "memory");
-    unsigned int seen;
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(seen) : "l"(&g_eig_barrier) : "memory");
-    } while (seen < target);
-  }
-  __syncthreads();
-}
 
 __global__ void __launch_bounds__(kEigThreads, 1)
 eig_block_jacobi_kernel(EigBatch batch) {
@@ -532,7 +505,7 @@ eig_block_jacobi_kernel(EigBatch batch) {
         base = (base + P.npairs) % gridDim.x;
       }
       t1 = clock64(); tA += t1 - t0;
-      round_barrier(bar_target);
+      grid_barrier(&g_eig_barrier, bar_target);
       t0 = clock64(); tS1 += t0 - t1;
       // ---- phase B: A_kl <- Q_k^T A_kl Q_l (k != l),  V[:, l] <- V[:, l] Q_l ----
       base = 0;
@@ -558,11 +531,11 @@ eig_block_jacobi_kernel(EigBatch batch) {
           for (int cidx = lane; cidx < EP * (EP / 2); cidx += 32) {
             const int i = cidx >> 4, jc = (cidx & 15) * 2;            // row, first of two columns
             const int gi = isV ? k * EP + i : pair_index(bik, bjk, i);
-            cp_async16_d(&T[i * ELD + jc], M + (int64_t)gi * P.np + pair_index(bil, bjl, jc));
+            cp_async16(&T[i * ELD + jc], M + (int64_t)gi * P.np + pair_index(bil, bjl, jc));
           }
           const bool sk = isV ? true : (P.skip[k] != 0);
           const bool sl = P.skip[l] != 0;
-          if (sk && sl) { cp_async_wait_all_d(); __syncwarp(); continue; }
+          if (sk && sl) { cp_async_wait_all(); __syncwarp(); continue; }
           const bool need_l = !sl, need_k = !isV && !sk;
           if (lane == 0 && (need_l || need_k)) {
             asm volatile("fence.proxy.async;\n" ::: "memory");     // generic accesses (smem reads, J written by other CTAs) before the async proxy
@@ -577,7 +550,7 @@ eig_block_jacobi_kernel(EigBatch batch) {
               if (!isV && sk) { Qk[i * ELD + jc] = (i == jc) ? 1.0 : 0.0; Qk[i * ELD + jc + 1] = (i == jc + 1) ? 1.0 : 0.0; }
             }
           }
-          cp_async_wait_all_d();
+          cp_async_wait_all();
           if (need_l || need_k) { tc::mbar_wait(&jbar[warp], jph); jph ^= 1u; }
           __syncwarp();
           // ---- X = T Ql ;  Y = Qk^T X  on the fp64 tensor cores ----
@@ -608,7 +581,7 @@ eig_block_jacobi_kernel(EigBatch batch) {
         base = (base + nA + nV) % nwarps;
       }
       t1 = clock64(); tB += t1 - t0;
-      round_barrier(bar_target);
+      grid_barrier(&g_eig_barrier, bar_target);
       t0 = clock64(); tS2 += t0 - t1;
     }
     // convergence: off-diagonal mass seen during this sweep (uniform decision: same memory, after sync)
@@ -677,13 +650,13 @@ EigLayout eig_layout(int n) {
   if (L.nb < 2) L.nb = 2;
   L.np = L.nb * EB;
   L.npairs = L.nb / 2;
-  size_t o = 0;
-  L.off_Ap = o; o += align_up(sizeof(double) * L.np * L.np, 256);
-  L.off_Vp = o; o += align_up(sizeof(double) * L.np * L.np, 256);
-  L.off_J = o; o += align_up(sizeof(double) * L.npairs * EP * ELD, 256);
-  L.off_skip = o; o += align_up(sizeof(int) * L.npairs, 256);
-  L.off_scal = o; o += align_up(sizeof(double) * (kPermSlot + L.np), 256);
-  L.total = o;
+  WsArena ws;
+  L.off_Ap = ws.take(sizeof(double) * L.np * L.np);
+  L.off_Vp = ws.take(sizeof(double) * L.np * L.np);
+  L.off_J = ws.take(sizeof(double) * L.npairs * EP * ELD);
+  L.off_skip = ws.take(sizeof(int) * L.npairs);
+  L.off_scal = ws.take(sizeof(double) * (kPermSlot + L.np));
+  L.total = ws.o;
   return L;
 }
 

@@ -25,7 +25,11 @@ namespace rt {
 
 constexpr float kLog2e = 1.4426950408889634f, kLn2 = 0.6931471805599453f;
 
+// the approximate special-function units (ftz): 2^x, log2 x, 1 / x; the softmax element and the branch-free BCE
+// epilogues of apply_tc.cu and score_bce_v3.cu use these
 __device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
+__device__ __forceinline__ float lg2_approx(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
+__device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 __device__ __forceinline__ float exact_logit(const float* __restrict__ q, const float* __restrict__ o, int r2) {
   float z = 0.0f;

@@ -11,7 +11,7 @@
 // memory (8 lanes read 32 contiguous bytes: full sectors; fp32 -> fp64 in registers), three k-steps in flight.  Warp
 // partials are summed through shared memory in a fixed order, chunk partials by a second kernel in a fixed order:
 // bit-identical on every replica.
-#include "common.h"
+#include "prims.cuh"
 
 namespace {
 
@@ -20,17 +20,6 @@ constexpr int GWARPS = 8, GTHREADS = 256;
 constexpr int GLD = 34;                   // padded row stride of a warp partial in shared memory
 constexpr int GMAX_T = 16;                // r <= 512
 
-__device__ __forceinline__ void dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-
-__device__ __forceinline__ void sym_tile(int u, int T, int& ti, int& tj) {   // u-th tile with ti <= tj
-  ti = 0;
-  while (u >= T - ti) { u -= T - ti; ++ti; }
-  tj = ti + u;
-}
-
 __global__ void __launch_bounds__(GTHREADS, 2)
 gram_sym_kernel(const float* __restrict__ X, int64_t ld, int n, int r, int T, int ntiles, int rows_per_chunk,
                 double* __restrict__ partial) {
@@ -38,7 +27,7 @@ gram_sym_kernel(const float* __restrict__ X, int64_t ld, int n, int r, int T, in
   const int unit = blockIdx.x;
   const int chunk = unit / ntiles, tile = unit - chunk * ntiles;
   int ti, tj;
-  sym_tile(tile, T, ti, tj);
+  rt::sym_tile(tile, T, ti, tj);
   const int i0 = ti * GT, j0 = tj * GT;
   const int row_beg = chunk * rows_per_chunk;
   const int row_end = min(n, row_beg + rows_per_chunk);
@@ -80,7 +69,7 @@ gram_sym_kernel(const float* __restrict__ X, int64_t ld, int n, int r, int T, in
 #pragma unroll
     for (int a = 0; a < 4; ++a)
 #pragma unroll
-      for (int b = 0; b < 4; ++b) dmma(c[a][b][0], c[a][b][1], da[a], db[b]);
+      for (int b = 0; b < 4; ++b) rt::dmma884(c[a][b][0], c[a][b][1], da[a], db[b]);
   };
   if (my_steps > 0) load(0, fa[0], fb[0]);
   if (my_steps > 1) load(1, fa[1], fb[1]);

@@ -138,12 +138,11 @@ RankLogitLayout rank_logit_layout(int B, int n_local, int r2) {
   L.chunk_len = (int)std::min<size_t>(std::max<size_t>(kChunkFloats / (size_t)B / 64 * 64, 64),
                                       (size_t)rt::align_up((size_t)std::max(n_local, 1), 64));
   L.nchunks = std::max(1, rt::cdiv(n_local, L.chunk_len));
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.part = take(sizeof(double) * (size_t)B * kSlices);
-  L.chunk = take(sizeof(float) * (size_t)B * L.chunk_len);
-  L.tc = L.use_tc ? take(rt::rank_tc_ws_bytes(B, n_local, r2)) : o;
-  L.total = o;
+  rt::WsArena ws;
+  L.part = ws.take(sizeof(double) * (size_t)B * kSlices);
+  L.chunk = ws.take(sizeof(float) * (size_t)B * L.chunk_len);
+  L.tc = L.use_tc ? ws.take(rt::rank_tc_ws_bytes(B, n_local, r2)) : ws.o;
+  L.total = ws.o;
   return L;
 }
 

@@ -14,7 +14,7 @@
 // batch in chunks of 64 queries:  Z = Q_chunk O_tile^T  ->  elementwise (p, loss, G)  ->
 // H_chunk += G O_tile (accumulated in this CTA's private workspace slice, summed over CTAs in a
 // fixed order afterwards)  and  dO_tile += G^T QP_chunk (registers, across the chunk loop).
-#include "common.h"
+#include "prims.cuh"
 #include "exact.cuh"
 #include <math.h>
 
@@ -321,24 +321,6 @@ score_kernel(ScoreArgs a) {
   }
 }
 
-__global__ void reduce_H_kernel(const float* __restrict__ H_ws, int nparts, int64_t count,
-                                float* __restrict__ H) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  float s = 0.0f;
-  for (int k = 0; k < nparts; ++k) s += H_ws[(int64_t)k * count + i];
-  H[i] = s;
-}
-
-__global__ void reduce_loss_kernel(const double* __restrict__ partial, int n, double* __restrict__ out,
-                                   int accumulate) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    double s = 0.0;
-    for (int i = 0; i < n; ++i) s += partial[i];
-    out[0] = accumulate ? out[0] + s : s;
-  }
-}
-
 __global__ void target_prob_kernel(const float* __restrict__ q, const float* __restrict__ O, int B,
                                    int r2, int n_begin, int n_local, const int32_t* __restrict__ target,
                                    float* __restrict__ p_target) {
@@ -435,9 +417,9 @@ int score_train_ffma(const float* q, const float* qp, const float* O, int B, int
   a.n_tiles = p.n_tiles;
   if (int rc = dispatch<false, CE>(a, p, s)) return rc;
   const int64_t count = (int64_t)B * r2;
-  reduce_H_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
+  rt::split_sum_kernel<float><<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, p.grid, count, H);
   RT_LAUNCH_CHECK();
-  reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, loss_sum, 0);
+  rt::split_sum_kernel<double><<<1, 32, 0, s>>>(a.loss_partial, p.grid, 1, loss_sum);
   RT_LAUNCH_CHECK();
   return 0;
 }
@@ -631,7 +613,7 @@ extern "C" int rt_score_rank_fused(const float* q, const float* O, int B, int r2
   if (rc) return rc;
   if (bce_sum) {
     if (gate) gated_reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, bce_sum, gate);
-    else reduce_loss_kernel<<<1, 32, 0, s>>>(a.loss_partial, p.grid, bce_sum, 0);
+    else rt::split_sum_kernel<double><<<1, 32, 0, s>>>(a.loss_partial, p.grid, 1, bce_sum);
     RT_LAUNCH_CHECK();
   }
   return 0;

@@ -13,7 +13,7 @@
 // Looser tolerance than the FFMA path: TF32 inputs (10-bit mantissa, round-to-nearest at staging).
 //
 // Work per launch 6*B*N*r2 flop; algorithmic bytes 8*N*r2.
-#include "common.h"
+#include "prims.cuh"
 #include "tc.cuh"
 #include <math.h>
 
@@ -91,11 +91,6 @@ __device__ __forceinline__ void stage_rows(unsigned char* dst, const float* __re
   }
 }
 
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" :: "r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
-
 // Whole [128 rows][r2 cols] operand (all of K) -> K-major interleaved block: every 16-byte chunk is one
 // cp.async (all in flight at once), then rounded to TF32 in place by the thread that copied it.
 // Requires r2 % 4 == 0 (16-byte aligned rows).  Invalid rows are zero filled.
@@ -107,7 +102,7 @@ __device__ __forceinline__ void stage_full_async(unsigned char* dst, const float
   for (int e = threadIdx.x; e < TB * nchp; e += kThreads) {
     const int row = e / nchp, ch = e - row * nchp;
     const uint32_t off = (uint32_t)ch * CS_ROW + (uint32_t)(row >> 3) * RS + (uint32_t)(row & 7) * 16u;
-    if (row < rows_valid && ch < nch) cp_async16(d0 + off, src + (int64_t)(row0 + row) * r2 + 4 * ch);
+    if (row < rows_valid && ch < nch) rt::cp_async16(d0 + off, src + (int64_t)(row0 + row) * r2 + 4 * ch);
     else *reinterpret_cast<uint4*>(dst + off) = make_uint4(0u, 0u, 0u, 0u);
   }
 }
@@ -186,11 +181,6 @@ pack_cols_kernel(const float* __restrict__ src, int n_rows, int r2, int ncb, uns
   }
 }
 
-// ---- TMA bulk copy (global -> shared), completion counted in bytes on an mbarrier ----
-__device__ __forceinline__ void bulk_g2s_split(unsigned char* dst, const unsigned char* src, uint32_t bytes, uint64_t* bar) {
-  for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(dst + o, src + o, min(32768u, bytes - o), bar);
-}
-
 __global__ void __launch_bounds__(kThreads, 1)
 score_tc_kernel(TcArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -263,7 +253,7 @@ score_tc_kernel(TcArgs a) {
         stage_full_async(sQ, a.q, r2, b0, b_valid);
         stage_full_async(sO, a.O, r2, n0, n_valid);
         RT_TC_PROF(8);    // cp.async issue
-        cp_async_wait_all();
+        rt::cp_async_wait_all();
         RT_TC_PROF(9);    // cp.async wait
         round_full_inplace(sQ, r2, b_valid);
         round_full_inplace(sO, r2, n_valid);
@@ -581,21 +571,6 @@ score_tc_kernel(TcArgs a) {
   if (warp == 0) tmem_dealloc<512>(tmem);
 }
 
-__global__ void reduce_H_tc_kernel(const float* __restrict__ H_ws, int nparts, int64_t count, float* __restrict__ H) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  float s = 0.0f;
-  for (int k = 0; k < nparts; ++k) s += H_ws[(int64_t)k * count + i];
-  H[i] = s;
-}
-__global__ void reduce_loss_tc_kernel(const double* __restrict__ partial, int n, double* __restrict__ out) {
-  if (threadIdx.x == 0 && blockIdx.x == 0) {
-    double s = 0.0;
-    for (int i = 0; i < n; ++i) s += partial[i];
-    out[0] = s;
-  }
-}
-
 long long* g_tc_prof = nullptr;
 
 int tc_grid(int n_local) {
@@ -623,13 +598,14 @@ static TcLayout tc_layout(int B, int n_local, int r2) {
   L.packed = (r2 % 4 == 0 && r2 <= 200) ? 1 : 0;
   const int nch = r2 >> 2, nchp = nch + (nch & 1);
   L.full_bytes = (uint32_t)nchp * CS_ROW;
-  size_t o = rt::align_up((size_t)L.grid * B * r2 * sizeof(float), 256);
-  L.off_loss = o; o += rt::align_up((size_t)L.grid * sizeof(double), 256);
-  L.off_Opk1 = o; if (L.packed) o += rt::align_up((size_t)L.n_tiles * L.full_bytes, 256);
-  L.off_Qpk1 = o; if (L.packed) o += rt::align_up((size_t)L.n_chunks * L.full_bytes, 256);
-  L.off_Opk2 = o; if (L.packed) o += rt::align_up((size_t)L.n_tiles * L.ncb * TBLK_BYTES, 256);
-  L.off_Qpk2 = o; if (L.packed) o += rt::align_up((size_t)L.n_chunks * L.ncb * TBLK_BYTES, 256);
-  L.total = o;
+  rt::WsArena ws;
+  ws.take((size_t)L.grid * B * r2 * sizeof(float));                        // partial H at offset 0
+  L.off_loss = ws.take((size_t)L.grid * sizeof(double));
+  L.off_Opk1 = L.packed ? ws.take((size_t)L.n_tiles * L.full_bytes) : ws.o;
+  L.off_Qpk1 = L.packed ? ws.take((size_t)L.n_chunks * L.full_bytes) : ws.o;
+  L.off_Opk2 = L.packed ? ws.take((size_t)L.n_tiles * L.ncb * TBLK_BYTES) : ws.o;
+  L.off_Qpk2 = L.packed ? ws.take((size_t)L.n_chunks * L.ncb * TBLK_BYTES) : ws.o;
+  L.total = ws.o;
   return L;
 }
 
@@ -674,9 +650,9 @@ int score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2,
   score_tc_kernel<<<grid, kThreads, SMEM_BYTES, s>>>(a);
   RT_LAUNCH_CHECK();
   const int64_t count = (int64_t)B * r2;
-  reduce_H_tc_kernel<<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, grid, count, H);
+  rt::split_sum_kernel<float><<<(int)((count + 255) / 256), 256, 0, s>>>(a.H_ws, grid, count, H);
   RT_LAUNCH_CHECK();
-  reduce_loss_tc_kernel<<<1, 32, 0, s>>>(a.loss_partial, grid, loss_sum);
+  rt::split_sum_kernel<double><<<1, 32, 0, s>>>(a.loss_partial, grid, 1, loss_sum);
   RT_LAUNCH_CHECK();
   return 0;
 }

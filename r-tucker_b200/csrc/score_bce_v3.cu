@@ -29,6 +29,7 @@
 //
 // Work per launch 6*B*N*r2 flop; algorithmic bytes 8*N*r2.
 #include "common.h"
+#include "exact.cuh"
 #include "tc.cuh"
 #include <cuda_fp16.h>
 #include <math.h>
@@ -89,12 +90,6 @@ struct ProfT<false> {
   __device__ __forceinline__ void dump(long long*) {}
 };
 
-__device__ __forceinline__ void bulk_g2s_split(unsigned char* dst, const unsigned char* src, uint32_t bytes, uint64_t* bar) {
-  for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(dst + o, src + o, min(32768u, bytes - o), bar);
-}
-__device__ __forceinline__ float ex2_approx(float x) { float y; asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float lg2_approx(float x) { float y; asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
-__device__ __forceinline__ float rcp_approx(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 __device__ __forceinline__ void red_add_v4(float* p, float x, float y, float z, float w) {
   asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};\n" :: "l"(p), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
 }
@@ -357,11 +352,11 @@ score_v3_kernel(V3Args a) {
               float gq[2];
 #pragma unroll
               for (int u = 0; u < 2; ++u) {
-                const float s = fmaf(ex2_approx(y[j + u]), 256.0f, 1.0f);    // 1 + e^{-z}
-                const float p = rcp_approx(s);
+                const float s = fmaf(rt::ex2_approx(y[j + u]), 256.0f, 1.0f);    // 1 + e^{-z}
+                const float p = rt::rcp_approx(s);
                 gsum += p;
                 prod *= s;
-                if ((j + u) % 3 == 2 || j + u == 15) { A1 += lg2_approx(prod); prod = 1.0f; }
+                if ((j + u) % 3 == 2 || j + u == 15) { A1 += rt::lg2_approx(prod); prod = 1.0f; }
                 Y2 += y[j + u];
                 gq[u] = fmaf(p, G_SCALE, gneg);
               }
@@ -761,17 +756,18 @@ V3Layout v3_layout(int B, int n_local, int r2) {
   // G3 reads 16 n-blocks of G whatever TN is: keep 32 KB addressable behind sG
   const uint32_t tail = (uint32_t)(L.TN / 8) * QCS;
   L.smem = 2 * L.OB + 2 * L.QB + (tail < 16 * QCS ? 16 * QCS : tail);
-  size_t o = rt::align_up((size_t)L.grid * L.n_chunks * L.r2p * TB * sizeof(float), 256);
-  L.off_loss = o; o += rt::align_up((size_t)L.grid * sizeof(double), 256);
-  L.off_gsum = o; o += rt::align_up((size_t)L.grid * sizeof(double), 256);
-  L.off_cq = o; o += rt::align_up((size_t)L.r2p * sizeof(float), 256);
-  L.off_hc = o; o += rt::align_up((size_t)L.r2p * sizeof(float), 256);
-  L.off_tcs = o; o += rt::align_up((size_t)(L.n_tiles > 0 ? L.n_tiles : 1) * L.r2p * sizeof(float), 256);
-  L.off_scal = o; o += 256;
-  L.off_abs = o; o += 256;
-  L.off_Opk = o; o += rt::align_up((size_t)(L.n_tiles > 0 ? L.n_tiles : 1) * L.OB, 256);
-  L.off_Qpk = o; o += rt::align_up((size_t)L.n_chunks * L.QB, 256);
-  L.total = o;
+  rt::WsArena ws;
+  ws.take((size_t)L.grid * L.n_chunks * L.r2p * TB * sizeof(float));     // partial H at offset 0
+  L.off_loss = ws.take((size_t)L.grid * sizeof(double));
+  L.off_gsum = ws.take((size_t)L.grid * sizeof(double));
+  L.off_cq = ws.take((size_t)L.r2p * sizeof(float));
+  L.off_hc = ws.take((size_t)L.r2p * sizeof(float));
+  L.off_tcs = ws.take((size_t)(L.n_tiles > 0 ? L.n_tiles : 1) * L.r2p * sizeof(float));
+  L.off_scal = ws.take(256);
+  L.off_abs = ws.take(256);
+  L.off_Opk = ws.take((size_t)(L.n_tiles > 0 ? L.n_tiles : 1) * L.OB);
+  L.off_Qpk = ws.take((size_t)L.n_chunks * L.QB);
+  L.total = ws.o;
   return L;
 }
 

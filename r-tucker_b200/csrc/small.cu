@@ -39,8 +39,8 @@ Layout make_layout(int r0, int r1, int r2, int B) {
   Layout L;
   L.r[0] = r0; L.r[1] = r1; L.r[2] = r2; L.B = B;
   L.c = (int64_t)r0 * r1 * r2;
-  size_t o = 0;
-  auto take = [&](size_t doubles) { size_t at = o; o += align_up(doubles * sizeof(double), 256); return at; };
+  rt::WsArena ws;
+  auto take = [&](size_t doubles) { return ws.take(doubles * sizeof(double)); };
   L.C64 = take(L.c);
   for (int i = 0; i < 3; ++i) { L.Gm[i] = take((size_t)L.r[i] * L.r[i]); L.Ainv[i] = take((size_t)L.r[i] * L.r[i]); }
   L.coresq = take(4);
@@ -55,13 +55,13 @@ Layout make_layout(int r0, int r1, int r2, int B) {
     L.Gs[i] = take(r * r);
     L.tmpM[i] = take(2 * r * r);
     L.tmpK[i] = take(2 * r * r);
-    size_t at = o; o += align_up(rt::subspace_ws_bytes(2 * (int)r, (int)r), 256); L.sub[i] = at;
+    L.sub[i] = ws.take(rt::subspace_ws_bytes(2 * (int)r, (int)r));
   }
-  { size_t at = o; o += align_up(rt::subspace_shared_ws_bytes(), 256); L.sub_shared = at; }
+  L.sub_shared = ws.take(rt::subspace_shared_ws_bytes());
   L.exec_bar = take(32);
   L.gemm_partial = take(kPartialArenaBytes / sizeof(double));
   int rmax = r0 > r1 ? r0 : r1; rmax = rmax > r2 ? rmax : r2;
-  { size_t at = o; o += align_up(rt_gram_ws_bytes(B > 0 ? B : 1, rmax, rmax), 256); L.gram_ws = at; }
+  L.gram_ws = ws.take(rt_gram_ws_bytes(B > 0 ? B : 1, rmax, rmax));
   // The largest dots (rt_small_norm) are one over the core and one over each r_i x r_i Gram, recorded together;
   // every partial of one dot must fit, or its two-stage sum would write past the slot.
   auto chunks = [](int64_t n) { return (n + kEwChunk - 1) / kEwChunk; };
@@ -70,7 +70,7 @@ Layout make_layout(int r0, int r1, int r2, int B) {
   L.dot_slots = (int)std::max<int64_t>(kMinDotSlots, slots);
   L.dot_partial = take((size_t)L.dot_slots);
   L.scal = take(16);
-  L.total = o;
+  L.total = ws.o;
   return L;
 }
 

@@ -19,7 +19,7 @@
 // contractions with few tiles are split over CTAs; the partial tiles are summed by a REDUCE
 // operation of the next level in split order -- deterministic, bit-identical on every replica.
 #pragma once
-#include "common.h"
+#include "prims.cuh"
 #include <math.h>
 
 namespace rt {
@@ -77,24 +77,6 @@ constexpr int kExecThreads = 256;
 constexpr int kExecWarps = 8;
 constexpr int kEwChunk = 2048;    // elements per elementwise unit
 constexpr int kReduceChunk = 1024;
-
-__device__ __forceinline__ void exec_dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-
-__device__ __forceinline__ void exec_barrier(unsigned int* bar, unsigned int& target) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    target += gridDim.x;
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;\n" :: "l"(bar) : "memory");
-    unsigned int seen;
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(seen) : "l"(bar) : "memory");
-    } while (seen < target);
-  }
-  __syncthreads();
-}
 
 __device__ __forceinline__ double ld_as_f64(const void* p, int64_t i, int t) {
   return t == DT_F64 ? __ldcg(reinterpret_cast<const double*>(p) + i) : (double)__ldcg(reinterpret_cast<const float*>(p) + i);
@@ -161,7 +143,7 @@ __device__ __noinline__ void gemm_unit(const GemmPart& op, int unit, double* red
 #pragma unroll
     for (int ti = 0; ti < 4; ++ti)
 #pragma unroll
-      for (int tj = 0; tj < 4; ++tj) exec_dmma(c[ti][tj][0], c[ti][tj][1], ra[ti], rb[tj]);
+      for (int tj = 0; tj < 4; ++tj) dmma884(c[ti][tj][0], c[ti][tj][1], ra[ti], rb[tj]);
   };
   // three register buffers: the loads of two steps ahead are in flight while a step is multiplied
   constexpr int W = kExecWarps;
@@ -361,19 +343,6 @@ __device__ __forceinline__ void ew_unit(const EwPart& op, int ew, int unit) {
   }
 }
 
-// deterministic CTA-wide sum (fixed shuffle tree, fixed warp order)
-__device__ __forceinline__ double exec_cta_sum(double v, double* sh) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  __syncthreads();
-  if ((threadIdx.x & 31) == 0) sh[threadIdx.x >> 5] = v;
-  __syncthreads();
-  double s = 0.0;
-#pragma unroll
-  for (int w = 0; w < kExecWarps; ++w) s += sh[w];
-  return s;
-}
-
 // DOT: z[unit] = sum over this unit's chunk of x[i] * y[i];  DOTFIN: z[0] = (p0 ? z[0] : 0) + s0 * sum_{i < count} x[i]
 __device__ __forceinline__ void dot_unit(const EwPart& op, int unit, double* sh) {
   const int64_t base = (int64_t)unit * kEwChunk;
@@ -383,14 +352,14 @@ __device__ __forceinline__ void dot_unit(const EwPart& op, int unit, double* sh)
     const int64_t i = base + threadIdx.x + kExecThreads * mI;
     if (i < op.count) s = fma(ld_as_f64(op.x, i, op.tx), ld_as_f64(op.y, i, op.tz), s);
   }
-  s = exec_cta_sum(s, sh);
+  s = cta_sum<kExecWarps>(s, sh);
   if (threadIdx.x == 0) reinterpret_cast<double*>(op.z)[unit] = s;
 }
 __device__ __forceinline__ void dotfin_unit(const EwPart& op, double* sh) {
   const double* part = reinterpret_cast<const double*>(op.x);
   double s = 0.0;
   for (int64_t i = threadIdx.x; i < op.count; i += kExecThreads) s += __ldcg(part + i);
-  s = exec_cta_sum(s, sh);
+  s = cta_sum<kExecWarps>(s, sh);
   if (threadIdx.x == 0) {
     double* out = reinterpret_cast<double*>(op.z);
     out[0] = (op.p0 ? __ldcg(out) : 0.0) + op.s0 * s;
@@ -450,7 +419,7 @@ small_exec_kernel(const __grid_constant__ Program prog) {
     const int i_first = i;
 #endif
     i = j;
-    if (i < nops) exec_barrier(prog.bar, bar_target);
+    if (i < nops) grid_barrier(prog.bar, bar_target);
 #ifdef RT_EXEC_PROF
     if (blockIdx.x == 0 && threadIdx.x == 0) {
       const long long now = clock64();

@@ -2,7 +2,7 @@
 // executor of small_exec.cuh: the SPD factorisation / inverse, and the rows-times-inverse product of
 // rt_rows_times_ainv.  Internal to small.cu.
 #pragma once
-#include "common.h"
+#include "prims.cuh"
 #include <math.h>
 
 namespace rt {
@@ -47,10 +47,6 @@ struct SpdProblem {
 struct SpdBatch { SpdProblem p[3]; int dmma; };   // dmma: O(n^3) phases on the fp64 tensor cores (needs 8 n more doubles of smem)
 
 __device__ __forceinline__ int pk(int i, int j) { return i * (i + 1) / 2 + j; }
-__device__ __forceinline__ void spd_dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 // sum of 8 interleaved partial accumulators in a fixed order
 __device__ __forceinline__ double spd_sum8(const double (&c)[8][2], int e) {
   return ((c[0][e] + c[1][e]) + (c[2][e] + c[3][e])) + ((c[4][e] + c[5][e]) + (c[6][e] + c[7][e]));
@@ -151,7 +147,7 @@ spd_blocked_kernel(SpdBatch batch) {
           for (int s0 = 0; s0 < nsteps; s0 += 8) {
 #pragma unroll
             for (int u = 0; u < 8; ++u)
-              if (s0 + u < nsteps) spd_dmma(c[u][0], c[u][1], av ? La[4 * (s0 + u)] : 0.0, bv ? Lb[4 * (s0 + u)] : 0.0);
+              if (s0 + u < nsteps) dmma884(c[u][0], c[u][1], av ? La[4 * (s0 + u)] : 0.0, bv ? Lb[4 * (s0 + u)] : 0.0);
           }
           // result element: row 8 tile + fg (the SAME row this lane fetched), columns 2 ft, 2 ft + 1
 #pragma unroll
@@ -316,7 +312,7 @@ spd_blocked_kernel(SpdBatch batch) {
           for (int u = 0; u < 8; ++u)
             if (s0 + u < nsteps) {
               const int k = j0 + 4 * (s0 + u) + ft;
-              spd_dmma(c[u][0], c[u][1], stage[fg * n + k], k >= jc ? Lp[pk(k, jc)] : 0.0);
+              dmma884(c[u][0], c[u][1], stage[fg * n + k], k >= jc ? Lp[pk(k, jc)] : 0.0);
             }
         }
 #pragma unroll
@@ -398,7 +394,7 @@ spd_blocked_kernel(SpdBatch batch) {
           if (s0 + u < nsteps) {
             const int k = i0 + 4 * (s0 + u) + ft;
             const bool kv = k < n;
-            spd_dmma(c[u][0], c[u][1], (kv && ic < n && k >= ic) ? Lp[pk(k, ic)] : 0.0, (kv && jc < n && k >= jc) ? Lp[pk(k, jc)] : 0.0);
+            dmma884(c[u][0], c[u][1], (kv && ic < n && k >= ic) ? Lp[pk(k, ic)] : 0.0, (kv && jc < n && k >= jc) ? Lp[pk(k, jc)] : 0.0);
           }
       }
 #pragma unroll

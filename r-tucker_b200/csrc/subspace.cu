@@ -26,7 +26,7 @@
 // in a fixed order through shared memory.  All reductions (traces, defects) go through per-tile
 // slots that every CTA sums in the same order: the result is bit-identical on every replica of an
 // entity-sharded run, which keeps the replicated cores identical.
-#include "common.h"
+#include "prims.cuh"
 #include <math.h>
 #include <stdlib.h>
 
@@ -63,24 +63,6 @@ struct SubBatch {
 
 enum SubState { S_TC2 = 0, S_COPY = 1, S_NSG = 2, S_NSZ = 3, S_DONE = 4 };
 
-__device__ __forceinline__ void sub_dmma(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
-
-__device__ __forceinline__ void sub_barrier(unsigned int* bar, unsigned int& target) {
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    target += gridDim.x;
-    asm volatile("red.release.gpu.global.add.u32 [%0], 1;\n" :: "l"(bar) : "memory");
-    unsigned int seen;
-    do {
-      asm volatile("ld.acquire.gpu.global.u32 %0, [%1];\n" : "=r"(seen) : "l"(bar) : "memory");
-    } while (seen < target);
-  }
-  __syncthreads();
-}
-
 // C(32 x 32) = A[i0.., :K] * B[j0.., :K]^T with rows of A and B contiguous in k.  The 8 warps split K
 // (K is a multiple of 32); the sum of their partials lands in red[0] (fixed order).  `out[m]` of thread t
 // is element e = t + 256 m, (row, col) = (e / 32, e % 32).
@@ -110,7 +92,7 @@ __device__ __forceinline__ void tile_nt(const double* __restrict__ A, int lda, i
 #pragma unroll
     for (int ti = 0; ti < 4; ++ti)
 #pragma unroll
-      for (int tj = 0; tj < 4; ++tj) sub_dmma(c[ti][tj][0], c[ti][tj][1], ra[ti], rb[tj]);
+      for (int tj = 0; tj < 4; ++tj) dmma884(c[ti][tj][0], c[ti][tj][1], ra[ti], rb[tj]);
   };
   load(0, a0, b0);
   if (steps > 1) load(1, a1, b1);
@@ -143,20 +125,6 @@ __device__ __forceinline__ void tile_nt(const double* __restrict__ A, int lda, i
   __syncthreads();
 }
 
-// deterministic CTA-wide sum (fixed shuffle tree, fixed warp order); result valid in every thread
-__device__ __forceinline__ double cta_sum(double v, double* sh) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  __syncthreads();
-  if (lane == 0) sh[warp] = v;
-  __syncthreads();
-  double s = 0.0;
-#pragma unroll
-  for (int w = 0; w < kSubWarps; ++w) s += sh[w];
-  return s;
-}
-
 // sum of `count` (<= 160) slots in a fixed order, by one warp; every warp of every CTA gets the same bits
 __device__ __forceinline__ double slot_sum(const double* slots, int count) {
   const int lane = threadIdx.x & 31;
@@ -165,12 +133,6 @@ __device__ __forceinline__ double slot_sum(const double* slots, int count) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
   return v;
-}
-
-__device__ __forceinline__ void sym_tile(int u, int T, int& ti, int& tj) {   // u-th tile with ti <= tj
-  ti = 0;
-  while (u >= T - ti) { u -= T - ti; ++ti; }
-  tj = ti + u;
 }
 
 // One CTA per SM: with two (296 CTAs, 128 registers) a round costs 18 us instead of 9 (spills in the tile routine and a
@@ -197,14 +159,14 @@ subspace_kernel(SubBatch batch) {
       const int i = e / P.n;
       if (e - i * P.n == i) tr += v;
     }
-    f2 = cta_sum(f2, sh_red);
-    tr = cta_sum(tr, sh_red);
+    f2 = cta_sum<kSubWarps>(f2, sh_red);
+    tr = cta_sum<kSubWarps>(tr, sh_red);
     if (tid == 0) {
       batch.scratch[(int64_t)blockIdx.x * (2 * kSubMaxProblems) + 2 * pi] = f2;
       batch.scratch[(int64_t)blockIdx.x * (2 * kSubMaxProblems) + 2 * pi + 1] = tr;
     }
   }
-  sub_barrier(batch.bar, bar_target);
+  grid_barrier(batch.bar, bar_target);
   // per-problem state: identical in every CTA (same inputs, same order of operations), kept in shared memory
   __shared__ double trace[kSubMaxProblems];
   __shared__ int state[kSubMaxProblems], iters[kSubMaxProblems], ns_iters[kSubMaxProblems], cur[kSubMaxProblems],
@@ -234,7 +196,7 @@ subspace_kernel(SubBatch batch) {
       P.X[0][e] = (i < P.n && j < P.n) ? P.N_in[(int64_t)i * P.n + j] * inv : 0.0;
     }
   }
-  sub_barrier(batch.bar, bar_target);
+  grid_barrier(batch.bar, bar_target);
 
   int round = 0;
   for (;;) {
@@ -291,7 +253,7 @@ subspace_kernel(SubBatch batch) {
           if (ti != tj) Xn[(int64_t)j * np + i] = v;
         }
         if (ti == tj) {                      // slot ti: trace of X^2 over this diagonal tile
-          trc = cta_sum(trc, sh_red);
+          trc = cta_sum<kSubWarps>(trc, sh_red);
           if (tid == 0) slots[ti] = trc;
         }
       } else if (state[pi] == S_COPY) {
@@ -324,7 +286,7 @@ subspace_kernel(SubBatch batch) {
             err2 = fma(d, d, err2);
           }
         }
-        err2 = cta_sum(err2, sh_red);
+        err2 = cta_sum<kSubWarps>(err2, sh_red);
         if (tid == 0) slots[lu] = (ti == tj) ? err2 : 2.0 * err2;
       } else if (state[pi] == S_NSZ) {
         const int ti = lu / Tr, tj = lu - ti * Tr;
@@ -351,7 +313,7 @@ subspace_kernel(SubBatch batch) {
         }
       }
     }
-    sub_barrier(batch.bar, bar_target);
+    grid_barrier(batch.bar, bar_target);
     // ---- state update: every CTA reads the same slots and takes the same decisions (warp 0, then broadcast
     //      through shared memory) ----
     if (tid < 32) {
@@ -411,15 +373,14 @@ static SubLayout sub_layout(int n, int r) {
   SubLayout L;
   L.np = cdiv(n, ST) * ST;
   L.rp = cdiv(r, ST) * ST;
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += align_up(bytes, 256); return at; };
-  for (int k = 0; k < 2; ++k) L.X[k] = take(sizeof(double) * L.np * L.np);
-  for (int k = 0; k < 2; ++k) L.Z[k] = take(sizeof(double) * L.np * L.rp);
-  for (int k = 0; k < 2; ++k) L.Zt[k] = take(sizeof(double) * L.np * L.rp);
-  L.G = take(sizeof(double) * L.rp * L.rp);
-  L.slots = take(sizeof(double) * 2 * kSlotsPerProblem);
-  L.info = take(sizeof(int) * 4);
-  L.total = o;
+  WsArena ws;
+  for (int k = 0; k < 2; ++k) L.X[k] = ws.take(sizeof(double) * L.np * L.np);
+  for (int k = 0; k < 2; ++k) L.Z[k] = ws.take(sizeof(double) * L.np * L.rp);
+  for (int k = 0; k < 2; ++k) L.Zt[k] = ws.take(sizeof(double) * L.np * L.rp);
+  L.G = ws.take(sizeof(double) * L.rp * L.rp);
+  L.slots = ws.take(sizeof(double) * 2 * kSlotsPerProblem);
+  L.info = ws.take(sizeof(int) * 4);
+  L.total = ws.o;
   return L;
 }
 

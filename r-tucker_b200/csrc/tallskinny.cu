@@ -5,7 +5,7 @@
 //
 // Bound: HBM for thin ranks; at r ~ 200 the N x r x r products are FP32-FFMA bound
 // (2*N*ra*rb flops per Gram, 2*N*rk*rc per update term).
-#include "common.h"
+#include "prims.cuh"
 #include <algorithm>
 
 namespace {
@@ -86,10 +86,6 @@ constexpr int GKC = 32;      // rows per smem chunk
 // its row split; warp w owns the 8 x 64 strip of A-columns [8w, 8w + 8): eight 8 x 8 accumulator tiles.
 // Row chunks are staged in shared memory as doubles (pitch 72: the four k-rows of a fragment load fall into
 // different bank halves).
-__device__ __forceinline__ void dmma884_g(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};\n"
-               : "+d"(c0), "+d"(c1) : "d"(a), "d"(b));
-}
 constexpr int DG_LD = GT + 8;
 __global__ void __launch_bounds__(256)
 gram_dmma_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict__ B, int64_t ldb,
@@ -139,7 +135,7 @@ gram_dmma_kernel(const float* __restrict__ A, int64_t lda, const float* __restri
         const double a = As[4 * kk + t][8 * warp + g];
 #pragma unroll
         for (int j = 0; j < 8; ++j)
-          if (j < nbj) dmma884_g(c[j][0], c[j][1], a, Bs[4 * kk + t][8 * j + g]);
+          if (j < nbj) rt::dmma884(c[j][0], c[j][1], a, Bs[4 * kk + t][8 * j + g]);
       }
     }
     __syncthreads();
@@ -158,15 +154,6 @@ gram_dmma_kernel(const float* __restrict__ A, int64_t lda, const float* __restri
       }
     }
   }
-}
-
-__global__ void gram_reduce_kernel(const double* __restrict__ partial, int nsplit, int count,
-                                   double* __restrict__ out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  double s = 0.0;
-  for (int k = 0; k < nsplit; ++k) s += partial[(int64_t)k * count + i];  // fixed order
-  out[i] = s;
 }
 
 struct GramPlan {
@@ -251,7 +238,7 @@ extern "C" int rt_gram(const float* A, int64_t lda, const float* B, int64_t ldb,
   gram_dmma_kernel<<<grid, 256, 0, s>>>(A, lda, B, ldb, n, ra, rb, p.tiles_b, p.rows_per_split, (double*)ws);
   RT_LAUNCH_CHECK();
   const int count = ra * rb;
-  gram_reduce_kernel<<<rt::cdiv(count, 256), 256, 0, s>>>((const double*)ws, p.nsplit, count, out);
+  rt::split_sum_kernel<double><<<rt::cdiv(count, 256), 256, 0, s>>>((const double*)ws, p.nsplit, count, out);
   RT_LAUNCH_CHECK();
   return 0;
 }

@@ -3,17 +3,9 @@
 //              operand rows streamed with cp.async (row-major input IS the k-major smem layout)
 //   apply_v2:  Y[n, rc] = a0 X0 + sum_t X_t K_t       128 x 104 tiles, 4 x 13 register tiles, double buffered
 // r = 200 is exactly two 104-wide tiles (4 % padding).  FFMA-bound: 2*n*ra*rb and 2*n*rc*sum(rk) flop.
-#include "common.h"
+#include "prims.cuh"
 
 namespace {
-
-__device__ __forceinline__ void cp_async16(void* dst_smem, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n"
-               :: "r"((uint32_t)__cvta_generic_to_shared(dst_smem)), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" :: "n"(N) : "memory"); }
 
 // =====================================================================================================
 // gram_v2
@@ -44,18 +36,18 @@ gram_v2_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict
       const int gr = row0 + rr;
       float* da = &As[stage][rr][c4];
       float* db = &Bs[stage][rr][c4];
-      if (gr < n1 && vec_ok && a0 + c4 + 4 <= ra) cp_async16(da, A + (int64_t)gr * lda + a0 + c4);
+      if (gr < n1 && vec_ok && a0 + c4 + 4 <= ra) rt::cp_async16(da, A + (int64_t)gr * lda + a0 + c4);
       else {
 #pragma unroll
         for (int j = 0; j < 4; ++j) da[j] = (gr < n1 && a0 + c4 + j < ra) ? __ldg(A + (int64_t)gr * lda + a0 + c4 + j) : 0.0f;
       }
-      if (gr < n1 && vec_ok && b0 + c4 + 4 <= rb) cp_async16(db, B + (int64_t)gr * ldb + b0 + c4);
+      if (gr < n1 && vec_ok && b0 + c4 + 4 <= rb) rt::cp_async16(db, B + (int64_t)gr * ldb + b0 + c4);
       else {
 #pragma unroll
         for (int j = 0; j < 4; ++j) db[j] = (gr < n1 && b0 + c4 + j < rb) ? __ldg(B + (int64_t)gr * ldb + b0 + c4 + j) : 0.0f;
       }
     }
-    cp_async_commit();
+    rt::cp_async_commit();
   };
 
   float acc[13][4];
@@ -64,11 +56,11 @@ gram_v2_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict
 #pragma unroll
     for (int j = 0; j < 4; ++j) acc[i][j] = 0.0f;
 
-  for (int c = 0; c < GST - 1; ++c) { if (c < nchunks) issue(c, c); else cp_async_commit(); }
+  for (int c = 0; c < GST - 1; ++c) { if (c < nchunks) issue(c, c); else rt::cp_async_commit(); }
   for (int c = 0; c < nchunks; ++c) {
-    cp_async_wait<GST - 2>();
+    rt::cp_async_wait<GST - 2>();
     __syncthreads();
-    if (c + GST - 1 < nchunks) issue(c + GST - 1, (c + GST - 1) % GST); else cp_async_commit();
+    if (c + GST - 1 < nchunks) issue(c + GST - 1, (c + GST - 1) % GST); else rt::cp_async_commit();
     const int st = c % GST;
 #pragma unroll 4
     for (int k = 0; k < GKC; ++k) {
@@ -88,7 +80,7 @@ gram_v2_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict
         for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
     }
   }
-  cp_async_wait<0>();
+  rt::cp_async_wait<0>();
   // partial[split][ra][rb]
   float* out = partial + (int64_t)split * ra * rb;
 #pragma unroll
@@ -101,14 +93,6 @@ gram_v2_kernel(const float* __restrict__ A, int64_t lda, const float* __restrict
       if (bj < rb) out[(int64_t)ai * rb + bj] = acc[i][j];
     }
   }
-}
-
-__global__ void gram_v2_reduce_kernel(const float* __restrict__ partial, int nsplit, int count, double* __restrict__ out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= count) return;
-  double s = 0.0;
-  for (int k = 0; k < nsplit; ++k) s += (double)partial[(int64_t)k * count + i];
-  out[i] = s;
 }
 
 struct GramV2Plan { int qa, qb, nsplit, rows_per_split; };
@@ -280,7 +264,7 @@ int gram_v2(const float* A, int64_t lda, const float* B, int64_t ldb, int n, int
   gram_v2_kernel<<<grid, GTHREADS, 0, s>>>(A, lda, B, ldb, n, ra, rb, p.qb, p.rows_per_split, (float*)ws, vec_ok);
   RT_LAUNCH_CHECK();
   const int count = ra * rb;
-  gram_v2_reduce_kernel<<<rt::cdiv(count, 256), 256, 0, s>>>((const float*)ws, p.nsplit, count, out);
+  rt::split_sum_kernel<double><<<rt::cdiv(count, 256), 256, 0, s>>>((const float*)ws, p.nsplit, count, out);
   RT_LAUNCH_CHECK();
   return 0;
 }

@@ -141,6 +141,10 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src, uint32
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n"
                :: "r"(smem_u32(dst_smem)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
+// a copy of any size as 32 KB bulk copies on one mbarrier
+__device__ __forceinline__ void bulk_g2s_split(unsigned char* dst, const unsigned char* src, uint32_t bytes, uint64_t* bar) {
+  for (uint32_t o = 0; o < bytes; o += 32768u) bulk_g2s(dst + o, src + o, min(32768u, bytes - o), bar);
+}
 __device__ __forceinline__ void bulk_s2g(void* dst, const void* src_smem, uint32_t bytes) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n"
                :: "l"(dst), "r"(smem_u32(src_smem)), "r"(bytes) : "memory");

@@ -213,17 +213,16 @@ TopkLayout topk_layout(int B, int n_local, int r2, int k) {
   L.chunk_len = (int)std::min<size_t>(std::max<size_t>(kChunkFloats / (size_t)B / 64 * 64, 64),
                                       (size_t)rt::align_up((size_t)std::max(n_local, 1), 64));
   L.nchunks = std::max(1, rt::cdiv(n_local, L.chunk_len));
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t at = o; o += rt::align_up(bytes, 256); return at; };
-  L.scal = take(256);                                   // [0] some query is flagged
-  L.pk = take(sizeof(float) * B);
-  L.flag = take(sizeof(int) * B);
-  L.cnt = take(sizeof(int) * B);
-  L.run = take(sizeof(u64) * (size_t)B * k);
-  L.chunk = take(sizeof(float) * (size_t)B * L.chunk_len);
-  L.tc = L.use_tc ? take(rt::topk_tc_ws_bytes(B, n_local, r2)) : o;
-  L.seg = L.use_tc ? take(sizeof(int32_t) * (size_t)B * kCap) : o;
-  L.total = o;
+  rt::WsArena ws;
+  L.scal = ws.take(256);                                // [0] some query is flagged
+  L.pk = ws.take(sizeof(float) * B);
+  L.flag = ws.take(sizeof(int) * B);
+  L.cnt = ws.take(sizeof(int) * B);
+  L.run = ws.take(sizeof(u64) * (size_t)B * k);
+  L.chunk = ws.take(sizeof(float) * (size_t)B * L.chunk_len);
+  L.tc = L.use_tc ? ws.take(rt::topk_tc_ws_bytes(B, n_local, r2)) : ws.o;
+  L.seg = L.use_tc ? ws.take(sizeof(int32_t) * (size_t)B * kCap) : ws.o;
+  L.total = ws.o;
   return L;
 }
 

@@ -124,15 +124,35 @@ def test_every_kernel_is_referenced():
 
 def test_exact_score_arithmetic_is_written_once():
     """The element arithmetic that the dense, fused and recheck kernels must share bit for bit (accurate sigmoid,
-    clamped BCE logs, guarded BCE gradient, ex2.approx of the softmax) is spelled out only in exact.cuh.  The fp16
-    score variant (score_bce_v3.cu) keeps its own approximate ex2."""
+    clamped BCE logs, guarded BCE gradient, ex2.approx of the softmax) is spelled out only in exact.cuh."""
     rules = {"log1pf(": r"\blog1pf\(", "fmaxf(.., 1e-12f)": r"\bfmaxf\([^();]*\b1e-12f",
              "expf(-": r"(?<!\w)expf\(\s*-", "ex2.approx": r"ex2\.approx"}
     found = {rule: sorted(f for f, text in csrc_sources().items() if re.search(pattern, text))
              for rule, pattern in rules.items()}
-    for rule in ("log1pf(", "fmaxf(.., 1e-12f)", "expf(-"):
+    for rule in rules:
         assert found[rule] == ["exact.cuh"], (rule, found[rule])
-    assert len([f for f in found["ex2.approx"] if f != "score_bce_v3.cu"]) <= 1, found["ex2.approx"]
+
+
+def first_ptx_mnemonic(ptx):
+    """The first instruction of an inline-PTX string, skipping braces, .reg declarations and labels."""
+    for stmt in re.split(r"[;{}]", ptx.replace("\\n", " ").replace("\\t", " ")):
+        stmt = re.sub(r"^\s*\w+:", "", stmt).strip()
+        if stmt and not stmt.startswith("."):
+            return stmt.split()[0]
+    return None
+
+
+def test_inline_ptx_is_written_once():
+    """Every inline-PTX instruction (the first mnemonic of each asm statement) is spelled out in one file: prims.cuh,
+    tc.cuh, exact.cuh or the one kernel that uses it.  A second copy would not receive a fix made to the first."""
+    files = {}
+    for name, text in csrc_sources().items():
+        for strings in re.findall(r"\basm\s*(?:volatile\s*)?\(\s*((?:\"(?:[^\"\\]|\\.)*\"\s*)+)", text):
+            ptx = "".join(re.findall(r"\"((?:[^\"\\]|\\.)*)\"", strings))
+            files.setdefault(first_ptx_mnemonic(ptx), set()).add(name)
+    assert None not in files, files[None]
+    copies = {m: sorted(f) for m, f in files.items() if len(f) > 1}
+    assert not copies, copies
 
 
 def test_no_cpu_fallback():

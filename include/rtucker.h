@@ -170,6 +170,17 @@ int rt_query_bwd(const float* core, const float* r_rows, const float* s_rows, co
 size_t rt_pair_ws_bytes(int B, int r0, int r1, int r2);
 int rt_pair_fwd(const float* core, const float* s_rows, const float* o_rows,
                 int B, int r0, int r1, int r2, float* t, void* ws, void* stream);
+/* Backward of rt_pair_fwd given H_t = dL/dt [B, r0] (the relation-prediction term of the training step):
+ * d_core[r0,r1,r2] = sum_b H_t[b] (x) s_rows[b] (x) o_rows[b];
+ * ds_rows[b,i] = sum_{a,j} core[a,i,j] H_t[b,a] o_rows[b,j]  [B, r1];
+ * do_rows[b,j] = sum_{a,i} core[a,i,j] H_t[b,a] s_rows[b,i]  [B, r2].
+ * Reads the core in place and writes d_core unpermuted (no permuted copies).  Bit-identical to rt_query_bwd on core
+ * permuted to (r1, r2, r0) with (s_rows, o_rows, H_t) in place of (r_rows, s_rows, H), its d_core permuted back, its
+ * ds_rows as do_rows and its dr_rows as ds_rows: same products, same split plan, same summation order.
+ * The workspace of rt_pair_ws_bytes covers both passes.  Deterministic; B == 0 launches nothing. */
+int rt_pair_bwd(const float* core, const float* s_rows, const float* o_rows, const float* H_t,
+                int B, int r0, int r1, int r2,
+                float* d_core, float* ds_rows, float* do_rows, void* ws, void* stream);
 
 /* ---- (b) fused 1-N score + sigmoid + label-smoothed BCE + backward ------------------- */
 /*

@@ -48,6 +48,7 @@ PROTOTYPES = {
     "rt_query_bwd": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
     "rt_pair_ws_bytes": (sz, [i32, i32, i32, i32]),
     "rt_pair_fwd": (i32, [vp, vp, vp, i32, i32, i32, i32, vp, vp, vp]),
+    "rt_pair_bwd": (i32, [vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp, vp]),
     "rt_score_bce_ws_bytes": (sz, [i32, i32, i32, i32]),
     "rt_score_bce_fwd_bwd": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, i32, vp, vp, f32, vp, vp, vp,
                                    i32, vp, vp]),

@@ -6,7 +6,8 @@
 //   r[b,a]*s[b,i] is generated on the fly (never stored), K = r0*r1, split-K for occupancy.
 // Backward is what autograd would compute for those two lines.
 // Pair contraction (relation prediction, (s, ?, o)): t[b,a] = sum_{i,j} core[a,i,j] s[b,i] o[b,j], the same GEMM with
-// K = r1*r2, the left operand s[b,i]*o[b,j] generated on the fly and the core read in place (no permuted copy).
+// K = r1*r2, the left operand s[b,i]*o[b,j] generated on the fly and the core read in place (no permuted copy); its
+// backward (the relation-prediction training term) is the query backward's two kernels with the same folding.
 //
 // FP32 FFMA, deterministic (split partials reduced in a fixed order).
 // Flops: fwd 2*B*r0*r1*r2, bwd 3x that.  Bytes: core once per pass (L2 resident) + rows.
@@ -142,6 +143,10 @@ __global__ void reduce_splits_kernel(const float* __restrict__ partial, int nspl
 // ---- backward (1): d_core[k=(a,i), j] = sum_b r[b,a] s[b,i] H[b,j] ----------------------------
 // grid.z splits the batch (few k x j tiles at small ranks: 128 CTAs walked all 512 rows, 98 us); the partial sums are
 // added in split order by reduce_splits_kernel
+// PAIR: the backward of the pair contraction, run as this kernel on the core permuted to (r1, r2, r0) (so r0, r1, r2
+// here are the permuted extents); only the store addressing differs: element (k, j) of the permuted core's gradient is
+// written where the unpermuted core keeps it, d_core[j * K + k].
+template <bool PAIR>
 __global__ void __launch_bounds__(256)
 query_bwd_core_kernel(const float* __restrict__ r_rows, const float* __restrict__ s_rows,
                       const float* __restrict__ H, int B, int r0, int r1, int r2, int b_per_split,
@@ -172,13 +177,16 @@ query_bwd_core_kernel(const float* __restrict__ r_rows, const float* __restrict_
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       const int jj = j0 + tx * 4 + j;
-      if (jj < r2) d_core[(int64_t)k * r2 + jj] = acc[i][j];
+      if (jj < r2) d_core[PAIR ? (int64_t)jj * K + k : (int64_t)k * r2 + jj] = acc[i][j];
     }
   }
 }
 
 // ---- backward (2): Y_a[b,i] = sum_j H[b,j] core[a,i,j];  ds[b,i] += r[b,a] Y_a;  dr[b,a] = sum_i s[b,i] Y_a
 // grid (b tiles, i tiles, a splits).  ds partial per a-split, dr partial per i-tile.
+// PAIR: as query_bwd_core_kernel<true>, the permuted core (r0, r1, r2 its extents) read in place: element (a, i, j) of
+// the permuted core is core[(j * r0 + a) * r1 + i], contiguous along i, so the B operand's lanes run along i.
+template <bool PAIR>
 __global__ void __launch_bounds__(256)
 query_bwd_rows_kernel(const float* __restrict__ core, const float* __restrict__ r_rows,
                       const float* __restrict__ s_rows, const float* __restrict__ H, int B, int r0,
@@ -207,9 +215,10 @@ query_bwd_rows_kernel(const float* __restrict__ core, const float* __restrict__ 
     zero_acc(y);
     auto lb = [&](int j, int cc) -> float {  // core[a, i0+cc, j]
       const int ii = i0 + cc;
-      return (ii < r1) ? __ldg(core + ((int64_t)a * r1 + ii) * r2 + j) : 0.0f;
+      if (ii >= r1) return 0.0f;
+      return __ldg(core + (PAIR ? ((int64_t)j * r0 + a) * r1 + ii : ((int64_t)a * r1 + ii) * r2 + j));
     };
-    tile_mainloop<true, false>(0, r2, la, lb, y, As, Bs);
+    tile_mainloop<true, PAIR>(0, r2, la, lb, y, As, Bs);
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int b = b0 + ty * 4 + i;
@@ -271,6 +280,40 @@ QueryPlan query_plan(int B, int r0, int r1, int r2) {
   return p;
 }
 
+// rt_query_bwd on (core, r_rows, s_rows, H) with extents (r0, r1, r2); PAIR: core is the unpermuted core of the pair
+// contraction and (r0, r1, r2) the extents of its permutation (r1, r2, r0), d_core is written unpermuted.
+template <bool PAIR>
+int query_bwd(const float* core, const float* r_rows, const float* s_rows, const float* H, int B, int r0, int r1,
+              int r2, float* d_core, float* ds_rows, float* dr_rows, void* ws, cudaStream_t s) {
+  QueryPlan p = query_plan(B, r0, r1, r2);
+  float* ds_partial = (float*)ws;
+  float* dr_partial = ds_partial + (size_t)p.asplit * B * r1;
+  {
+    float* core_partial = dr_partial + (size_t)p.itiles * B * r0;
+    dim3 grid(rt::cdiv(r0 * r1, T), rt::cdiv(r2, T), p.bsplit);
+    query_bwd_core_kernel<PAIR><<<grid, 256, 0, s>>>(r_rows, s_rows, H, B, r0, r1, r2, p.b_per_split,
+                                                     p.bsplit > 1 ? core_partial : d_core);
+    RT_LAUNCH_CHECK();
+    if (p.bsplit > 1) {
+      const int64_t cc = (int64_t)r0 * r1 * r2;
+      reduce_splits_kernel<<<(int)((cc + 255) / 256), 256, 0, s>>>(core_partial, p.bsplit, cc, d_core);
+      RT_LAUNCH_CHECK();
+    }
+  }
+  {
+    dim3 grid(rt::cdiv(B, T), p.itiles, p.asplit);
+    query_bwd_rows_kernel<PAIR><<<grid, 256, 0, s>>>(core, r_rows, s_rows, H, B, r0, r1, r2,
+                                                     p.a_per_split, ds_partial, dr_partial);
+    RT_LAUNCH_CHECK();
+  }
+  const int64_t c1 = (int64_t)B * r1, c0 = (int64_t)B * r0;
+  reduce_splits_kernel<<<(int)((c1 + 255) / 256), 256, 0, s>>>(ds_partial, p.asplit, c1, ds_rows);
+  RT_LAUNCH_CHECK();
+  reduce_splits_kernel<<<(int)((c0 + 255) / 256), 256, 0, s>>>(dr_partial, p.itiles, c0, dr_rows);
+  RT_LAUNCH_CHECK();
+  return 0;
+}
+
 }  // namespace
 
 extern "C" size_t rt_query_ws_bytes(int B, int r0, int r1, int r2) {
@@ -298,12 +341,9 @@ extern "C" int rt_query_fwd(const float* core, const float* r_rows, const float*
   return 0;
 }
 
-// The forward split plan of the permuted core (r1, r2, r0): the plan, and so the partial sums, of rt_query_fwd there.
-extern "C" size_t rt_pair_ws_bytes(int B, int r0, int r1, int r2) {
-  if (B <= 0) return 16;
-  QueryPlan p = query_plan(B, r1, r2, r0);
-  return sizeof(float) * (size_t)p.ksplit * B * r0;
-}
+// The split plan of the permuted core (r1, r2, r0): the plan, and so the partial sums, of rt_query_fwd / rt_query_bwd
+// there.  The workspace covers both passes.
+extern "C" size_t rt_pair_ws_bytes(int B, int r0, int r1, int r2) { return rt_query_ws_bytes(B, r1, r2, r0); }
 
 extern "C" int rt_pair_fwd(const float* core, const float* s_rows, const float* o_rows, int B, int r0, int r1,
                            int r2, float* t, void* ws, void* stream) {
@@ -326,32 +366,18 @@ extern "C" int rt_query_bwd(const float* core, const float* r_rows, const float*
                             float* ds_rows, float* dr_rows, void* ws, void* stream) {
   RT_REQUIRE(B > 0 && r0 > 0 && r1 > 0 && r2 > 0, "rt_query_bwd: bad shape");
   RT_REQUIRE(ws != nullptr, "rt_query_bwd: workspace is NULL");
-  cudaStream_t s = (cudaStream_t)stream;
-  QueryPlan p = query_plan(B, r0, r1, r2);
-  float* ds_partial = (float*)ws;
-  float* dr_partial = ds_partial + (size_t)p.asplit * B * r1;
-  {
-    float* core_partial = dr_partial + (size_t)p.itiles * B * r0;
-    dim3 grid(rt::cdiv(r0 * r1, T), rt::cdiv(r2, T), p.bsplit);
-    query_bwd_core_kernel<<<grid, 256, 0, s>>>(r_rows, s_rows, H, B, r0, r1, r2, p.b_per_split,
-                                               p.bsplit > 1 ? core_partial : d_core);
-    RT_LAUNCH_CHECK();
-    if (p.bsplit > 1) {
-      const int64_t cc = (int64_t)r0 * r1 * r2;
-      reduce_splits_kernel<<<(int)((cc + 255) / 256), 256, 0, s>>>(core_partial, p.bsplit, cc, d_core);
-      RT_LAUNCH_CHECK();
-    }
-  }
-  {
-    dim3 grid(rt::cdiv(B, T), p.itiles, p.asplit);
-    query_bwd_rows_kernel<<<grid, 256, 0, s>>>(core, r_rows, s_rows, H, B, r0, r1, r2,
-                                               p.a_per_split, ds_partial, dr_partial);
-    RT_LAUNCH_CHECK();
-  }
-  const int64_t c1 = (int64_t)B * r1, c0 = (int64_t)B * r0;
-  reduce_splits_kernel<<<(int)((c1 + 255) / 256), 256, 0, s>>>(ds_partial, p.asplit, c1, ds_rows);
-  RT_LAUNCH_CHECK();
-  reduce_splits_kernel<<<(int)((c0 + 255) / 256), 256, 0, s>>>(dr_partial, p.itiles, c0, dr_rows);
-  RT_LAUNCH_CHECK();
-  return 0;
+  return query_bwd<false>(core, r_rows, s_rows, H, B, r0, r1, r2, d_core, ds_rows, dr_rows, ws,
+                          (cudaStream_t)stream);
+}
+
+// rt_query_bwd of the permuted core (r1, r2, r0) with (s_rows, o_rows) in place of (r_rows, s_rows): its ds is do, its
+// dr is ds.
+extern "C" int rt_pair_bwd(const float* core, const float* s_rows, const float* o_rows, const float* H_t, int B,
+                           int r0, int r1, int r2, float* d_core, float* ds_rows, float* do_rows, void* ws,
+                           void* stream) {
+  RT_REQUIRE(B >= 0 && r0 > 0 && r1 > 0 && r2 > 0, "rt_pair_bwd: bad shape");
+  if (B == 0) return 0;
+  RT_REQUIRE(ws != nullptr, "rt_pair_bwd: workspace is NULL");
+  return query_bwd<true>(core, s_rows, o_rows, H_t, B, r1, r2, r0, d_core, do_rows, ds_rows, ws,
+                         (cudaStream_t)stream);
 }

@@ -202,3 +202,11 @@ def relation_datasets_from_ids(ids):
     m = ids["n_relations"]
     return tuple(SparseKGDataset(np.asarray(ids[split])[:, cols], m, all_triples=allt, test_set=True)
                  for split in ("valid", "test"))
+
+
+def relation_train_dataset(ids, label_smoothing=0.0):
+    """The training data of the relation-prediction term (optim.RelationTerm): a SparseKGDataset over the train split's
+    directed triples (reverse triples included) with the columns permuted to (s, o, r).  Its features are the unique
+    (s, o) pairs (first-occurrence order), its targets their train relations (ascending), its n_entities the number of
+    relations M; ``label_smoothing`` is the term's.  DeviceEpoch iterates it like the entity split."""
+    return SparseKGDataset(np.asarray(ids["train"])[:, [0, 2, 1]], ids["n_relations"], label_smoothing=label_smoothing)

@@ -93,6 +93,40 @@ class SparseTargets:
     idx: torch.Tensor  # int32 [nnz]
 
 
+class RelationTerm:
+    """The relation-prediction term of the training loss (Chen et al., AKBC 2021): ``weight`` times the softmax
+    cross-entropy over the M relations of B' subject-object pairs,
+      t_b = W x_2 S[s_b] x_3 O[o_b],  z_bm = R[m] . t_b,
+      tau_bm = (1 - ls) [m in Y_b] / |Y_b| + ls / M,  L_rel = (1/B') sum_b (lse_b - sum_m tau_bm z_bm)
+    i.e. F.cross_entropy(z, y / |y|, label_smoothing=ls).  ``pairs`` int32 [B', 2] = (s_b, o_b) (global entity ids);
+    ``targets`` the CSR of the relations Y_b of each pair (global relation ids, reverse relations included, unique per
+    pair).  The term has no state."""
+
+    def __init__(self, pairs: torch.Tensor, targets: SparseTargets, weight: float, label_smoothing: float = 0.0):
+        weight, label_smoothing = float(weight), float(label_smoothing)
+        if not (weight >= 0.0 and weight != float("inf")):
+            raise ValueError(f"RelationTerm: weight must be finite and >= 0, got {weight}")
+        if not 0.0 <= label_smoothing < 1.0:
+            raise ValueError(f"RelationTerm: label_smoothing must be in [0, 1), got {label_smoothing}")
+        if not isinstance(pairs, torch.Tensor) or pairs.dtype != torch.int32 or pairs.dim() != 2 or pairs.shape[1] != 2:
+            raise ValueError("RelationTerm: pairs must be an int32 tensor [B', 2] of (subject, object) ids, got "
+                             f"{getattr(pairs, 'dtype', type(pairs))} {tuple(getattr(pairs, 'shape', ()))}")
+        if pairs.shape[0] == 0:
+            raise ValueError("RelationTerm: the relation batch is empty (B' == 0)")
+        if not isinstance(targets, SparseTargets):
+            raise TypeError("RelationTerm: targets must be a SparseTargets (CSR of relation ids per pair)")
+        off, idx = targets.off, targets.idx
+        if off.dtype != torch.int32 or idx.dtype != torch.int32 or off.dim() != 1 or idx.dim() != 1:
+            raise ValueError("RelationTerm: targets.off and targets.idx must be 1-D int32 tensors")
+        if off.shape[0] != pairs.shape[0] + 1:
+            raise ValueError(f"RelationTerm: targets.off must have B' + 1 = {pairs.shape[0] + 1} entries, "
+                             f"got {off.shape[0]}")
+        if off.device != pairs.device or idx.device != pairs.device:
+            raise ValueError("RelationTerm: pairs and targets must be on the same device")
+        self.pairs, self.targets = pairs, targets
+        self.weight, self.label_smoothing = weight, label_smoothing
+
+
 class Direction:
     """The optimiser's ``direction``: a tangent vector at ``point`` = (core, [R, S, O])."""
 
@@ -165,6 +199,13 @@ class StepEngine:
         self.score_centre = torch.tensor([0.0, 0.5], dtype=f32, device=dev)
         self.loss_buf = torch.zeros(1, dtype=f64, device=dev)
         self.norm_buf = torch.zeros(1, dtype=f64, device=dev)
+        # relation-prediction term: [weight, 1.0] on the device (the scale the term's kernels read) and L_rel
+        self.rel_w = torch.tensor([0.0, 1.0], dtype=f64, device=dev)
+        self._rel_w_host = None
+        self._rel_w_val = None
+        self.rel_loss_buf = torch.zeros(1, dtype=f64, device=dev)
+        self.rel_loss = None
+        self._static_rel = {}
         self.has_old = False
         # CUDA graphs (single GPU, CUDA ops only): captured after the first eager step
         self.use_graphs = False
@@ -211,6 +252,15 @@ class StepEngine:
             self.hyper.copy_(host, non_blocking=True)
             self._hyper_vals = vals
 
+    def _set_rel_weight(self, weight):
+        if weight != self._rel_w_val:
+            host = torch.tensor([weight, 1.0], dtype=f64)
+            if self.dev.type == "cuda":
+                host = host.pin_memory()
+            self._rel_w_host = host            # keep alive until replaced
+            self.rel_w.copy_(host, non_blocking=True)
+            self._rel_w_val = weight
+
     def _allreduce(self, *tensors):
         if self.group is None:
             return
@@ -246,12 +296,24 @@ class StepEngine:
         return self._U(2) if not self.sym else self._U(1)
 
     # -------------------------------------------------------------------------------------------
+    def _check_relation(self, relation):
+        """``relation`` with a weight of 0 is no term at all: None is returned and nothing of it runs."""
+        if relation is None:
+            return None
+        if not isinstance(relation, RelationTerm):
+            raise TypeError("relation must be a RelationTerm")
+        if relation.pairs.device != self.dev:
+            raise ValueError(f"RelationTerm on device {relation.pairs.device}, the model on device {self.dev}")
+        return relation if relation.weight != 0.0 else None
+
     def fit(self, rel_idx, sub_idx, targets: SparseTargets, label_smoothing, reg, lr_hint=0.0,
-            normalize_grad=1.0, loss="bce"):
+            normalize_grad=1.0, loss="bce", relation: Optional[RelationTerm] = None):
         """Riemannian gradient and step direction of ``loss`` at the current point: "bce" (the reference's
         label-smoothed sigmoid BCE, the default) or "ce" (1-N softmax cross-entropy over all entities,
-        rtucker.h: rt_score_ce_fwd_bwd)."""
+        rtucker.h: rt_score_ce_fwd_bwd), plus ``relation.weight`` times the relation-prediction cross-entropy when a
+        RelationTerm is given (its value alone in ``rel_loss``)."""
         check_loss(loss)
+        relation = self._check_relation(relation)
         loss_kind = loss
         ops, small, sym = self.ops, self.small, self.sym
         r0, r1, r2 = self.rank
@@ -307,11 +369,17 @@ class StepEngine:
         with self._stage("small_grad"):
             dS_g, loss, drA, dsA, P_R, P_S, P_O = small.grad(core, d_core, qp, H, r_rows, s_rows, dr_rows,
                                                              ds_rows, bce_sum, inv_count, self.hyper)
+        dR_rel, rel_rows = None, []
+        if relation is not None:
+            dR_rel, rel_rows = self._relation_term(relation, core, dS_g, loss, P_R, P_S, P_O)
         t_tall = self._stage("tall_skinny_fit")
         t_tall.__enter__()
         # ---- factor parts of the Riemannian gradient: dV_i = g_i A_i - U_i (U_i^T g_i A_i) ----
         dV_g = [None] * self.nf
-        dV_g[0] = ops.apply(self.spare[0], None, None, [(R, P_R)])
+        if dR_rel is None:
+            dV_g[0] = ops.apply(self.spare[0], None, None, [(R, P_R)])
+        else:
+            dV_g[0] = ops.apply(self.spare[0], dR_rel, self.rel_w[0:1], [(R, P_R)])
         ops.scatter_rows_add(dV_g[0], rel_idx, drA)
         obj_terms = [(dO_raw, small.ainv(2)), (O, P_O)] if fold_a else None
         if not sym:
@@ -324,6 +392,8 @@ class StepEngine:
         for k, v in zip(self._entity_factor_ids(), out):
             dV_g[k] = v
         ops.scatter_rows_add(dV_g[1], sub_idx, dsA, self.n_begin)
+        for k, idx, rows in rel_rows:
+            ops.scatter_rows_add(dV_g[k], idx, rows, self.n_begin)
         # ---- norm of the Riemannian gradient ----
         grams = [ops.gram(v, v, out=self._gram_view[0][k]) for k, v in enumerate(dV_g)]
         self._allreduce(self._gram_flat[0][self._gram_ent:])
@@ -357,7 +427,50 @@ class StepEngine:
         self.norm_buf.copy_(norm)
         self.loss = self.loss_buf
         self.rgrad_norm = self.norm_buf
+        self.rel_loss = self.rel_loss_buf if relation is not None else None
         return self.norm_buf
+
+    def _relation_term(self, relation, core, dS_g, loss, P_R, P_S, P_O):
+        """Adds the relation-prediction term to the parts of the Riemannian gradient (DESIGN.md 4.10): with
+        Gbar = (softmax - tau) / B' and H_t = weight * Gbar R (scaled once: every part below is linear in H_t),
+          dS_g += pair_bwd's d_core;  P_R -= H_t^T (t A_0);  P_S -= S[s]^T (ds A_1);  P_O -= O[o]^T (do A_2)
+        (SF-Tucker: both into the shared P_S), and ``loss`` += weight * L_rel.  Returns dR = Gbar^T (t A_0) (the
+        caller adds weight * dR to dV_R) and the row terms [(factor, ids, rows . A)] to scatter into dV_S / dV_O.
+        Entity-sharded: the subject and object rows are gathered zero-filled on their owner shards and all-reduced
+        in one [B', r1 + r2] buffer; the rest is replicated (core and R are) and the scatters land on the owners."""
+        ops, small = self.ops, self.small
+        r1 = self.rank[1]
+        R, S, O = self._U(0), self._U(1), self._obj()
+        self._set_rel_weight(relation.weight)
+        s_idx = relation.pairs[:, 0].contiguous()
+        o_idx = relation.pairs[:, 1].contiguous()
+        Bp = s_idx.shape[0]
+        tg = relation.targets
+        with self._stage("relation_fwd"):
+            s_rows = ops.gather_rows(S, s_idx, self.n_begin)
+            o_rows = ops.gather_rows(O, o_idx, self.n_begin)
+            if self.group is not None:
+                so = torch.cat([s_rows, o_rows], 1)
+                self._allreduce(so)
+                s_rows, o_rows = so[:, :r1].contiguous(), so[:, r1:].contiguous()
+            t = ops.pair_fwd(core, s_rows, o_rows)
+            tA = small.rows_times_ainv(t, 0)
+            parts = ops.score_lse(t, R, variant=0)
+            rel_sum, H_t, dR = ops.score_ce_fwd_bwd(t, tA, R, tg.off, tg.idx, relation.label_smoothing, parts,
+                                                    n_total=R.shape[0], b_total=Bp, n_begin=0, variant=0)
+            ops.apply(H_t, H_t, self.rel_w[0:1], [])
+        with self._stage("relation_bwd"):
+            d_core, ds_rows, do_rows = ops.pair_bwd(core, s_rows, o_rows, H_t)
+            ops.core_axpby(dS_g, self.rel_w[1:2], d_core, out=dS_g)
+            dsA = small.rows_times_ainv(ds_rows, 1)
+            doA = small.rows_times_ainv(do_rows, 2)
+            P_R.sub_(ops.gram(H_t, tA))
+            P_S.sub_(ops.gram(s_rows, dsA))
+            P_O.sub_(ops.gram(o_rows, doA))        # SF-Tucker: P_O is P_S
+        torch.div(rel_sum, Bp, out=self.rel_loss_buf)
+        loss.add_(self.rel_loss_buf, alpha=relation.weight)
+        k_obj = 2 if not self.sym else 1
+        return dR, [(1, s_idx, dsA), (k_obj, o_idx, doA)]
 
     def _score_ce(self, q, qp, O, targets, label_smoothing, variant, out):
         """1-N softmax cross-entropy: the log-sum-exp pass over this shard, the (m, s) parts of every shard (one
@@ -520,13 +633,15 @@ class StepEngine:
                 and self.ops is cuda_ops and getattr(self, "timers", None) is None)
 
     def fit_auto(self, rel_idx, sub_idx, targets: SparseTargets, label_smoothing, reg, lr_hint=0.0,
-                 normalize_grad=1.0, loss="bce"):
+                 normalize_grad=1.0, loss="bce", relation: Optional[RelationTerm] = None):
         """fit() through a captured CUDA graph once the state machine is in steady state (one graph per batch size,
-        label smoothing and loss kind)."""
+        label smoothing and loss kind, and per relation batch size, label smoothing and weight)."""
         check_loss(loss)
+        relation = self._check_relation(relation)
         steady = self._eager_steps >= 1 and (self.beta is None or self.has_old)
         if not (self._graphs_ok() and steady):
-            return self.fit(rel_idx, sub_idx, targets, label_smoothing, reg, lr_hint, normalize_grad, loss=loss)
+            return self.fit(rel_idx, sub_idx, targets, label_smoothing, reg, lr_hint, normalize_grad, loss=loss,
+                            relation=relation)
         B, nnz = rel_idx.shape[0], targets.idx.shape[0]
         si = self._static_in
         if si is None or si["B"] != B or si["cap"] < nnz:
@@ -544,17 +659,43 @@ class StepEngine:
         si["idx"][:nnz].copy_(targets.idx, non_blocking=True)
         self._set_hyper(self._hyper_vals[0], reg, self.beta, normalize_grad if normalize_grad else 0.0)
         key = ("fit", B, float(label_smoothing), loss)
+        static_rel = None
+        if relation is not None:
+            static_rel = self._stage_relation(relation)
+            self._set_rel_weight(relation.weight)
+            key = key + (relation.pairs.shape[0], relation.label_smoothing, relation.weight)
         g = self._graphs.get(key)
         if g is None:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self.fit(si["rel"], si["sub"], SparseTargets(si["off"], si["idx"]), label_smoothing, reg,
-                         lr_hint, normalize_grad, loss=loss)
+                         lr_hint, normalize_grad, loss=loss, relation=static_rel)
             self._graphs[key] = g
         g.replay()
         self.pending = (self.dS_dir, self.dV_new)
         self.loss, self.rgrad_norm = self.loss_buf, self.norm_buf
+        self.rel_loss = self.rel_loss_buf if relation is not None else None
         return self.norm_buf
+
+    def _stage_relation(self, relation):
+        """Copies the relation batch into the fixed buffers (one set per B') the captured fit graphs read; returns the
+        RelationTerm over them.  New buffers for a B' (more targets than they hold) drop the fit graphs that read the
+        old ones."""
+        Bp, nnz = relation.pairs.shape[0], relation.targets.idx.shape[0]
+        sr = self._static_rel.get(Bp)
+        if sr is None or sr["cap"] < nnz:
+            cap = max(2 * nnz, 4 * Bp, 1024)
+            i32 = torch.int32
+            sr = dict(cap=cap, pairs=torch.zeros(Bp, 2, dtype=i32, device=self.dev),
+                      off=torch.zeros(Bp + 1, dtype=i32, device=self.dev),
+                      idx=torch.zeros(cap, dtype=i32, device=self.dev))
+            self._static_rel[Bp] = sr
+            self._graphs = {k: v for k, v in self._graphs.items() if not (k[0] == "fit" and len(k) > 4 and k[4] == Bp)}
+        sr["pairs"].copy_(relation.pairs, non_blocking=True)
+        sr["off"].copy_(relation.targets.off, non_blocking=True)
+        sr["idx"][:nnz].copy_(relation.targets.idx, non_blocking=True)
+        return RelationTerm(sr["pairs"], SparseTargets(sr["off"], sr["idx"]), relation.weight,
+                            relation.label_smoothing)
 
     def step_auto(self, lr):
         steady = self._eager_steps >= 1 and (self.beta is None or self.has_old)

@@ -175,6 +175,23 @@ def pair_fwd(core, s_rows, o_rows, ws=None):
     return t
 
 
+def pair_bwd(core, s_rows, o_rows, H_t, ws=None):
+    """Backward of pair_fwd given H_t = dL/dt [B, r0] (rt_pair_bwd): returns (d_core [r0, r1, r2], ds_rows [B, r1],
+    do_rows [B, r2]), bit-identical to query_bwd(core.permute(1, 2, 0).contiguous(), s_rows, o_rows, H_t) with its
+    d_core permuted back, its ds_rows as do_rows and its dr_rows as ds_rows."""
+    require_cuda(core, s_rows, o_rows, H_t)
+    r0, r1, r2 = core.shape
+    B = s_rows.shape[0]
+    d_core = torch.empty_like(core)
+    ds_rows = torch.empty(B, r1, dtype=f32, device=core.device)
+    do_rows = torch.empty(B, r2, dtype=f32, device=core.device)
+    ws = ws if ws is not None else _ws(lib().rt_pair_ws_bytes(B, r0, r1, r2), core.device)
+    check(lib().rt_pair_bwd(ptr(_c(core, f32)), ptr(_c(s_rows, f32)), ptr(_c(o_rows, f32)), ptr(_c(H_t, f32)),
+                            B, r0, r1, r2, ptr(d_core), ptr(ds_rows), ptr(do_rows), ptr(ws), stream_ptr()),
+          "rt_pair_bwd")
+    return d_core, ds_rows, do_rows
+
+
 def query_bwd(core, r_rows, s_rows, H, ws=None):
     require_cuda(core, r_rows, s_rows, H)
     r0, r1, r2 = core.shape

@@ -7,7 +7,8 @@
 
 Kept: torch.optim.Optimizer subclasses (OneCycleLR drives param_groups[0]["lr"], train.py:213-215),
 ``fit(loss_fn, x_k, normalize_grad=1.) -> ||rgrad||``, ``step(closure=None)``, attributes ``loss``,
-``direction``, ``momentum_beta``.  ``loss_fn`` must be a ``FusedLoss`` (the reference's opaque lambda
+``direction``, ``momentum_beta``; ``rel_loss`` is the relation-prediction cross-entropy of the last fit (None without a
+``RelationTerm``).  ``loss_fn`` must be a ``FusedLoss`` (the reference's opaque lambda
 would need autodiff through dense B x N tensors; that path does not exist here and fit() says so).
 Note the reference's asymmetric RGD.step is broken (unpacks 3 of 4 params, optim.py:49-57,
 SURVEY.md App. D-2); here it performs the step its docstring describes.
@@ -17,7 +18,7 @@ from typing import Optional
 import torch
 from torch.optim import Optimizer
 
-from .engine import SparseTargets, StepEngine, check_loss
+from .engine import RelationTerm, SparseTargets, StepEngine, check_loss
 from .model import ScoreFn
 
 
@@ -27,14 +28,19 @@ class FusedLoss:
     Stands where the reference passes ``lambda T: criterion(score_fn(T), targets) + reg * T.norm()**2``.
     ``loss="ce"`` selects the 1-N softmax cross-entropy over all entities instead of the BCE (the same targets,
     normalised to 1 per query, with the same label smoothing; include/rtucker.h, rt_score_ce_fwd_bwd).
+    ``relation``: a ``RelationTerm`` adds ``relation.weight`` times the relation-prediction cross-entropy of a batch of
+    (s, o) pairs over all relations; with None or a weight of 0 nothing of it runs.
     """
 
     def __init__(self, score_fn: ScoreFn, targets: SparseTargets, label_smoothing: float, reg_coeff: float,
-                 loss: str = "bce"):
+                 loss: str = "bce", relation: Optional[RelationTerm] = None):
         check_loss(loss)
+        if relation is not None and not isinstance(relation, RelationTerm):
+            raise TypeError(f"FusedLoss: relation must be a RelationTerm or None, got {type(relation).__name__}")
         self.score_fn, self.targets = score_fn, targets
         self.label_smoothing, self.reg_coeff = float(label_smoothing), float(reg_coeff)
         self.loss = loss
+        self.relation = relation
 
 
 class _RiemannianBase(Optimizer):
@@ -56,6 +62,7 @@ class _RiemannianBase(Optimizer):
         self.direction = None
         self.momentum = None
         self.loss = None
+        self.rel_loss = None
         self._engine = None
         self._pending_engine_state = None
         self._use_graphs = bool(use_graphs)
@@ -118,8 +125,9 @@ class _RiemannianBase(Optimizer):
             normalize_grad = 0.0       # SFTuckerAdam.fit never normalises (its normalize_grad argument is unused)
         norm = eng.fit_auto(sf.relation_idx, sf.subject_idx, loss_fn.targets, loss_fn.label_smoothing,
                             loss_fn.reg_coeff, lr_hint=self.param_groups[0]["lr"], normalize_grad=normalize_grad,
-                            loss=loss_fn.loss)
+                            loss=loss_fn.loss, relation=loss_fn.relation)
         self.loss = eng.loss.float().reshape(())
+        self.rel_loss = eng.rel_loss.float().reshape(()) if eng.rel_loss is not None else None
         self.direction = eng.pending
         return norm.float().reshape(())
 

@@ -26,6 +26,7 @@ from torch import nn
 from . import checkpoint
 from .evaluation import _check_space, _sums_from_ranks, rank_batch
 from .manifold import SFTucker, Tucker
+from .engine import RelationTerm
 from .optim import FusedLoss
 from .rank import set_rank
 
@@ -51,24 +52,58 @@ def _check_criterion(criterion):
                     "(the smoothing comes from the loader); got %r" % (criterion,))
 
 
-def train_one_epoch(model, optimizer, criterion, train_loader, regularization_coeff=1e-4):
-    """One pass over ``train_loader``; returns (mean loss, mean ||rgrad||) like train.py:91."""
+def _relation_batches(loader):
+    """Relation batches without end: the loader restarts (a new permutation) whenever it runs out."""
+    while True:
+        empty = True
+        for batch in loader:
+            empty = False
+            yield batch
+        if empty:
+            raise ValueError("relation_loader yields no batches")
+
+
+def train_one_epoch(model, optimizer, criterion, train_loader, regularization_coeff=1e-4, relation_loader=None,
+                    relation_weight=0.0):
+    """One pass over ``train_loader``; returns (mean loss, mean ||rgrad||) like train.py:91.
+
+    ``relation_loader`` (a DeviceEpoch over data.relation_train_dataset) adds the relation-prediction term with weight
+    ``relation_weight`` to every step (optim.RelationTerm; the loss then includes it): each step draws the loader's next
+    (s, o) batch, restarting it when it runs out.  The return value is then (mean loss, mean ||rgrad||, mean relation
+    cross-entropy), the last None when the weight is 0 (nothing of the term runs)."""
     loss_kind = _check_criterion(criterion)
+    relation_weight = float(relation_weight)
+    if not (relation_weight >= 0.0 and relation_weight != float("inf")):
+        raise ValueError(f"relation_weight must be finite and >= 0, got {relation_weight}")
+    if relation_loader is None and relation_weight != 0.0:
+        raise ValueError("relation_weight > 0 needs a relation_loader")
     model.train()
     device = model.core.device
     n_batches = len(train_loader)
     train_loss = torch.zeros((), device=device)
     train_grad_norm = torch.zeros((), device=device)
+    rel_batches = _relation_batches(relation_loader) if relation_loader is not None else None
+    rel_loss = torch.zeros((), device=device) if rel_batches is not None and relation_weight > 0 else None
     for features, targets in train_loader:
         score_fn = model(features[:, 0], features[:, 1])
-        loss_fn = FusedLoss(score_fn, targets, train_loader.label_smoothing, regularization_coeff, loss=loss_kind)
+        relation = None
+        if rel_batches is not None:
+            pairs, rel_targets = next(rel_batches)
+            relation = RelationTerm(pairs, rel_targets, relation_weight, relation_loader.label_smoothing)
+        loss_fn = FusedLoss(score_fn, targets, train_loader.label_smoothing, regularization_coeff, loss=loss_kind,
+                            relation=relation)
         x_k = extract_tensor(model)
         grad_norm = optimizer.fit(loss_fn, x_k)
         optimizer.step()
         train_grad_norm += grad_norm.detach()
         train_loss += optimizer.loss.detach()
+        if rel_loss is not None:
+            rel_loss += optimizer.rel_loss.detach()
         optimizer.zero_grad(set_to_none=True)
-    return train_loss.item() / n_batches, train_grad_norm.item() / n_batches      # the epoch's only host sync
+    if relation_loader is None:
+        return train_loss.item() / n_batches, train_grad_norm.item() / n_batches      # the epoch's only host sync
+    return (train_loss.item() / n_batches, train_grad_norm.item() / n_batches,
+            rel_loss.item() / n_batches if rel_loss is not None else None)
 
 
 @torch.no_grad()
@@ -101,7 +136,8 @@ def evaluate(model, criterion, dataloader, n_begin=0, group=None, space="prob"):
 
 
 def train(model, optimizer, train_loader, val_loader, test_loader, config, regulizer, scheduler=None, log_fn=None,
-          start_epoch=None, num_epoches=None, history=None, criterion=None, eval_space="prob", rank_schedule=None):
+          start_epoch=None, num_epoches=None, history=None, criterion=None, eval_space="prob", rank_schedule=None,
+          relation_loader=None, relation_weight=0.0):
     """train.py:128-167: evaluate once, then per epoch: regulariser step, train epoch, validate, test, snapshot
     (now with the optimiser state), scheduler step.  ``config`` needs ``train_cfg.num_epoches`` and
     ``train_cfg.checkpoint_path`` (configs/base_config.py); ``log_fn(record)`` replaces wandb_log.  ``criterion``:
@@ -110,7 +146,8 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
     ``evaluate`` ("prob", the default: BCE and probability ranks whichever the criterion; "logit"); each record
     names it.  ``rank_schedule``: {epoch: (r0, r1, r2)}; ``rank.set_rank(model, rank, optimizer)`` runs at the start of
     that epoch (truncation or growth; the optimiser's momentum restarts, the scheduler is untouched).  Each record
-    names the rank the epoch trained at."""
+    names the rank the epoch trained at.  ``relation_loader`` / ``relation_weight``: the relation-prediction term of
+    train_one_epoch; each record then carries its mean (``train_rel_loss``)."""
     criterion = nn.BCELoss(reduction="mean") if criterion is None else criterion
     _check_criterion(criterion)
     _check_space(eval_space, ("prob", "logit"))
@@ -124,8 +161,14 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
             set_rank(model, rank_schedule[epoch], optimizer)
         regularization_coeff = regulizer.step()
         t0 = time.perf_counter()
-        train_loss, train_norm = train_one_epoch(model, optimizer, criterion, train_loader,
-                                                 regularization_coeff=regularization_coeff)
+        rel = {}
+        if relation_loader is None:
+            train_loss, train_norm = train_one_epoch(model, optimizer, criterion, train_loader,
+                                                     regularization_coeff=regularization_coeff)
+        else:
+            train_loss, train_norm, rel["train_rel_loss"] = train_one_epoch(
+                model, optimizer, criterion, train_loader, regularization_coeff=regularization_coeff,
+                relation_loader=relation_loader, relation_weight=relation_weight)
         epoch_time = time.perf_counter() - t0
         val_metrics, val_loss = evaluate(model, criterion, val_loader, space=eval_space)
         t0 = time.perf_counter()
@@ -135,6 +178,7 @@ def train(model, optimizer, train_loader, val_loader, test_loader, config, regul
         record = dict(epoch=epoch, train_loss=train_loss, grad_norm=train_norm, val_loss=float(val_loss),
                       test_loss=float(test_loss), lr=optimizer.param_groups[0]["lr"], reg_coeff=regularization_coeff,
                       epoch_time=epoch_time, eval_time=eval_time, eval_space=eval_space, rank=list(model.core.shape),
+                      **rel,
                       **{"val_" + k: v for k, v in val_metrics.items()},
                       **{"test_" + k: v for k, v in test_metrics.items()})
         history.append(record)

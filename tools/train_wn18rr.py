@@ -21,7 +21,11 @@ kernel variant 2 (fp16-operand tcgen05) and variant 0 (fp32 FFMA, the 1e-5 parit
 and batches (host shuffle = the reference's RandomSampler draw) so that their curves can be compared point by point.
 --relation-eval adds relation prediction (s, ?, o) over all relations, reverse relations included, per split: the
 filtered probability-space metrics (<split>_rel_mrr, <split>_rel_hits@k), the BCE over the relations
-(<split>_rel_loss) and the seconds the two splits took (rel_eval_s); the model is trained as before (1-N over entities).
+(<split>_rel_loss) and the seconds the two splits took (rel_eval_s); the model is trained as before (1-N over entities)
+unless --relation-weight > 0 adds the relation-prediction term (optim.RelationTerm: softmax cross-entropy of (s, ?, o)
+over all relations, weight lambda) to every step, on batches of --relation-batch train pairs (default: the pairs spread
+evenly over the epoch's entity batches); each record then carries train_rel_loss.  With --loss bce the BCE's mean over
+B x N makes its gradient about N times smaller than the relation term's: state the lambda of such a run.
 """
 import argparse
 import json
@@ -36,7 +40,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from rtucker_b200 import asymmetric, symmetric                      # noqa: E402
 from rtucker_b200 import train as T                                  # noqa: E402
-from rtucker_b200.data import DeviceEpoch, datasets_from_ids, relation_datasets_from_ids, wn18rr_fixture  # noqa: E402
+from rtucker_b200.data import (DeviceEpoch, datasets_from_ids, relation_datasets_from_ids,  # noqa: E402
+                               relation_train_dataset, wn18rr_fixture)
 from rtucker_b200.evaluation import evaluate_relations, rank_batch  # noqa: E402
 from rtucker_b200.rank import DEFAULT_GROWTH, set_rank              # noqa: E402
 
@@ -111,6 +116,10 @@ def main():
                     help="logit: also report logit-space ranks, the cross-entropy evaluation loss and tie counts")
     ap.add_argument("--relation-eval", action="store_true",
                     help="also report filtered relation prediction (s, ?, o) metrics and loss per split")
+    ap.add_argument("--relation-weight", type=float, default=0.0,
+                    help="lambda of the relation-prediction training term (0: entity loss only)")
+    ap.add_argument("--relation-batch", type=int, default=0,
+                    help="(s, o) pairs per step of the relation term (default: ceil(pairs / entity batches per epoch))")
     ap.add_argument("--rank", type=parse_rank, default=(10, 200, 200), help="starting rank r0,r1,r2")
     ap.add_argument("--rank-schedule", type=parse_schedule, default={},
                     help='rank changes at the start of epochs: "epoch:r0,r1,r2;epoch:r0,r1,r2"')
@@ -143,6 +152,11 @@ def main():
     train_loader = DeviceEpoch(train_ds, 512, dev, shuffle="host", drop_last=True)
     val_loader = DeviceEpoch(valid_ds, 512, dev, shuffle=False)
     test_loader = DeviceEpoch(test_ds, 512, dev, shuffle=False)
+    rel_loader, rel_batch = None, 0
+    if args.relation_weight > 0:
+        rel_train = relation_train_dataset(ids)
+        rel_batch = args.relation_batch or math.ceil(len(rel_train) / len(train_loader))
+        rel_loader = DeviceEpoch(rel_train, rel_batch, dev, shuffle="device", drop_last=True, seed=args.seed)
     crit = torch.nn.CrossEntropyLoss(reduction="mean") if args.loss == "ce" else torch.nn.BCELoss(reduction="mean")
     hist = []
     t_start = time.perf_counter()
@@ -159,10 +173,16 @@ def main():
         r = reg.step()
         torch.cuda.synchronize()
         t0 = time.perf_counter()
-        loss, gnorm = T.train_one_epoch(model, opt, crit, train_loader, regularization_coeff=r)
+        rel_rec = {}
+        if rel_loader is None:
+            loss, gnorm = T.train_one_epoch(model, opt, crit, train_loader, regularization_coeff=r)
+        else:
+            loss, gnorm, rel_rec["train_rel_loss"] = T.train_one_epoch(
+                model, opt, crit, train_loader, regularization_coeff=r, relation_loader=rel_loader,
+                relation_weight=args.relation_weight)
         torch.cuda.synchronize()
         rec = dict(epoch=epoch, rank=list(model.core.shape), train_loss=loss, grad_norm=gnorm,
-                   lr=opt.param_groups[0]["lr"], reg=r, epoch_s=time.perf_counter() - t0)
+                   lr=opt.param_groups[0]["lr"], reg=r, epoch_s=time.perf_counter() - t0, **rel_rec)
         if change is not None:
             rec["after_change"] = change
         if epoch % args.eval_every == 0 or epoch == 1 or epoch == args.epochs:
@@ -204,6 +224,7 @@ def main():
                                batch=512, optim="rsgd", recipe=args.recipe,
                                momentum=0.8, label_smoothing=0.1, seed=args.seed, score_variant=args.variant,
                                loss=args.loss, eval_space=args.eval_space, relation_eval=args.relation_eval,
+                               relation_weight=args.relation_weight, relation_batch=rel_batch,
                                device=torch.cuda.get_device_name(dev), power_limit_w=_power_limit(),
                                epochs=args.epochs, steps_per_epoch=len(train_loader)),
                    wall_s=time.perf_counter() - t_start, history=hist)

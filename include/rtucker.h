@@ -194,9 +194,10 @@ int rt_pair_bwd(const float* core, const float* s_rows, const float* o_rows, con
  *   dO = G^T qp     [n_local, r2]      (qp = q for the raw partial; pass q.A to fold a right factor)
  * O holds global entity rows [n_begin, n_begin+n_local); tgt_idx holds GLOBAL entity ids.
  * loss_sum is a double[1] (un-normalised sum over the shard; divide by B_total*n_total).
- * variant: 0 = fp32 FFMA (parity path), 1 = tcgen05 TF32 tensor cores (looser tolerance),
+ * variant: 0 = fp32 FFMA (parity path),
  *          2 = warp-specialised tcgen05 kernel with power-of-two-scaled fp16 operands (same 11 significant
  *              bits as TF32, stated tolerance 2e-3); qp must be NULL or q (dO = G^T q).
+ *          Any other variant returns an error (the 3xTF32 tensor-core path is rt_score_bce_tc3).
  */
 size_t rt_score_bce_ws_bytes(int B, int n_local, int r2, int variant);
 int rt_score_bce_fwd_bwd(const float* q, const float* qp, const float* O,

@@ -18,8 +18,6 @@ int rt_score_bce_v3_phases(const float* q, const float* O, int B, int r2, int n_
 
 /* Debug: per-CTA, per-role (producer, MMA issuer, epilogue, flush) cycle counters [grid][4][10] int64; NULL = off. */
 int rt_score_v3_set_profile(long long* dev_buf);
-/* Debug: per-CTA, per-phase cycle counters of the variant-1 score kernel ([grid][12] int64); NULL = off. */
-int rt_score_tc_set_profile(long long* dev_buf);
 /* Debug: per-CTA cycle counters of rt_eigh's block Jacobi kernel ([grid][4] int64: phase A, sync, phase B, sync);
  * NULL = off. */
 int rt_eigh_set_profile(long long* dev_buf);

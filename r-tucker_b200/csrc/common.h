@@ -121,12 +121,6 @@ int score_dense(const float* q, const float* O, int B, int r2, int n_local, floa
 int lse_combine(const float2* part, int ngroups, int64_t ld, int B, float* out, cudaStream_t s);
 int ce_row_stats(const float* parts, int nparts, int B, int ld, float* stats, cudaStream_t s);
 
-// score_bce_tc.cu: BCE score variant 1 (TF32 tensor cores)
-size_t score_bce_tc_ws_bytes(int B, int n_local, int r2);
-int score_bce_tc(const float* q, const float* qp, const float* O, int B, int r2, int n_begin, int n_local, int n_total,
-                 int b_total, const int32_t* tgt_off, const int32_t* tgt_idx, float label_smoothing, double* loss_sum,
-                 float* H, float* dO, void* ws, void* stream);
-
 // gram_sym.cu: X^T X on the fp64 tensor cores
 bool gram_sym_supported(int r);
 size_t gram_sym_ws_bytes(int n, int r);

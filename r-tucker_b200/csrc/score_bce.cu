@@ -8,7 +8,7 @@
 //
 // This file is the FP32-FFMA variant (parity path, and the thin-rank path r2 ~ 20).
 // Work per launch: 6*B*N*r2 flops (three B x N x r2 contractions), algorithmic bytes 8*N*r2
-// (read O once, write dO once).  The tcgen05 variant lives in score_bce_tc.cu.
+// (read O once, write dO once).  The tcgen05 variants live in apply_tc.cu (3) and score_bce_v3.cu (2).
 //
 // Decomposition: persistent CTAs; a CTA owns entity tiles of 64 rows; per tile it loops over the
 // batch in chunks of 64 queries:  Z = Q_chunk O_tile^T  ->  elementwise (p, loss, G)  ->
@@ -522,9 +522,8 @@ __global__ void ce_empty_rows_kernel(const int32_t* __restrict__ off, int B, con
 
 }  // namespace
 
-// variant 1: tcgen05 TF32 (score_bce_tc.cu); variant 2: warp-specialised fp16 tcgen05 (score_bce_v3.cu)
+// variant 2: warp-specialised fp16 tcgen05 (score_bce_v3.cu)
 extern "C" size_t rt_score_bce_ws_bytes(int B, int n_local, int r2, int variant) {
-  if (variant == 1) return rt::score_bce_tc_ws_bytes(B, n_local, r2);
   if (variant == 2) return rt_score_bce_v3_ws_bytes(B, n_local, r2);
   Plan p = make_plan(n_local, r2, false);
   return rt::align_up((size_t)p.grid * B * r2 * sizeof(float), 256) + (size_t)p.grid * sizeof(double);
@@ -538,9 +537,6 @@ extern "C" int rt_score_bce_fwd_bwd(const float* q, const float* qp, const float
   RT_REQUIRE(B > 0 && r2 > 0 && r2 <= 256 && n_local >= 0 && n_total > 0 && b_total > 0,
              "rt_score_bce_fwd_bwd: bad shape B=%d r2=%d n_local=%d", B, r2, n_local);
   RT_REQUIRE(ws != nullptr, "rt_score_bce_fwd_bwd: workspace is NULL");
-  if (variant == 1)
-    return rt::score_bce_tc(q, qp, O, B, r2, n_begin, n_local, n_total, b_total, tgt_off, tgt_idx,
-                            label_smoothing, loss_sum, H, dO, ws, stream);
   if (variant == 2) {
     RT_REQUIRE(qp == nullptr || qp == q, "rt_score_bce_fwd_bwd: variant 2 computes dO = G^T q only (pass qp = NULL and "
                "fold the right factor into the following rt_apply)");

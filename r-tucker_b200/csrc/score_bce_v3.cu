@@ -24,8 +24,8 @@
 //   Query chunks are visited in boustrophedon order over the tiles, so the chunk at a tile boundary repeats: its Q
 //   image stays in shared memory and its H accumulator stays in TMEM (one flush and one reload less per tile).
 // Operands are fp16 scaled by powers of two (exact) chosen from the arrays' absolute maxima: 11 significant
-// bits like TF32 at twice the tensor rate and half the shared-memory footprint.  Stated tolerance: 2e-3 (same as
-// the TF32 kernel of score_bce_tc.cu); the fp32-FFMA kernel of score_bce.cu is the 1e-5 path.
+// bits like TF32 at twice the tensor rate and half the shared-memory footprint.  Stated tolerance: 2e-3; the
+// fp32-FFMA kernel of score_bce.cu and the 3xTF32 kernels of apply_tc.cu are the 1e-5 paths.
 //
 // Work per launch 6*B*N*r2 flop; algorithmic bytes 8*N*r2.
 #include "common.h"

@@ -40,6 +40,15 @@ def check_loss(loss):
         raise ValueError(f"loss must be one of {LOSSES}, got {loss!r}")
 
 
+SCORE_VARIANTS = (0, 2, 3)
+
+
+def check_score_variant(variant):
+    """The fused score kernels a step can select: 0 (fp32 FFMA), 2 (fp16-operand tcgen05) and 3 (3xTF32 tcgen05)."""
+    if variant not in SCORE_VARIANTS:
+        raise ValueError(f"score_variant must be one of {SCORE_VARIANTS}, got {variant!r}")
+
+
 def core_mode_product(ops, core, K, mode):
     """``core`` x_mode K^T, i.e. core[.., j, ..] <- sum_j' core[.., j', ..] K[j', j] for K fp64 [r_mode, rc]: ONE
     ops.apply over a permuted copy of the core that puts ``mode`` last.  Returns a (possibly non-contiguous) view of
@@ -156,6 +165,7 @@ class StepEngine:
         self.n_begin = int(n_begin)
         self.n_local = self.params[1].shape[0]
         self.n_total = int(n_total) if n_total is not None else self.n_local
+        check_score_variant(score_variant)
         self.score_variant = int(score_variant)
         dev = core.device
         self.dev = dev
@@ -337,17 +347,20 @@ class StepEngine:
         H = torch.empty(B, r2, dtype=core.dtype, device=self.dev)
         # variant 2 (warp-specialised fp16 tcgen05 kernel) returns dO = G^T q; the right factor A_O is folded into
         # the projection apply below (dO_raw lands in the not-yet-used direction buffer)
-        # variant 3 = the same at fp32 accuracy (3xTF32 tensor-core kernels); it falls back to variant 0 on shapes the
-        # tensor-core path does not take (thin ranks, short shards)
+        # variant 3 = the same at fp32 accuracy (3xTF32 tensor-core kernels)
+        # One order of fallbacks on shapes a path does not take: 2 -> 3 (r2 > 208) -> 0 (thin ranks, short shards)
         variant = self.score_variant
         if loss_kind == "ce" and variant not in (0, 3):
             raise ValueError(f"loss='ce' runs on score variants 0 (FFMA) and 3 (tensor cores), not {variant}")
-        if variant == 3 and not (getattr(ops, "HAS_SCORE_V3", False) and ops.score_tc3_supported(B, O.shape[0], r2)):
+        has_tc = getattr(ops, "HAS_SCORE_V3", False)
+        if variant == 2 and not (has_tc and ops.score_v3_supported(r2)):
+            variant = 3
+        if variant == 3 and not (has_tc and ops.score_tc3_supported(B, O.shape[0], r2)):
             variant = 0
         # variant 2 returns dO = G^T q and leaves the right factor A_O to the projection apply ("fold"): measured on real
         # WN18RR this is what keeps it from learning -- rounding G^T q to fp32 BEFORE the ill-conditioned A_O loses the
         # components along the weak directions of the core; variants 0 and 3 contract with qp = q A_O directly
-        fold_a = variant == 2 and getattr(ops, "HAS_SCORE_V3", False) and ops.score_v3_supported(r2)
+        fold_a = variant == 2
         dO_raw = self.dV_new[k_obj] if fold_a else None
         if loss_kind == "ce":
             self._score_ce(q, qp, O, targets, label_smoothing, variant, (bce_sum, H, dOp))
@@ -360,8 +373,7 @@ class StepEngine:
                                           centre=self.score_centre)
                 else:
                     ops.score_bce_fwd_bwd(q, qp, O, targets.off, targets.idx, label_smoothing, n_total=self.n_total,
-                                          b_total=B, n_begin=self.n_begin, variant=variant if variant == 3 else min(variant, 1),
-                                          out=(bce_sum, H, dOp))
+                                          b_total=B, n_begin=self.n_begin, variant=variant, out=(bce_sum, H, dOp))
         self._allreduce(H, bce_sum)
         with self._stage("query_bwd"):
             d_core, ds_rows, dr_rows = ops.query_bwd(core, r_rows, s_rows, H)

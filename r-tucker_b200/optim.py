@@ -18,7 +18,7 @@ from typing import Optional
 import torch
 from torch.optim import Optimizer
 
-from .engine import RelationTerm, SparseTargets, StepEngine, check_loss
+from .engine import RelationTerm, SparseTargets, StepEngine, check_loss, check_score_variant
 from .model import ScoreFn
 
 
@@ -51,6 +51,7 @@ class _RiemannianBase(Optimizer):
 
     def __init__(self, params, rank, max_lr, momentum_beta: Optional[float] = None, group=None,
                  n_total=None, n_begin=0, score_variant=3, ops=None, use_graphs=False):
+        check_score_variant(score_variant)      # the engine is built at the first fit: reject a bad value here
         self.rank = rank
         self.max_lr = max_lr
         self.lr = max_lr

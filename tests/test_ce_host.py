@@ -151,7 +151,7 @@ def _cpu_engine(variant):
     return eng, rel, sub, off, idx
 
 
-@pytest.mark.parametrize("variant", [1, 2])
+@pytest.mark.parametrize("variant", [2])
 def test_engine_rejects_ce_on_score_variants_without_it(variant):
     from rtucker_b200.engine import SparseTargets
     eng, rel, sub, off, idx = _cpu_engine(variant)

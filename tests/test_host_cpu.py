@@ -119,6 +119,21 @@ def _small_problem(sym, seed=4):
     return N, M, rank, B, core, R, S, O, batches
 
 
+@pytest.mark.parametrize("variant", [1, 4, -1])
+def test_unknown_score_variants_are_rejected_on_construction(variant):
+    """Score variants 0, 2 and 3 exist; the engine and the optimisers (which build their engine at the first fit)
+    reject any other value when they are constructed."""
+    from rtucker_b200 import asymmetric
+    N, M, rank, B, core, R, S, O, _ = _small_problem(False)
+    P = torch.nn.Parameter
+    with pytest.raises(ValueError, match="score_variant"):
+        StepEngine(P(core.clone()), [P(R.clone()), P(S.clone()), P(O.clone())], False, B, 0.8, score_variant=variant,
+                   ops=cpu_ops)
+    with pytest.raises(ValueError, match="score_variant"):
+        asymmetric.RSGDwithMomentum([P(core.clone()), P(S.clone()), P(R.clone()), P(O.clone())], rank, 10.0, 0.8,
+                                    score_variant=variant, ops=cpu_ops)
+
+
 @pytest.mark.parametrize("sym", [True, False])
 def test_engine_adam_matches_analytic_twin(sym):
     """SFTuckerAdam's state machine in the engine (device-side coefficients, kept DIRECTION + ratio instead of the

@@ -9,7 +9,7 @@ w = bench.WORKLOADS['wn18rr']; dev = torch.device('cuda')
 torch.manual_seed(20)
 model = asymmetric.R_TuckER((w['N'], w['M']), w['rank']); model.init(None); model.to(dev)
 opt = asymmetric.RSGDwithMomentum([model.core, model.S.weight, model.R.weight, model.O.weight], w['rank'], bench.LR, 0.8,
-                                  score_variant=int(sys.argv[1]) if len(sys.argv) > 1 else 1)
+                                  score_variant=int(sys.argv[1]) if len(sys.argv) > 1 else 3)
 g = torch.Generator().manual_seed(0)
 for it in range(4):
     sub = torch.randint(0, w['N'], (512,), generator=g).int().to(dev); rel = torch.randint(0, w['M'], (512,), generator=g).int().to(dev)

@@ -34,20 +34,19 @@ def case(B, N, r2, nnz_per=2, zstd=4.0, o_absmax=None, seed=1):
     off = torch.arange(0, (B + 1) * nnz_per, nnz_per).int().to(dev)
     idx = torch.randint(0, N, (B * nnz_per,), generator=g).int().to(dev)
     l0, H0, d0 = ops.score_bce_fwd_bwd(q, q, O, off, idx, 0.1, variant=0)
-    l1, H1, d1 = ops.score_bce_fwd_bwd(q, q, O, off, idx, 0.1, variant=1)
     l2, H2, d2 = ops.score_bce_fwd_bwd(q, None, O, off, idx, 0.1, variant=2, o_absmax=o_absmax)
     torch.cuda.synchronize()
     rel = lambda x, y: float((x.double() - y.double()).norm() / y.double().norm())
-    return (rel(l2, l0), rel(H2, H0), rel(d2, d0)), (rel(l1, l0), rel(H1, H0), rel(d1, d0))
+    return rel(l2, l0), rel(H2, H0), rel(d2, d0)
 
 quick = len(sys.argv) > 1
 shapes = [(128, 96, 16, 1, 4.0), (100, 1000, 20, 2, 4.0), (512, 5000, 200, 2, 4.0), (300, 777, 52, 3, 4.0),
           (512, 40943, 200, 2, 4.0), (512, 40943, 200, 2, 12.0), (64, 200, 176, 1, 4.0), (512, 3000, 208, 2, 4.0), (1, 5, 3, 1, 2.0),
           (130, 97, 7, 1, 3.0)]
 for (B, N, r2, nn, zs) in shapes:
-    e2, e1 = case(B, N, r2, nn, zs)
-    print(f"B={B} N={N} r2={r2} zstd={zs}: v2 rel err loss/H/dO =", ["%.2e" % e for e in e2], " v1:", ["%.2e" % e for e in e1], flush=True)
-print("hint=1.0:", ["%.2e" % e for e in case(512, 40943, 200, 2, 4.0, o_absmax=1.0)[0]])
+    e2 = case(B, N, r2, nn, zs)
+    print(f"B={B} N={N} r2={r2} zstd={zs}: v2 rel err loss/H/dO =", ["%.2e" % e for e in e2], flush=True)
+print("hint=1.0:", ["%.2e" % e for e in case(512, 40943, 200, 2, 4.0, o_absmax=1.0)])
 
 def timeit(fn, n=20):
     for _ in range(3): fn()
@@ -65,7 +64,7 @@ for (B, N, r2) in [(512, 40943, 200)] + ([] if quick else [(512, 1000000, 200)])
     q = (torch.randn(B, r2, generator=g) * 600).to(dev)
     off = torch.arange(0, (B + 1) * 2, 2).int().to(dev); idx = torch.randint(0, N, (B * 2,), generator=g).int().to(dev)
     outs = (torch.empty(1, dtype=torch.float64, device=dev), torch.empty(B, r2, device=dev), torch.empty(N, r2, device=dev))
-    for v in (0, 1, 2):
+    for v in (0, 2):
         ws = torch.empty(int(lib().rt_score_bce_ws_bytes(B, N, r2, v)) + 16, dtype=torch.uint8, device=dev)
         ms = timeit(lambda: ops.score_bce_fwd_bwd(q, None if v == 2 else q, O, off, idx, 0.1, variant=v, out=outs, ws=ws, o_absmax=1.0 if v == 2 else None))
         print(f"N={N} variant {v}: {ms*1e3:.1f} us  {6.0*B*N*r2/ms/1e9:.1f} TFLOP/s", flush=True)

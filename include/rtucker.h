@@ -366,6 +366,24 @@ int rt_small_project(const float* core, const float* core_old, const float* dS_o
                      const double* hyper, int r0, int r1, int r2, int sym,
                      float* pS_beta, double* K_R, double* K_S, double* K_O,
                      double* L_R, double* L_S, double* L_O, void* small_ws, void* stream);
+/*
+ * The same projection in two calls, for a step with momentum: the part that needs neither A_i nor hyper runs while
+ * rt_small_prepare's factorisation does, on the SMs the factorisation leaves idle.  Outputs are bit-identical to
+ * rt_small_prepare followed by rt_small_project.
+ * rt_small_prepare_project: rt_small_prepare plus the head of the projection (the transport of dS_old and the
+ *   products with the current core).  Its inputs must stay unchanged until rt_small_norm_project.
+ * rt_small_norm_project: rt_small_norm (adam == NULL) or rt_small_norm_adam, then the tail of the projection in the
+ *   same program: pS_beta, K_i and L_i exactly as rt_small_project returns them, with the beta that hyper[2] holds
+ *   after the norm.  M_i must be the matrices given to rt_small_prepare_project.
+ */
+int rt_small_prepare_project(const float* core, const float* core_old, const float* dS_old,
+                             const double* M_R, const double* M_S, const double* M_O,
+                             int r0, int r1, int r2, int sym, void* small_ws, void* stream);
+int rt_small_norm_project(const float* dS_g, const double* gram_R, const double* gram_S, const double* gram_O,
+                          double* hyper, double* adam, const double* M_R, const double* M_S, const double* M_O,
+                          int r0, int r1, int r2, int sym, double* norm_out, double* alpha_out,
+                          float* pS_beta, double* K_R, double* K_S, double* K_O,
+                          double* L_R, double* L_S, double* L_O, void* small_ws, void* stream);
 /* dS_dir = alpha * dS_g + pS_beta (pS_beta may be NULL).  asymmetric/optim.py:92 (core part). */
 int rt_core_axpby(const float* dS_g, const double* alpha_dev, const float* pS_beta, int count,
                   float* dS_dir, void* stream);

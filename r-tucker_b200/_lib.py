@@ -70,6 +70,8 @@ PROTOTYPES = {
     "rt_small_norm": (i32, [vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp]),
     "rt_small_norm_adam": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp, vp, vp, vp]),
     "rt_small_project": (i32, [vp] * 7 + [i32, i32, i32, i32] + [vp] * 9),
+    "rt_small_prepare_project": (i32, [vp] * 6 + [i32, i32, i32, i32] + [vp] * 2),
+    "rt_small_norm_project": (i32, [vp] * 9 + [i32, i32, i32, i32] + [vp] * 11),
     "rt_core_axpby": (i32, [vp, vp, vp, i32, vp, vp]),
     "rt_small_retract": (i32, [vp] * 6 + [i32, i32, i32, i32] + [vp] * 12),
     "rt_epoch_batch": (i32, [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp, i32, vp]),

@@ -30,6 +30,13 @@ __device__ __forceinline__ void grid_barrier(unsigned int* bar, unsigned int& ta
   __syncthreads();
 }
 
+// Programmatic dependent launch.  launch_dependents lets the next kernel of the stream, if it was launched with
+// programmatic stream serialization, start once every CTA of this grid has signalled (or exited).  wait blocks until
+// the grids this one depends on programmatically have completed and their writes are visible; without such a
+// dependency it returns at once.
+__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;\n" ::: "memory"); }
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;\n" ::: "memory"); }
+
 // 16-byte asynchronous global -> shared copy (L2 only), to a shared-memory address or a generic pointer into shared
 // memory; completion through commit / wait_group or wait_all
 __device__ __forceinline__ void cp_async16(uint32_t dst_smem, const void* src) {

@@ -58,7 +58,7 @@ Layout make_layout(int r0, int r1, int r2, int B) {
     L.sub[i] = ws.take(rt::subspace_ws_bytes(2 * (int)r, (int)r));
   }
   L.sub_shared = ws.take(rt::subspace_shared_ws_bytes());
-  L.exec_bar = take(32);
+  L.exec_bar = take(32);        // two grid-barrier counters, 128 bytes apart (Ctx::flush)
   L.gemm_partial = take(kPartialArenaBytes / sizeof(double));
   int rmax = r0 > r1 ? r0 : r1; rmax = rmax > r2 ? rmax : r2;
   L.gram_ws = ws.take(rt_gram_ws_bytes(B > 0 ? B : 1, rmax, rmax));
@@ -77,7 +77,7 @@ Layout make_layout(int r0, int r1, int r2, int B) {
 // ---- recording context: operations are RECORDED with the byte ranges they touch, scheduled into dependency
 // levels and executed by one persistent launch per flush() (small_exec.cuh) ------------------------------------------
 struct Range { const char* lo; const char* hi; };
-struct Rec { Op op; Range rd[4]; int nrd; Range wr[2]; int nwr; };
+struct Rec { Op op; Range rd[4]; int nrd; Range wr[4]; int nwr; };
 
 // C[m,n] = alpha * sum_{k1<K1,k2<K2} A[m,(k1,k2)] B[(k1,k2),n] + beta * C[m,n]      (batched): what Ctx::mode_prod and
 // Ctx::unfold_gram hand to Ctx::gemm
@@ -97,6 +97,8 @@ template <typename T> struct DT;
 template <> struct DT<float> { static constexpr int v = DT_F32; };
 template <> struct DT<double> { static constexpr int v = DT_F64; };
 static inline size_t dsize(int t) { return t == DT_F64 ? 8 : 4; }
+
+enum class Launch { kCooperative, kAfterPrimary };
 
 struct Ctx {
   Layout L;
@@ -132,25 +134,43 @@ struct Ctx {
     recs.push_back(rec);
   }
 
-  // Execute what has been recorded (one cooperative launch); direct launches may follow on the stream.
-  void flush() {
+  // Execute what has been recorded as one cooperative launch of `ctas` CTAs (0: kExecCtasPerSm per SM); direct
+  // launches may follow on the stream.  Launch::kAfterPrimary makes the program the programmatic dependent of the
+  // kernel enqueued just before it: it may start while that kernel runs, on the SMs that kernel leaves free, and it
+  // ends only after that kernel has completed (pdl_wait).  No memset may come between the two launches, so such a
+  // program counts on the second counter of exec_bar instead: every cooperative flush zeroes both, and only a
+  // dependent program advances the second.
+  void flush(int ctas = 0, Launch mode = Launch::kCooperative) {
     if (err || recs.empty()) { recs.clear(); return; }
     std::stable_sort(recs.begin(), recs.end(), [](const Rec& a, const Rec& b) { return a.op.level < b.op.level; });
     static Program prog;     // host staging of the parameter block (copied by the launch)
+    const bool dependent = mode == Launch::kAfterPrimary;
     prog.nops = (int)recs.size();
-    prog.bar = reinterpret_cast<unsigned int*>(base + L.exec_bar);
+    prog.bar = reinterpret_cast<unsigned int*>(base + L.exec_bar) + (dependent ? 32 : 0);
     for (int i = 0; i < prog.nops; ++i) prog.ops[i] = recs[i].op;
     recs.clear();
     partial_off = 0;
     dot_off = 0;
     const size_t smem = sizeof(double) * kExecWarps * XT * XLD;
-    if (cudaMemsetAsync(prog.bar, 0, 256, s) != cudaSuccess ||
-        cudaFuncSetAttribute(small_exec_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    if ((!dependent && cudaMemsetAsync(base + L.exec_bar, 0, 256, s) != cudaSuccess) ||
+        cudaFuncSetAttribute(small_exec_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) !=
+            cudaSuccess) {
       err = 1; return;
     }
+    cudaLaunchAttribute attr[2];
+    attr[0].id = cudaLaunchAttributeCooperative;
+    attr[0].val.cooperative = 1;
+    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[1].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(ctas > 0 ? ctas : kExecCtasPerSm * rt::sm_count());
+    cfg.blockDim = dim3(kExecThreads);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = s;
+    cfg.attrs = attr;
+    cfg.numAttrs = dependent ? 2 : 1;
     void* args[] = {(void*)&prog};
-    if (cudaLaunchCooperativeKernel((const void*)small_exec_kernel, dim3(kExecCtasPerSm * rt::sm_count()), dim3(kExecThreads), args,
-                                    smem, s) != cudaSuccess) err = 1;
+    if (cudaLaunchKernelExC(&cfg, (const void*)small_exec_kernel, args) != cudaSuccess) err = 1;
     ++rt::g_launches;
   }
 
@@ -349,6 +369,8 @@ struct Ctx {
     rec.rd[rec.nrd++] = range(adam, 64);
     rec.wr[rec.nwr++] = range(norm_out, 8);
     rec.wr[rec.nwr++] = range(alpha_out, 8);
+    rec.wr[rec.nwr++] = range(hyper + 2, 8);     // the momentum coefficient
+    rec.wr[rec.nwr++] = range(adam, 64);         // the state, updated in place
     push(rec);
   }
   void zero64(double* z, int64_t n) { ew(EW_ZERO64, nullptr, DT_F64, 0, nullptr, 0, z, DT_F64, n * 8, n, 0.0, nullptr, 0.0, nullptr); }
@@ -434,6 +456,98 @@ void grouped_contract(Ctx& c, const T* X, const T* const B[3], const T* const Wa
   c.mode_prod(2, Wb[2], st_o[2], st_i[2], d[2], d[2], U2, d, out, 1.0, 1.0);
 }
 
+// Records rt_small_prepare's program (the fp64 core, its unfolding Grams, ||core||^2) and fills the batch of the
+// factorisation that follows it.  Returns its largest order.
+int prepare_program(Ctx& c, const float* core, int sym, SpdBatch& b) {
+  const int d[3] = {c.r(0), c.r(1), c.r(2)};
+  double* C64 = c.p(c.L.C64);
+  c.to64(core, C64, c.L.c);
+  for (int i = 0; i < 3; ++i) c.unfold_gram(i, C64, d, C64, d[i], c.p(c.L.Gm[i]), d[i], 1.0, 0.0);
+  if (sym) {
+    c.axpby(c.p(c.L.Gm[1]), c.p(c.L.Gm[2]), c.p(c.L.Gm[1]), (int64_t)d[1] * d[1], 1.0, nullptr, 1.0, nullptr);
+    c.axpby(c.p(c.L.Gm[1]), nullptr, c.p(c.L.Gm[2]), (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
+  }
+  int nmax = 0;
+  for (int i = 0; i < 3; ++i) {
+    b.p[i].G = c.p(c.L.Gm[i]); b.p[i].L = nullptr; b.p[i].Linv = nullptr; b.p[i].Ginv = c.p(c.L.Ainv[i]);
+    b.p[i].n = d[i];
+    nmax = d[i] > nmax ? d[i] : nmax;
+  }
+  c.dot(C64, DT_F64, C64, DT_F64, c.L.c, 1.0, c.p(c.L.coresq), 0);
+  return nmax;
+}
+
+// The projection of rt_small_project in two parts.  The head transports the previous direction: pS (fp32, in T6) and
+// KC_i (fp64).  It reads neither the factorisation's Grams nor its inverses, nor hyper, so it can run alongside
+// rt_small_prepare's factorisation (rt_small_prepare_project).  The tail scales by beta = hyper[2] and applies the
+// inverses: pS_beta = beta pS, K_i = beta KC_i Ainv_i, L_i = -M_i K_i.
+void project_head(Ctx& c, const float* core, const float* core_old, const float* dS_old, const double* const M[3],
+                  int sym) {
+  const int d[3] = {c.r(0), c.r(1), c.r(2)};
+  // All O(r^4) contractions of the projection run in fp32 (inputs are the fp32 parameters themselves and
+  // the result only needs fp32 accuracy); the r x r solves with (S_(i)S_(i)^T)^-1 stay in fp64.
+  const float* Cf = core;
+  const float* Co = core_old;
+  const float* Xo = dS_old;
+  float* Mf[3];
+  for (int i = 0; i < 3; ++i) Mf[i] = reinterpret_cast<float*>(c.p(c.L.tmpM[i]));
+  for (int i = 0; i < (sym ? 2 : 3); ++i) c.to32plain(M[i], Mf[i], 2 * (int64_t)d[i] * d[i]);
+  if (sym) Mf[2] = Mf[1];
+  const float* Wa[3]; const float* Wb[3]; int64_t st_o[3], st_i[3];
+  for (int i = 0; i < 3; ++i) { Wa[i] = Mf[i]; Wb[i] = Mf[i] + d[i]; st_o[i] = 2 * d[i]; st_i[i] = 1; }
+  const float* Cb[3] = {Co, Co, Co};
+  float* D = c.Tf(2); float* Ta = c.Tf(3); float* U1 = c.Tf(4); float* U2 = c.Tf(5);
+  float* pS = c.Tf(6);
+  grouped_contract<float>(c, Xo, Cb, Wa, Wb, st_o, st_i, D, Ta, Ta, U1, U2, pS);
+  // KC_i (2 r_i x r_i) in fp32 scratch (the eigenvector slots are idle here), converted to fp64 afterwards
+  float* KCf[3] = {reinterpret_cast<float*>(c.p(c.L.Vf[0])), reinterpret_cast<float*>(c.p(c.L.Vf[1])),
+                   reinterpret_cast<float*>(c.p(c.L.Vf[2]))};
+  double* KC[3] = {c.p(c.L.KC[0]), c.p(c.L.KC[1]), c.p(c.L.KC[2])};
+  // KC_2 = [U1_(2) ; U2_(2)] C_(2)^T
+  c.unfold_gram<float>(2, U1, d, Cf, d[2], KCf[2], d[2], 1.0, 0.0);
+  c.unfold_gram<float>(2, U2, d, Cf, d[2], KCf[2] + (int64_t)d[2] * d[2], d[2], 1.0, 0.0);
+  // KC_1: V1 = D x2 W2a + Ta x2 W2b ; V2 = Ta x2 W2a     (reuse U1/U2 storage after KC_2)
+  // Every intermediate has its own buffer (T0, T1, T7 and both halves are idle during the projection): the levels come
+  // from byte-range hazards, so REUSING U1 / U2 / Ta / D here serialised the three KC chains behind each other
+  // (16 levels); with private buffers the KC_0 chain starts at level 0 and KC_1 right after the first mode products.
+  float* V1 = c.Tf(0); float* V2 = c.Tf(0) + c.L.c;
+  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], D, d, V1, 1.0, 0.0);
+  c.mode_prod<float>(2, Wb[2], st_o[2], st_i[2], d[2], d[2], Ta, d, V1, 1.0, 1.0);
+  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], Ta, d, V2, 1.0, 0.0);
+  c.unfold_gram<float>(1, V1, d, Cf, d[1], KCf[1], d[1], 1.0, 0.0);
+  c.unfold_gram<float>(1, V2, d, Cf, d[1], KCf[1] + (int64_t)d[1] * d[1], d[1], 1.0, 0.0);
+  // KC_0: Ea = Co x1 W1a, Eb = Co x1 W1b, F = Xo x1 W1a + Eb ; Z1 = F x2 W2a + Ea x2 W2b ; Z2 = Ea x2 W2a
+  float* Ea = c.Tf(1); float* F = c.Tf(1) + c.L.c;
+  c.mode_prod<float>(1, Wa[1], st_o[1], st_i[1], d[1], d[1], Co, d, Ea, 1.0, 0.0);
+  c.mode_prod<float>(1, Wa[1], st_o[1], st_i[1], d[1], d[1], Xo, d, F, 1.0, 0.0);
+  c.mode_prod<float>(1, Wb[1], st_o[1], st_i[1], d[1], d[1], Co, d, F, 1.0, 1.0);
+  float* Z1 = c.Tf(7); float* Z2 = c.Tf(7) + c.L.c;
+  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], F, d, Z1, 1.0, 0.0);
+  c.mode_prod<float>(2, Wb[2], st_o[2], st_i[2], d[2], d[2], Ea, d, Z1, 1.0, 1.0);
+  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], Ea, d, Z2, 1.0, 0.0);
+  c.unfold_gram<float>(0, Z1, d, Cf, d[0], KCf[0], d[0], 1.0, 0.0);
+  c.unfold_gram<float>(0, Z2, d, Cf, d[0], KCf[0] + (int64_t)d[0] * d[0], d[0], 1.0, 0.0);
+  for (int i = 0; i < 3; ++i) c.to64(KCf[i], KC[i], 2 * (int64_t)d[i] * d[i]);
+  if (sym) c.axpby(KC[1], KC[2], KC[1], 2 * (int64_t)d[1] * d[1], 1.0, nullptr, 1.0, nullptr);
+}
+
+void project_tail(Ctx& c, const double* const M[3], const double* hyper, int sym, float* pS_beta, double* const K[3],
+                  double* const L[3]) {
+  const int d[3] = {c.r(0), c.r(1), c.r(2)};
+  c.scale32(c.Tf(6), pS_beta, c.L.c, 1.0, hyper + 2);
+  const int nm = sym ? 2 : 3;
+  for (int i = 0; i < nm; ++i) {
+    // K_i = beta * KC_i Ainv_i ;  L_i = -M_i K_i
+    c.matmul(c.p(c.L.KC[i]), d[i], false, c.p(c.L.Ainv[i]), d[i], false, K[i], d[i], 2 * d[i], d[i], d[i], 1.0, 0.0,
+             hyper + 2);
+    c.matmul(M[i], 2 * d[i], false, K[i], d[i], false, L[i], d[i], d[i], d[i], 2 * d[i], -1.0, 0.0);
+  }
+  if (sym && K[2] && K[2] != K[1]) {
+    c.axpby(K[1], nullptr, K[2], 2 * (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
+    c.axpby(L[1], nullptr, L[2], (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
+  }
+}
+
 }  // namespace
 
 extern "C" size_t rt_small_ws_bytes(int r0, int r1, int r2, int B) {
@@ -447,25 +561,29 @@ extern "C" int rt_small_prepare(const float* core, int r0, int r1, int r2, int s
   RT_REQUIRE(!sym || r1 == r2, "rt_small_prepare: SF-Tucker needs r1 == r2");
   Ctx c{make_layout(r0, r1, r2, 0), (char*)small_ws, (cudaStream_t)stream};
   // layout must not depend on B for the persistent slots: they precede every B-dependent slot
-  double* C64 = c.p(c.L.C64);
-  c.to64(core, C64, c.L.c);
-  const int d[3] = {r0, r1, r2};
-  for (int i = 0; i < 3; ++i) c.unfold_gram(i, C64, d, C64, d[i], c.p(c.L.Gm[i]), d[i], 1.0, 0.0);
-  if (sym) {
-    c.axpby(c.p(c.L.Gm[1]), c.p(c.L.Gm[2]), c.p(c.L.Gm[1]), (int64_t)r1 * r1, 1.0, nullptr, 1.0, nullptr);
-    c.axpby(c.p(c.L.Gm[1]), nullptr, c.p(c.L.Gm[2]), (int64_t)r1 * r1, 1.0, nullptr, 0.0, nullptr);
-  }
   SpdBatch b{};
-  int nmax = 0;
-  for (int i = 0; i < 3; ++i) {
-    b.p[i].G = c.p(c.L.Gm[i]); b.p[i].L = nullptr; b.p[i].Linv = nullptr; b.p[i].Ginv = c.p(c.L.Ainv[i]);
-    b.p[i].n = d[i];
-    nmax = d[i] > nmax ? d[i] : nmax;
-  }
-  c.dot(C64, DT_F64, C64, DT_F64, c.L.c, 1.0, c.p(c.L.coresq), 0);
+  const int nmax = prepare_program(c, core, sym, b);
   int rc = c.spd(b, 3, nmax);
   if (rc) return rc;
   return finish(c, "rt_small_prepare");
+}
+
+extern "C" int rt_small_prepare_project(const float* core, const float* core_old, const float* dS_old,
+                                        const double* M_R, const double* M_S, const double* M_O, int r0, int r1,
+                                        int r2, int sym, void* small_ws, void* stream) {
+  RT_REQUIRE(small_ws != nullptr && r0 > 0 && r1 > 0 && r2 > 0, "rt_small_prepare_project: bad arguments");
+  RT_REQUIRE(!sym || r1 == r2, "rt_small_prepare_project: SF-Tucker needs r1 == r2");
+  Ctx c{make_layout(r0, r1, r2, 0), (char*)small_ws, (cudaStream_t)stream};
+  SpdBatch b{};
+  const int nmax = prepare_program(c, core, sym, b);
+  int rc = c.spd(b, 3, nmax);
+  if (rc) return rc;
+  // The factorisation occupies one SM per problem and leaves the others idle for ~0.3 ms at r = 200.  The head runs
+  // there, as its programmatic dependent on a grid that fits beside it; its results do not depend on the grid size.
+  const double* M[3] = {M_R, M_S, sym ? M_S : M_O};
+  project_head(c, core, core_old, dS_old, M, sym);
+  c.flush(kExecCtasPerSm * std::max(1, rt::sm_count() - 3), Launch::kAfterPrimary);
+  return finish(c, "rt_small_prepare_project");
 }
 
 extern "C" size_t rt_small_ainv_offset(int mode, int r0, int r1, int r2) {
@@ -522,9 +640,13 @@ extern "C" int rt_small_grad(const float* core, const float* d_core, const float
   return finish(c, "rt_small_grad");
 }
 
+// The norm's program.  With `tail` it also records the projection's tail (project_tail) after it: for TuckerAdam
+// the tail reads the momentum coefficient that adam_finish writes.
+struct ProjectTail { const double* M[3]; float* pS_beta; double* K[3]; double* L[3]; };
+
 static int small_norm_impl(const float* dS_g, const double* gram_R, const double* gram_S, const double* gram_O,
                            double* hyper, double* adam, int r0, int r1, int r2, int sym, double* norm_out,
-                           double* alpha_out, void* small_ws, void* stream) {
+                           double* alpha_out, const ProjectTail* tail, void* small_ws, void* stream) {
   Ctx c{make_layout(r0, r1, r2, 0), (char*)small_ws, (cudaStream_t)stream};
   double* sq = c.p(c.L.scal);
   c.dot(dS_g, DT_F32, dS_g, DT_F32, c.L.c, 1.0, sq, 0);
@@ -533,7 +655,8 @@ static int small_norm_impl(const float* dS_g, const double* gram_R, const double
   if (!sym) c.dot(gram_O, DT_F64, c.p(c.L.Gm[2]), DT_F64, (int64_t)r2 * r2, 1.0, sq, 1);
   if (adam) c.adam_finish(sq, hyper, adam, norm_out, alpha_out);
   else c.norm_finish(sq, hyper, norm_out, alpha_out);
-  return finish(c, "rt_small_norm");
+  if (tail) project_tail(c, tail->M, hyper, sym, tail->pS_beta, tail->K, tail->L);
+  return finish(c, tail ? "rt_small_norm_project" : "rt_small_norm");
 }
 
 extern "C" int rt_small_norm(const float* dS_g, const double* gram_R, const double* gram_S,
@@ -541,15 +664,27 @@ extern "C" int rt_small_norm(const float* dS_g, const double* gram_R, const doub
                              double* norm_out, double* alpha_out, void* small_ws, void* stream) {
   RT_REQUIRE(small_ws != nullptr, "rt_small_norm: workspace is NULL");
   return small_norm_impl(dS_g, gram_R, gram_S, gram_O, const_cast<double*>(hyper), nullptr, r0, r1, r2, sym, norm_out,
-                         alpha_out, small_ws, stream);
+                         alpha_out, nullptr, small_ws, stream);
 }
 
 extern "C" int rt_small_norm_adam(const float* dS_g, const double* gram_R, const double* gram_S,
                                   const double* gram_O, double* hyper, double* adam, int r0, int r1, int r2, int sym,
                                   double* norm_out, double* alpha_out, void* small_ws, void* stream) {
   RT_REQUIRE(small_ws != nullptr && adam != nullptr, "rt_small_norm_adam: NULL argument");
-  return small_norm_impl(dS_g, gram_R, gram_S, gram_O, hyper, adam, r0, r1, r2, sym, norm_out, alpha_out, small_ws,
-                         stream);
+  return small_norm_impl(dS_g, gram_R, gram_S, gram_O, hyper, adam, r0, r1, r2, sym, norm_out, alpha_out, nullptr,
+                         small_ws, stream);
+}
+
+extern "C" int rt_small_norm_project(const float* dS_g, const double* gram_R, const double* gram_S,
+                                     const double* gram_O, double* hyper, double* adam, const double* M_R,
+                                     const double* M_S, const double* M_O, int r0, int r1, int r2, int sym,
+                                     double* norm_out, double* alpha_out, float* pS_beta, double* K_R, double* K_S,
+                                     double* K_O, double* L_R, double* L_S, double* L_O, void* small_ws,
+                                     void* stream) {
+  RT_REQUIRE(small_ws != nullptr, "rt_small_norm_project: workspace is NULL");
+  const ProjectTail tail{{M_R, M_S, sym ? M_S : M_O}, pS_beta, {K_R, K_S, K_O}, {L_R, L_S, L_O}};
+  return small_norm_impl(dS_g, gram_R, gram_S, gram_O, hyper, adam, r0, r1, r2, sym, norm_out, alpha_out, &tail,
+                         small_ws, stream);
 }
 
 extern "C" int rt_small_project(const float* core, const float* core_old, const float* dS_old,
@@ -558,68 +693,12 @@ extern "C" int rt_small_project(const float* core, const float* core_old, const 
                                 double* K_R, double* K_S, double* K_O, double* L_R, double* L_S,
                                 double* L_O, void* small_ws, void* stream) {
   RT_REQUIRE(small_ws != nullptr, "rt_small_project: workspace is NULL");
-  (void)core;  // the current core is already resident as C64 (rt_small_prepare)
   Ctx c{make_layout(r0, r1, r2, 0), (char*)small_ws, (cudaStream_t)stream};
-  const int d[3] = {r0, r1, r2};
   const double* M[3] = {M_R, M_S, sym ? M_S : M_O};
-  double* Kout[3] = {K_R, K_S, K_O};
-  double* Lout[3] = {L_R, L_S, L_O};
-  // All O(r^4) contractions of the projection run in fp32 (inputs are the fp32 parameters themselves and
-  // the result only needs fp32 accuracy); the r x r solves with (S_(i)S_(i)^T)^-1 stay in fp64.
-  const float* Cf = core;
-  const float* Co = core_old;
-  const float* Xo = dS_old;
-  float* Mf[3];
-  for (int i = 0; i < 3; ++i) Mf[i] = reinterpret_cast<float*>(c.p(c.L.tmpM[i]));
-  for (int i = 0; i < (sym ? 2 : 3); ++i) c.to32plain(M[i], Mf[i], 2 * (int64_t)d[i] * d[i]);
-  if (sym) Mf[2] = Mf[1];
-  const float* Wa[3]; const float* Wb[3]; int64_t st_o[3], st_i[3];
-  for (int i = 0; i < 3; ++i) { Wa[i] = Mf[i]; Wb[i] = Mf[i] + d[i]; st_o[i] = 2 * d[i]; st_i[i] = 1; }
-  const float* Cb[3] = {Co, Co, Co};
-  float* D = c.Tf(2); float* Ta = c.Tf(3); float* U1 = c.Tf(4); float* U2 = c.Tf(5);
-  float* pS = c.Tf(6);
-  grouped_contract<float>(c, Xo, Cb, Wa, Wb, st_o, st_i, D, Ta, Ta, U1, U2, pS);
-  c.scale32(pS, pS_beta, c.L.c, 1.0, hyper + 2);
-  // KC_i (2 r_i x r_i) in fp32 scratch (the eigenvector slots are idle here), converted to fp64 afterwards
-  float* KCf[3] = {reinterpret_cast<float*>(c.p(c.L.Vf[0])), reinterpret_cast<float*>(c.p(c.L.Vf[1])),
-                   reinterpret_cast<float*>(c.p(c.L.Vf[2]))};
-  double* KC[3] = {c.p(c.L.KC[0]), c.p(c.L.KC[1]), c.p(c.L.KC[2])};
-  // KC_2 = [U1_(2) ; U2_(2)] C_(2)^T
-  c.unfold_gram<float>(2, U1, d, Cf, d[2], KCf[2], d[2], 1.0, 0.0);
-  c.unfold_gram<float>(2, U2, d, Cf, d[2], KCf[2] + (int64_t)d[2] * d[2], d[2], 1.0, 0.0);
-  // KC_1: V1 = D x2 W2a + Ta x2 W2b ; V2 = Ta x2 W2a     (reuse U1/U2 storage after KC_2)
-  // Every intermediate has its own buffer (T0, T1, T7 and both halves are idle during the projection): the levels come
-  // from byte-range hazards, so REUSING U1 / U2 / Ta / D here serialised the three KC chains behind each other
-  // (16 levels); with private buffers the KC_0 chain starts at level 0 and KC_1 right after the first mode products.
-  float* V1 = c.Tf(0); float* V2 = c.Tf(0) + c.L.c;
-  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], D, d, V1, 1.0, 0.0);
-  c.mode_prod<float>(2, Wb[2], st_o[2], st_i[2], d[2], d[2], Ta, d, V1, 1.0, 1.0);
-  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], Ta, d, V2, 1.0, 0.0);
-  c.unfold_gram<float>(1, V1, d, Cf, d[1], KCf[1], d[1], 1.0, 0.0);
-  c.unfold_gram<float>(1, V2, d, Cf, d[1], KCf[1] + (int64_t)d[1] * d[1], d[1], 1.0, 0.0);
-  // KC_0: Ea = Co x1 W1a, Eb = Co x1 W1b, F = Xo x1 W1a + Eb ; Z1 = F x2 W2a + Ea x2 W2b ; Z2 = Ea x2 W2a
-  float* Ea = c.Tf(1); float* F = c.Tf(1) + c.L.c;
-  c.mode_prod<float>(1, Wa[1], st_o[1], st_i[1], d[1], d[1], Co, d, Ea, 1.0, 0.0);
-  c.mode_prod<float>(1, Wa[1], st_o[1], st_i[1], d[1], d[1], Xo, d, F, 1.0, 0.0);
-  c.mode_prod<float>(1, Wb[1], st_o[1], st_i[1], d[1], d[1], Co, d, F, 1.0, 1.0);
-  float* Z1 = c.Tf(7); float* Z2 = c.Tf(7) + c.L.c;
-  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], F, d, Z1, 1.0, 0.0);
-  c.mode_prod<float>(2, Wb[2], st_o[2], st_i[2], d[2], d[2], Ea, d, Z1, 1.0, 1.0);
-  c.mode_prod<float>(2, Wa[2], st_o[2], st_i[2], d[2], d[2], Ea, d, Z2, 1.0, 0.0);
-  c.unfold_gram<float>(0, Z1, d, Cf, d[0], KCf[0], d[0], 1.0, 0.0);
-  c.unfold_gram<float>(0, Z2, d, Cf, d[0], KCf[0] + (int64_t)d[0] * d[0], d[0], 1.0, 0.0);
-  for (int i = 0; i < 3; ++i) c.to64(KCf[i], KC[i], 2 * (int64_t)d[i] * d[i]);
-  if (sym) c.axpby(KC[1], KC[2], KC[1], 2 * (int64_t)d[1] * d[1], 1.0, nullptr, 1.0, nullptr);
-  const int nm = sym ? 2 : 3;
-  for (int i = 0; i < nm; ++i) {
-    // K_i = beta * KC_i Ainv_i ;  L_i = -M_i K_i
-    c.matmul(KC[i], d[i], false, c.p(c.L.Ainv[i]), d[i], false, Kout[i], d[i], 2 * d[i], d[i], d[i], 1.0, 0.0, hyper + 2);
-    c.matmul(M[i], 2 * d[i], false, Kout[i], d[i], false, Lout[i], d[i], d[i], d[i], 2 * d[i], -1.0, 0.0);
-  }
-  if (sym && K_O && K_O != K_S) {
-    c.axpby(K_S, nullptr, K_O, 2 * (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
-    c.axpby(L_S, nullptr, L_O, (int64_t)d[1] * d[1], 1.0, nullptr, 0.0, nullptr);
-  }
+  double* const K[3] = {K_R, K_S, K_O};
+  double* const L[3] = {L_R, L_S, L_O};
+  project_head(c, core, core_old, dS_old, M, sym);
+  project_tail(c, M, hyper, sym, pS_beta, K, L);
   return finish(c, "rt_small_project");
 }
 

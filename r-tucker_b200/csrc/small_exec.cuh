@@ -444,6 +444,9 @@ small_exec_kernel(const __grid_constant__ Program prog) {
     printf("program end (%d ops)\n", nops);
   }
 #endif
+  // A program launched as a programmatic dependent (Ctx::flush, Launch::kAfterPrimary) ends only after the kernel
+  // before it has completed, so everything later on the stream sees that kernel's results.  Otherwise a no-op.
+  pdl_wait();
 }
 
 }  // namespace small

@@ -67,6 +67,9 @@ constexpr int SPD_NB = 8;
 constexpr int SPD_THREADS = 512, SPD_TPR = 2;
 __global__ void __launch_bounds__(SPD_THREADS, 1)
 spd_blocked_kernel(SpdBatch batch) {
+  // an executor program launched as this kernel's programmatic dependent (rt_small_prepare_project) starts on the SMs
+  // the batch leaves idle; it must not touch the batch's matrices, and its end waits for this grid
+  pdl_launch_dependents();
   extern __shared__ double sm[];
   const SpdProblem P = batch.p[blockIdx.x];
   const int n = P.n;

@@ -331,8 +331,20 @@ class StepEngine:
         B = rel_idx.shape[0]
         self._set_hyper(self._hyper_vals[0] if self._hyper_vals else lr_hint, reg, self.beta,
                         normalize_grad if normalize_grad else 0.0)
+        # momentum: the previous direction is transported to the current point.  The transport Grams
+        # M_k = U_k^T [U_old_k | dV_dir_k] come from the previous retraction's own small matrices (no N-sized pass, no
+        # all-reduce: replicated); see rt_small_retract.  Most of the projection depends on nothing this fit() computes
+        # and runs alongside the factorisation of the Gram inverses; norm_project() finishes it.  A small stage without
+        # that split (the fp64 stand-in the CPU tests inject as ``ops``) computes the projection in one project() call.
+        use_momentum = self.beta is not None and self.has_old
+        split = use_momentum and hasattr(small, "norm_project")
+        M = self.M_next
+        M_O = M[2] if not sym else M[1]
         with self._stage("small_prepare"):
-            small.prepare(core)
+            if split:
+                small.prepare_project(core, self.core_old, self.dS_dir_old, M[0], M[1], M_O)
+            else:
+                small.prepare(core)
         R, S, O = self._U(0), self._U(1), self._obj()
         with self._stage("query_fwd"):
             r_rows = ops.gather_rows(R, rel_idx)
@@ -409,18 +421,17 @@ class StepEngine:
         # ---- norm of the Riemannian gradient ----
         grams = [ops.gram(v, v, out=self._gram_view[0][k]) for k, v in enumerate(dV_g)]
         self._allreduce(self._gram_flat[0][self._gram_ent:])
-        norm, alpha = small.norm(dS_g, grams[0], grams[1], grams[2] if not sym else grams[1], self.hyper,
-                                 adam=self.adam)
-        # ---- momentum: transport the previous direction, then combine ----
-        use_momentum = self.beta is not None and self.has_old
+        gram_O = grams[2] if not sym else grams[1]
+        # ---- momentum: the transported previous direction, then combine ----
         dV_new = self.dV_new
+        if split:
+            norm, alpha, pS_beta, K, L = small.norm_project(dS_g, grams[0], grams[1], gram_O, self.hyper, M[0], M[1],
+                                                            M_O, adam=self.adam)
+        else:
+            norm, alpha = small.norm(dS_g, grams[0], grams[1], gram_O, self.hyper, adam=self.adam)
+            if use_momentum:
+                pS_beta, K, L = small.project(core, self.core_old, self.dS_dir_old, M[0], M[1], M_O, self.hyper)
         if use_momentum:
-            # transport Grams M_k = U_k^T [U_old_k | dV_dir_k]: produced by the previous retraction from its
-            # own small matrices (no N-sized pass, no all-reduce: replicated); see rt_small_retract
-            M = self.M_next
-            with self._stage("small_project"):
-                pS_beta, K, L = small.project(core, self.core_old, self.dS_dir_old, M[0], M[1],
-                                              M[2] if not sym else M[1], self.hyper)
             dS_dir = ops.core_axpby(dS_g, alpha, pS_beta, out=self.dS_dir)
 
             def mom(k):

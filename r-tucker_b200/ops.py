@@ -430,7 +430,7 @@ class SmallStage:
 
     def norm(self, dS_g, gram_R, gram_S, gram_O, hyper, adam=None):
         """(||rgrad||, alpha): alpha = normalize / ||rgrad|| (RGD / RSGD, optim.py:92).  With ``adam`` (device state of
-        SFTuckerAdam) alpha and hyper[2] (the momentum coefficient rt_small_project reads) become the Adam ones."""
+        SFTuckerAdam) alpha and hyper[2] (the momentum coefficient of the projection) become the Adam ones."""
         out = torch.empty(2, dtype=f64, device=self.device)
         if adam is not None:
             check(lib().rt_small_norm_adam(ptr(dS_g), ptr(gram_R), ptr(gram_S), ptr(gram_O), ptr(hyper), ptr(adam),
@@ -442,18 +442,30 @@ class SmallStage:
               "rt_small_norm")
         return out[0:1], out[1:2]
 
-    def project(self, core, core_old, dS_old, M_R, M_S, M_O, hyper):
+    def prepare_project(self, core, core_old, dS_old, M_R, M_S, M_O):
+        """prepare(core) and the head of the projection of the previous direction (``dS_old`` at ``core_old``,
+        transport Grams M_i), which runs alongside the factorisation of the Gram inverses.  norm_project() finishes
+        the projection: until then the inputs must stay unchanged."""
+        check(lib().rt_small_prepare_project(ptr(_c(core, f32)), ptr(_c(core_old, f32)), ptr(_c(dS_old, f32)), ptr(M_R),
+                                             ptr(M_S), ptr(M_O), *self._r(), self.sym, ptr(self.ws), stream_ptr()),
+              "rt_small_prepare_project")
+
+    def norm_project(self, dS_g, gram_R, gram_S, gram_O, hyper, M_R, M_S, M_O, adam=None):
+        """norm() and then the tail of the projection that prepare_project() began, in one program.  Returns
+        (||rgrad||, alpha, pS_beta, K, L): the projection pre-scaled by the momentum coefficient hyper[2] as norm()
+        leaves it, K_i [2 r_i, r_i] and L_i [r_i, r_i] fp64 with pV_i = [U_old_i | dV_old_i] K_i + U_i L_i."""
         dev, (r0, r1, r2) = self.device, self._r()
-        pS = torch.empty_like(core)
+        out = torch.empty(2, dtype=f64, device=dev)
+        pS = torch.empty_like(dS_g)
         K = [torch.empty(2 * r, r, dtype=f64, device=dev) for r in (r0, r1, r2)]
         L = [torch.empty(r, r, dtype=f64, device=dev) for r in (r0, r1, r2)]
         if self.sym:
             K[2], L[2] = K[1], L[1]
-        check(lib().rt_small_project(ptr(core), ptr(core_old), ptr(dS_old), ptr(M_R), ptr(M_S), ptr(M_O),
-                                     ptr(hyper), r0, r1, r2, self.sym, ptr(pS), ptr(K[0]), ptr(K[1]),
-                                     ptr(K[2]), ptr(L[0]), ptr(L[1]), ptr(L[2]), ptr(self.ws), stream_ptr()),
-              "rt_small_project")
-        return pS, K, L
+        check(lib().rt_small_norm_project(ptr(dS_g), ptr(gram_R), ptr(gram_S), ptr(gram_O), ptr(hyper), ptr(adam),
+                                          ptr(M_R), ptr(M_S), ptr(M_O), r0, r1, r2, self.sym, ptr(out[0:1]),
+                                          ptr(out[1:2]), ptr(pS), ptr(K[0]), ptr(K[1]), ptr(K[2]), ptr(L[0]),
+                                          ptr(L[1]), ptr(L[2]), ptr(self.ws), stream_ptr()), "rt_small_norm_project")
+        return out[0:1], out[1:2], pS, K, L
 
     def retract(self, core, dS_dir, gram_R, gram_S, gram_O, hyper, transport_out=None):
         dev, (r0, r1, r2) = self.device, self._r()

@@ -28,7 +28,7 @@ from test_gpu_step import CONFIGS, make_batch, ortho, probes   # noqa: E402
 
 f64 = torch.float64
 BOUNDS = {"loss": 1e-5, "norm": 1e-5, "point": 1e-5, "traj_point": 1e-3, "traj_norm": 1e-3, "ortho": 5e-6}
-CALLS = ("prepare", "grad", "norm", "project", "retract")
+CALLS = ("prepare", "prepare_project", "grad", "norm", "norm_project", "retract")
 
 
 def _host(x):
@@ -66,6 +66,9 @@ def replay(calls, rank, B, sym):
     for name, ins, out in calls:
         if name == "prepare":
             ref.prepare(ins[0])
+        elif name == "prepare_project":
+            ref.prepare(ins[0])
+            project_in = ins[:3]
         elif name == "grad":
             r = ref.grad(*ins)
             res["grad"] = max(chk.tile_relerr(o, x) for o, x in zip(out, r))
@@ -74,9 +77,12 @@ def replay(calls, rank, B, sym):
             adam = ins[5].clone() if len(ins) > 5 and ins[5] is not None else None
             r = ref.norm(*ins[:4], hyper, adam=adam)
             res["norm"] = max(chk.tile_relerr(o, x) for o, x in zip(out, r))
-        elif name == "project":
-            pS, K, L = ref.project(*ins)
-            res["project"] = max([chk.tile_relerr(out[0], pS)] + [chk.tile_relerr(a, b) for a, b in zip(out[1] + out[2], K + L)])
+        elif name == "norm_project":       # TuckerAdam's state is passed by keyword and not recorded: RSGD only
+            hyper = ins[4].clone()
+            nrm, alpha = ref.norm(*ins[:4], hyper)
+            pS, K, L = ref.project(*project_in, *ins[5:8], hyper)
+            res["norm"] = max(chk.tile_relerr(o, x) for o, x in zip(out[:2], (nrm, alpha)))
+            res["project"] = max([chk.tile_relerr(out[2], pS)] + [chk.tile_relerr(a, b) for a, b in zip(out[3] + out[4], K + L)])
         elif name == "retract":
             spectra = []
             core_new, Z1, Z2, _ = ref.retract(*ins[:6], spectra=spectra)
